@@ -24,6 +24,8 @@ e2e     : the same step through the C ABI with HOST (pinned) frames: H2D of the 
 parity_in_bench : the reference (oracle/_ref) runs the same unit on sample pairs of the same frames on the host; corner
           counts, survivor counts, li, RANSAC status / inlier lists must be identical, lj within 1e-3 px.
 --impl reference : the reference's own CPU implementation of the unit on all host cores, bounded sample per step.
+--dump-outputs DIR : the results of the last timed resident step as .npy files (dump_outputs); the inputs depend on the
+          arguments only, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -415,6 +417,38 @@ def decode_gathered(hbuf, shards, P, cap):
     return out
 
 
+DUMP_PAIRS = 128  # pairs whose full lists are dumped: 128 x 8000 corners x (li, lj, inliers) = 40 MB as float64
+
+
+def dump_outputs(unit, torch, out_dir):
+    """What the resident step hands its caller, as DIR/<name>.npy (float64; integers are exact).  Per pair of the sequence:
+    n_corners, n_kept, status (0 skipped, 1 no pose, 2 pose), best_h, best_n, R [9], t [3].  For a fixed seeded sample of
+    DUMP_PAIRS pairs (pairs.npy): li, lj [cap, 2] and inliers [cap].  Entries the library leaves undefined are zeroed
+    (li / lj past n_kept; R, t when status != 2) or -1 (inliers past best_n, or when status != 2)."""
+    P = unit.npairs
+    v_li, v_lj, v_nk, v_nc = unit.pairs.torch_views(P)
+    v_st, v_best, v_inl, v_R, v_t = unit.pairs.ransac_torch_views(P)
+    unit.ctx.sync()
+    sample = np.sort(np.random.default_rng(SEED0).choice(P, min(P, DUMP_PAIRS), replace=False))
+    sel = torch.as_tensor(sample, device=v_li.device)
+    nk, st, best = v_nk.cpu().numpy(), v_st.cpu().numpy(), v_best.cpu().numpy()
+    ok = st == 2
+    out = {"n_corners": v_nc.cpu().numpy(), "n_kept": nk, "status": st, "best_h": best[:, 0], "best_n": best[:, 1],
+           "R": np.where(ok[:, None], v_R.cpu().numpy(), 0.0), "t": np.where(ok[:, None], v_t.cpu().numpy(), 0.0), "pairs": sample}
+    col = np.arange(unit.cap)
+    valid = col[None, :] < nk[sample, None]
+    out["li"] = np.where(valid[..., None], v_li[sel].cpu().numpy(), 0.0)
+    out["lj"] = np.where(valid[..., None], v_lj[sel].cpu().numpy(), 0.0)
+    out["inliers"] = np.where(ok[sample, None] & (col[None, :] < best[sample, 1:2]), v_inl[sel].cpu().numpy(), -1)
+    nbytes = sum(a.size * 8 for a in out.values())
+    if nbytes > 64 << 20:
+        raise ValueError(f"dump of {nbytes} bytes exceeds 64 MB: nothing written")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, np.float64))
+    log(f"dumped {len(out)} arrays ({nbytes / 1e6:.1f} MB) of the last timed step to {out_dir}")
+
+
 def parity_check(chk, gen, wl, sample_pairs, frames_of, got, threads):
     """Reference (chk) on the sampled pairs vs the GPU results `got` (dict of arrays indexed by global pair).  Returns the
     parity_in_bench object."""
@@ -492,6 +526,8 @@ def measure_workload(args, ctx, wl, nframes_total, rank, local, world, torch, di
     clocks = sampler.stop() if sampler else None
     n_tracks, n_kept, n_it = unit.pairs.totals()
     early_pairs = unit.pairs.ransac_early()  # pair-steps whose RANSAC scoring stopped at a full count (exact, see DESIGN.md §4)
+    if full and args.dump_outputs:
+        dump_outputs(unit, torch, args.dump_outputs)  # before the passes below overwrite the results
 
     # ---- the same step with every hypothesis of every pair solved and scored (early stop off) --------------------------------
     fs_steps = max(1, min(steps, 3))
@@ -810,7 +846,14 @@ def main():
     ap.add_argument("--pipe", type=int, default=-1, help="pairs per sub-chunk of the stage pipeline (-1: library default, 0: off)")
     ap.add_argument("--klt-mode", type=int, default=0, help="sfmgpu_klt_set_mode value (A/B timing of kernel variants)")
     ap.add_argument("--chunk", type=int, default=0, help="frames per chunk of the streaming e2e call (0: library default, about 100 frames)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the results of the last timed step to DIR/<name>.npy (float64, at most 64 MB; c3 / c2, one process), "
+                         "so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "c5" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs covers the two-view workloads (c3, c2) of --impl ours in one process")
     args.warmup = max(args.warmup, 0)
     wl = WORKLOADS["c3" if args.workload == "c5" else args.workload]
     nframes_total = args.frames or wl["frames"]

@@ -45,6 +45,48 @@ def test_wire_layout_roundtrip():
         assert np.array_equal(got[key], full[key]), key
 
 
+def test_dump_outputs(tmp_path):
+    """--dump-outputs: float64 arrays of the resident step's results, entries the library leaves undefined masked, the
+    same seeded pair sample every run (CPU tensors stand in for the device views)."""
+    import torch
+    rng = np.random.default_rng(2)
+    P, cap = 300, 40
+    nk = rng.integers(0, cap + 1, P).astype(np.int32)
+    st = rng.integers(0, 3, P).astype(np.int32)
+    best = np.stack([rng.integers(-1, 4000, P), rng.integers(0, cap + 1, P)], 1).astype(np.int32)
+    dev = [rng.normal(0, 100, (P, cap, 2)), rng.normal(0, 100, (P, cap, 2)), nk, rng.integers(0, 999, P).astype(np.int32),
+           st, best, rng.integers(0, cap, (P, cap)).astype(np.int32), rng.normal(size=(P, 9)), rng.normal(size=(P, 3))]
+
+    class _Pairs:
+        def torch_views(self, n):
+            return [torch.from_numpy(a) for a in dev[:4]]
+
+        def ransac_torch_views(self, n):
+            return [torch.from_numpy(a) for a in dev[4:]]
+
+    class _Ctx:
+        def sync(self):
+            pass
+
+    class _Unit:
+        npairs, pairs, ctx = P, _Pairs(), _Ctx()
+    _Unit.cap = cap
+    for d in ("a", "b"):
+        bench.dump_outputs(_Unit, torch, str(tmp_path / d))
+    got = {f[:-4]: np.load(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))}
+    assert all(np.array_equal(got[k], np.load(str(tmp_path / "b" / f"{k}.npy"))) for k in got)
+    assert all(a.dtype == np.float64 for a in got.values())
+    s = got["pairs"].astype(int)
+    assert len(s) == bench.DUMP_PAIRS and np.all(np.diff(s) > 0) and s[-1] < P
+    assert np.array_equal(got["n_kept"], nk) and np.array_equal(got["status"], st) and np.array_equal(got["best_n"], best[:, 1])
+    ok = st == 2
+    assert np.array_equal(got["R"][ok], dev[7][ok]) and not got["R"][~ok].any() and not got["t"][~ok].any()
+    for k, p in enumerate(s):
+        n, m = nk[p], best[p, 1] if st[p] == 2 else 0
+        assert np.array_equal(got["li"][k, :n], dev[0][p, :n]) and not got["li"][k, n:].any() and not got["lj"][k, n:].any()
+        assert np.array_equal(got["inliers"][k, :m], dev[6][p, :m]) and np.all(got["inliers"][k, m:] == -1)
+
+
 def test_reference_arm_line_tiny():
     """`bench.py --impl reference` prints ONE JSON line with the contract's keys (tiny frames so that it runs in seconds)."""
     env = dict(os.environ)
