@@ -77,7 +77,7 @@ int sfmgpu_flush_l2(sfmgpu_ctx* ctx, size_t bytes);
  * Reading synchronises the stream and resets the accumulators. */
 int sfmgpu_profile(sfmgpu_ctx* ctx, int enable);
 int sfmgpu_stage_times(sfmgpu_ctx* ctx, float* ms4);
-/* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac). */
+/* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac). */
 int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n);
 /* Measured non-tensor FP64 throughput of this GPU (DFMA micro-benchmark, ~10 ms): the KLT / RANSAC roofline. */
 int sfmgpu_fp64_peak(sfmgpu_ctx* ctx, double* tflops);
@@ -300,6 +300,19 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
 int sfmgpu_multitracker_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t);
 int sfmgpu_multitracker_tracks(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int sequence, double* xy, int32_t* ids, int cap, int* n_out);
 int sfmgpu_multitracker_totals(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long long* n_track_steps, long long* n_lk_iters);
+/* find_E_ransac(K, prev_pts, cur_pts, iters, thr, min_inliers) (:1739) on every sequence's survivors, inside every later
+ * step; rc == NULL: off.  rc->min_points = 1 is the reference's `prev_pts.empty()` guard (:1715).  Singular K: SFMGPU_E_ARG.
+ * The stage is the one of sfmgpu_pairs_set_ransac (same results for the same survivors; early stop and solver mode follow
+ * the context) and runs before the step's one synchronisation.  A sequence that the step resets instead of tracking (the
+ * first step, the first after sfmgpu_multitracker_reset, a sequence without tracks) is SFMGPU_TV_SKIPPED. */
+int sfmgpu_multitracker_set_ransac(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const double* K, const sfmgpu_ransac_cfg* rc);
+/* Results of the last step: status / best_n [S], inliers [S][ROWS] (indices into that step's survivor list, ascending),
+ * R [S][9], t [S][3] (valid for SFMGPU_TV_OK); any may be NULL.  SFMGPU_E_STATE when the last step ran without the stage
+ * (never enabled, switched off, or no step since set_ransac / reset). */
+int sfmgpu_multitracker_ransac_download_all(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int32_t* status, int32_t* best_n,
+                                            int32_t* inliers, double* R, double* t3);
+/* Sets stopped early since the last call (reads and resets). */
+int sfmgpu_multitracker_ransac_early(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long long* sets_stopped);
 
 /* ---- RANSAC scoring: sampson_err + the loop at :667-676 ------------------------------------------------- */
 /* xi/xj: n normalised correspondences; E: H hypotheses, 9 doubles each.  counts[h] = #{i : e_i < thr};

@@ -106,10 +106,18 @@ struct sfmgpu_pairs {
   int last_npairs = 0;
   TwoViewState* tv = nullptr;  // allocated by the first sfmgpu_pairs_ransac call
 };
-void sfm_two_view_free(sfmgpu_ctx* ctx, sfmgpu_pairs* p);
-bool sfm_two_view_enabled(const sfmgpu_pairs* p);
-int sfm_two_view_stage(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npairs, const double* E_host);
-int sfm_two_view_download(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npairs, cudaStream_t s);
+// The stage works on result sets of `cap` rows: the pairs of a batch, or the sequences of the lock-step tracker.
+void sfm_two_view_free(sfmgpu_ctx* ctx, TwoViewState** tv);
+bool sfm_two_view_enabled(const TwoViewState* tv);
+int sfm_two_view_configure(sfmgpu_ctx* ctx, TwoViewState** tv, int max_sets, int cap, const double* K, const sfmgpu_ransac_cfg* rc,
+                           const char* who);
+int sfm_two_view_stage(sfmgpu_ctx* ctx, TwoViewState* tv, const double2* li, const double2* lj, const int* nkept, int cap, int set_off,
+                       int nsets, const double* E_host);
+int sfm_two_view_skip(sfmgpu_ctx* ctx, TwoViewState* tv, const int* n_in, int nsets);
+int sfm_two_view_download(sfmgpu_ctx* ctx, TwoViewState* tv, int cap, int set_off, int nsets, cudaStream_t s);
+int sfm_two_view_download_all(sfmgpu_ctx* ctx, TwoViewState* tv, int cap, int nsets, int32_t* status, int32_t* best_n, int32_t* inliers,
+                              double* R, double* t, const char* who);
+int sfm_two_view_early(sfmgpu_ctx* ctx, TwoViewState* tv, long long* stopped);
 
 int sfm_fail(sfmgpu_ctx* ctx, int code, const char* fmt, ...);
 int sfm_reserve(sfmgpu_ctx* ctx, DevBuf& b, size_t bytes);

@@ -222,7 +222,7 @@ void sfmgpu_pairs_destroy(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
   SFM_ENTER_VOID(ctx);
   if (!p) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
-  sfm_two_view_free(ctx, p);
+  sfm_two_view_free(ctx, &p->tv);
   void* ptrs[] = {p->xy0, p->p1, p->pb, p->li, p->lj, p->nit, p->keep, p->ncorn, p->nkept, p->totals, p->work[0].p, p->work[1].p};
   for (void* q : ptrs)
     if (q) cudaFree(q);
@@ -282,9 +282,9 @@ static int stage_klt(sfmgpu_ctx* ctx, const ChunkArgs& c) {
     SFM_LAUNCH(ctx, totals_kernel, 256, 256, 0, out->ncorn + c.pair_off, out->nkept + c.pair_off, out->nit + so, c.npairs, out->cap,
                out->totals);
   }
-  if (sfm_two_view_enabled(out)) {  // the unit's last step: find_E_ransac on the survivors of every pair (:1855-1857)
+  if (sfm_two_view_enabled(out->tv)) {  // the unit's last step: find_E_ransac on the survivors of every pair (:1855-1857)
     StageTimer rt(ctx, 4);
-    SFM_TRY(sfm_two_view_stage(ctx, out, c.pair_off, c.npairs, nullptr));
+    SFM_TRY(sfm_two_view_stage(ctx, out->tv, out->li, out->lj, out->nkept, out->cap, c.pair_off, c.npairs, nullptr));
   }
   return 0;
 }
@@ -596,7 +596,7 @@ int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* 
       SFM_CUDA(ctx, cudaMemcpyAsync(lj_xy + 2 * o * cap, out->lj + o * cap, np_ * cap * 16, cudaMemcpyDeviceToHost, ctx->back_stream));
     if (n_kept) SFM_CUDA(ctx, cudaMemcpyAsync(n_kept + o, out->nkept + o, np_ * 4, cudaMemcpyDeviceToHost, ctx->back_stream));
     if (n_corners) SFM_CUDA(ctx, cudaMemcpyAsync(n_corners + o, out->ncorn + o, np_ * 4, cudaMemcpyDeviceToHost, ctx->back_stream));
-    if (sfm_two_view_enabled(out)) SFM_TRY(sfm_two_view_download(ctx, out, P0, P1 - P0, ctx->back_stream));
+    if (sfm_two_view_enabled(out->tv)) SFM_TRY(sfm_two_view_download(ctx, out->tv, out->cap, P0, P1 - P0, ctx->back_stream));
   }
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->back_stream));
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->klt_stream));
@@ -611,7 +611,7 @@ int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* 
     if (lj_xy) SFM_CUDA(ctx, cudaMemcpyAsync(lj_xy + 2 * o * cap, out->lj + o * cap, cap * 16, cudaMemcpyDeviceToHost, ctx->stream));
     if (n_kept) SFM_CUDA(ctx, cudaMemcpyAsync(n_kept + o, out->nkept + o, 4, cudaMemcpyDeviceToHost, ctx->stream));
     if (n_corners) SFM_CUDA(ctx, cudaMemcpyAsync(n_corners + o, out->ncorn + o, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (sfm_two_view_enabled(out)) SFM_TRY(sfm_two_view_download(ctx, out, q, 1, ctx->stream));
+    if (sfm_two_view_enabled(out->tv)) SFM_TRY(sfm_two_view_download(ctx, out->tv, out->cap, q, 1, ctx->stream));
   }
   if (!redone.empty()) SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
@@ -959,6 +959,8 @@ struct sfmgpu_multitracker {
   uint8_t *keep = nullptr, *ok = nullptr;
   long long track_steps = 0;
   unsigned long long* tot = nullptr;
+  TwoViewState* tv = nullptr;       // find_E_ransac on every sequence's survivors inside the step (sfmgpu_multitracker_set_ransac)
+  bool tv_fresh = false;            // the last step ran the stage: its results can be downloaded
 };
 
 namespace {
@@ -1049,6 +1051,7 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   SFM_ENTER_VOID(ctx);
   if (!t) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
+  sfm_two_view_free(ctx, &t->tv);
   void* ptrs[] = {t->trk, t->p1, t->pb, t->oa, t->ob, t->ids, t->oid, t->nit, t->keep, t->fresh, t->ok, t->dn, t->dnk, t->scal, t->tot};
   for (void* q : ptrs)
     if (q) cudaFree(q);
@@ -1083,6 +1086,7 @@ int sfmgpu_multitracker_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   if (ctx->copy_stream) SFM_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
   t->parity = -1;
   t->prefetched = false;
+  t->tv_fresh = false;
   t->n.assign(t->S, 0);
   t->next_id.assign(t->S, 0);
   t->track_steps = 0;
@@ -1111,6 +1115,8 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   if (host_pix && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: frames given but others are prefetched");
   const int S = t->S, cap = t->cap;
   const int par = t->parity < 0 ? 0 : (t->parity + 1) % 3;
+  const bool stage = sfm_two_view_enabled(t->tv);
+  t->tv_fresh = false;
   if (host_pix) {
     SFM_TRY(sfmgpu_frames_upload(ctx, t->frames, par * S, S, host_pix));
     SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, par * S, S));
@@ -1122,7 +1128,12 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   if (next_host_pix) SFM_TRY(multi_prefetch(ctx, t, par, next_host_pix));
   if (n_out)
     for (int s = 0; s < S; s++) n_out[s] = 0;
-  if (t->parity < 0) return multi_reset(ctx, t, par);  // first frames: reset every sequence (:341-344)
+  if (t->parity < 0) {  // first frames: reset every sequence (:341-344); find_E_ransac is not called (:1715)
+    SFM_TRY(multi_reset(ctx, t, par));
+    if (stage) SFM_TRY(sfm_two_view_skip(ctx, t->tv, nullptr, S));
+    t->tv_fresh = stage;
+    return 0;
+  }
   std::vector<int> empties;  // sequences without tracks are reset on this frame instead of stepped (:341-344)
   for (int s = 0; s < S; s++)
     if (t->n[s] == 0) empties.push_back(s);
@@ -1150,6 +1161,12 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   SFM_LAUNCH(ctx, compact_kernel, S, 1024, 0, t->trk, t->p1, t->keep, (const int*)t->ids, (const int*)t->dn, cap, t->oa, t->ob, t->oid,
              t->dnk);
   SFM_LAUNCH(ctx, totals_kernel, 64, 256, 0, (const int*)t->dn, (const int*)t->dnk, (const int*)t->nit, S, cap, t->tot);
+  if (stage) {  // find_E_ransac(K, prev_pts, cur_pts, ...) on every sequence's survivors (:1739), inside the step's one synchronisation
+    StageTimer rt(ctx, 4);
+    SFM_TRY(sfm_two_view_stage(ctx, t->tv, t->oa, t->ob, t->dnk, cap, 0, S, nullptr));
+    // sequences reset on this frame instead of stepped (dn == 0) return no step: SKIPPED whatever min_points says
+    if (!empties.empty()) SFM_TRY(sfm_two_view_skip(ctx, t->tv, t->dn, S));
+  }
   SFM_CUDA(ctx, cudaMemcpyAsync(t->n.data(), t->dnk, (size_t)S * 4, cudaMemcpyDeviceToHost, ctx->stream));
   const size_t rows = (size_t)S * cap;
   if (prev_xy) SFM_CUDA(ctx, cudaMemcpyAsync(prev_xy, t->oa, rows * 16, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1159,6 +1176,7 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   SFM_CUDA(ctx, cudaMemcpyAsync(t->ids, t->oid, rows * 4, cudaMemcpyDeviceToDevice, ctx->stream));
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   t->parity = par;
+  t->tv_fresh = stage;
   if (n_out)
     for (int s = 0; s < S; s++) n_out[s] = t->n[s];
   for (int s : empties) {
@@ -1185,6 +1203,28 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
                             &t->next_id[s], t->fresh, t->fresh_cap, t->ok, t->scal, cap));
   }
   return 0;
+}
+
+int sfmgpu_multitracker_set_ransac(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const double* K, const sfmgpu_ransac_cfg* rc) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  t->tv_fresh = false;  // results of earlier steps are not those of this configuration
+  return sfm_two_view_configure(ctx, &t->tv, t->S, t->cap, K, rc, "multitracker_set_ransac");
+}
+
+int sfmgpu_multitracker_ransac_download_all(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int32_t* status, int32_t* best_n, int32_t* inliers,
+                                            double* R, double* tr) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  if (!t->tv || !t->tv_fresh)
+    return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_ransac_download_all: the last step ran without the RANSAC stage");
+  return sfm_two_view_download_all(ctx, t->tv, t->cap, t->S, status, best_n, inliers, R, tr, "multitracker_ransac");
+}
+
+int sfmgpu_multitracker_ransac_early(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long long* sets_stopped) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t || !sets_stopped) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_ransac_early: null pointer");
+  return sfm_two_view_early(ctx, t->tv, sets_stopped);
 }
 
 int sfmgpu_multitracker_tracks(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int sequence, double* xy, int32_t* ids, int cap, int* n_out) {

@@ -180,10 +180,22 @@ int raw_stream(sfmgpu_ctx* ctx, DevBuf& buf, int& have, long long draws, double 
   return 0;
 }
 
-int tv_alloc(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
-  if (p->tv) return 0;
+// Result sets that did not go through the stage (a tracker step that reset the sequence instead of tracking it): status
+// SKIPPED and winner / count (-1, 0), what the stage leaves for a set below min_points.  n_in: only sets with n_in[s] == 0
+// (nullptr: every set).
+__global__ void tv_skip_kernel(const int* __restrict__ n_in, int nsets, int* __restrict__ status, int* __restrict__ best) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= nsets || (n_in && n_in[s] != 0)) return;
+  status[s] = SFMGPU_TV_SKIPPED;
+  best[2 * s] = -1;
+  best[2 * s + 1] = 0;
+}
+
+// The stage's state for max_sets result sets of cap rows each (no-op when *tvp exists).
+int tv_alloc(sfmgpu_ctx* ctx, TwoViewState** tvp, int max_sets, int cap) {
+  if (*tvp) return 0;
   TwoViewState* tv = new TwoViewState();
-  const size_t n = (size_t)p->max_pairs * p->cap, P = (size_t)p->max_pairs;
+  const size_t n = (size_t)max_sets * cap, P = (size_t)max_sets;
   cudaError_t e = cudaSuccess;
   auto al = [&](void** q, size_t bytes) {
     if (e == cudaSuccess) e = cudaMalloc(q, bytes + 256);
@@ -200,34 +212,36 @@ int tv_alloc(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
   al((void**)&tv->flags, 64);
   if (e == cudaSuccess) e = cudaMemsetAsync(tv->flags, 0, 64, ctx->stream);
   if (e == cudaSuccess) e = cudaMemsetAsync(tv->status, 0, P * 4, ctx->stream);
-  p->tv = tv;
+  *tvp = tv;
   if (e != cudaSuccess) {
-    sfm_two_view_free(ctx, p);
-    return sfm_fail(ctx, SFMGPU_E_CUDA, "pairs_ransac: cudaMalloc failed: %s", cudaGetErrorString(e));
+    sfm_two_view_free(ctx, tvp);
+    return sfm_fail(ctx, SFMGPU_E_CUDA, "ransac stage: cudaMalloc failed: %s", cudaGetErrorString(e));
   }
   return 0;
 }
 
 }  // namespace
 
-void sfm_two_view_free(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
+void sfm_two_view_free(sfmgpu_ctx* ctx, TwoViewState** tvp) {
   (void)ctx;
-  TwoViewState* tv = p->tv;
+  TwoViewState* tv = *tvp;
   if (!tv) return;
   void* ptrs[] = {tv->xi, tv->xj, tv->inl, tv->neff, tv->status, tv->best, tv->bestE, tv->R, tv->t, tv->flags, tv->idx8.p, tv->E.p, tv->counts.p, tv->neff2.p, tv->raw.p};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   delete tv;
-  p->tv = nullptr;
+  *tvp = nullptr;
 }
 
-// The stage for pairs [pair_off, pair_off + npairs) of `p` on the context's CURRENT stream (the KLT stream of the chunk
-// pipeline: the scratch is used by one chunk at a time).  E_host: optional caller hypotheses [npairs][iters][9].
-int sfm_two_view_stage(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npairs, const double* E_host) {
-  TwoViewState* tv = p->tv;
+// The stage for result sets [pair_off, pair_off + npairs) on the context's CURRENT stream (the KLT stream of the chunk
+// pipeline: the scratch is used by one chunk at a time).  Set k's correspondences are li/lj [k][cap], the first nkept[k]
+// valid (a pairs batch: its survivors per pair; the lock-step tracker: the survivors of every sequence in track order).
+// E_host: optional caller hypotheses [npairs][iters][9].
+int sfm_two_view_stage(sfmgpu_ctx* ctx, TwoViewState* tv, const double2* li, const double2* lj, const int* nkept, int cap, int pair_off,
+                       int npairs, const double* E_host) {
   if (!tv || npairs <= 0) return 0;
   const sfmgpu_ransac_cfg& rc = tv->rc;
-  const int H = rc.iters > 0 ? rc.iters : 0, cap = p->cap;
+  const int H = rc.iters > 0 ? rc.iters : 0;
   const int Hs = H > 0 ? H : 1;
   const int chunk = npairs < TV_CHUNK ? npairs : TV_CHUNK;
   SFM_TRY(sfm_reserve(ctx, tv->E, (size_t)chunk * Hs * 72));
@@ -245,9 +259,8 @@ int sfm_two_view_stage(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npair
   for (int c0 = 0; c0 < npairs; c0 += chunk) {
     const int pc = npairs - c0 < chunk ? npairs - c0 : chunk, po = pair_off + c0;
     const size_t so = (size_t)po * cap;
-    SFM_LAUNCH(ctx, tv_normalize_kernel, dim3(sfm_cdiv(cap, 256), pc), 256, 0, (const double2*)(p->li + so), (const double2*)(p->lj + so),
-               (const int*)(p->nkept + po), cap, mp, k[0], k[1], k[2], k[3], k[4], k[5], k[6], k[7], k[8], tv->xi + so, tv->xj + so,
-               tv->neff + po);
+    SFM_LAUNCH(ctx, tv_normalize_kernel, dim3(sfm_cdiv(cap, 256), pc), 256, 0, li + so, lj + so, nkept + po, cap, mp, k[0], k[1], k[2],
+               k[3], k[4], k[5], k[6], k[7], k[8], tv->xi + so, tv->xj + so, tv->neff + po);
     if (H > 0) {
       if (E_host) {
         SFM_CUDA(ctx, cudaMemcpyAsync(tv->E.p, E_host + (size_t)c0 * H * 9, (size_t)pc * H * 72, cudaMemcpyHostToDevice, ctx->stream));
@@ -278,7 +291,7 @@ int sfm_two_view_stage(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npair
       SFM_TRY(sfm_ransac_score_batched(ctx, tv->xi + so, tv->xj + so, (size_t)cap, tv->neff + po, cap, pc, (double*)tv->E.p, H, rc.thr,
                                        (int*)tv->counts.p, tv->best + 2 * po, tv->inl + so, screen ? (const int*)tv->idx8.p : nullptr));
     }
-    SFM_LAUNCH(ctx, tv_finalize_kernel, sfm_cdiv(pc, 128), 128, 0, (const int*)(p->nkept + po), (const int*)(tv->neff + po),
+    SFM_LAUNCH(ctx, tv_finalize_kernel, sfm_cdiv(pc, 128), 128, 0, nkept + po, (const int*)(tv->neff + po),
                (const int*)(tv->best + 2 * po), (const double*)tv->E.p, Hs, pc, mp, rc.min_inliers, tv->status + po, tv->bestE + 9 * (size_t)po);
     SFM_TRY(sfm_pose_batched(ctx, tv->xi + so, tv->xj + so, (size_t)cap, pc, tv->status + po, tv->best + 2 * po, tv->inl + so,
                              tv->bestE + 9 * (size_t)po, tv->R + 9 * (size_t)po, tv->t + 3 * (size_t)po));
@@ -286,7 +299,13 @@ int sfm_two_view_stage(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npair
   return 0;
 }
 
-bool sfm_two_view_enabled(const sfmgpu_pairs* p) { return p->tv && p->tv->enabled; }
+bool sfm_two_view_enabled(const TwoViewState* tv) { return tv && tv->enabled; }
+
+int sfm_two_view_skip(sfmgpu_ctx* ctx, TwoViewState* tv, const int* n_in, int nsets) {
+  if (!tv || nsets <= 0) return 0;
+  SFM_LAUNCH(ctx, tv_skip_kernel, sfm_cdiv(nsets, 128), 128, 0, n_in, nsets, tv->status, tv->best);
+  return 0;
+}
 
 // H index octets of find_E_ransac's seeded sampling (:657-665) for ONE set of n correspondences into d_idx8 [H][8], from the
 // context's resident mt19937(12345) stream; *d_flag (device, 4 bytes, zeroed here) becomes non-zero if the stream was too
@@ -300,11 +319,11 @@ int sfm_sample_octets(sfmgpu_ctx* ctx, int n, int H, int* d_idx8, int* d_flag) {
   return 0;
 }
 
-// D2H of the stage's per-pair results for pairs [pair_off, pair_off + npairs) into the registered host outputs, on `s`.
-int sfm_two_view_download(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int npairs, cudaStream_t s) {
-  TwoViewState* tv = p->tv;
+// D2H of the stage's per-set results for sets [pair_off, pair_off + npairs) (cap inlier rows each) into the registered host
+// outputs, on `s`.
+int sfm_two_view_download(sfmgpu_ctx* ctx, TwoViewState* tv, int cap_rows, int pair_off, int npairs, cudaStream_t s) {
   if (!tv || npairs <= 0) return 0;
-  const size_t o = (size_t)pair_off, np_ = (size_t)npairs, cap = (size_t)p->cap;
+  const size_t o = (size_t)pair_off, np_ = (size_t)npairs, cap = (size_t)cap_rows;
   if (tv->h_status) SFM_CUDA(ctx, cudaMemcpyAsync(tv->h_status + o, tv->status + o, np_ * 4, cudaMemcpyDeviceToHost, s));
   if (tv->h_best_n)
     SFM_CUDA(ctx, cudaMemcpy2DAsync(tv->h_best_n + o, 4, tv->best + 2 * o + 1, 8, 4, np_, cudaMemcpyDeviceToHost, s));
@@ -314,24 +333,68 @@ int sfm_two_view_download(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair_off, int np
   return 0;
 }
 
+// Checks K and the configuration, allocates *tvp for max_sets sets of cap rows on first use, stores both and switches the
+// stage on (rc == nullptr: off again).  `who` names the entry point in error messages.
+int sfm_two_view_configure(sfmgpu_ctx* ctx, TwoViewState** tvp, int max_sets, int cap, const double* K, const sfmgpu_ransac_cfg* rc,
+                           const char* who) {
+  if (!rc) {
+    if (*tvp) (*tvp)->enabled = false;
+    return 0;
+  }
+  if (!K) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null K", who);
+  if (rc->iters < 0 || rc->iters > (1 << 24)) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: bad iteration count", who);
+  double Ki[9];
+  if (!invert_K_host(K, Ki)) return sfm_fail(ctx, SFMGPU_E_ARG, "Singular K");  // the reference throws "Singular K" (:474)
+  SFM_TRY(tv_alloc(ctx, tvp, max_sets, cap));
+  TwoViewState* tv = *tvp;
+  tv->rc = *rc;
+  for (int i = 0; i < 9; i++) tv->Kinv[i] = Ki[i];
+  tv->enabled = true;
+  return 0;
+}
+
+// Sets stopped early since the last call (reads and resets the counter; synchronises).
+int sfm_two_view_early(sfmgpu_ctx* ctx, TwoViewState* tv, long long* stopped) {
+  *stopped = 0;
+  if (!tv) return 0;
+  int v = 0;
+  SFM_CUDA(ctx, cudaMemcpyAsync(&v, tv->flags + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaMemsetAsync(tv->flags + 1, 0, 4, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  *stopped = v;
+  return 0;
+}
+
+// Results of sets [0, nsets) into the given host arrays (any may be null; layout of sfmgpu_pairs_ransac_host_outputs with
+// cap inlier rows per set); synchronises.
+int sfm_two_view_download_all(sfmgpu_ctx* ctx, TwoViewState* tv, int cap, int nsets, int32_t* status, int32_t* best_n, int32_t* inliers,
+                              double* R, double* t, const char* who) {
+  TwoViewState saved = *tv;
+  tv->h_status = status;
+  tv->h_best_n = best_n;
+  tv->h_inl = inliers;
+  tv->h_R = R;
+  tv->h_t = t;
+  int rcode = sfm_two_view_download(ctx, tv, cap, 0, nsets, ctx->stream);
+  tv->h_status = saved.h_status;
+  tv->h_best_n = saved.h_best_n;
+  tv->h_inl = saved.h_inl;
+  tv->h_R = saved.h_R;
+  tv->h_t = saved.h_t;
+  SFM_TRY(rcode);
+  int flag = 0;
+  SFM_CUDA(ctx, cudaMemcpyAsync(&flag, tv->flags, 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (flag) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "%s: the random stream was too short (internal)", who);
+  return 0;
+}
+
 extern "C" {
 
 int sfmgpu_pairs_set_ransac(sfmgpu_ctx* ctx, sfmgpu_pairs* p, const double* K, const sfmgpu_ransac_cfg* rc) {
   SFM_ENTER(ctx);
   if (!ctx || !p) return SFMGPU_E_ARG;
-  if (!rc) {  // switch the stage off again
-    if (p->tv) p->tv->enabled = false;
-    return 0;
-  }
-  if (!K) return sfm_fail(ctx, SFMGPU_E_ARG, "pairs_set_ransac: null K");
-  if (rc->iters < 0 || rc->iters > (1 << 24)) return sfm_fail(ctx, SFMGPU_E_ARG, "pairs_set_ransac: bad iteration count");
-  double Ki[9];
-  if (!invert_K_host(K, Ki)) return sfm_fail(ctx, SFMGPU_E_ARG, "Singular K");  // the reference throws "Singular K" (:474)
-  SFM_TRY(tv_alloc(ctx, p));
-  p->tv->rc = *rc;
-  for (int i = 0; i < 9; i++) p->tv->Kinv[i] = Ki[i];
-  p->tv->enabled = true;
-  return 0;
+  return sfm_two_view_configure(ctx, &p->tv, p->max_pairs, p->cap, K, rc, "pairs_set_ransac");
 }
 
 int sfmgpu_ransac_set_early_stop(sfmgpu_ctx* ctx, int on) {
@@ -343,21 +406,14 @@ int sfmgpu_ransac_set_early_stop(sfmgpu_ctx* ctx, int on) {
 int sfmgpu_pairs_ransac_early(sfmgpu_ctx* ctx, sfmgpu_pairs* p, long long* pairs_stopped) {
   SFM_ENTER(ctx);
   if (!ctx || !p || !pairs_stopped) return sfm_fail(ctx, SFMGPU_E_ARG, "pairs_ransac_early: null pointer");
-  *pairs_stopped = 0;
-  if (!p->tv) return 0;
-  int v = 0;
-  SFM_CUDA(ctx, cudaMemcpyAsync(&v, p->tv->flags + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaMemsetAsync(p->tv->flags + 1, 0, 4, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  *pairs_stopped = v;
-  return 0;
+  return sfm_two_view_early(ctx, p->tv, pairs_stopped);
 }
 
 int sfmgpu_pairs_ransac_host_outputs(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int32_t* status, int32_t* best_n, int32_t* inliers, double* R,
                                      double* t) {
   SFM_ENTER(ctx);
   if (!ctx || !p) return SFMGPU_E_ARG;
-  SFM_TRY(tv_alloc(ctx, p));
+  SFM_TRY(tv_alloc(ctx, &p->tv, p->max_pairs, p->cap));
   p->tv->h_status = status;
   p->tv->h_best_n = best_n;
   p->tv->h_inl = inliers;
@@ -372,7 +428,7 @@ int sfmgpu_pairs_ransac(sfmgpu_ctx* ctx, sfmgpu_pairs* p, const double* K, const
   const bool was_enabled = p->tv && p->tv->enabled;
   SFM_TRY(sfmgpu_pairs_set_ransac(ctx, p, K, rc));
   p->tv->enabled = was_enabled;  // an explicit call does not change what the front end does
-  SFM_TRY(sfm_two_view_stage(ctx, p, 0, p->last_npairs, E_host));
+  SFM_TRY(sfm_two_view_stage(ctx, p->tv, p->li, p->lj, p->nkept, p->cap, 0, p->last_npairs, E_host));
   if (E_host) SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller's hypotheses were read asynchronously
   return 0;
 }
@@ -407,25 +463,7 @@ int sfmgpu_pairs_ransac_download_all(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int32_t* 
                                      double* t) {
   SFM_ENTER(ctx);
   if (!ctx || !p || !p->tv) return sfm_fail(ctx, SFMGPU_E_STATE, "pairs_ransac_download_all: the RANSAC stage has not run");
-  TwoViewState* tv = p->tv;
-  TwoViewState saved = *tv;
-  tv->h_status = status;
-  tv->h_best_n = best_n;
-  tv->h_inl = inliers;
-  tv->h_R = R;
-  tv->h_t = t;
-  int rcode = sfm_two_view_download(ctx, p, 0, p->last_npairs, ctx->stream);
-  tv->h_status = saved.h_status;
-  tv->h_best_n = saved.h_best_n;
-  tv->h_inl = saved.h_inl;
-  tv->h_R = saved.h_R;
-  tv->h_t = saved.h_t;
-  SFM_TRY(rcode);
-  int flag = 0;
-  SFM_CUDA(ctx, cudaMemcpyAsync(&flag, tv->flags, 4, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (flag) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "pairs_ransac: the random stream was too short (internal)");
-  return 0;
+  return sfm_two_view_download_all(ctx, p->tv, p->cap, p->last_npairs, status, best_n, inliers, R, t, "pairs_ransac");
 }
 
 int sfmgpu_pairs_ransac_device_ptrs(sfmgpu_pairs* p, void** status, void** best, void** inliers, void** R, void** t) {

@@ -505,6 +505,18 @@ class MultiKLTTracker {
     return out;
   }
 
+  // find_E_ransac(K, step.prev_pts, step.cur_pts, iters, thr, min_inliers) (:1739) on every sequence's survivors inside every
+  // later step, skipped where a sequence has none (:1715); the results of a step: two_view_results(*this), sfmgpu_two_view.hpp
+  void set_two_view(const Mat33& K, int iters, double thr, int min_inliers) {
+    auto* ctx = sfmgpu_shim::context();
+    const sfmgpu_ransac_cfg rc{iters, thr, min_inliers, 1};
+    sfmgpu_shim::check(ctx, sfmgpu_multitracker_set_ransac(ctx, trk_.get(), K.a.data(), &rc), "multitracker_set_ransac");
+  }
+
+  sfmgpu_multitracker* handle() const { return trk_.get(); }
+  int n_sequences() const { return S_; }
+  int rows() const { return cap_; }
+
  private:
   int S_, w_, h_, cap_ = 0;
   std::shared_ptr<sfmgpu_multitracker> trk_;

@@ -183,3 +183,26 @@ static std::optional<RelPose> find_E_ransac(const Mat33& K, const std::vector<Ve
   rp.inliers.assign(inl.begin(), inl.begin() + best_n);
   return rp;
 }
+
+// find_E_ransac's answer for every sequence of the last MultiKLTTracker::step (set_two_view on), computed inside the step on
+// the device: std::nullopt where the reference has none (no survivors, :1715; fewer than 8 points or min_inliers, :648 /
+// :678), else R_ji, t_ji and the inlier indices into that sequence's step.prev_pts / cur_pts.
+static std::vector<std::optional<RelPose>> two_view_results(const MultiKLTTracker& mt) {
+  using namespace sfmgpu_shim;
+  const int S = mt.n_sequences(), rows = mt.rows();
+  std::vector<std::int32_t> st((size_t)S), bn((size_t)S), inl((size_t)S * rows);
+  std::vector<double> R(9 * (size_t)S), t(3 * (size_t)S);
+  sfmgpu_ctx* ctx = context();
+  check(ctx, sfmgpu_multitracker_ransac_download_all(ctx, mt.handle(), st.data(), bn.data(), inl.data(), R.data(), t.data()),
+        "multitracker_ransac_download_all");
+  std::vector<std::optional<RelPose>> out((size_t)S);
+  for (int s = 0; s < S; s++) {
+    if (st[s] != SFMGPU_TV_OK) continue;
+    RelPose rp;
+    for (int k = 0; k < 9; k++) rp.R_ji.a[k] = R[9 * (size_t)s + k];
+    rp.t_ji = Vec3{t[3 * (size_t)s], t[3 * (size_t)s + 1], t[3 * (size_t)s + 2]};
+    rp.inliers.assign(inl.begin() + (size_t)s * rows, inl.begin() + (size_t)s * rows + bn[s]);
+    out[s] = std::move(rp);
+  }
+  return out;
+}

@@ -40,6 +40,7 @@ SYMBOLS = [
     "sfmgpu_pairs_set_matches", "sfmgpu_ransac_set_early_stop", "sfmgpu_pairs_ransac_early",
     "sfmgpu_sched_shard", "sfmgpu_sched_unique_id", "sfmgpu_sched_create", "sfmgpu_sched_destroy", "sfmgpu_sched_pair_shard",
     "sfmgpu_sched_gather_pairs", "sfmgpu_frames_device_ptr", "sfmgpu_multitracker_reset",
+    "sfmgpu_multitracker_set_ransac", "sfmgpu_multitracker_ransac_download_all", "sfmgpu_multitracker_ransac_early",
 ]
 
 
@@ -156,6 +157,9 @@ def load_library():
         "sfmgpu_pairs_set_matches": (_i, [_vp, _vp, _i, _f64p, _f64p, _i32p]),
         "sfmgpu_frames_device_ptr": (_i, [_vp, _i, C.POINTER(_vp), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
         "sfmgpu_multitracker_reset": (_i, [_vp, _vp]),
+        "sfmgpu_multitracker_set_ransac": (_i, [_vp, _vp, _vp, C.POINTER(RansacCfg)]),
+        "sfmgpu_multitracker_ransac_download_all": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+        "sfmgpu_multitracker_ransac_early": (_i, [_vp, _vp, C.POINTER(_ll)]),
         "sfmgpu_sched_shard": (_i, [_i, _i, _i, C.POINTER(_i), C.POINTER(_i)]),
         "sfmgpu_sched_unique_id": (_i, [_vp]),
         "sfmgpu_sched_create": (_i, [_vp, _i, _i, _vp, _vp, C.POINTER(_vp)]),
@@ -661,6 +665,34 @@ class MultiTracker:
 
     def reset(self):
         self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_reset(self.ctx.h, self.h_))
+
+    # ---- RANSAC stage: find_E_ransac(K, prev_pts, cur_pts, ...) on every sequence's survivors inside the step -------------
+    def set_ransac(self, K, iters=2500, thr=1e-3, min_inliers=60, min_points=1):
+        """Make find_E_ransac(K, prev_pts, cur_pts, iters, thr, min_inliers) part of every later step (K None: off again);
+        min_points=1 skips sequences without survivors, as the reference's `prev_pts.empty()` guard does."""
+        if K is None:
+            self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_set_ransac(self.ctx.h, self.h_, None, None))
+            return
+        K = np.ascontiguousarray(K, np.float64).reshape(9)
+        rc = RansacCfg(iters, thr, min_inliers, min_points)
+        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_set_ransac(self.ctx.h, self.h_, K.ctypes.data_as(_vp), C.byref(rc)))
+
+    def ransac_results(self):
+        """Results of the last step: status [S] (SKIPPED 0 / NONE 1 / OK 2), best_n [S], per sequence its ascending inlier
+        indices into that step's survivors, R [S, 3, 3] and t [S, 3] (valid where status is OK)."""
+        S = self.S
+        st, bn = np.zeros(S, np.int32), np.zeros(S, np.int32)
+        inl = np.zeros((S, self.cap), np.int32)
+        R, t = np.zeros((S, 9)), np.zeros((S, 3))
+        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_ransac_download_all(self.ctx.h, self.h_, _ptr(st), _ptr(bn), _ptr(inl), _ptr(R),
+                                                                          _ptr(t)))
+        return st, bn, [inl[s, :max(bn[s], 0)].copy() for s in range(S)], R.reshape(S, 3, 3), t
+
+    def ransac_early(self):
+        """Sequences whose scoring stopped early (a hypothesis explained all survivors) since the last call; resets the counter."""
+        v = _ll(0)
+        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_ransac_early(self.ctx.h, self.h_, C.byref(v)))
+        return int(v.value)
 
     def tracks(self, s):
         xy, ids = np.zeros((self.cap, 2)), np.zeros(self.cap, np.int32)
