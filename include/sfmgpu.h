@@ -77,7 +77,8 @@ int sfmgpu_flush_l2(sfmgpu_ctx* ctx, size_t bytes);
  * Reading synchronises the stream and resets the accumulators. */
 int sfmgpu_profile(sfmgpu_ctx* ctx, int enable);
 int sfmgpu_stage_times(sfmgpu_ctx* ctx, float* ms4);
-/* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac). */
+/* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac),
+ * ms[5] = the frame gather of sfmgpu_pair_frontend_list. */
 int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n);
 /* Measured non-tensor FP64 throughput of this GPU (DFMA micro-benchmark, ~10 ms): the KLT / RANSAC roofline. */
 int sfmgpu_fp64_peak(sfmgpu_ctx* ctx, double* tflops);
@@ -149,6 +150,19 @@ int sfmgpu_pairs_create(sfmgpu_ctx* ctx, int max_pairs, int max_corners, sfmgpu_
 void sfmgpu_pairs_destroy(sfmgpu_ctx* ctx, sfmgpu_pairs* p);
 int sfmgpu_pair_frontend(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int npairs, const sfmgpu_lkcfg* cfg,
                          sfmgpu_pairs* out);
+/* The same unit over an explicit list of frame pairs (loop-closure verification: old keyframe, current frame).  Pair k =
+ * (frame_a[k], frame_b[k]) of f, k < npairs: any indices, repeats, a == b and a > b allowed; pyramids built.  Detect on
+ * frame_a[k], track a -> b and back, fb filter, compaction - and the RANSAC stage when sfmgpu_pairs_set_ransac is on - into
+ * slot k of `out`: per pair the results sfmgpu_pair_frontend gives for (a, b) when they are adjacent, bit for bit, including
+ * the redo of frames that overflow the candidate lists.  Every reader of a pairs object (download(_all), totals,
+ * ransac_download(_all), ransac_early, device_ptrs, sfmgpu_sched_gather_pairs) works on the result unchanged.
+ * The pyramids of both frames of every pair of a chunk are copied into a scratch batch (about 2.7*W*H bytes per pair with 3
+ * levels; chunks follow sfmgpu_pair_frontend's rule, <= 1024 pairs); chunks run back to back on the context stream
+ * (sfmgpu_pipeline_set does not apply).  An index outside [0, f->n), npairs > max_pairs,
+ * NULL arrays with npairs > 0, or a cfg that does not match `out` / `f` is SFMGPU_E_ARG, reported before any work is queued.
+ * Returns when the batch has finished. */
+int sfmgpu_pair_frontend_list(sfmgpu_ctx* ctx, sfmgpu_frames* f, const int32_t* frame_a, const int32_t* frame_b, int npairs,
+                              const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out);
 /* Stage pipeline: with pairs_per_chunk > 0, a resident batch of at least 2*pairs_per_chunk pairs is cut into chunks
  * that flow through three streams (score -> select on a high-priority stream -> KLT), so the latency-bound corner
  * selection of one chunk shares the SMs with the score / KLT kernels of its neighbours (results are identical).
@@ -364,6 +378,27 @@ int sfmgpu_global_desc32(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count
  * best_id = first index with the strictly largest score above 0 (-1: none), best_score (0 when none). */
 int sfmgpu_desc_search(sfmgpu_ctx* ctx, const float* descs, int n_search, const float* query, float* scores, int* best_id,
                        float* best_score);
+
+/* ---- device-resident descriptor bank and batched candidate search (loop closure for a whole sequence) ----------------
+ * A bank holds `capacity` descriptors of 1024 floats in HBM, zero-filled at create: a zero descriptor scores 0 against
+ * anything, so an unfilled slot can never become a candidate. */
+typedef struct sfmgpu_descs sfmgpu_descs;
+int sfmgpu_descs_create(sfmgpu_ctx* ctx, int capacity, sfmgpu_descs** out);
+void sfmgpu_descs_destroy(sfmgpu_ctx* ctx, sfmgpu_descs* d);
+/* global_desc_32 (:1100-1122) of frames [first, first+count) of f into slots [slot, slot+count), without a host round trip
+ * (same values as sfmgpu_global_desc32).  Stream-ordered: returns before the kernels finish. */
+int sfmgpu_descs_compute(sfmgpu_ctx* ctx, sfmgpu_descs* d, int slot, sfmgpu_frames* f, int first, int count);
+/* Host <-> slots [slot, slot+count): count * 1024 floats.  Both return when the copy is done. */
+int sfmgpu_descs_upload(sfmgpu_ctx* ctx, sfmgpu_descs* d, int slot, int count, const float* host);
+int sfmgpu_descs_download(sfmgpu_ctx* ctx, sfmgpu_descs* d, int slot, int count, float* host);
+/* For every query q: the loop of :1823-1831 with query = slot query_slot[q] over slots [0, n_search[q]):
+ * best_id[q] = first slot with the strictly largest score above 0 (-1: none), best_score[q] (0 when none).
+ * scores (optional): [nq][ld], ld = max n_search; entries k >= n_search[q] are 0.  Every score is dot_desc (:1124-1129)
+ * bit for bit.  The caller keeps the reference's keyframe gap (n_search = k - gap for keyframe k) and its gate (a
+ * comparison on best_score).  query_slot outside [0, capacity) or n_search outside [0, capacity] is SFMGPU_E_ARG.
+ * best_id / best_score may be NULL; returns when the outputs are in host memory. */
+int sfmgpu_descs_search(sfmgpu_ctx* ctx, sfmgpu_descs* d, const int32_t* query_slot, const int32_t* n_search, int nq,
+                        int32_t* best_id, float* best_score, float* scores);
 
 #ifdef __cplusplus
 }

@@ -74,7 +74,7 @@ struct sfmgpu_ctx {
   bool profile = false;
   struct StageEv { int stage; cudaEvent_t a, b; };
   std::vector<StageEv> stage_evs;
-  float stage_ms[5] = {0, 0, 0, 0, 0};  // corner score, corner select, KLT, compaction, RANSAC stage
+  float stage_ms[6] = {0, 0, 0, 0, 0, 0};  // corner score, corner select, KLT, compaction, RANSAC stage, list-call gather
   void* pinned = nullptr;  // staging for small D2H results
   size_t pinned_cap = 0;
   // kernels whose >48 KB dynamic shared memory opt-in has been set ON THIS CONTEXT'S DEVICE (the attribute is per device)
@@ -103,6 +103,8 @@ struct sfmgpu_pairs {
   uint8_t* keep = nullptr;
   unsigned long long* totals = nullptr;
   DevBuf work[2];  // corner work areas (two, so that the stage pipeline can score one chunk while it selects another)
+  DevBuf gather;   // list call: the pyramids of both frames of every pair of a chunk
+  DevBuf idx;      // list call: frame_a, frame_b (device copies for the gather)
   int last_npairs = 0;
   TwoViewState* tv = nullptr;  // allocated by the first sfmgpu_pairs_ransac call
 };

@@ -299,13 +299,13 @@ extern "C" int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n) {
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   for (auto& e : ctx->stage_evs) {
     float t = 0;
-    if (cudaEventElapsedTime(&t, e.a, e.b) == cudaSuccess && e.stage >= 0 && e.stage < 5) ctx->stage_ms[e.stage] += t;
+    if (cudaEventElapsedTime(&t, e.a, e.b) == cudaSuccess && e.stage >= 0 && e.stage < 6) ctx->stage_ms[e.stage] += t;
     cudaEventDestroy(e.a);
     cudaEventDestroy(e.b);
   }
   ctx->stage_evs.clear();
-  for (int i = 0; i < n; i++) ms[i] = i < 5 ? ctx->stage_ms[i] : 0.f;
-  for (int i = 0; i < 5; i++) ctx->stage_ms[i] = 0;
+  for (int i = 0; i < n; i++) ms[i] = i < 6 ? ctx->stage_ms[i] : 0.f;
+  for (int i = 0; i < 6; i++) ctx->stage_ms[i] = 0;
   return 0;
 }
 

@@ -176,6 +176,17 @@ int track_rows(const sfmgpu_lkcfg& c) {
   return m + 1;
 }
 
+// List call, one pyramid level: frame idx_a[y] of src -> frame y of dst and frame idx_b[y] -> frame b_off + y (grid.z = 0 / 1),
+// whole frames with their row padding, 16 B per thread and step.
+__global__ void __launch_bounds__(256) gather_frames_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, size_t fstride,
+                                                           const int* __restrict__ idx_a, const int* __restrict__ idx_b, int b_off) {
+  const size_t n16 = fstride / 16;  // pitch is a multiple of 16
+  const int y = blockIdx.y, sf = blockIdx.z ? idx_b[y] : idx_a[y], df = blockIdx.z ? b_off + y : y;
+  const uint4* s = reinterpret_cast<const uint4*>(src + (size_t)sf * fstride);
+  uint4* d = reinterpret_cast<uint4*>(dst + (size_t)df * fstride);
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (size_t)gridDim.x * blockDim.x) d[i] = s[i];
+}
+
 int default_cand_cap(int w, int h) {
   long long px = (long long)w * h;
   long long cap = px / 6;
@@ -223,7 +234,8 @@ void sfmgpu_pairs_destroy(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
   if (!p) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
   sfm_two_view_free(ctx, &p->tv);
-  void* ptrs[] = {p->xy0, p->p1, p->pb, p->li, p->lj, p->nit, p->keep, p->ncorn, p->nkept, p->totals, p->work[0].p, p->work[1].p};
+  void* ptrs[] = {p->xy0, p->p1, p->pb, p->li, p->lj, p->nit, p->keep, p->ncorn, p->nkept, p->totals, p->work[0].p, p->work[1].p,
+                  p->gather.p, p->idx.p};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   delete p;
@@ -232,6 +244,9 @@ void sfmgpu_pairs_destroy(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
 // ---- the three stages of a chunk of pairs --------------------------------------------------------------------------
 // Pairs (first_frame + k, first_frame + k + 1), k < npairs, go to slots [pair_off, pair_off + npairs) of `out`;
 // totals are accumulated (the caller zeroes them).  A chunk is at most 1024 frames (the corner work area).
+// The stages read the pairs' frames from `cf`: image A of pair k is frame cfirst + k, image B frame cfirst + b_off + k.  The
+// consecutive calls use cf = f, cfirst = first_frame, b_off = 1; the list call (explicit frame pairs) a gathered copy of
+// both frames' pyramids, A frames first, B frames b_off later.
 struct ChunkArgs {
   sfmgpu_frames* f;
   int first_frame, pair_off, npairs;
@@ -239,15 +254,17 @@ struct ChunkArgs {
   sfmgpu_pairs* out;
   DevBuf* work;
   int cand_cap, md;
+  const sfmgpu_frames* cf;
+  int cfirst, b_off;
 };
 
 static int stage_score(sfmgpu_ctx* ctx, const ChunkArgs& c) {
-  return sfm_corners_score_stage(ctx, c.f, c.first_frame, c.npairs, c.cfg->quality, c.md, c.cand_cap, c.work->p, c.work->cap);
+  return sfm_corners_score_stage(ctx, c.cf, c.cfirst, c.npairs, c.cfg->quality, c.md, c.cand_cap, c.work->p, c.work->cap);
 }
 
 static int stage_select(sfmgpu_ctx* ctx, const ChunkArgs& c) {
   const size_t so = (size_t)c.pair_off * c.out->cap;
-  return sfm_corners_select_stage(ctx, c.f, c.first_frame, c.npairs, c.cfg->max_tracks, c.cfg->quality, c.md, c.cand_cap, c.work->p, c.work->cap, c.out->xy0 + so,
+  return sfm_corners_select_stage(ctx, c.cf, c.cfirst, c.npairs, c.cfg->max_tracks, c.cfg->quality, c.md, c.cand_cap, c.work->p, c.work->cap, c.out->xy0 + so,
                                   c.out->ncorn + c.pair_off);
 }
 
@@ -255,14 +272,14 @@ static int stage_klt(sfmgpu_ctx* ctx, const ChunkArgs& c) {
   sfmgpu_pairs* out = c.out;
   const size_t so = (size_t)c.pair_off * out->cap;
   KltLaunch k;
-  k.pv = c.f->view();
+  k.pv = c.cf->view();
   k.p0 = out->xy0 + so;
   k.counts = out->ncorn + c.pair_off;
   k.npairs = c.npairs;
   k.cap = out->cap;
-  k.fa0 = c.first_frame;
+  k.fa0 = c.cfirst;
   k.fa_step = 1;
-  k.fb0 = c.first_frame + 1;
+  k.fb0 = c.cfirst + c.b_off;
   k.fb_step = 1;
   k.radius = c.cfg->win_radius;
   k.iters = c.cfg->iters;
@@ -301,21 +318,29 @@ static ChunkArgs chunk_args(sfmgpu_frames* f, int first_frame, int pair_off, int
   c.work = work;
   c.cand_cap = default_cand_cap(f->w, f->h);
   c.md = cfg->min_distance < 0 ? -cfg->min_distance : cfg->min_distance;
+  c.cf = f;
+  c.cfirst = first_frame;
+  c.b_off = 1;
   return c;
+}
+
+// Pairs per corner launch: >= 4 blocks per SM keeps the one-block-per-frame selection kernels busy; large frames are
+// limited by the work area instead (57 MB per 4K frame: 16 GiB hold 280 of them - still two waves of blocks)
+static int pair_chunk(sfmgpu_ctx* ctx, sfmgpu_frames* f, int npairs, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
+  ChunkArgs c1 = chunk_args(f, 0, 0, 1, cfg, out, &out->work[0]);
+  const size_t per_frame = sfm_corner_work_bytes_md(f->w, f->h, 1, c1.cand_cap, c1.md);
+  long long by_mem = (long long)(((size_t)16 << 30) / (per_frame ? per_frame : 1));
+  if (by_mem < 2 * ctx->n_sm) by_mem = 2 * ctx->n_sm;
+  int chunk = npairs < 1024 ? npairs : 1024;
+  if (chunk > by_mem) chunk = (int)by_mem;
+  return chunk;
 }
 
 // Everything back to back on the context stream (chunks of <= 1024 frames).
 static int pair_range(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int pair_off, int npairs, const sfmgpu_lkcfg* cfg,
                       sfmgpu_pairs* out) {
   if (npairs == 0) return 0;
-  // frames per corner launch: >= 4 blocks per SM keeps the one-block-per-frame selection kernels busy; large frames are
-  // limited by the work area instead (57 MB per 4K frame: 16 GiB hold 280 of them - still two waves of blocks)
-  ChunkArgs c1 = chunk_args(f, first_frame, pair_off, 1, cfg, out, &out->work[0]);
-  const size_t per_frame = sfm_corner_work_bytes_md(f->w, f->h, 1, c1.cand_cap, c1.md);
-  long long by_mem = (long long)(((size_t)16 << 30) / (per_frame ? per_frame : 1));
-  if (by_mem < 2 * ctx->n_sm) by_mem = 2 * ctx->n_sm;
-  int chunk = npairs < 1024 ? npairs : 1024;
-  if (chunk > by_mem) chunk = (int)by_mem;
+  const int chunk = pair_chunk(ctx, f, npairs, cfg, out);
   ChunkArgs c0 = chunk_args(f, first_frame, pair_off, chunk, cfg, out, &out->work[0]);
   SFM_TRY(sfm_reserve(ctx, out->work[0], sfm_corner_work_bytes_md(f->w, f->h, chunk, c0.cand_cap, c0.md)));
   for (int p = 0; p < npairs; p += chunk) {
@@ -442,23 +467,28 @@ static int pipe_chunk(Pipe& p, sfmgpu_frames* f, int first_frame, int pair_off, 
   return 0;
 }
 
-static int pair_args_ok(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int npairs, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
-  if (npairs < 0 || npairs > out->max_pairs || first_frame < 0 || first_frame + npairs + (npairs > 0 ? 1 : 0) > f->n)
-    return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend: pair range [%d,%d) does not fit (frames %d, max_pairs %d)", first_frame,
-                    first_frame + npairs, f->n, out->max_pairs);
+static int pair_cfg_ok(sfmgpu_ctx* ctx, sfmgpu_frames* f, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
   const int cap_out = cfg->max_tracks < 1 ? 1 : cfg->max_tracks;
   if (cap_out != out->cap) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend: cfg->max_tracks != pairs capacity");
   if (cfg->pyr_levels != f->levels) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend: cfg->pyr_levels != frames levels");
   return 0;
 }
 
+static int pair_args_ok(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int npairs, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
+  if (npairs < 0 || npairs > out->max_pairs || first_frame < 0 || first_frame + npairs + (npairs > 0 ? 1 : 0) > f->n)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend: pair range [%d,%d) does not fit (frames %d, max_pairs %d)", first_frame,
+                    first_frame + npairs, f->n, out->max_pairs);
+  return pair_cfg_ok(ctx, f, cfg, out);
+}
+
 // Batch calls size the candidate lists for W*H/6 entries per frame.  A frame whose FINAL list is longer (flat or
 // weak-texture image: thr = 0 makes every pixel a candidate, :274-285) comes back with n_corners < 0; it is redone here
 // through the single-frame path, whose work area holds the worst case (W*H candidates), so the batch returns what the
 // reference returns for every frame.  Synchronises the context stream (the overflow flags are read on the host).
-// redone (optional) receives the pair slots that were recomputed.
+// redone (optional) receives the pair slots that were recomputed.  The list call passes its frame pairs (h_fa, h_fb: host);
+// the consecutive calls pass none (pair p = (first_frame + p, first_frame + p + 1)).  Either way the frames are read from f.
 static int pair_fix_overflow(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int npairs, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out,
-                             std::vector<int>* redone) {
+                             std::vector<int>* redone, const int* h_fa = nullptr, const int* h_fb = nullptr) {
   if (npairs <= 0) return 0;
   SFM_TRY(sfm_pinned(ctx, (size_t)npairs * sizeof(int)));
   int* hn = (int*)ctx->pinned;
@@ -471,9 +501,13 @@ static int pair_fix_overflow(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame,
   const int full_cap = f->w * f->h, md = cfg->min_distance < 0 ? -cfg->min_distance : cfg->min_distance;
   SFM_TRY(sfm_reserve(ctx, ctx->cs_work, sfm_corner_work_bytes_md(f->w, f->h, 1, full_cap, md)));
   for (int p : bad) {
-    SFM_TRY(sfm_corners_batch(ctx, f, first_frame + p, 1, cfg->max_tracks, cfg->quality, cfg->min_distance, full_cap, ctx->cs_work.p,
-                              ctx->cs_work.cap, out->xy0 + (size_t)p * out->cap, out->ncorn + p));
+    SFM_TRY(sfm_corners_batch(ctx, f, h_fa ? h_fa[p] : first_frame + p, 1, cfg->max_tracks, cfg->quality, cfg->min_distance, full_cap,
+                              ctx->cs_work.p, ctx->cs_work.cap, out->xy0 + (size_t)p * out->cap, out->ncorn + p));
     ChunkArgs c = chunk_args(f, first_frame + p, p, 1, cfg, out, nullptr);
+    if (h_fa) {
+      c.cfirst = h_fa[p];
+      c.b_off = h_fb[p] - h_fa[p];
+    }
     SFM_TRY(stage_klt(ctx, c));  // adds this pair's corners / survivors / iterations to the totals
   }
   SFM_CUDA(ctx, cudaMemcpyAsync(hn, out->ncorn, (size_t)npairs * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -521,6 +555,65 @@ int sfmgpu_pair_frontend(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int
   }
   SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, last, 0));  // the KLT stream is in order: its last event covers all chunks
   return pair_fix_overflow(ctx, f, first_frame, npairs, cfg, out, nullptr);
+}
+
+// Explicit frame pairs (loop-closure verification): pair k = (frame_a[k], frame_b[k]) of resident frames.  Per chunk, the
+// pyramids of both frames of every pair are gathered into a scratch batch (A frames, then B frames) and the three stages run
+// on it unchanged, as they run on consecutive frames; chunks run back to back on the context stream.
+int sfmgpu_pair_frontend_list(sfmgpu_ctx* ctx, sfmgpu_frames* f, const int32_t* frame_a, const int32_t* frame_b, int npairs,
+                              const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
+  SFM_ENTER(ctx);
+  if (!ctx || !f || !cfg || !out) return SFMGPU_E_ARG;
+  if (npairs < 0 || npairs > out->max_pairs)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_list: %d pairs, room for %d", npairs, out->max_pairs);
+  if (npairs > 0 && (!frame_a || !frame_b)) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_list: null frame index array");
+  for (int k = 0; k < npairs; k++)
+    if (frame_a[k] < 0 || frame_a[k] >= f->n || frame_b[k] < 0 || frame_b[k] >= f->n)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_list: pair %d = (%d, %d) outside frames [0,%d)", k, frame_a[k], frame_b[k], f->n);
+  SFM_TRY(pair_cfg_ok(ctx, f, cfg, out));
+  const int chunk = npairs > 0 ? pair_chunk(ctx, f, npairs, cfg, out) : 0;
+  // scratch batch of 2 * chunk frames with f's geometry: level l at gather + lofs[l]
+  size_t lofs[SFM_MAXL], gbytes = 0;
+  for (int l = 0; l < f->levels; l++) {
+    lofs[l] = gbytes;
+    gbytes += (f->fstride[l] * 2 * chunk + 255) & ~(size_t)255;
+  }
+  if (npairs > 0) {  // scratch is sized before any work is queued
+    const ChunkArgs c0 = chunk_args(f, 0, 0, chunk, cfg, out, nullptr);
+    SFM_TRY(sfm_reserve(ctx, out->idx, 2 * (size_t)npairs * sizeof(int)));
+    SFM_TRY(sfm_reserve(ctx, out->work[0], sfm_corner_work_bytes_md(f->w, f->h, chunk, c0.cand_cap, c0.md)));
+    SFM_TRY(sfm_reserve(ctx, out->gather, gbytes));
+  }
+  out->last_npairs = npairs;
+  SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
+  if (npairs == 0) return 0;
+  int* d_fa = (int*)out->idx.p;
+  int* d_fb = d_fa + npairs;
+  SFM_CUDA(ctx, cudaMemcpyAsync(d_fa, frame_a, (size_t)npairs * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  SFM_CUDA(ctx, cudaMemcpyAsync(d_fb, frame_b, (size_t)npairs * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  sfmgpu_frames g = *f;  // same geometry and levels, 2 * chunk frames in the scratch
+  g.n = 2 * chunk;
+  for (int l = 0; l < f->levels; l++) g.lvl[l] = (uint8_t*)out->gather.p + lofs[l];
+  for (int p = 0; p < npairs; p += chunk) {
+    const int cnt = npairs - p < chunk ? npairs - p : chunk;
+    {
+      StageTimer st(ctx, 5);
+      for (int l = 0; l < f->levels; l++) {
+        if (f->fstride[l] == 0) continue;  // level of zero size
+        const unsigned gx = sfm_cdiv((long long)(f->fstride[l] / 16), 256 * 8);
+        SFM_LAUNCH(ctx, gather_frames_kernel, dim3(gx, cnt, 2), 256, 0, f->lvl[l], g.lvl[l], f->fstride[l], (const int*)(d_fa + p),
+                   (const int*)(d_fb + p), chunk);
+      }
+    }
+    ChunkArgs c = chunk_args(f, 0, p, cnt, cfg, out, &out->work[0]);
+    c.cf = &g;
+    c.cfirst = 0;
+    c.b_off = chunk;
+    SFM_TRY(stage_score(ctx, c));
+    SFM_TRY(stage_select(ctx, c));
+    SFM_TRY(stage_klt(ctx, c));
+  }
+  return pair_fix_overflow(ctx, f, 0, npairs, cfg, out, nullptr, frame_a, frame_b);
 }
 
 // Streaming variant for frames that live in HOST memory: frames [0, nframes) of `f` are filled from host_pix in

@@ -41,6 +41,8 @@ SYMBOLS = [
     "sfmgpu_sched_shard", "sfmgpu_sched_unique_id", "sfmgpu_sched_create", "sfmgpu_sched_destroy", "sfmgpu_sched_pair_shard",
     "sfmgpu_sched_gather_pairs", "sfmgpu_frames_device_ptr", "sfmgpu_multitracker_reset",
     "sfmgpu_multitracker_set_ransac", "sfmgpu_multitracker_ransac_download_all", "sfmgpu_multitracker_ransac_early",
+    "sfmgpu_pair_frontend_list", "sfmgpu_descs_create", "sfmgpu_descs_destroy", "sfmgpu_descs_compute", "sfmgpu_descs_upload",
+    "sfmgpu_descs_download", "sfmgpu_descs_search",
 ]
 
 
@@ -160,6 +162,13 @@ def load_library():
         "sfmgpu_multitracker_set_ransac": (_i, [_vp, _vp, _vp, C.POINTER(RansacCfg)]),
         "sfmgpu_multitracker_ransac_download_all": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
         "sfmgpu_multitracker_ransac_early": (_i, [_vp, _vp, C.POINTER(_ll)]),
+        "sfmgpu_pair_frontend_list": (_i, [_vp, _vp, _vp, _vp, _i, C.POINTER(LKCfg), _vp]),
+        "sfmgpu_descs_create": (_i, [_vp, _i, C.POINTER(_vp)]),
+        "sfmgpu_descs_destroy": (None, [_vp, _vp]),
+        "sfmgpu_descs_compute": (_i, [_vp, _vp, _i, _vp, _i, _i]),
+        "sfmgpu_descs_upload": (_i, [_vp, _vp, _i, _i, _vp]),
+        "sfmgpu_descs_download": (_i, [_vp, _vp, _i, _i, _vp]),
+        "sfmgpu_descs_search": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
         "sfmgpu_sched_shard": (_i, [_i, _i, _i, C.POINTER(_i), C.POINTER(_i)]),
         "sfmgpu_sched_unique_id": (_i, [_vp]),
         "sfmgpu_sched_create": (_i, [_vp, _i, _i, _vp, _vp, C.POINTER(_vp)]),
@@ -366,6 +375,10 @@ class Context:
                                              C.byref(bid), C.byref(bs)))
         return bid.value, np.float32(bs.value), scores[:n]
 
+    def descs(self, capacity):
+        """Device-resident bank of `capacity` loop-closure descriptors (zero-filled)."""
+        return DescBank(self, capacity)
+
     def sort_perm_desc(self, keys):
         keys = np.ascontiguousarray(keys, np.float64)
         perm = np.zeros(max(len(keys), 1), np.int32)
@@ -491,6 +504,15 @@ class Pairs:
     def run(self, frames, first_frame, npairs, cfg):
         self.ctx._ck(self.ctx.lib.sfmgpu_pair_frontend(self.ctx.h, frames.h_, first_frame, npairs, C.byref(cfg), self.h_))
 
+    def run_list(self, frames, frame_a, frame_b, cfg):
+        """The two-view unit over explicit frame pairs: pair k = (frame_a[k], frame_b[k]) goes to slot k."""
+        fa = np.ascontiguousarray(frame_a, np.int32).reshape(-1)
+        fb = np.ascontiguousarray(frame_b, np.int32).reshape(-1)
+        if len(fa) != len(fb):
+            raise ValueError("frame_a and frame_b differ in length")
+        self.ctx._ck(self.ctx.lib.sfmgpu_pair_frontend_list(self.ctx.h, frames.h_, _ptr(fa) if len(fa) else None,
+                                                            _ptr(fb) if len(fb) else None, len(fa), C.byref(cfg), self.h_))
+
     def run_host(self, frames, host, cfg, li=None, lj=None, nkept=None, ncorn=None, chunk=0):
         """Streaming front end over host frames [n, h, w] (uint8, ideally pinned): upload, pyramids, corners, KLT and
         the download of the results are overlapped chunk by chunk; returns when li/lj/nkept/ncorn are filled."""
@@ -602,6 +624,56 @@ class Pairs:
         nk, nc = _i(0), _i(0)
         self.ctx._ck(self.ctx.lib.sfmgpu_pairs_download(self.ctx.h, self.h_, pair, li, lj, self.cap, C.byref(nk), C.byref(nc)))
         return li[:nk.value].copy(), lj[:nk.value].copy(), nc.value
+
+
+class DescBank:
+    """sfmgpu_descs: loop-closure descriptors (1024 floats each) resident on the device, searched in one launch."""
+
+    def __init__(self, ctx, capacity):
+        self.ctx, self.capacity = ctx, capacity
+        p = _vp()
+        ctx._ck(ctx.lib.sfmgpu_descs_create(ctx.h, capacity, C.byref(p)))
+        self.h_ = p
+
+    def close(self):
+        if getattr(self, "h_", None) and self.ctx.h:
+            self.ctx.lib.sfmgpu_descs_destroy(self.ctx.h, self.h_)
+        self.h_ = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def compute(self, frames, first, count, slot=0):
+        """global_desc_32 of frames [first, first+count) into slots [slot, slot+count) (no host round trip)."""
+        self.ctx._ck(self.ctx.lib.sfmgpu_descs_compute(self.ctx.h, self.h_, slot, frames.h_, first, count))
+
+    def upload(self, descs, slot=0):
+        descs = np.ascontiguousarray(descs, np.float32).reshape(-1, 1024)
+        self.ctx._ck(self.ctx.lib.sfmgpu_descs_upload(self.ctx.h, self.h_, slot, len(descs), _ptr(descs) if len(descs) else None))
+
+    def download(self, slot=0, count=None):
+        count = self.capacity - slot if count is None else count
+        out = np.zeros((max(count, 1), 1024), np.float32)
+        self.ctx._ck(self.ctx.lib.sfmgpu_descs_download(self.ctx.h, self.h_, slot, count, _ptr(out)))
+        return out[:count]
+
+    def search(self, query_slots, n_search, want_scores=False):
+        """Candidate search of every query (:1823-1831): (best_id [nq] int32, -1 = none; best_score [nq] float32; scores
+        [nq, max n_search] float32 or None)."""
+        qs = np.ascontiguousarray(query_slots, np.int32).reshape(-1)
+        ns = np.ascontiguousarray(n_search, np.int32).reshape(-1)
+        if len(qs) != len(ns):
+            raise ValueError("query_slots and n_search differ in length")
+        nq = len(qs)
+        ld = int(ns.max()) if nq else 0
+        bid, bs = np.full(max(nq, 1), -1, np.int32), np.zeros(max(nq, 1), np.float32)
+        scores = np.zeros((max(nq, 1), max(ld, 1)), np.float32) if want_scores else None
+        self.ctx._ck(self.ctx.lib.sfmgpu_descs_search(self.ctx.h, self.h_, _ptr(qs) if nq else None, _ptr(ns) if nq else None, nq,
+                                                      _ptr(bid), _ptr(bs), _ptr(scores)))
+        return bid[:nq], bs[:nq], (scores[:nq, :ld] if want_scores else None)
 
 
 class MultiTracker:
