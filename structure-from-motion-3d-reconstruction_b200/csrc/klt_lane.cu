@@ -23,6 +23,8 @@
 //     the image).  A feature whose window touches the border, or whose position is not finite, is appended to a
 //     "deferred" list and recomputed from scratch by the exact warp-per-feature kernel of klt.cu (which implements
 //     the out-of-bounds rule :188 tap by tap).
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace {
@@ -175,6 +177,7 @@ __device__ __forceinline__ void stage_load(StageRegs& r, const uint8_t* __restri
   if (o > 2) r.hi = __ldg(reinterpret_cast<const uint4*>(rowp + c1));  // needed bytes reach the next chunk
 }
 
+// Bytes 14 and 15 of a staged row are zero: the Gram build of klt_quad_kernel masks a pixel by selecting byte 15.
 __device__ __forceinline__ void stage_store(const StageRegs& r, unsigned char* tile_s, int x0, int lane) {
   const int img = lane >= LN ? 1 : 0, row = lane - img * LN;
   const int o = x0 & 15, q = o >> 2, sh = (o & 3) * 8;
@@ -185,7 +188,7 @@ __device__ __forceinline__ void stage_store(const StageRegs& r, unsigned char* t
   out.x = __funnelshift_r(W[0], W[1], sh);
   out.y = __funnelshift_r(W[1], W[2], sh);
   out.z = __funnelshift_r(W[2], W[3], sh);
-  out.w = __funnelshift_r(W[3], W[4], sh);
+  out.w = __funnelshift_r(W[3], W[4], sh) & 0xFFFFu;
   *reinterpret_cast<uint4*>(tile_s + img * LIMG + row * 16) = out;
 }
 
@@ -344,7 +347,8 @@ __global__ void __launch_bounds__(32 * LWARPS, MINB) klt_lane_kernel(KltLaunch k
 // of :443-447 are therefore quadratic forms  w^T M w  with 4x4 INTEGER matrices M = sum over the window of v v'^T that
 // depend only on the two images and the integer window position.  While the position stays inside one pixel - steps
 // are a few hundredths of a pixel - an LK iteration costs ~90 FP64 instructions instead of ~2,500; the matrices are
-// rebuilt (exact int32 arithmetic, ~5,000 IMAD) only when floor(position) or the pyramid level changes.  The matrices
+// rebuilt (exact integer arithmetic: one Gram matrix of raw taps per feature on the tensor cores, below) only when
+// floor(position) or the pyramid level changes.  The matrices
 // are exact, so the sums differ from the reference's 121-term FP64 loops only by rounding (measured: DESIGN.md §4).
 //
 // Build: with D[r][c] the tap-difference images (DX[r][c] = T1[r][c+1] - T1[r][c-1], DY[r][c] = T1[r+1][c] - T1[r-1][c],
@@ -543,6 +547,155 @@ __device__ __forceinline__ void quad_build(const unsigned char* tile, double* m)
   quad_store<false>(b, m + 40);
 }
 
+// ---- Gram build (the default) -------------------------------------------------------------------------------------------
+// Every difference is a +-1 combination of raw taps, so every matrix entry is an integer combination of the entries of ONE
+// 16 x 16 Gram matrix G = sum over the window of t(p) t(p)^T, where t(p) holds the 16 u8 taps that any component at window
+// pixel p = (r, c) touches (tile coordinates; (dr, dc) = offset from p):
+//   taps 0..7    I1, rows r, r+1 (dr = j >> 2), columns c-1 .. c+2 (dc = (j & 3) - 1)
+//   taps 8..11   I1, rows r-1 (8, 9) and r+2 (10, 11), columns c, c+1
+//   taps 12..15  I0, rows r, r+1, columns c, c+1
+// A diagonal entry of a family is a_k' G b_k, an off-diagonal one a_k' G b_l + a_l' G b_k (a_k, b_l: the +-1 tap vectors of the
+// two differences; for XX and YY that is 2 a_k' G a_l, the doubling of quad_store).  G <= 121 * 255^2 and an entry sums at most
+// 8 of them, so s32 is exact: the entries are the integers the FFMA build computes, and the same doubles.
+//
+// G = R'R, R = one row per window pixel (K), one column per tap, is one warp-wide integer MMA per k-step and n8 half
+// (mma.sync m16n8k32 u8 x u8 -> s32, IMMA.16832): 5 k-steps, 10 IMMA per feature.  K order: groups of 4 consecutive pixels of
+// one window row, columns 1-4, 5-8, 9-12 (classes 0, 1, 2); column 12 is outside the window and its byte comes from the zeroed
+// byte 15 of the tile row.  A 32-bit fragment word is one group of one tap: one PRMT of two words of one tile row, since the
+// tap offset only shifts the bytes.  Slot u = 2 * kstep + half (16 K) holds class u / 3 (u < 9) and window row
+// 1 + t + 4 (u % 3) for lane t of a quad; row 12 and slot 9 are zero (33 groups + 7 zero groups = 5 x 32 K).  The A words of
+// taps g and g + 8 of lane (g, t) are also the B fragments of the two n8 halves.
+// Cost: the FFMA build costs the same per round whatever the number of lanes that build; this one costs per building lane.
+// In a fully packed round (32 lanes) it is 1.19x the FFMA build (scripts/klt_build_bench.py, DESIGN.md §9-1): its shared
+// memory traffic (fragment loads of every lane from the same tile, G lookups with bank conflicts) and the per-feature chain
+// bound it, not instruction issue.  It wins on the partly packed rounds: KLT stage 114.1 -> 107.4 ms on C3.
+struct GramBuild {};                    // build tag of klt_quad_kernel
+constexpr int GRAM_SCRATCH = 3 * 256;   // G as three 8 x 8 s32 blocks: G[0..7][0..7], G[0..7][8..15], G[8..15][8..15]
+constexpr int ZROW = 2 * LIMG;          // the 16 bytes after a lane's tiles: zeroed once, never written
+
+__device__ __forceinline__ void gram_tap(int j, int& dr, int& dc, int& img) {
+  if (j < 8) { dr = j >> 2; dc = (j & 3) - 1; img = 0; }
+  else if (j < 12) { dr = j < 10 ? -1 : 2; dc = j & 1; img = 0; }
+  else { dr = (j - 12) >> 1; dc = j & 1; img = 1; }
+}
+
+// tap of the + / - term of difference component k (at offset (k >> 1, k & 1) from the pixel); side 0 = DX, 1 = DY, 2 = DE
+__device__ __forceinline__ int gram_diff_tap(int side, int k, bool plus) {
+  const int a = k >> 1, b = k & 1;
+  if (side == 0) return a * 4 + b + (plus ? 2 : 0);
+  if (side == 1) return plus ? (a ? 10 + b : 5 + b) : (a ? 1 + b : 8 + b);
+  return plus ? 12 + 2 * a + b : a * 4 + b + 1;
+}
+
+// byte offset of G[i][j] in the scratch
+__device__ __forceinline__ int gram_at(int i, int j) {
+  if (i >= 8 && j < 8) { const int s = i; i = j; j = s; }
+  return i < 8 ? (j < 8 ? (i * 8 + j) * 4 : 256 + (i * 8 + j - 8) * 4) : 512 + ((i - 8) * 8 + j - 8) * 4;
+}
+
+struct GramLane {
+  int rb[2], r2[2];          // tile byte offsets of taps g, g + 8 at window row 1 + t (u % 3 == 0); row 9 + t or ZROW (u % 3 == 2)
+  uint32_t sel[2], selm[2];  // PRMT selectors of the two taps; selm: class 2, the column-12 byte taken from byte 15
+  int ga[2][8];              // scratch byte offsets of the G entries of matrix entries lane, lane + 32 (+ + - - pattern below)
+};
+
+// zero_off: scratch-relative offset of a zero word (the second half of a diagonal entry and lanes without a second entry)
+__device__ __forceinline__ void gram_lane_init(GramLane& L, int lane, int zero_off) {
+  const int g = lane >> 2, t = lane & 3;
+#pragma unroll
+  for (int x = 0; x < 2; x++) {
+    int dr, dc, img;
+    gram_tap(g + 8 * x, dr, dc, img);
+    L.rb[x] = img * LIMG + (dr + t + 1) * 16;
+    L.r2[x] = t == 3 ? ZROW : L.rb[x] + 128;
+    L.sel[x] = 0x3210u + 0x1111u * (uint32_t)(dc + 1);
+    L.selm[x] = (L.sel[x] & 0x0FFFu) | 0x7000u;
+  }
+#pragma unroll
+  for (int h = 0; h < 2; h++) {
+    const int e = lane + 32 * h, f = e / 10, q = e % 10;
+    const int k = q < 4 ? 0 : q < 7 ? 1 : q < 9 ? 2 : 3;
+    const int l = k + q - (q < 4 ? 0 : q < 7 ? 4 : q < 9 ? 7 : 9);
+    const int sa = (f == 1 || f == 4) ? 1 : 0, sb = f == 0 ? 0 : f <= 2 ? 1 : 2;  // XX, YY, XY, XE, YE
+#pragma unroll
+    for (int d = 0; d < 2; d++) {  // a_k' G b_l, then a_l' G b_k
+      const int ka = d ? l : k, kb = d ? k : l;
+      const int ap = gram_diff_tap(sa, ka, true), am = gram_diff_tap(sa, ka, false);
+      const int bp = gram_diff_tap(sb, kb, true), bm = gram_diff_tap(sb, kb, false);
+      const bool z = e >= QM || (d == 1 && k == l);
+      L.ga[h][4 * d + 0] = z ? zero_off : gram_at(ap, bp);
+      L.ga[h][4 * d + 1] = z ? zero_off : gram_at(ap, bm);
+      L.ga[h][4 * d + 2] = z ? zero_off : gram_at(am, bp);
+      L.ga[h][4 * d + 3] = z ? zero_off : gram_at(am, bm);
+    }
+  }
+}
+
+// fragment word of slot U for tap g + 8x of this lane
+template <int U>
+__device__ __forceinline__ uint32_t gram_word(const unsigned char* ftile, const GramLane& L, int x) {
+  constexpr int CLS = U / 3, J = U % 3;
+  if (U >= 9) return 0u;
+  const unsigned char* rowp = ftile + (J == 2 ? L.r2[x] : L.rb[x] + 64 * J);
+  const uint32_t sel = CLS == 2 ? L.selm[x] : L.sel[x];
+  if (CLS == 1) {
+    const uint4 q = *reinterpret_cast<const uint4*>(rowp);
+    return __byte_perm(q.y, q.z, sel);
+  }
+  const uint2 q = *reinterpret_cast<const uint2*>(rowp + 4 * CLS);
+  return __byte_perm(q.x, q.y, sel);
+}
+
+__device__ __forceinline__ void imma_16832(int (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
+  asm("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+      : "+r"(d[0]), "+r"(d[1]), "+r"(d[2]), "+r"(d[3])
+      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+}
+
+// Warp-cooperative: the 50 doubles of the feature whose staged tile is ftile, written over that tile.  Every lane calls it.
+__device__ __forceinline__ void gram_build(unsigned char* ftile, unsigned char* scratch, const GramLane& L, int lane) {
+  uint32_t w[2][10];
+#pragma unroll
+  for (int x = 0; x < 2; x++) {
+    w[x][0] = gram_word<0>(ftile, L, x);
+    w[x][1] = gram_word<1>(ftile, L, x);
+    w[x][2] = gram_word<2>(ftile, L, x);
+    w[x][3] = gram_word<3>(ftile, L, x);
+    w[x][4] = gram_word<4>(ftile, L, x);
+    w[x][5] = gram_word<5>(ftile, L, x);
+    w[x][6] = gram_word<6>(ftile, L, x);
+    w[x][7] = gram_word<7>(ftile, L, x);
+    w[x][8] = gram_word<8>(ftile, L, x);
+    w[x][9] = gram_word<9>(ftile, L, x);
+  }
+  int d0[4] = {0, 0, 0, 0}, d1[4] = {0, 0, 0, 0};  // n8 halves: taps 0..7, 8..15
+#pragma unroll
+  for (int s = 0; s < 5; s++) {
+    const uint32_t a0 = w[0][2 * s], a1 = w[1][2 * s], a2 = w[0][2 * s + 1], a3 = w[1][2 * s + 1];
+    imma_16832(d0, a0, a1, a2, a3, a0, a2);
+    imma_16832(d1, a0, a1, a2, a3, a1, a3);
+  }
+  // accumulator (g, 2t..2t+1) of half 0 is G[g][2t..], of half 1 G[g][8+2t..]; rows g + 8 of half 1 are G[8+g][8+2t..]
+  const int o = (lane >> 2) * 8 + 2 * (lane & 3);
+  int* G = reinterpret_cast<int*>(scratch);
+  *reinterpret_cast<int2*>(G + o) = make_int2(d0[0], d0[1]);
+  *reinterpret_cast<int2*>(G + 64 + o) = make_int2(d1[0], d1[1]);
+  *reinterpret_cast<int2*>(G + 128 + o) = make_int2(d1[2], d1[3]);
+  __syncwarp();
+#pragma unroll
+  for (int h = 0; h < 2; h++) {
+    const int e = lane + 32 * h;
+    if (e < QM) {
+      const int* a = L.ga[h];
+#define GR(i) (*reinterpret_cast<const int*>(scratch + a[i]))
+      const int v = (GR(0) - GR(1) - GR(2) + GR(3)) + (GR(4) - GR(5) - GR(6) + GR(7));
+#undef GR
+      reinterpret_cast<double*>(ftile)[e] = (double)v;
+    }
+  }
+  __syncwarp();  // the scratch is rewritten by the next feature
+}
+
 // the five sums from the matrices: 4*Sxx, 4*Sxy, 4*Syy, 2*bx, 2*by in the conventions of window_sums
 __device__ __forceinline__ void quad_eval(const double* m, double fx, double fy, double& a00, double& a01, double& a11, double& b0,
                                           double& b1) {
@@ -585,6 +738,13 @@ __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __
   double* mq = reinterpret_cast<double*>(tile);  // the matrices replace the taps they were built from (400 B <= 448 B)
   const long long total = (long long)k.npairs * k.cap;
   const int ndir = k.pb ? 2 : 1;
+  constexpr bool GRAM = std::is_same<T, GramBuild>::value;
+  unsigned char* scratch = smem_raw + 32 * LSTRIDE;
+  GramLane gl;
+  if (GRAM) {
+    gram_lane_init(gl, lane, ZROW - 32 * LSTRIDE);  // lane 0's zero row
+    *reinterpret_cast<uint4*>(tile + ZROW) = make_uint4(0u, 0u, 0u, 0u);
+  }
   for (long long wbase = (long long)blockIdx.x * 32; wbase < total; wbase += (long long)gridDim.x * 32) {
     const long long g = wbase + lane;
     const int pair = g < total ? (int)(g / k.cap) : 0;
@@ -676,6 +836,7 @@ __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __
 #ifdef KLT_ROUND_STATS
       if (lane == 0) atomicAdd(&klt_round_hist[0][__popc(need)], 1ull);
 #endif
+      const unsigned build = need;
       __syncwarp();
       while (need) {
         int ss[LSTAGE], sx0[LSTAGE];
@@ -700,8 +861,12 @@ __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __
           if (ss[j] >= 0 && lane < 2 * LN) stage_store(sr[j], wtile + ss[j] * LSTRIDE, sx0[j], lane);
       }
       __syncwarp();
-      if (act) {
+      if constexpr (GRAM) {
+        for (unsigned todo = build; todo; todo &= todo - 1) gram_build(wtile + (__ffs(todo) - 1) * LSTRIDE, scratch, gl, lane);
+      } else if (act) {
         quad_build<T>(tile, mq);
+      }
+      if (act) {
         tFX = FX;
         tFY = FY;
         tkey = key;
@@ -750,7 +915,7 @@ static int lane_launch(sfmgpu_ctx* ctx, const KltLaunch& k, const int* in_list, 
 // *defer_count (device, zeroed by the caller on the same stream).  variant: tuning builds (A/B runs).
 template <int MINB, int LSTAGE, typename T>
 static int quad_launch(sfmgpu_ctx* ctx, const KltLaunch& k, int* defer_count, int* defer_list) {
-  const size_t smem = (size_t)32 * LSTRIDE;
+  const size_t smem = (size_t)32 * LSTRIDE + (std::is_same<T, GramBuild>::value ? GRAM_SCRATCH : 0);
   static const int cfg_id = sfm_next_cfg_id();  // one per template instantiation
   SFM_SMEM_OPTIN(ctx, cfg_id, (klt_quad_kernel<MINB, LSTAGE, T>), smem);
   const long long total = (long long)k.npairs * k.cap;
@@ -772,7 +937,12 @@ int sfm_klt_lane_launch(sfmgpu_ctx* ctx, const KltLaunch& k, int* defer_count, i
     // Measured on B200 (C2, KLT stage incl. the border pass): <8,4,int> 16.8 ms, <8,4,float> 16.6, <10,4,float> 15.6,
     // <12,4,float> 15.0, <12,2,float> 14.8 (no spills), <16,4,float> 24.2 (spills), staging rounds of 8: 20.2 (spills); a
     // single-sweep build (255 registers, 8 warps) 15.2 ms.
-    default: return quad_launch<12, 2, float>(ctx, k, defer_count, defer_list);  // quadratic forms over integer matrices
+    // Gram build, measured on B200 (1000 W, C3 KLT stage incl. the border pass, 3 alternated runs): <14,2,Gram> 107.4 ms
+    // (128 registers, 16 B spilled outside the build loop, 14 warps/SM), <12,2,Gram> 107.1 (156 registers, no spills),
+    // the FFMA build <12,2,float> 114.1.
+    case 7: return quad_launch<12, 2, float>(ctx, k, defer_count, defer_list);  // the FFMA build
+    case 8: return quad_launch<12, 2, GramBuild>(ctx, k, defer_count, defer_list);
+    default: return quad_launch<14, 2, GramBuild>(ctx, k, defer_count, defer_list);  // quadratic forms over integer matrices
   }
 }
 
