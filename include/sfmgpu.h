@@ -122,10 +122,10 @@ int sfmgpu_sort_perm_desc(sfmgpu_ctx* ctx, const double* keys, int n, int32_t* p
 /* How every later corner selection of this context orders its candidates (results are bit-identical either way):
  * 0 = bucket selection (candidates grouped by score bucket, blocked ones dropped unsorted, the survivors sorted and
  * selected bucket group by bucket group), and the exact introsort emulation only for frames where two candidates with
- * identical scores are both still selectable (default); 1 = introsort emulation for every frame; 2 = full radix sort by
- * score + selection over the sorted list; 12..34 = bucket selection with that many order-code bits (tests: short codes
- * exercise the equal-code path); 1064..5096 = bucket selection with gathers of (mode - 1000) words (tests: small gathers
- * exercise the walk of an oversized bucket by sub-buckets). */
+ * identical scores are both still selectable (default); 1 = introsort emulation for every frame; 12..34 = bucket
+ * selection with that many order-code bits (tests: short codes exercise the equal-code path); 1064..5096 = bucket
+ * selection with gathers of (mode - 1000) words (tests: small gathers exercise the walk of an oversized bucket by
+ * sub-buckets).  Any other mode returns SFMGPU_E_ARG. */
 int sfmgpu_select_set_mode(sfmgpu_ctx* ctx, int mode);
 
 /* ---- KLT: track_one / lk_step / sample_bilinear (:183-198, :396-460) ------------------------------- */

@@ -59,7 +59,7 @@ struct sfmgpu_ctx {
   DevBuf flush;
   DevBuf klt_in, klt_p1, klt_pb, klt_nit, klt_keep, klt_defer;
   int klt_mode = 0;  // 0 auto, 1 warp-per-feature, 2 lane-per-feature (tests / profiling)
-  int select_mode = 0;  // 0 bucket selection + tie fallback, 1 introsort emulation only, 2 full radix sort + selection, 12..34 bucket selection with that many code bits, 1064..5096 bucket selection with a gather of (mode - 1000) words (tests / profiling)
+  int select_mode = 0;  // 0 bucket selection + tie fallback, 1 introsort emulation only, 12..34 bucket selection with that many code bits, 1064..5096 bucket selection with a gather of (mode - 1000) words (tests / profiling)
   DevBuf cs_work;    // corner-score work area for single-frame calls
   DevBuf sel_work;   // corner-select work area
   DevBuf misc;       // small scalars
@@ -214,7 +214,6 @@ int sfm_klt_launch(sfmgpu_ctx* ctx, const KltLaunch& k);
 
 // corner_score.cu / corner_select.cu
 struct CornerWork;  // opaque per-batch work area
-size_t sfm_corner_work_bytes(int w, int h, int nframes, int cand_cap);
 size_t sfm_corner_work_bytes_md(int w, int h, int nframes, int cand_cap, int min_dist);
 // Detect corners for frames [first, first+count): out_xy [count][max_corners] (double2, integer valued),
 // out_n[count].  cand_cap = per-frame candidate capacity (overflow -> E_CAPACITY, reported via status word).

@@ -80,10 +80,6 @@ __device__ __forceinline__ float est_u(float a, float b, float c) {
 }
 
 // One tile of one frame.  MODE 0: frame maximum only.  MODE 1: candidates against the FINAL threshold (maximum known).
-// MODE 2: maximum AND candidates in one pass, against a PROVISIONAL threshold quality * L where L <= final maximum is what
-// is known when the block starts (running maximum, which a sparse probe pass has seeded, and this tile's own estimate):
-// multiplication by quality > 0 is monotone, so the provisional threshold never exceeds the final one and the list is a
-// superset of the candidates; candidate_finalize_kernel drops the surplus once the maximum is final.
 template <int MODE>
 __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restrict__ im, int w, int h, int pitch, int X0, int Y0,
                                            int fr, const CornerWorkView& wv, double quality) {
@@ -178,25 +174,13 @@ __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restr
   unsigned long long* maxbits = wv.maxbits + fr;
   double thr8 = 0.0;
   float bound;
-  unsigned long long maxkey = 0;
-  int shift = 0;
-  double runmax = 0.0;
-  if (MODE == 0 || MODE == 2) {
-    runmax = __longlong_as_double(*(volatile unsigned long long*)maxbits);  // what earlier blocks found
-    bound = __double2float_rd(runmax);
+  if (MODE == 0) {
+    bound = __double2float_rd(__longlong_as_double(*(volatile unsigned long long*)maxbits));  // what earlier blocks found
   } else {
     const double maxv = 0.125 * __longlong_as_double(*maxbits);
     const double thr = maxv * quality;  // (:275)
     thr8 = 8.0 * thr;                   // s >= thr  <=>  u >= 8*thr
     bound = __double2float_rd(thr8);
-    // order code of the radix selection path: distance of the score's bit pattern below the frame maximum, shifted so
-    // that the whole candidate range [thr, max] fits CORNER_CODE_BITS bits (ascending code = descending score; scores are
-    // non-negative doubles, so bit order is value order)
-    maxkey = (unsigned long long)__double_as_longlong(maxv);
-    const unsigned long long thrkey = thr > 0.0 ? (unsigned long long)__double_as_longlong(thr) : 0ull;
-    const unsigned long long range = maxkey > thrkey ? maxkey - thrkey : 0ull;
-    const int bits = 64 - __clzll((long long)range);
-    shift = bits > CORNER_CODE_BITS ? bits - CORNER_CODE_BITS : 0;
   }
   const bool col_in = x < w, col_interior = x >= 2 && x < w - 2;
   const bool tile_inner = X0 >= 2 && X0 + TW <= w - 2 && Y0 >= 2 && Y0 + TH <= h - 2;  // no border pixel in this tile
@@ -223,7 +207,7 @@ __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restr
       const int y = Y0 + q * VRUN + j;
       const bool interior = INNER || (col_interior && y >= 2 && y < h - 2);
       const float u = est_u(a, b, c);
-      if (MODE == 0 || MODE == 2) {
+      if (MODE == 0) {
         uf[j] = interior ? u : -1.0e30f;
         tmax = fmaxf(tmax, uf[j]);
       } else {
@@ -248,7 +232,7 @@ __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restr
   else
     walk(std::false_type{});
 
-  if (MODE == 0 || MODE == 2) {
+  if (MODE == 0) {
     // tile maximum of the estimates
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) tmax = fmaxf(tmax, __shfl_xor_sync(0xffffffffu, tmax, o));
@@ -258,33 +242,6 @@ __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restr
 #pragma unroll
     for (int k = 1; k < 8; k++) bm = fmaxf(bm, sm.wmaxf[k]);
     bound = fmaxf(bound, bm) - EST_MARGIN;  // a pixel below this cannot be the frame maximum
-    if (MODE == 2) {
-      // provisional threshold from a lower bound of the frame maximum: the running maximum (an exact score) or this
-      // tile's best estimate minus the margin (estimate error < 0.72 < margin)
-      const double lb = fmax(runmax, fmax(0.0, (double)bm - (double)EST_MARGIN));
-      thr8 = 8.0 * ((0.125 * lb) * quality);
-      bound = fminf(bound, __double2float_rd(thr8) - EST_MARGIN);
-      if (tile_inner) {
-#pragma unroll
-        for (int j = 0; j < VRUN; j++)
-          if (uf[j] >= bound) pmask |= 1u << j;
-      } else {
-#pragma unroll
-        for (int j = 0; j < VRUN; j++) {
-          const int y = Y0 + q * VRUN + j;
-          if (col_in && y < h) {
-            const bool interior = col_interior && y >= 2 && y < h - 2;
-            if (interior) {
-              if (uf[j] >= bound) pmask |= 1u << j;
-            } else if (0.0 >= thr8) {
-              pmask |= (1u << j) | (1u << (16 + j));  // border score is exactly 0 (:240, :253-254)
-            }
-          }
-        }
-      }
-    }
-  }
-  if (MODE == 0) {
     // queue every pixel that can still be the frame maximum
 #pragma unroll
     for (int j = 0; j < VRUN; j++)
@@ -340,28 +297,25 @@ __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restr
         cand = u >= thr8;
       }
     }
-    if (MODE == 0 || MODE == 2) best = fmax(best, u);
-    if (MODE != 0) {
+    if (MODE == 0) best = fmax(best, u);
+    if (MODE == 1) {
       const unsigned m = __ballot_sync(0xffffffffu, cand);
       if (m) {
         unsigned base = 0;
-        if (lane == 0) base = atomicAdd((MODE == 1 ? wv.nfinal : wv.ncand) + fr, (unsigned)__popc(m));
+        if (lane == 0) base = atomicAdd(wv.nfinal + fr, (unsigned)__popc(m));
         base = __shfl_sync(0xffffffffu, base, 0);
         if (cand) {
           atomicOr(&sm.tile_bm[row * 2 + (col >> 5)], 1u << (col & 31));
           const unsigned slot = base + __popc(m & ((1u << lane) - 1u));
           if (slot < (unsigned)wv.cand_cap) {
-            const unsigned long long k = (unsigned long long)__double_as_longlong(0.125 * u);
             wv.tmp_idx[(size_t)fr * wv.cand_cap + slot] = ((unsigned)(Y0 + row) << 16) | (unsigned)(X0 + col);
-            wv.tmp_key[(size_t)fr * wv.cand_cap + slot] = k;
-            if (MODE == 1)  // k in [thr, max]: code < 2^CORNER_CODE_BITS (MODE 2: candidate_finalize_kernel writes the sort words)
-              wv.pk_a[(size_t)fr * wv.cand_cap + slot] = (((maxkey - k) >> shift) << 32) | slot;
+            wv.tmp_key[(size_t)fr * wv.cand_cap + slot] = (unsigned long long)__double_as_longlong(0.125 * u);
           }
         }
       }
     }
   }
-  if (MODE == 0 || MODE == 2) {
+  if (MODE == 0) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) best = fmax(best, __shfl_xor_sync(0xffffffffu, best, o));
     if (lane == 0) sm.wmax[warp] = best;
@@ -373,7 +327,7 @@ __device__ __forceinline__ void score_tile(ScoreSmem& sm, const uint8_t* __restr
       if (mb > *(volatile unsigned long long*)maxbits) atomicMax(maxbits, mb);  // u >= 0: bit order == value order
     }
   }
-  if (MODE != 0) {
+  if (MODE == 1) {
     __syncthreads();
     if (tid < TH * 2) {
       const int y = Y0 + (tid >> 1), xw = X0 + 32 * (tid & 1);
@@ -409,9 +363,11 @@ __global__ void __launch_bounds__(256, 3) score_tile_kernel(const uint8_t* __res
 // which comes from a per-warp ring in shared memory (lane-contiguous float4: conflict-free, no block barrier anywhere
 // in the kernel).  ~31 instructions per pixel against ~82 of the tile kernel (3 rows converted per thread and row
 // there, two shared-memory round trips, three block barriers per tile).
-// Candidates: as in score_tile<2> - FP32 estimate for every pixel, the exact FP64 score for pixels within the estimate's
-// error of the provisional threshold quality * L, L = max(frame maximum so far, this warp's own exact maximum) <= final
-// maximum; the screened pixels are queued per warp and evaluated densely (see drain below).
+// Candidates: FP32 estimate for every pixel, the exact FP64 score for pixels within the estimate's error of the
+// provisional threshold quality * L, L = max(frame maximum so far, this warp's own exact maximum) <= final maximum:
+// multiplication by quality > 0 is monotone, so the provisional threshold never exceeds the final one and the list is a
+// superset of the candidates (the selection drops the surplus once the maximum is final).  The screened pixels are
+// queued per warp and evaluated densely (see drain below).
 constexpr int WK_COLS = 8, WK_WARPS = 4, WK_MINB = 3, WK_STRIP = 32 * WK_COLS;  // 12 warps per SM: 222 KB of rings + queues, <= 170 registers
 constexpr int WK_RING = 5 * 6 * 32;  // float4 per warp: 5 rows x (24 sums = 6 float4) x 32 lanes
 constexpr int WK_QUEUE = 224;        // screened pixels queued per warp before they are evaluated densely
@@ -760,41 +716,18 @@ __global__ void __launch_bounds__(256) bitmap_clear_kernel(CornerWorkView wv, in
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < wv.words_per_frame; i += (size_t)gridDim.x * blockDim.x) bm[i] = 0u;
 }
 
-// Provisional list -> final list: sets the candidate-bitmap bit of every entry that reaches the final threshold and, for the
-// paths that do not run the selection's own sweep (flagged_only == 0), produces the final count and the sort words of
-// the radix path (order code << 32 | slot in pk_a, count in nfinal).
+// Provisional list -> candidate bitmap: sets the bit of every entry that reaches the final threshold.
 __global__ void __launch_bounds__(256) candidate_finalize_kernel(CornerWorkView wv, double quality, int flagged_only) {
-  const int fr = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
+  const int fr = blockIdx.y;
   if (wv.exact_list[fr]) return;
   if (flagged_only && wv.status[fr] != 3) return;
   const unsigned nprov = wv.ncand[fr];
   const size_t cb = (size_t)fr * wv.cand_cap, wb = (size_t)fr * wv.words_per_frame;
-  const double maxv = 0.125 * __longlong_as_double(wv.maxbits[fr]);
-  const double thr = maxv * quality;
-  const unsigned long long maxkey = (unsigned long long)__double_as_longlong(maxv);
-  const unsigned long long thrkey = thr > 0.0 ? (unsigned long long)__double_as_longlong(thr) : 0ull;
-  const unsigned long long range = maxkey > thrkey ? maxkey - thrkey : 0ull;
-  const int bits = 64 - __clzll((long long)range);
-  const int shift = bits > CORNER_CODE_BITS ? bits - CORNER_CODE_BITS : 0;
-  for (unsigned e0 = blockIdx.x * blockDim.x; e0 < nprov; e0 += gridDim.x * blockDim.x) {  // warp-uniform trip count
-    const unsigned e = e0 + tid;
-    unsigned long long k = 0;
-    bool keep = false;
-    if (e < nprov) {
-      k = wv.tmp_key[cb + e];
-      keep = __longlong_as_double((long long)k) >= thr;  // s >= thr (:282)
-      if (keep) {
-        const unsigned yx = wv.tmp_idx[cb + e], x = yx & 0xFFFFu, y = yx >> 16;
-        atomicOr(wv.bitmap + wb + (size_t)y * wv.wpr + (x >> 5), 1u << (x & 31));
-      }
-    }
-    const unsigned m = __ballot_sync(0xffffffffu, keep && !flagged_only);
-    if (m) {
-      unsigned base = 0;
-      if (lane == 0) base = atomicAdd(wv.nfinal + fr, (unsigned)__popc(m));
-      base = __shfl_sync(0xffffffffu, base, 0);
-      if (keep) wv.pk_a[cb + base + __popc(m & ((1u << lane) - 1u))] = (((maxkey - k) >> shift) << 32) | e;
-    }
+  const double thr = (0.125 * __longlong_as_double(wv.maxbits[fr])) * quality;
+  for (unsigned e = blockIdx.x * blockDim.x + threadIdx.x; e < nprov; e += gridDim.x * blockDim.x) {
+    if (!(__longlong_as_double((long long)wv.tmp_key[cb + e]) >= thr)) continue;  // s >= thr (:282)
+    const unsigned yx = wv.tmp_idx[cb + e], x = yx & 0xFFFFu, y = yx >> 16;
+    atomicOr(wv.bitmap + wb + (size_t)y * wv.wpr + (x >> 5), 1u << (x & 31));
   }
 }
 
@@ -862,18 +795,11 @@ __global__ void __launch_bounds__(256) order_kernel(CornerWorkView wv, double qu
 
 }  // namespace
 
-// ---- work-area carving -------------------------------------------------------------------------------------
-size_t sfm_corner_work_bytes(int w, int h, int nframes, int cand_cap) {
-  CornerWorkView v;
-  return corner_work_carve(v, nullptr, w, h, nframes, cand_cap);
-}
-
 // Raster order for the frames of the batch (all of them, or only those the selection flagged with status 3): ntotal,
-// key[], idx[].  Needed by the introsort emulation and the candidate-list API; the radix selection path works on the
+// key[], idx[].  Needed by the introsort emulation and the candidate-list API; bucket_select_kernel works on the
 // unordered list.
 int sfm_corner_raster_order(sfmgpu_ctx* ctx, int count, const CornerWorkView& wv, double quality, int only_flagged) {
-  // provisional lists (fused score pass): drop the surplus bits from the candidate bitmap; without the radix sort
-  // (only_flagged == 0) also produce the final count and sort words
+  // provisional lists (walk-down score pass): build the candidate bitmap from the entries that reach the final threshold
   SFM_LAUNCH(ctx, bitmap_clear_kernel, dim3(32, count), 256, 0, wv, only_flagged);
   SFM_LAUNCH(ctx, candidate_finalize_kernel, dim3(32, count), 256, 0, wv, quality, only_flagged);
   SFM_LAUNCH(ctx, bitmap_scan_kernel, count, 1024, 0, wv, only_flagged);
@@ -881,9 +807,10 @@ int sfm_corner_raster_order(sfmgpu_ctx* ctx, int count, const CornerWorkView& wv
   return 0;
 }
 
-// Maximum and candidates for frames [first, first+count); leaves the candidate bitmap, the unordered (pixel, score) list,
-// the packed sort words (pk_a, nfinal of them) in the work area.  quality > 0: sparse probe pass + ONE fused pass + a
-// sweep over the list; otherwise (the provisional-threshold argument needs quality > 0) the two full passes.
+// Maximum and candidates for frames [first, first+count); leaves the unordered (pixel, score) list in the work area.
+// quality in (0, 1]: sparse probe pass + ONE walk-down pass against a provisional threshold (a superset of the candidates,
+// ncand entries, no candidate bitmap) + the rescue of frames whose list overflowed; otherwise (the provisional-threshold
+// argument needs quality > 0) the two full tile passes, which leave the exact list (nfinal entries) and its bitmap.
 int sfm_corner_candidates_batch(sfmgpu_ctx* ctx, const sfmgpu_frames* f, int first, int count, double quality,
                                 const CornerWorkView& wv) {
   SFM_CUDA(ctx, cudaMemsetAsync(wv.maxbits, 0, sizeof(unsigned long long) * count, ctx->stream));
@@ -892,32 +819,24 @@ int sfm_corner_candidates_batch(sfmgpu_ctx* ctx, const sfmgpu_frames* f, int fir
   SFM_CUDA(ctx, cudaMemsetAsync(wv.rescue_count, 0, sizeof(int), ctx->stream));
   const int ntx = sfm_cdiv(f->w, TW), nty = sfm_cdiv(f->h, TH);
   dim3 grid(ntx, nty, count);
-  static const int cfg_id[4] = {sfm_next_cfg_id(), sfm_next_cfg_id(), sfm_next_cfg_id(), sfm_next_cfg_id()};
+  static const int cfg_id[3] = {sfm_next_cfg_id(), sfm_next_cfg_id(), sfm_next_cfg_id()};
   SFM_SMEM_OPTIN(ctx, cfg_id[0], score_tile_kernel<0>, sizeof(ScoreSmem));
   SFM_SMEM_OPTIN(ctx, cfg_id[1], score_tile_kernel<1>, sizeof(ScoreSmem));
-  SFM_SMEM_OPTIN(ctx, cfg_id[2], score_tile_kernel<2>, sizeof(ScoreSmem));
-  SFM_SMEM_OPTIN(ctx, cfg_id[3], score_rescue_kernel, sizeof(ScoreSmem));
-  static const bool two_pass = getenv("SFMGPU_SCORE_TWO_PASS") != nullptr;  // A/B timing
-  if (quality > 0.0 && quality <= 1.0 && !two_pass) {  // (quality > 1: a pixel between the maximum and the threshold would be skipped)
+  SFM_SMEM_OPTIN(ctx, cfg_id[2], score_rescue_kernel, sizeof(ScoreSmem));
+  if (quality > 0.0 && quality <= 1.0) {  // (quality > 1: a pixel between the maximum and the threshold would be skipped)
     // every 6th tile in x and y seeds the running maximum (1/36 of a pass; measured per 999 1080p frames: every 4th tile 6.78 ms
     // for the stage, every 6th or 8th 6.45 ms)
     constexpr int PROBE = 6;
     SFM_CUDA(ctx, cudaMemsetAsync(wv.exact_list, 0, sizeof(int) * count, ctx->stream));
     SFM_LAUNCH(ctx, score_tile_kernel<0>, dim3(sfm_cdiv(ntx, PROBE), sfm_cdiv(nty, PROBE), count), 256, sizeof(ScoreSmem), f->lvl[0], f->w,
                f->h, f->pitch[0], f->fstride[0], first, wv, quality, PROBE);
-    static const bool use_tiles = getenv("SFMGPU_SCORE_TILES") != nullptr;  // A/B: the tile kernel of the earlier sessions
-    if (use_tiles) {
-      SFM_LAUNCH(ctx, score_tile_kernel<2>, grid, 256, sizeof(ScoreSmem), f->lvl[0], f->w, f->h, f->pitch[0], f->fstride[0], first, wv,
-                 quality, 1);
-    } else {
-      // segments of ~270 rows (6 warm-up rows each: 2 %), 4 strips of 256 columns per block
-      const int nseg = f->h > 400 ? (f->h + 269) / 270 : 1, seg_rows = (f->h + nseg - 1) / nseg;
-      static const int walk_id = sfm_next_cfg_id();
-      const size_t wsm = (size_t)WK_WARPS * WK_SMEM_WARP;
-      SFM_SMEM_OPTIN(ctx, walk_id, score_walk_kernel, wsm);
-      SFM_LAUNCH(ctx, score_walk_kernel, dim3(sfm_cdiv(f->w, WK_WARPS * WK_STRIP), sfm_cdiv(f->h, seg_rows), count), WK_WARPS * 32, wsm,
-                 f->lvl[0], f->w, f->h, f->pitch[0], f->fstride[0], first, wv, quality, seg_rows);
-    }
+    // segments of ~270 rows (6 warm-up rows each: 2 %), 4 strips of 256 columns per block
+    const int nseg = f->h > 400 ? (f->h + 269) / 270 : 1, seg_rows = (f->h + nseg - 1) / nseg;
+    static const int walk_id = sfm_next_cfg_id();
+    const size_t wsm = (size_t)WK_WARPS * WK_SMEM_WARP;
+    SFM_SMEM_OPTIN(ctx, walk_id, score_walk_kernel, wsm);
+    SFM_LAUNCH(ctx, score_walk_kernel, dim3(sfm_cdiv(f->w, WK_WARPS * WK_STRIP), sfm_cdiv(f->h, seg_rows), count), WK_WARPS * 32, wsm,
+               f->lvl[0], f->w, f->h, f->pitch[0], f->fstride[0], first, wv, quality, seg_rows);
     SFM_LAUNCH(ctx, rescue_mark_kernel, sfm_cdiv(count, 256), 256, 0, wv, count);
     SFM_LAUNCH(ctx, score_rescue_kernel, dim3(ntx, nty, count < 2 ? count : 2), 256, sizeof(ScoreSmem), f->lvl[0], f->w, f->h,
                f->pitch[0], f->fstride[0], first, wv, quality);
@@ -942,7 +861,7 @@ int sfm_candidates_single(sfmgpu_ctx* ctx, const sfmgpu_frames* f, int frame, do
                           int cap, int* n_out, double* max_score) {
   if (f->w > 32767 || f->h > 32767) return sfm_fail(ctx, SFMGPU_E_ARG, "corner_candidates: image larger than 32767 px");
   const int cand_cap = f->w * f->h;
-  const size_t bytes = sfm_corner_work_bytes(f->w, f->h, 1, cand_cap);
+  const size_t bytes = sfm_corner_work_bytes_md(f->w, f->h, 1, cand_cap, 0);
   SFM_TRY(sfm_reserve(ctx, ctx->cs_work, bytes));
   CornerWorkView wv;
   corner_work_carve(wv, ctx->cs_work.p, f->w, f->h, 1, cand_cap);

@@ -5,24 +5,25 @@
 // accepts a candidate iff no already accepted corner lies at squared distance < min_dist^2, capped at
 // max_corners (tested after the push, so at least one corner comes back whenever a candidate exists).
 //
-// Fast path (default): radix_sort_frame_kernel + nms_kernel.  The order std::sort produces is unique wherever the scores
-// are distinct, so the candidates are sorted by a per-frame LSD radix sort (8-bit passes over a 24-bit order code, then
-// the candidates that share a code are ordered by their full 64-bit score) and the selection walks that list.  Inside a
-// group of IDENTICAL scores introsort's order is only observable if at least two members are still unblocked when the
-// selection reaches them (DESIGN.md §4); nms_kernel detects that conservatively and such a frame (status 3) is redone by
-// the exact emulation below (select_kernel mode 3).  Results are bit-identical either way (tests force both paths).
+// Default: bucket_select_kernel.  The order std::sort produces is unique wherever the scores are distinct, so the
+// candidates are put into order-code buckets and only the still unblocked ones of the buckets the selection reaches are
+// sorted (see the kernel).  Inside a group of IDENTICAL scores introsort's order is only observable if at least two
+// members are still unblocked when the selection reaches them (DESIGN.md §4); the kernel detects that conservatively and
+// such a frame (status 3) is redone by the exact emulation below (select_kernel mode 3).
 //
-// Exact emulation (select_kernel): the introsort segment tree is walked LEFT-FIRST and LAZILY (sort_emul.h facts 1-4):
-// only as much of the array is sorted as the selection consumes.  Segments larger than SMALL are partitioned by the
-// whole block (two ordered compactions of the misfits + pairwise swaps); smaller ones are handed to warps, up to 32 at a
-// time, each warp finishing its segment completely (warp partitions, then one leaf per lane with the stable insertion
-// sort).  Depth-limit exhaustion takes the sequential heap-sort restatement.
+// Exact emulation (select_kernel): runs for the frames flagged with status 3, for every frame under select_set_mode(1),
+// and as the sort of sfmgpu_sort_perm_desc.  The introsort segment tree is walked LEFT-FIRST and LAZILY (sort_emul.h
+// facts 1-4): only as much of the array is sorted as the selection consumes.  Segments larger than SMALL are partitioned
+// by the whole block (two ordered compactions of the misfits + pairwise swaps); smaller ones are handed to warps, up to
+// 32 at a time, each warp finishing its segment completely (warp partitions, then one leaf per lane with the stable
+// insertion sort).  Depth-limit exhaustion takes the sequential heap-sort restatement.
 //
-// Selection (both paths): greedy acceptance only ever depends on higher-priority candidates, so a chunk of the sorted
-// prefix is decided in parallel: (1) kill candidates within min_dist of corners accepted in earlier chunks (nms_kernel: one
-// bit per pixel, accepted corners mark their disc; select_kernel: a min_dist-cell grid holding <= 2 corners per cell),
-// (2) resolve conflicts inside the chunk by rounds (a candidate is accepted once every closer, higher-priority survivor
-// is decided), (3) append the accepted ones in priority order.  Coordinates are integers: the arithmetic is exact.
+// Selection (both kernels): greedy acceptance only ever depends on higher-priority candidates, so a chunk of the sorted
+// prefix is decided in parallel: (1) kill candidates within min_dist of corners accepted in earlier chunks
+// (bucket_select_kernel: one bit per pixel, accepted corners mark their disc; select_kernel: a min_dist-cell grid holding
+// <= 2 corners per cell), (2) resolve conflicts inside the chunk by rounds (a candidate is accepted once every closer,
+// higher-priority survivor is decided), (3) append the accepted ones in priority order.  Coordinates are integers: the
+// arithmetic is exact.
 #include "common.cuh"
 #include "corner_work.cuh"
 #include "sort_emul.h"
@@ -362,526 +363,6 @@ __device__ void produce_sorted(SelSmem& sm, sfm_key_t* key, uint32_t* idx, uint3
   }
 }
 
-// ---- radix path -------------------------------------------------------------------------------------------------------
-// One block owns one frame: a stable LSD radix sort of the packed words (order code << 32 | slot in the frame's unordered
-// candidate list, as the candidate pass appended them), 8-bit digits of the code.  Because the block sees the whole frame, the four digit histograms are order-independent and come from
-// ONE sweep; every pass is then a single sweep over the frame in tiles of THREADS*ITEMS words: rank inside the warp by
-// ballot rounds (round r of a warp covers 32 consecutive words, so rank order = position order), across warps and
-// tiles by running per-digit offsets in shared memory.  Passes whose digit is the same for every word are skipped.  A
-// final sweep puts runs of equal codes into descending order of the full 64-bit score (one thread per run, in place; a
-// run is a handful of words) and flags the candidates whose score is IDENTICAL to a neighbour's.
-constexpr int RX_PASSES = CORNER_CODE_BITS / 8;  // 8-bit digits of the order code
-constexpr int RX_MAXRUN = 64;  // equal-code runs longer than this are treated like score ties
-
-constexpr int RX_TILE = 4096;  // words per tile (THREADS * ITEMS)
-
-template <int THREADS>
-struct RadixSmem {
-  __align__(16) unsigned long long tile[2][RX_TILE];  // double buffer filled by the TMA engine (cp.async.bulk), one mbarrier each
-  __align__(8) unsigned long long bar[2];
-  unsigned hist[RX_PASSES][256];
-  unsigned goff[256];
-  unsigned wc[THREADS / 32][256];
-  unsigned wsum[8];
-  int skip[RX_PASSES];
-  unsigned nkeep;
-};
-
-__device__ __forceinline__ unsigned rx_digit(unsigned long long v, int pass) { return (unsigned)(v >> (32 + 8 * pass)) & 255u; }
-
-// score bits of the candidate in slot `slot` of the frame's unordered list
-// Low word of a sort word: list slot (< 2^30: images are at most 32767 x 32767) and, after the final sweep, two flags:
-// RX_TIE = identical score as the predecessor in the sorted list, RX_BIG = member of a group of >= 3 identical scores.
-constexpr unsigned RX_SLOT = 0x3FFFFFFFu, RX_TIE = 0x80000000u, RX_BIG = 0x40000000u;
-
-__device__ __forceinline__ unsigned long long rx_key_of(const CornerWorkView& wv, int fr, unsigned low) {
-  return wv.tmp_key[(size_t)fr * wv.cand_cap + (low & RX_SLOT)];
-}
-
-// ---- bulk asynchronous copies (the 1-D form of TMA, sm_90+ / sm_100a: UBLKCP in SASS) -----------------------------------------
-// One thread hands a whole tile (up to 32 KB) to the copy engine and the bytes are counted on an mbarrier; the other 511 /
-// 1023 threads issue nothing (the cp.async version cost every thread 4-8 copy instructions + a commit per tile).
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem, const void* gmem, unsigned bytes, unsigned long long* bar) {
-  const unsigned b = (unsigned)__cvta_generic_to_shared(bar), d = (unsigned)__cvta_generic_to_shared(smem);
-  // generic-proxy accesses made so far (this block's global stores of the previous pass, shared-memory reads of the
-  // buffer's previous tile) are ordered before the async-proxy copy
-  asm volatile("fence.proxy.async;" ::: "memory");
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(b), "r"(bytes) : "memory");
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(d), "l"(gmem), "r"(bytes),
-               "r"(b)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-  const unsigned b = (unsigned)__cvta_generic_to_shared(bar);
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}\n" ::"r"(b),
-      "r"(parity)
-      : "memory");
-}
-
-template <int THREADS, int ITEMS>
-__global__ void __launch_bounds__(THREADS, 1024 / THREADS) radix_sort_frame_kernel(CornerWorkView wv, double quality) {
-  constexpr int WARPS = THREADS / 32, TILE = THREADS * ITEMS, WTILE = 32 * ITEMS;
-  static_assert(TILE == RX_TILE, "tile buffer size");
-  extern __shared__ __align__(16) unsigned char rx_raw[];
-  RadixSmem<THREADS>& sm = *reinterpret_cast<RadixSmem<THREADS>*>(rx_raw);
-  const int fr = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const size_t cb = (size_t)fr * wv.cand_cap;
-  unsigned long long* A = wv.pk_a + cb;
-  unsigned long long* B = wv.pk_b + cb;
-  if (tid == 0) wv.sorted_in_b[fr] = 0;
-  for (int i = tid; i < RX_PASSES * 256; i += THREADS) (&sm.hist[0][0])[i] = 0;
-  if (tid == 0) {
-    sm.nkeep = 0;
-    mbar_init(&sm.bar[0], 1);
-    mbar_init(&sm.bar[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  unsigned bar_parity = 0;  // bit b: parity the next completion of buffer b's barrier will have
-  __syncthreads();
-  unsigned n;
-  if (wv.exact_list[fr]) {
-    // the list is exact and the candidate pass wrote the sort words: sweep 0 only builds the four digit histograms
-    n = wv.nfinal[fr];
-    if (n > (unsigned)wv.cand_cap || n == 0) return;  // overflow is reported by nms_kernel
-    const unsigned* hi = reinterpret_cast<const unsigned*>(A) + 1;
-    for (unsigned i0 = 0; i0 < n; i0 += THREADS * 8) {
-      unsigned c[8];
-#pragma unroll
-      for (int k = 0; k < 8; k++) {
-        const unsigned i = i0 + k * THREADS + tid;
-        c[k] = i < n ? __ldcg(hi + 2 * (size_t)i) : 0u;
-      }
-#pragma unroll
-      for (int k = 0; k < 8; k++)
-        if (i0 + k * THREADS + tid < n) {
-#pragma unroll
-          for (int p = 0; p < RX_PASSES; p++) atomicAdd(&sm.hist[p][(c[k] >> (8 * p)) & 255u], 1u);
-        }
-    }
-  } else {
-    // provisional list of the fused score pass: the frame maximum is final now.  Sweep 0 keeps the entries that reach
-    // the final threshold (s >= thr, :282) as sort words (order code << 32 | list slot) and builds the histograms on the
-    // way (the candidate bitmap keeps the surplus bits: only the raster path needs it exact and cleans it itself).  The order code is the distance of the score's bit
-    // pattern below the maximum, shifted so that [thr, max] fits CORNER_CODE_BITS bits (ascending code = descending score).
-    const unsigned nprov = wv.ncand[fr];
-    if (nprov > (unsigned)wv.cand_cap) return;  // such frames are on the rescue list (exact_list) - unreachable
-    const double maxv = 0.125 * __longlong_as_double(wv.maxbits[fr]);
-    const double thr = maxv * quality;
-    const unsigned long long maxkey = (unsigned long long)__double_as_longlong(maxv);
-    const unsigned long long thrkey = thr > 0.0 ? (unsigned long long)__double_as_longlong(thr) : 0ull;
-    const unsigned long long range = maxkey > thrkey ? maxkey - thrkey : 0ull;
-    const int bits = 64 - __clzll((long long)range);
-    const int shift = bits > CORNER_CODE_BITS ? bits - CORNER_CODE_BITS : 0;
-    const unsigned long long* lkey = wv.tmp_key + cb;
-    for (unsigned i0 = 0; i0 < nprov; i0 += THREADS * 4) {  // block-uniform trip count
-      unsigned long long k[4];
-#pragma unroll
-      for (int q = 0; q < 4; q++) {
-        const unsigned e = i0 + q * THREADS + tid;
-        k[q] = e < nprov ? __ldcg(lkey + e) : 0ull;
-      }
-#pragma unroll
-      for (int q = 0; q < 4; q++) {
-        const unsigned e = i0 + q * THREADS + tid;
-        const bool in = e < nprov;
-        const bool keep = in && __longlong_as_double((long long)k[q]) >= thr;
-        const unsigned m = __ballot_sync(0xffffffffu, keep);
-        if (m) {
-          unsigned base = 0;
-          if (lane == 0) base = atomicAdd(&sm.nkeep, (unsigned)__popc(m));
-          base = __shfl_sync(0xffffffffu, base, 0);
-          if (keep) {
-            const unsigned code = (unsigned)((maxkey - k[q]) >> shift);
-            A[base + __popc(m & ((1u << lane) - 1u))] = ((unsigned long long)code << 32) | e;
-#pragma unroll
-            for (int p = 0; p < RX_PASSES; p++) atomicAdd(&sm.hist[p][(code >> (8 * p)) & 255u], 1u);
-          }
-        }
-      }
-    }
-    __threadfence();  // the first pass reads A back through the copy engine (L2)
-    __syncthreads();
-    n = sm.nkeep;
-    if (tid == 0) wv.nfinal[fr] = n;
-    if (n == 0) return;
-  }
-  __syncthreads();
-  if (tid < RX_PASSES) sm.skip[tid] = 0;
-  __syncthreads();
-  for (int i = tid; i < RX_PASSES * 256; i += THREADS)
-    if ((&sm.hist[0][0])[i] == n) sm.skip[i >> 8] = 1;  // every word carries this digit: the pass is the identity
-  __syncthreads();
-
-  unsigned long long* src = A;
-  unsigned long long* dst = B;
-  for (int pass = 0; pass < RX_PASSES; pass++) {
-    if (sm.skip[pass]) continue;  // block-uniform
-    // exclusive scan of this pass's histogram -> running output offset per digit
-    if (tid < 256) {
-      const unsigned c = sm.hist[pass][tid];
-      unsigned inc = c;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const unsigned u = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += u;
-      }
-      if (lane == 31) sm.wsum[warp] = inc;
-      sm.goff[tid] = inc - c;
-    }
-    __syncthreads();
-    if (tid < 256) {
-      unsigned base = 0;
-      for (int k = 0; k < warp; k++) base += sm.wsum[k];
-      sm.goff[tid] += base;
-    }
-    // tiles stream through a double buffer filled by bulk copies: tile t+1 is in flight while tile t is ranked and scattered
-    auto fetch = [&](int buf, unsigned t0) {
-      const unsigned words = n - t0 < (unsigned)TILE ? n - t0 : (unsigned)TILE, chunks = (words + 1) / 2;  // 16-byte chunks
-      if (tid == 0) bulk_load(&sm.tile[buf][0], src + t0, chunks * 16u, &sm.bar[buf]);
-    };
-    fetch(0, 0);
-    int it = 0;
-    for (unsigned t0 = 0; t0 < n; t0 += TILE, it++) {
-      if (t0 + TILE < n) fetch((it + 1) & 1, t0 + TILE);
-      mbar_wait(&sm.bar[it & 1], (bar_parity >> (it & 1)) & 1u);  // the tile's bytes have landed
-      bar_parity ^= 1u << (it & 1);
-      __syncthreads();  // goff ready / previous tile's scatter has read wc
-#pragma unroll
-      for (int k = 0; k < WARPS; k += THREADS / 256) {
-        const int row = k + (tid >> 8);
-        if (row < WARPS) sm.wc[row][tid & 255] = 0;
-      }
-      unsigned long long v[ITEMS];
-      unsigned d[ITEMS], peers[ITEMS], old[ITEMS];
-      const unsigned base = t0 + warp * WTILE;
-#pragma unroll
-      for (int r = 0; r < ITEMS; r++) v[r] = sm.tile[it & 1][warp * WTILE + r * 32 + lane];
-      __syncthreads();
-#pragma unroll
-      for (int r = 0; r < ITEMS; r++) {  // all matches first: they do not depend on each other
-        // positions past the end sit behind every valid word of the last tile: digit 255 keeps them behind, never stored
-        d[r] = base + r * 32 + lane < n ? rx_digit(v[r], pass) : 255u;
-        // lanes holding the same digit, from eight ballots (measured faster than __match_any_sync here: 5.1 vs 5.7 ms per
-        // 999 frames for the whole select stage)
-        unsigned pm = 0xffffffffu;
-#pragma unroll
-        for (int b = 0; b < 8; b++) {
-          const bool bit = (d[r] >> b) & 1u;
-          const unsigned bal = __ballot_sync(0xffffffffu, bit);
-          pm &= bit ? bal : ~bal;
-        }
-        peers[r] = pm;
-      }
-#pragma unroll
-      for (int r = 0; r < ITEMS; r++) {  // the leader of every digit group bumps the warp's counter, in round order
-        // (plain load + store: shared-memory atomics cost 2 cycles per active lane and were the bottleneck)
-        old[r] = 0;
-        if (lane == __ffs(peers[r]) - 1) {
-          old[r] = sm.wc[warp][d[r]];
-          sm.wc[warp][d[r]] = old[r] + (unsigned)__popc(peers[r]);
-        }
-        __syncwarp();
-      }
-      const unsigned lt = (1u << lane) - 1u;
-#pragma unroll
-      for (int r = 0; r < ITEMS; r++) old[r] = __shfl_sync(0xffffffffu, old[r], __ffs(peers[r]) - 1) + __popc(peers[r] & lt);
-      __syncthreads();
-      if (tid < 256) {
-        unsigned run = sm.goff[tid];
-#pragma unroll
-        for (int k = 0; k < WARPS; k++) {
-          const unsigned c = sm.wc[k][tid];
-          sm.wc[k][tid] = run;
-          run += c;
-        }
-        sm.goff[tid] = run;
-      }
-      __syncthreads();
-#pragma unroll
-      for (int r = 0; r < ITEMS; r++)
-        if (base + r * 32 + lane < n) dst[sm.wc[warp][d[r]] + old[r]] = v[r];
-    }
-    __threadfence();  // the next pass reads these words back through the copy engine (L2)
-    __syncthreads();
-    unsigned long long* t = src;
-    src = dst;
-    dst = t;
-  }
-  if (tid == 0) wv.sorted_in_b[fr] = src != A;  // nms_kernel reads the list where the last pass left it
-  A = src;
-
-  // final sweep: order the equal-code runs by the full score, note score ties.  Eight consecutive positions per thread.
-  const unsigned* hi = reinterpret_cast<const unsigned*>(A) + 1;
-  for (unsigned i0 = 0; i0 < n; i0 += THREADS * 8) {
-    const unsigned ib = i0 + tid * 8;
-    unsigned c[10];  // codes of positions ib-1 .. ib+8
-#pragma unroll
-    for (int k = 0; k < 10; k++) {
-      const unsigned i = ib + k - 1;  // wraps for ib == 0, k == 0: rejected by i < n
-      c[k] = i < n ? __ldcg(hi + 2 * (size_t)i) : 0u;
-    }
-    unsigned starts = 0;
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      const unsigned i = ib + k;
-      if (i + 1 < n && c[k + 1] == c[k + 2] && !(i > 0 && c[k] == c[k + 1])) starts |= 1u << k;
-    }
-    while (starts) {  // rare
-      const unsigned i = ib + __ffs(starts) - 1;
-      starts &= starts - 1;
-      const unsigned code = (unsigned)(A[i] >> 32);
-      unsigned j = i + 2;
-      while (j < n && j - i < RX_MAXRUN && (unsigned)(__ldcg(A + j) >> 32) == code) j++;
-      if (j < n && (unsigned)(__ldcg(A + j) >> 32) == code) {  // pathological pile-up: let the exact path decide
-        atomicMin(wv.tiepos + fr, i);
-        continue;
-      }
-      for (unsigned p = i + 1; p < j; p++) {
-        const unsigned long long e = A[p];
-        const unsigned long long ke = rx_key_of(wv, fr, (unsigned)e);
-        unsigned q = p;
-        while (q > i) {
-          const unsigned long long f = A[q - 1];
-          if (!(rx_key_of(wv, fr, (unsigned)f) < ke)) break;
-          A[q] = f;
-          q--;
-        }
-        A[q] = e;
-      }
-      // identical scores inside the run: flag the later member of every pair, every member of larger groups
-      for (unsigned p = i; p + 1 < j; p++)
-        if (rx_key_of(wv, fr, (unsigned)A[p]) == rx_key_of(wv, fr, (unsigned)A[p + 1])) {
-          A[p + 1] |= RX_TIE;
-          if (p > i && (A[p] & RX_TIE)) {
-            A[p - 1] |= RX_BIG;
-            A[p] |= RX_BIG;
-            A[p + 1] |= RX_BIG;
-          }
-        }
-    }
-  }
-}
-
-// ---- greedy selection over the sorted list ---------------------------------------------------------------------------
-// Same chunk scheme as select_kernel, but "is an accepted corner closer than min_dist?" is ONE bit: every accepted corner
-// marks the open disc dx^2 + dy^2 < min_dist^2 around it in a per-frame pixel bitmap (the storage of the bitmap's prefix
-// sums, unused unless a frame falls back), one (corner, row) pair per thread.  Integer arithmetic throughout: exact.
-constexpr int NMS_THREADS = 256, NMS_EPT = 8, NMS_CHUNK = NMS_THREADS * NMS_EPT, NMS_ALIVE = 256, NMS_WARPS = NMS_THREADS / 32;
-
-struct NmsSmem {
-  __align__(16) unsigned pxy[NMS_ALIVE];  // survivors of the chunk in priority order, y << 16 | x
-  unsigned accm[NMS_ALIVE / 32], deadm[NMS_ALIVE / 32];  // decided survivors, one bit each
-  unsigned short accl[NMS_ALIVE];
-  int wcnt[NMS_WARPS];
-  int consumed, accepted, cut, tiehit;
-};
-
-__device__ __forceinline__ int nms_block_scan(NmsSmem& sm, int c, int& total) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  int inc = c;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int u = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += u;
-  }
-  if (lane == 31) sm.wcnt[warp] = inc;
-  __syncthreads();
-  int pre = 0, tot = 0;
-#pragma unroll
-  for (int k = 0; k < NMS_WARPS; k++) {
-    const int v = sm.wcnt[k];
-    if (k < warp) pre += v;
-    tot += v;
-  }
-  __syncthreads();  // wcnt is reused by the next scan
-  total = tot;
-  return inc - c + pre;
-}
-
-__global__ void __launch_bounds__(NMS_THREADS) nms_kernel(CornerWorkView wv, int w, int h, int max_corners, int min_dist,
-                                                          double2* __restrict__ out_xy, int* __restrict__ out_n) {
-  __shared__ NmsSmem sm;
-  const int fr = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const unsigned ntot = wv.nfinal[fr];
-  if (ntot > (unsigned)wv.cand_cap) {  // capacity exceeded: report, never truncate silently
-    if (tid == 0) {
-      wv.status[fr] = 1;
-      if (out_n) out_n[fr] = -1;
-    }
-    return;
-  }
-  const int n = (int)ntot;
-  const int cap_out = max_corners < 1 ? 1 : max_corners;  // the cap is tested after the push (:298-299)
-  const unsigned long long* sorted = (wv.sorted_in_b[fr] ? wv.pk_b : wv.pk_a) + (size_t)fr * wv.cand_cap;  // low word: list slot
-  const unsigned* slot_yx = wv.tmp_idx + (size_t)fr * wv.cand_cap;
-  unsigned* blocked = wv.wordoff + (size_t)fr * wv.words_per_frame;  // free until a fallback frame needs raster ranks
-  double2* out = out_xy + (size_t)fr * cap_out;
-  const int d = min_dist, d2 = min_dist * min_dist, rows = 2 * d - 1;
-  const bool suppress = wv.cell > 0;
-  if (tid == 0) {
-    sm.consumed = 0;
-    sm.accepted = 0;
-    sm.tiehit = 0;
-  }
-  __syncthreads();
-  while (true) {
-    const int consumed = sm.consumed, acc0 = sm.accepted;
-    if (consumed >= n || acc0 >= cap_out) break;
-    const int cnt = min(NMS_CHUNK, n - consumed);
-    // (1) this chunk's candidates against the corners accepted in earlier chunks: NMS_EPT consecutive candidates per thread
-    unsigned yx[NMS_EPT], bw[NMS_EPT];
-#pragma unroll
-    for (int e = 0; e < NMS_EPT; e++) {
-      const int t = tid * NMS_EPT + e;
-      yx[e] = t < cnt ? (unsigned)__ldcg(sorted + consumed + t) : 0u;
-    }
-    unsigned tie = 0, big = 0;  // per candidate of this thread: RX_TIE / RX_BIG
-#pragma unroll
-    for (int e = 0; e < NMS_EPT; e++) {
-      const int t = tid * NMS_EPT + e;
-      tie |= (yx[e] >> 31) << e;
-      big |= ((yx[e] >> 30) & 1u) << e;
-      yx[e] = t < cnt ? __ldg(slot_yx + (yx[e] & RX_SLOT)) : 0u;
-    }
-#pragma unroll
-    for (int e = 0; e < NMS_EPT; e++) {
-      const int t = tid * NMS_EPT + e;
-      const unsigned x = yx[e] & 0xFFFFu, y = yx[e] >> 16;
-      bw[e] = (suppress && t < cnt) ? __ldcg(blocked + (size_t)y * wv.wpr + (x >> 5)) : 0u;
-    }
-    unsigned am = 0;
-#pragma unroll
-    for (int e = 0; e < NMS_EPT; e++)
-      if (tid * NMS_EPT + e < cnt && !((bw[e] >> (yx[e] & 31u)) & 1u)) am |= 1u << e;
-    {
-      // std::sort's order inside a group of identical scores is only observable if at least two of its members are still
-      // unblocked: they would be accepted in that order, or one would suppress the other.  Conservative test on the
-      // survivors of the bitmap check (predecessors outside the warp / chunk count as unblocked).
-      const unsigned up = __shfl_up_sync(0xffffffffu, am, 1);
-      const unsigned prev_alive = (am << 1) | (lane > 0 ? (up >> (NMS_EPT - 1)) & 1u : 1u);
-      if (am & (big | (tie & prev_alive))) sm.tiehit = 1;
-    }
-    // ordered compaction of the survivors; at most NMS_ALIVE are resolved now, the chunk is cut after the last one
-    int na;
-    const int exc = nms_block_scan(sm, __popc(am), na);
-    if (tid == 0) sm.cut = cnt;
-    __syncthreads();
-    {
-      int r = exc;
-#pragma unroll
-      for (int e = 0; e < NMS_EPT; e++)
-        if (am & (1u << e)) {
-          if (r < NMS_ALIVE) sm.pxy[r] = yx[e];
-          if (r == NMS_ALIVE) sm.cut = tid * NMS_EPT + e;  // first candidate that does not fit: it starts the next chunk
-          r++;
-        }
-    }
-    if (tid < NMS_ALIVE / 32) sm.accm[tid] = sm.deadm[tid] = 0;
-    na = na < NMS_ALIVE ? na : NMS_ALIVE;
-    __syncthreads();
-    const int used = sm.cut;
-    // (2) conflicts inside the chunk.  Thread i first collects the set C_i of higher-priority survivors closer than
-    // min_dist as a bit row (branch-free, broadcast loads; warp w only needs words 0..w), then rounds of pure bit
-    // logic: dead if C_i meets an accepted survivor, accepted once every member of C_i is dead.
-    const unsigned me = sm.pxy[tid];
-    const int mx = (int)(me & 0xFFFFu), my = (int)(me >> 16);
-    unsigned C[NMS_ALIVE / 32];
-#pragma unroll
-    for (int wd = 0; wd < NMS_ALIVE / 32; wd++) {
-      C[wd] = 0;
-      if (suppress && wd <= warp && wd * 32 < na) {
-        unsigned bits = 0;
-#pragma unroll
-        for (int q = 0; q < 8; q++) {
-          const uint4 o = *reinterpret_cast<const uint4*>(&sm.pxy[wd * 32 + q * 4]);
-          const unsigned ov[4] = {o.x, o.y, o.z, o.w};
-#pragma unroll
-          for (int k = 0; k < 4; k++) {
-            const int dx = (int)(ov[k] & 0xFFFFu) - mx, dy = (int)(ov[k] >> 16) - my;
-            if (dx * dx + dy * dy < d2) bits |= 1u << (q * 4 + k);
-          }
-        }
-        if (wd == warp) bits &= (1u << lane) - 1u;  // strictly higher priority only
-        C[wd] = bits;
-      }
-    }
-    int state = tid < na ? ST_UNDEC : ST_DEAD;
-    if (!suppress && tid < na) state = ST_ACC;
-    while (true) {
-      if (state == ST_UNDEC) {
-        unsigned hit = 0, und = 0;
-#pragma unroll
-        for (int wd = 0; wd < NMS_ALIVE / 32; wd++) {
-          const unsigned a = sm.accm[wd], dd = sm.deadm[wd];
-          hit |= C[wd] & a;
-          und |= C[wd] & ~(a | dd);
-        }
-        state = hit ? ST_DEAD : (und ? ST_UNDEC : ST_ACC);
-      }
-      __syncthreads();  // everybody has read the masks of the previous round
-      const unsigned ba = __ballot_sync(0xffffffffu, state == ST_ACC), bd = __ballot_sync(0xffffffffu, state == ST_DEAD);
-      if (lane == 0) {
-        sm.accm[warp] = ba;
-        sm.deadm[warp] = bd;
-      }
-      if (__syncthreads_or(state == ST_UNDEC) == 0) break;
-    }
-    // (3) append accepted survivors in priority order, stop at the cap; mark their discs
-    const bool acc = state == ST_ACC;
-    int nacc;
-    const int rank = nms_block_scan(sm, acc ? 1 : 0, nacc);
-    if (acc && acc0 + rank < cap_out) {
-      out[acc0 + rank] = make_double2((double)mx, (double)my);
-      sm.accl[rank] = (unsigned short)tid;
-    }
-    __syncthreads();
-    const int nnew = min(nacc, cap_out - acc0);
-    if (suppress && acc0 + nnew < cap_out) {  // nothing is looked up once the cap is reached
-      for (int i = tid; i < nnew * rows; i += NMS_THREADS) {
-        const int c = i / rows, dy = i - c * rows - (d - 1);
-        const unsigned sp = sm.pxy[sm.accl[c]];
-        const int px = (int)(sp & 0xFFFFu), py = (int)(sp >> 16) + dy;
-        if (py < 0 || py >= h) continue;
-        const int r2 = d2 - 1 - dy * dy;  // dx^2 <= r2  <=>  dx^2 + dy^2 < d^2
-        int r = (int)sqrtf((float)r2);
-        while (r * r > r2) r--;
-        while ((r + 1) * (r + 1) <= r2) r++;
-        const int xa = max(px - r, 0), xb = min(px + r, w - 1);
-        unsigned* rowp = blocked + (size_t)py * wv.wpr;
-        for (int wd = xa >> 5; wd <= (xb >> 5); wd++) {
-          const int lo = max(xa - wd * 32, 0), hi = min(xb - wd * 32, 31);
-          atomicOr(rowp + wd, (0xFFFFFFFFu >> (31 - hi)) & (0xFFFFFFFFu << lo));
-        }
-      }
-      __threadfence_block();
-    }
-    __syncthreads();
-    if (tid == 0) {
-      sm.accepted = acc0 + nnew;
-      sm.consumed = consumed + used;
-    }
-    __syncthreads();
-  }
-  if (tid == 0) {
-    wv.status[fr] = 0;
-    if (out_n) out_n[fr] = sm.accepted;
-    // an observable tie (above), or a pile-up of equal order codes the sort did not resolve, inside the consumed prefix:
-    // the frame is redone by select_kernel mode 3
-    if (sm.tiehit || wv.tiepos[fr] < (unsigned)sm.consumed) wv.status[fr] = 3;
-  }
-}
-
 // ---- bucket selection (default path) ------------------------------------------------------------------------------------------
 // The greedy loop only ever accepts candidates that no accepted corner blocks, and a candidate that is blocked once stays
 // blocked.  With ~50 candidates per accepted corner almost every candidate is blocked by the time its turn comes, so the
@@ -892,8 +373,8 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(CornerWorkView wv, int
 //   (2) scatters the words into bucket order (one pass, unordered inside a bucket);
 //   (3) walks the buckets from the best score down in gathers of <= 4096 words: a word whose pixel is already blocked is
 //       dropped at once (order-independent, exact); the SURVIVORS of the gather - all of them early on, a few per cent
-//       later - are sorted in shared memory (bitonic, 64-bit words) and go through the greedy rounds (conflict bit rows,
-//       as nms_kernel); accepted corners mark their discs; the walk stops when max_corners are accepted.
+//       later - are sorted in shared memory (bitonic, 64-bit words) and go through the greedy rounds (conflict bit rows);
+//       accepted corners mark their discs; the walk stops when max_corners are accepted.
 // Buckets the selection never reaches are never sorted, blocked candidates are never sorted, and nothing is gathered
 // through a slot index: the word carries the pixel.
 // (Tried and dropped: the blocked-pixel map in 8 x 4 pixel tiles, a 32-byte sector = 16 x 16 pixels, so that a disc touches
@@ -992,7 +473,7 @@ __global__ void __launch_bounds__(BK_THREADS, 4) bucket_select_kernel(CornerWork
   BucketSmem& sm = *reinterpret_cast<BucketSmem*>(bk_raw);
   const int fr = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const size_t cb = (size_t)fr * wv.cand_cap;
-  unsigned long long* B = wv.pk_b + cb;
+  unsigned long long* B = wv.words + cb;
   const bool exact = wv.exact_list[fr] != 0;
   const unsigned nlist = exact ? wv.nfinal[fr] : wv.ncand[fr];
   if (nlist > (unsigned)wv.cand_cap) {  // capacity exceeded: report, never truncate silently
@@ -1452,7 +933,7 @@ __global__ void __launch_bounds__(BK_THREADS, 4) bucket_select_kernel(CornerWork
 }
 
 // mode 0: full shi_tomasi selection; mode 1: sort only (sfmgpu_sort_perm_desc).
-// mode 3: redo exactly the frames nms_kernel marked with status 3 (a consumed score tie) through the emulation.
+// mode 3: redo exactly the frames bucket_select_kernel marked with status 3 (a consumed score tie) through the emulation.
 __global__ void __launch_bounds__(SEL_THREADS, 4) select_kernel(CornerWorkView wv, int w, int max_corners, int min_dist, int mode,
                                                                double2* __restrict__ out_xy, int* __restrict__ out_n) {
   extern __shared__ __align__(16) unsigned char sel_raw[];
@@ -1632,10 +1113,8 @@ __global__ void __launch_bounds__(SEL_THREADS, 4) select_kernel(CornerWorkView w
 }
 
 int select_smem_config(sfmgpu_ctx* ctx) {
-  static const int cfg_id[3] = {sfm_next_cfg_id(), sfm_next_cfg_id(), sfm_next_cfg_id()};
-  SFM_SMEM_OPTIN(ctx, cfg_id[0], select_kernel, sizeof(SelSmem));
-  SFM_SMEM_OPTIN(ctx, cfg_id[1], (radix_sort_frame_kernel<512, 8>), sizeof(RadixSmem<512>));
-  SFM_SMEM_OPTIN(ctx, cfg_id[2], (radix_sort_frame_kernel<1024, 4>), sizeof(RadixSmem<1024>));
+  static const int sel_id = sfm_next_cfg_id();
+  SFM_SMEM_OPTIN(ctx, sel_id, select_kernel, sizeof(SelSmem));
   static const int bk_id = sfm_next_cfg_id();
   SFM_SMEM_OPTIN(ctx, bk_id, bucket_select_kernel, sizeof(BucketSmem));
   return 0;
@@ -1679,20 +1158,11 @@ int sfm_corners_select_stage(sfmgpu_ctx* ctx, const sfmgpu_frames* f, int first,
     return 0;
   }
   SFM_CUDA(ctx, cudaMemsetAsync(wv.wordoff, 0, sizeof(unsigned) * wv.words_per_frame * count, ctx->stream));  // the blocked-pixel map
-  if (ctx->select_mode == 2) {  // the full radix sort + selection over the sorted list (A/B timing)
-    SFM_CUDA(ctx, cudaMemsetAsync(wv.tiepos, 0xFF, sizeof(unsigned) * count, ctx->stream));
-    if (count >= 2 * ctx->n_sm)
-      SFM_LAUNCH(ctx, (radix_sort_frame_kernel<512, 8>), count, 512, sizeof(RadixSmem<512>), wv, quality);
-    else  // few frames: the widest block per frame
-      SFM_LAUNCH(ctx, (radix_sort_frame_kernel<1024, 4>), count, 1024, sizeof(RadixSmem<1024>), wv, quality);
-    SFM_LAUNCH(ctx, nms_kernel, count, NMS_THREADS, 0, wv, f->w, f->h, max_corners, min_dist, out_xy, out_n);
-  } else {
-    // tests: short codes make equal codes common (modes 12..34); small gathers make the sub-bucket walk common (modes 1000 + g)
-    const int code_bits = (ctx->select_mode >= 12 && ctx->select_mode <= BK_CODE_BITS) ? ctx->select_mode : BK_CODE_BITS;
-    const int gather_cap = ctx->select_mode >= 1000 ? ctx->select_mode - 1000 : BK_T;
-    SFM_LAUNCH(ctx, bucket_select_kernel, count, BK_THREADS, sizeof(BucketSmem), wv, f->lvl[0], f->pitch[0], f->fstride[0], first, f->w, f->h,
-               max_corners, min_dist, quality, code_bits, gather_cap, out_xy, out_n);
-  }
+  // tests: short codes make equal codes common (modes 12..34); small gathers make the sub-bucket walk common (modes 1000 + g)
+  const int code_bits = (ctx->select_mode >= 12 && ctx->select_mode <= BK_CODE_BITS) ? ctx->select_mode : BK_CODE_BITS;
+  const int gather_cap = ctx->select_mode >= 1000 ? ctx->select_mode - 1000 : BK_T;
+  SFM_LAUNCH(ctx, bucket_select_kernel, count, BK_THREADS, sizeof(BucketSmem), wv, f->lvl[0], f->pitch[0], f->fstride[0], first, f->w, f->h,
+             max_corners, min_dist, quality, code_bits, gather_cap, out_xy, out_n);
   // frames where a score tie was consumed (status 3): raster order, then the exact emulation.  Blocks of all other
   // frames return at once.
   SFM_TRY(sfm_corner_raster_order(ctx, count, wv, quality, 1));
@@ -1714,8 +1184,8 @@ size_t sfm_corner_work_bytes_md(int w, int h, int nframes, int cand_cap, int min
 extern "C" int sfmgpu_select_set_mode(sfmgpu_ctx* ctx, int mode) {
   SFM_ENTER(ctx);
   if (!ctx) return SFMGPU_E_ARG;
-  if (mode != 0 && mode != 1 && mode != 2 && !(mode >= 12 && mode <= BK_CODE_BITS) && !(mode >= 1000 + 64 && mode <= 1000 + BK_T))
-    return sfm_fail(ctx, SFMGPU_E_ARG, "select_set_mode: mode %d not in {0, 1, 2, 12..%d, %d..%d}", mode, BK_CODE_BITS, 1000 + 64, 1000 + BK_T);
+  if (mode != 0 && mode != 1 && !(mode >= 12 && mode <= BK_CODE_BITS) && !(mode >= 1000 + 64 && mode <= 1000 + BK_T))
+    return sfm_fail(ctx, SFMGPU_E_ARG, "select_set_mode: mode %d not in {0, 1, 12..%d, %d..%d}", mode, BK_CODE_BITS, 1000 + 64, 1000 + BK_T);
   ctx->select_mode = mode;
   return 0;
 }

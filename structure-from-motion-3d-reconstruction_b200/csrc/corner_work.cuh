@@ -3,14 +3,10 @@
 #include <stddef.h>
 #include <stdint.h>
 
-// Width of the radix selection path's order code (a multiple of 8: one LSD pass per byte).  24 bits: ~10^3 pairs of
-// candidates per 1080p frame share a code and are ordered by their full score afterwards, one pass less than 32 bits.
-constexpr int CORNER_CODE_BITS = 24;
-
 struct CornerWorkView {
   unsigned long long* maxbits;  // [nframes] bit pattern of max u = 8*lmin
   unsigned* ncand;              // [nframes] entries appended to the provisional list by the fused pass (may exceed cand_cap)
-  unsigned* nfinal;             // [nframes] candidates = sort words in pk_a (may exceed cand_cap: overflow)
+  unsigned* nfinal;             // [nframes] candidates that reach the final threshold (may exceed cand_cap: overflow)
   int* exact_list;              // [nframes] != 0: the unordered list holds exactly the nfinal candidates (two-pass / rescued)
   int* rescue_list;             // [nframes] frames whose provisional list overflowed
   int* rescue_count;            // [1]
@@ -22,15 +18,10 @@ struct CornerWorkView {
   unsigned long long* tmp_key;  // [nframes][cand_cap] unordered list: score bits
   unsigned long long* key;      // [nframes][cand_cap] raster order, then sorted in place
   unsigned* idx;                // [nframes][cand_cap] pixel as y << 16 | x
-  unsigned* lpos;               // [nframes][cand_cap] partition scratch of the emulation (aliases pk_b)
+  unsigned* lpos;               // [nframes][cand_cap] partition scratch of the emulation (aliases words)
   unsigned* rpos;               // [nframes][cand_cap]
   unsigned* grid;               // [nframes][grid_cells][2] accepted corners per min_dist cell (packed y<<16|x)
-  // radix selection path (corner_select.cu): packed (order code << 32 | slot in the unordered list) ping-pong buffers
-  // and the first sorted position holding two candidates with identical scores
-  unsigned long long* pk_a;     // [nframes][cand_cap] written by the candidate pass, holds the sorted result
-  unsigned long long* pk_b;     // [nframes][cand_cap]
-  unsigned* tiepos;             // [nframes]
-  int* sorted_in_b;             // [nframes] != 0: the sorted list ended in pk_b (odd number of passes ran)
+  unsigned long long* words;    // [nframes][cand_cap] bucket_select_kernel: order code << 30 | y << 15 | x in bucket order
   int wpr;
   size_t words_per_frame;
   int cand_cap;
@@ -48,7 +39,7 @@ static inline size_t corner_work_carve(CornerWorkView& v, void* base, int w, int
     off += (bytes + 255) / 256 * 256;
     return p;
   };
-  cand_cap = (cand_cap + 1) & ~1;  // per-frame strides of the 8-byte arrays stay 16-byte aligned (cp.async)
+  cand_cap = (cand_cap + 1) & ~1;  // per-frame strides of the 8-byte arrays stay 16-byte aligned
   v.wpr = (w + 31) / 32;
   v.words_per_frame = (size_t)v.wpr * h;
   v.cand_cap = cand_cap;
@@ -71,11 +62,8 @@ static inline size_t corner_work_carve(CornerWorkView& v, void* base, int w, int
   v.key = (unsigned long long*)take(sizeof(unsigned long long) * (size_t)cand_cap * nframes);
   v.idx = (unsigned*)take(sizeof(unsigned) * (size_t)cand_cap * nframes);
   v.grid = (unsigned*)take(sizeof(unsigned) * (v.grid_per_frame ? v.grid_per_frame : 1) * nframes);
-  v.pk_a = (unsigned long long*)take(sizeof(unsigned long long) * (size_t)cand_cap * nframes);
-  v.pk_b = (unsigned long long*)take(sizeof(unsigned long long) * (size_t)cand_cap * nframes);
-  v.lpos = (unsigned*)v.pk_b;  // the emulation runs after (or instead of) the radix sort
+  v.words = (unsigned long long*)take(sizeof(unsigned long long) * (size_t)cand_cap * nframes);
+  v.lpos = (unsigned*)v.words;  // the emulation redoes a frame only after the bucket selection is done with every frame
   v.rpos = v.lpos ? v.lpos + (size_t)cand_cap * nframes : nullptr;
-  v.tiepos = (unsigned*)take(sizeof(unsigned) * nframes);
-  v.sorted_in_b = (int*)take(sizeof(int) * nframes);
   return off + 256;
 }

@@ -325,7 +325,7 @@ static ChunkArgs chunk_args(sfmgpu_frames* f, int first_frame, int pair_off, int
 }
 
 // Pairs per corner launch: >= 4 blocks per SM keeps the one-block-per-frame selection kernels busy; large frames are
-// limited by the work area instead (57 MB per 4K frame: 16 GiB hold 280 of them - still two waves of blocks)
+// limited by the work area instead (47 MB per 4K frame at min_distance 8: 16 GiB hold 362 of them, ~2.4 blocks per SM)
 static int pair_chunk(sfmgpu_ctx* ctx, sfmgpu_frames* f, int npairs, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
   ChunkArgs c1 = chunk_args(f, 0, 0, 1, cfg, out, &out->work[0]);
   const size_t per_frame = sfm_corner_work_bytes_md(f->w, f->h, 1, c1.cand_cap, c1.md);

@@ -229,7 +229,9 @@ class Context:
         self._ck(self.lib.sfmgpu_klt_set_mode(self.h, mode))
 
     def select_set_mode(self, mode):
-        """0 radix sort + exact fallback on consumed score ties (default), 1 introsort emulation for every frame."""
+        """0 bucket selection + exact fallback on consumed score ties (default), 1 introsort emulation for every frame,
+        12..34 bucket selection with that many order-code bits, 1064..5096 bucket selection with gathers of (mode - 1000)
+        words (tests).  Other modes raise SfmGpuError."""
         self._ck(self.lib.sfmgpu_select_set_mode(self.h, mode))
 
     def solver_set_mode(self, mode):

@@ -100,12 +100,12 @@ def test_device_std_sort_permutation(ctx, port, n, distinct):
 @pytest.mark.parametrize("name", list(_images()))
 @pytest.mark.parametrize("mc,q,d", [(2200, 0.01, 8), (50, 0.2, 3), (0, 0.01, 8), (300, 0.0, 1), (100, 0.01, 0), (4000, 0.001, 2),
                                     (500, 0.01, 25)])
-@pytest.mark.parametrize("select_mode", [0, 1, 2, 14, 20, 1064, 1300])
+@pytest.mark.parametrize("select_mode", [0, 1, 14, 20, 1064, 1300])
 def test_corners_bit_exact(ctx, checker, name, mc, q, d, select_mode):
-    """select_mode 0: bucket selection + exact introsort fallback on observable score ties; 1: introsort emulation; 2: full
-    radix sort + selection; 14 / 20: bucket selection with 14- / 20-bit order codes (equal codes everywhere: the exact-score
-    path orders them; with 14 bits a bucket is a few codes wide); 1064 / 1300: gathers of 64 / 300 words (every bucket is
-    oversized: walked in runs of its sub-buckets, or handed to the exact emulation where a sub-bucket alone is too large)."""
+    """select_mode 0: bucket selection + exact introsort fallback on observable score ties; 1: introsort emulation;
+    14 / 20: bucket selection with 14- / 20-bit order codes (equal codes everywhere: the exact-score path orders them;
+    with 14 bits a bucket is a few codes wide); 1064 / 1300: gathers of 64 / 300 words (every bucket is oversized: walked
+    in runs of its sub-buckets, or handed to the exact emulation where a sub-bucket alone is too large)."""
     img = _images()[name]
     f = _frames(ctx, [img], 1)
     ctx.select_set_mode(select_mode)
@@ -120,7 +120,8 @@ def test_corners_bit_exact(ctx, checker, name, mc, q, d, select_mode):
 @pytest.mark.parametrize("period,mc,d", [(32, 3000, 8), (48, 500, 3), (17, 20000, 0), (64, 8000, 12)])
 def test_corners_periodic_image_ties(ctx, checker, period, mc, d):
     """A periodic image: every score occurs dozens of times, so std::sort's tie order decides the corners from the first
-    candidate on (the radix path must hand every such frame to the exact emulation), next to tie-free frames in one batch."""
+    candidate on (the bucket selection must hand every such frame to the exact emulation), next to tie-free frames in one
+    batch."""
     rng = np.random.default_rng(period)
     cell = rng.integers(0, 256, (period, period), dtype=np.uint8)
     w, h = 1280, 720
@@ -570,15 +571,15 @@ def test_pair_frontend_bench_shape_pair(ctx, checker):
 
 
 def test_pair_frontend_batch_with_score_ties(ctx, checker):
-    """Quantised frames (many identical scores) between plain ones in ONE batch: the radix selection redoes exactly the
-    frames whose consumed prefix holds a tie, inside the batched launch."""
+    """Quantised frames (many identical scores) between plain ones in ONE batch: the bucket selection hands exactly the
+    frames whose consumed prefix holds a tie to the exact emulation, inside the batched launch."""
     imgs = [synth.frame(31, t, W, H) for t in range(7)]
     for t in (1, 2, 5):
         imgs[t] = imgs[t] >> 4 << 4
     f = _frames(ctx, imgs)
     cfg = sfmgpu.lkcfg(max_tracks=900)
     pairs = ctx.pairs(6, 900)
-    for mode in (0, 1, 2, 16, 1100):
+    for mode in (0, 1, 16, 1100):
         ctx.select_set_mode(mode)
         try:
             pairs.run(f, 0, 6, cfg)
@@ -651,11 +652,11 @@ def test_c3_shape_4k_pair(ctx, checker):
     assert np.array_equal(kept_all[sel], keep) and _klt_close(p1[sel], w1) and _klt_close(pb[sel], wb)
 
 
-@pytest.mark.parametrize("select_mode", [0, 1300, 3048, 20, 2])
+@pytest.mark.parametrize("select_mode", [0, 1300, 3048, 20])
 def test_c3_shape_4k_corners_select_modes(ctx, checker, select_mode):
     """One 3840x2160 frame, 8000 corners (~400 k candidates): the bucket selection with its default geometry, with gathers
-    of 300 / 2048 words (every bucket oversized: the sub-bucket walk at scale, or the exact emulation), with 20-bit order
-    codes (equal codes by the exact score recomputed from the image) and the full radix sort: bit-exact corners."""
+    of 300 / 2048 words (every bucket oversized: the sub-bucket walk at scale, or the exact emulation) and with 20-bit
+    order codes (equal codes by the exact score recomputed from the image): bit-exact corners."""
     w, h, nmax = 3840, 2160, 8000
     f0 = synth.frame(SEED, 3, w, h)
     f = _frames(ctx, [f0], 1)
@@ -676,3 +677,5 @@ def test_errors_are_loud(ctx):
         f.klt_track(0, 1, np.zeros((1, 2)), radius=50)
     with pytest.raises(sfmgpu.SfmGpuError):
         ctx.frames(0, 48, 2, 3)
+    with pytest.raises(sfmgpu.SfmGpuError):  # not a selection mode: an error, never a silent default
+        ctx.select_set_mode(2)

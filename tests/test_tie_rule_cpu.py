@@ -1,4 +1,5 @@
-"""CPU check of the "observable tie" rule behind the radix selection path (csrc/corner_select.cu: nms_kernel, DESIGN.md §4).
+"""CPU check of the "observable tie" rule behind the default selection (csrc/corner_select.cu: bucket_select_kernel,
+DESIGN.md §4).
 
 std::sort may leave a group of candidates with IDENTICAL scores in any order.  The rule: the order inside a group can only
 change the result of the greedy min-distance selection if at least TWO members of the group are unblocked (farther than
@@ -22,8 +23,8 @@ def greedy(points, d, cap):
 
 
 def observable(groups, d, cap):
-    """The device's criterion, evaluated in the radix order: a group is flagged iff >= 2 of its members are unblocked by the
-    corners accepted BEFORE the group (the kernel tests a superset: unblocked by the corners of earlier chunks)."""
+    """The device's criterion, evaluated in score order: a group is flagged iff >= 2 of its members are unblocked by the
+    corners accepted BEFORE the group (the kernel tests a superset: unblocked by the corners of earlier rounds)."""
     acc = []
     for g in groups:
         free = [p for p in g if all((p[0] - ax) ** 2 + (p[1] - ay) ** 2 >= d * d for ax, ay in acc)]
