@@ -78,7 +78,7 @@ int sfmgpu_flush_l2(sfmgpu_ctx* ctx, size_t bytes);
 int sfmgpu_profile(sfmgpu_ctx* ctx, int enable);
 int sfmgpu_stage_times(sfmgpu_ctx* ctx, float* ms4);
 /* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac),
- * ms[5] = the frame gather of sfmgpu_pair_frontend_list. */
+ * ms[5] = the frame gather of sfmgpu_pair_frontend_list and sfmgpu_multitracker_step_frames. */
 int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n);
 /* Measured non-tensor FP64 throughput of this GPU (DFMA micro-benchmark, ~10 ms): the KLT / RANSAC roofline. */
 int sfmgpu_fp64_peak(sfmgpu_ctx* ctx, double* tflops);
@@ -194,6 +194,25 @@ int sfmgpu_pairs_set_matches(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int npairs, const
                              const int32_t* n_kept);
 /* Device addresses of the same arrays (for NCCL gathers by the scheduler); valid until pairs_destroy. */
 int sfmgpu_pairs_device_ptrs(sfmgpu_pairs* p, void** li_xy, void** lj_xy, void** n_kept, void** n_corners);
+/* Segment mode (SURVEY.md §8e): nseg segments of one resident sequence, each a fresh KLTTracker (:323-391) with cfg: reset on
+ * frame seg_first[j], then step(frame seg_first[j] + k) for k = 1 .. steps.  Step k of segment j goes to row j * steps + (k - 1)
+ * of `out` (segment-major: a contiguous block of segments owns contiguous rows): li / lj = the step's prev / cur points of its
+ * survivors in track order, n_kept, n_corners = the size of the track list entering the step (the tracks attempted), and the
+ * survivors' track ids (sfmgpu_pairs_ids_download_all; ids count from 0 in every segment).  Rows [0, nseg * steps) become the
+ * last batch: every reader of the pairs object works on them unchanged.  With sfmgpu_pairs_set_ransac on `out` every row also
+ * gets find_E_ransac on its survivors (:1739 uses iters 2500, thr 1e-3, min_inliers 60, min_points 1); a step that resets its
+ * segment instead of tracking it (empty track list) is SFMGPU_TV_SKIPPED.  Per segment the rows equal a sfmgpu_multitracker run
+ * fed that segment's frames; they are NOT the rows of one unsegmented run (tracker state chains frame to frame).  Repeated and
+ * overlapping seg_first are allowed.  Segments run as sfmgpu_multitracker slots in lock step, chunks of them back to back (the
+ * number of slots is bounded by the reset's corner work area, W*H candidates per slot).  seg_first[j] + steps >= f->n,
+ * nseg * steps > max_pairs, out's max_corners below ROWS = max(max_tracks, min_tracks, 1) + 1, steps < 1 or a cfg that does not
+ * match f is SFMGPU_E_ARG, reported before any work is queued.  Returns when the batch has finished. */
+int sfmgpu_pair_frontend_segments(sfmgpu_ctx* ctx, sfmgpu_frames* f, const int32_t* seg_first, int nseg, int steps,
+                                  const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out);
+/* Track ids of the segment call's rows: ids [npairs][max_corners], the first n_kept of each row valid.  SFMGPU_E_STATE when the
+ * last batch came from another call (those carry no ids).  The device pointer is the same array, valid until the next batch. */
+int sfmgpu_pairs_ids_download_all(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int32_t* ids);
+int sfmgpu_pairs_ids_device_ptr(sfmgpu_pairs* p, void** ids);
 
 /* ---- RANSAC stage of the two-view unit, batched over the pairs of a batch (:1855-1857; find_E_ransac :640-761) -----------
  * What the loop-closure block does with the survivors of a pair:
@@ -274,6 +293,19 @@ int sfmgpu_sched_pair_shard(const sfmgpu_sched* s, int n_frames, int* pair_begin
 int sfmgpu_sched_gather_pairs(sfmgpu_ctx* ctx, sfmgpu_sched* s, sfmgpu_pairs* p, int n_pairs_total, int root, int with_ransac,
                               double* li_xy, double* lj_xy, int32_t* n_kept, int32_t* n_corners, int32_t* status,
                               int32_t* best_n, int32_t* inliers, double* R, double* t);
+/* Segment-mode shard of a sequence of n_frames (T) into n_segments (G) segments of *steps = L = ceil((T-1)/G) steps:
+ * seg_first[j] = G == 1 ? 0 : floor(j * (T-1-L) / (G-1)) (all G of them; may be NULL), so every pair (t, t+1) is a step of some
+ * segment, the last segment ends on frame T-1 and G*L - (T-1) < G steps are done twice.  This rank runs segments
+ * [seg_begin, seg_end) (sfmgpu_sched_shard's block rule) and must hold frames [frame_begin, frame_end) = [seg_first[seg_begin],
+ * seg_first[seg_end-1] + L + 1) (empty when it has no segment).  T < 2 or G outside [1, T-1]: SFMGPU_E_ARG.  Its rows
+ * (sfmgpu_pair_frontend_segments) are a contiguous block of the G * L rows; sfmgpu_sched_gather_pairs / _gather_pair_ids with
+ * n_pairs_total = G * L take the same blocks when world divides G. */
+int sfmgpu_sched_segment_shard(const sfmgpu_sched* s, int n_frames, int n_segments, int* steps, int* seg_begin, int* seg_end,
+                               int32_t* seg_first, int* frame_begin, int* frame_end);
+/* Collective like sfmgpu_sched_gather_pairs (same block rule, same grouped send / recv; world = 1: a local copy): the track ids of
+ * every rank's segment call into ids [n_pairs_total][max_corners] on the root.  SFMGPU_E_STATE on a rank whose last batch carries
+ * no ids. */
+int sfmgpu_sched_gather_pair_ids(sfmgpu_ctx* ctx, sfmgpu_sched* s, sfmgpu_pairs* p, int n_pairs_total, int root, int32_t* ids);
 
 /* ---- stateful tracker: KLTTracker (:323-391) ----------------------------------------------------------
  * A track list never holds more than ROWS = max(max_tracks, min_tracks, 1) + 1 entries; `cap` arguments of that size
@@ -310,6 +342,13 @@ int sfmgpu_multitracker_step(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint
 int sfmgpu_multitracker_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* host_pix);
 int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* host_pix, const uint8_t* next_host_pix,
                                        double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
+/* Resident frames: the next frame of sequence s is frame frame_idx[s] of f (pyramids built; same w, h and level count as the
+ * tracker), any indices, repeats allowed - no host-to-device copy of images.  The S pyramids are copied into the tracker's own
+ * slots (about 1.33 * w * h bytes read and written per sequence with 3 levels; sfmgpu_stage_times_n ms[5]).  Results identical to
+ * sfmgpu_multitracker_step with those images.  Prefetched frames pending: SFMGPU_E_STATE; a NULL frame_idx, an index outside
+ * [0, f->n) or a size / level mismatch: SFMGPU_E_ARG; both before any work is queued. */
+int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* f, const int32_t* frame_idx,
+                                    double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 /* Back to the state after create (the next step resets every sequence, ids restart at 0). */
 int sfmgpu_multitracker_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t);
 int sfmgpu_multitracker_tracks(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int sequence, double* xy, int32_t* ids, int cap, int* n_out);

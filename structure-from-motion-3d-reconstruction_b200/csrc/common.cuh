@@ -107,6 +107,9 @@ struct sfmgpu_pairs {
   DevBuf idx;      // list call: frame_a, frame_b (device copies for the gather)
   int last_npairs = 0;
   TwoViewState* tv = nullptr;  // allocated by the first sfmgpu_pairs_ransac call
+  int* ids = nullptr;          // segment call: track ids [max_pairs][cap] (allocated by its first use)
+  bool ids_valid = false;      // the last batch came from the segment call (other batches carry no ids)
+  sfmgpu_multitracker* seg = nullptr;  // segment call: the lock-step tracker it drives (kept for the next call)
 };
 // The stage works on result sets of `cap` rows: the pairs of a batch, or the sequences of the lock-step tracker.
 void sfm_two_view_free(sfmgpu_ctx* ctx, TwoViewState** tv);

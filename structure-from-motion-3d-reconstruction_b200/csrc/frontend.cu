@@ -234,8 +234,9 @@ void sfmgpu_pairs_destroy(sfmgpu_ctx* ctx, sfmgpu_pairs* p) {
   if (!p) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
   sfm_two_view_free(ctx, &p->tv);
+  if (p->seg) sfmgpu_multitracker_destroy(ctx, p->seg);
   void* ptrs[] = {p->xy0, p->p1, p->pb, p->li, p->lj, p->nit, p->keep, p->ncorn, p->nkept, p->totals, p->work[0].p, p->work[1].p,
-                  p->gather.p, p->idx.p};
+                  p->gather.p, p->idx.p, p->ids};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   delete p;
@@ -533,6 +534,7 @@ int sfmgpu_pair_frontend(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame, int
   if (!ctx || !f || !cfg || !out) return SFMGPU_E_ARG;
   SFM_TRY(pair_args_ok(ctx, f, first_frame, npairs, cfg, out));
   out->last_npairs = npairs;
+  out->ids_valid = false;
   SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
   const int sub = ctx->pipe_chunk;
   if (sub <= 0 || ctx->profile || npairs < 2 * sub) {  // stage profiling wants the stages back to back on one stream
@@ -585,6 +587,7 @@ int sfmgpu_pair_frontend_list(sfmgpu_ctx* ctx, sfmgpu_frames* f, const int32_t* 
     SFM_TRY(sfm_reserve(ctx, out->gather, gbytes));
   }
   out->last_npairs = npairs;
+  out->ids_valid = false;
   SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
   if (npairs == 0) return 0;
   int* d_fa = (int*)out->idx.p;
@@ -628,6 +631,7 @@ int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* 
   const int npairs = nframes > 0 ? nframes - 1 : 0;
   SFM_TRY(pair_args_ok(ctx, f, 0, npairs, cfg, out));
   out->last_npairs = npairs;
+  out->ids_valid = false;
   SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
   if (nframes == 0) return 0;
   SFM_TRY(pipe_streams(ctx));
@@ -755,6 +759,7 @@ int sfmgpu_pairs_set_matches(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int npairs, const
     SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller's arrays may be pageable / reused
   }
   p->last_npairs = npairs;
+  p->ids_valid = false;
   return 0;
 }
 
@@ -764,6 +769,24 @@ int sfmgpu_pairs_device_ptrs(sfmgpu_pairs* p, void** li_xy, void** lj_xy, void**
   if (lj_xy) *lj_xy = p->lj;
   if (n_kept) *n_kept = p->nkept;
   if (n_corners) *n_corners = p->ncorn;
+  return 0;
+}
+
+int sfmgpu_pairs_ids_device_ptr(sfmgpu_pairs* p, void** ids) {
+  if (!p || !ids) return SFMGPU_E_ARG;
+  if (!p->ids_valid) return SFMGPU_E_STATE;
+  *ids = p->ids;
+  return 0;
+}
+
+int sfmgpu_pairs_ids_download_all(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int32_t* ids) {
+  SFM_ENTER(ctx);
+  if (!ctx || !p || !ids) return SFMGPU_E_ARG;
+  if (!p->ids_valid) return sfm_fail(ctx, SFMGPU_E_STATE, "pairs_ids_download_all: the last batch carries no track ids (not a segment call)");
+  const size_t np_ = (size_t)p->last_npairs;
+  if (np_ == 0) return 0;
+  SFM_CUDA(ctx, cudaMemcpyAsync(ids, p->ids, np_ * p->cap * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 
@@ -1049,6 +1072,7 @@ struct sfmgpu_multitracker {
   std::vector<int> n, next_id;      // host copies
   double2 *trk = nullptr, *p1 = nullptr, *pb = nullptr, *oa = nullptr, *ob = nullptr, *fresh = nullptr;
   int *ids = nullptr, *oid = nullptr, *nit = nullptr, *dn = nullptr, *dnk = nullptr, *scal = nullptr;
+  int* didx = nullptr;              // step_frames: the frame index of every sequence (device copy for the gather)
   uint8_t *keep = nullptr, *ok = nullptr;
   long long track_steps = 0;
   unsigned long long* tot = nullptr;
@@ -1128,6 +1152,7 @@ int sfmgpu_multitracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_s
   al((void**)&t->ok, (size_t)t->fresh_cap);
   al((void**)&t->dn, (size_t)n_sequences * 4);
   al((void**)&t->dnk, (size_t)n_sequences * 4);
+  al((void**)&t->didx, (size_t)n_sequences * 4);
   al((void**)&t->scal, 64);
   al((void**)&t->tot, 64);
   if (e == cudaSuccess) e = cudaMemsetAsync(t->tot, 0, 64, ctx->stream);
@@ -1145,13 +1170,17 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   if (!t) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
   sfm_two_view_free(ctx, &t->tv);
-  void* ptrs[] = {t->trk, t->p1, t->pb, t->oa, t->ob, t->ids, t->oid, t->nit, t->keep, t->fresh, t->ok, t->dn, t->dnk, t->scal, t->tot};
+  void* ptrs[] = {t->trk, t->p1, t->pb, t->oa, t->ob, t->ids, t->oid, t->nit, t->keep, t->fresh, t->ok, t->dn, t->dnk, t->didx, t->scal, t->tot};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   if (t->frames) sfmgpu_frames_destroy(ctx, t->frames);
   if (t->pf_done) cudaEventDestroy(t->pf_done);
   delete t;
 }
+
+// Slot group of the next step's frames.
+static int multi_next_group(const sfmgpu_multitracker* t) { return t->parity < 0 ? 0 : (t->parity + 1) % 3; }
+static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 
 // Upload + pyramids of the frames of a LATER step on the copy stream, into the slot group after `after_group`.
 static int multi_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int after_group, const uint8_t* host_pix) {
@@ -1206,9 +1235,8 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   if (!ctx || !t) return SFMGPU_E_ARG;
   if (!host_pix && !t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: no frames given and none prefetched");
   if (host_pix && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: frames given but others are prefetched");
-  const int S = t->S, cap = t->cap;
-  const int par = t->parity < 0 ? 0 : (t->parity + 1) % 3;
-  const bool stage = sfm_two_view_enabled(t->tv);
+  const int S = t->S;
+  const int par = multi_next_group(t);
   t->tv_fresh = false;
   if (host_pix) {
     SFM_TRY(sfmgpu_frames_upload(ctx, t->frames, par * S, S, host_pix));
@@ -1219,6 +1247,46 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   }
   // the frames of the NEXT step travel while this one computes (their slot group is neither previous nor current)
   if (next_host_pix) SFM_TRY(multi_prefetch(ctx, t, par, next_host_pix));
+  return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
+}
+
+// Resident frames: the pyramids of frame frame_idx[s] of f are copied into the current slot group (one gather launch per level),
+// so that every kernel of the step reads its frames exactly as it reads uploaded ones.
+int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* f, const int32_t* frame_idx, double* prev_xy,
+                                    double* cur_xy, int32_t* ids, int32_t* n_out) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t || !f) return SFMGPU_E_ARG;
+  if (!frame_idx) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: null frame index array");
+  if (t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step_frames: frames are prefetched; step them first");
+  const sfmgpu_frames* g = t->frames;
+  if (f->w != g->w || f->h != g->h || f->levels != g->levels)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: frames are %dx%d with %d levels, the tracker %dx%d with %d", f->w, f->h,
+                    f->levels, g->w, g->h, g->levels);
+  const int S = t->S;
+  for (int s = 0; s < S; s++)
+    if (frame_idx[s] < 0 || frame_idx[s] >= f->n)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: sequence %d: frame %d outside [0,%d)", s, frame_idx[s], f->n);
+  const int par = multi_next_group(t);
+  t->tv_fresh = false;
+  SFM_CUDA(ctx, cudaMemcpyAsync(t->didx, frame_idx, (size_t)S * 4, cudaMemcpyHostToDevice, ctx->stream));
+  {
+    StageTimer st(ctx, 5);
+    for (int l = 0; l < g->levels; l++) {
+      if (g->fstride[l] == 0) continue;  // level of zero size
+      const unsigned gx = sfm_cdiv((long long)(g->fstride[l] / 16), 256 * 8);
+      SFM_LAUNCH(ctx, gather_frames_kernel, dim3(gx, S, 1), 256, 0, f->lvl[l], g->lvl[l] + (size_t)par * S * g->fstride[l], g->fstride[l],
+                 (const int*)t->didx, (const int*)t->didx, 0);
+    }
+  }
+  return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
+}
+
+}  // extern "C"
+
+// One step of every sequence on the frames in slot group `par` (uploaded, prefetched or gathered there).
+static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out) {
+  const int S = t->S, cap = t->cap;
+  const bool stage = sfm_two_view_enabled(t->tv);
   if (n_out)
     for (int s = 0; s < S; s++) n_out[s] = 0;
   if (t->parity < 0) {  // first frames: reset every sequence (:341-344); find_E_ransac is not called (:1715)
@@ -1298,6 +1366,8 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   return 0;
 }
 
+extern "C" {
+
 int sfmgpu_multitracker_set_ransac(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const double* K, const sfmgpu_ransac_cfg* rc) {
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
@@ -1347,3 +1417,105 @@ int sfmgpu_multitracker_totals(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long lon
 }
 
 }  // extern "C"
+
+// ---- segment mode: contiguous segments of one resident sequence, each a fresh KLTTracker (SURVEY.md §8e) -------------------
+// A chunk of segments is one lock step: slot s of the tracker runs segment j0 + s, reset on its first frame and stepped through
+// the next `steps` frames, read from the resident batch by sfmgpu_multitracker_step_frames.  Every segment of a call has the
+// same length, so the slots start and finish together.  Step k of segment j is written to row j * steps + (k - 1) of the pairs
+// object; the RANSAC stage then runs once over all rows, as it does after the other batch calls.
+namespace {
+
+// Survivors (the first n_kept of slot s), their ids and the counts of slot s -> row row0 + s * row_stride of the pairs arrays.
+__global__ void __launch_bounds__(256) segment_rows_kernel(const double2* __restrict__ oa, const double2* __restrict__ ob,
+                                                          const int* __restrict__ oid, const int* __restrict__ n_in,
+                                                          const int* __restrict__ n_kept, int src_cap, double2* __restrict__ li,
+                                                          double2* __restrict__ lj, int* __restrict__ ids, int* __restrict__ ncorn,
+                                                          int* __restrict__ nkept, int dst_cap, long long row0, int row_stride) {
+  const int s = blockIdx.y, n = n_kept[s];
+  const long long row = row0 + (long long)s * row_stride;
+  const size_t so = (size_t)s * src_cap, d = (size_t)row * dst_cap;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    li[d + i] = oa[so + i];
+    lj[d + i] = ob[so + i];
+    ids[d + i] = oid[so + i];
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    ncorn[row] = n_in[s];
+    nkept[row] = n;
+  }
+}
+
+bool same_lkcfg(const sfmgpu_lkcfg& a, const sfmgpu_lkcfg& b) {
+  return a.max_tracks == b.max_tracks && a.min_tracks == b.min_tracks && a.quality == b.quality && a.min_distance == b.min_distance &&
+         a.pyr_levels == b.pyr_levels && a.win_radius == b.win_radius && a.iters == b.iters && a.fb_thresh == b.fb_thresh;
+}
+
+}  // namespace
+
+extern "C" int sfmgpu_pair_frontend_segments(sfmgpu_ctx* ctx, sfmgpu_frames* f, const int32_t* seg_first, int nseg, int steps,
+                                             const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out) {
+  SFM_ENTER(ctx);
+  if (!ctx || !f || !cfg || !out) return SFMGPU_E_ARG;
+  if (steps < 1) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: %d steps per segment (at least 1)", steps);
+  if (nseg < 0 || (long long)nseg * steps > out->max_pairs)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: %d segments x %d steps, room for %d rows", nseg, steps, out->max_pairs);
+  if (nseg > 0 && !seg_first) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: null seg_first");
+  for (int j = 0; j < nseg; j++)
+    if (seg_first[j] < 0 || (long long)seg_first[j] + steps >= f->n)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: segment %d = frames [%d, %lld] outside [0,%d)", j, seg_first[j],
+                      (long long)seg_first[j] + steps, f->n);
+  if (cfg->pyr_levels != f->levels) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: cfg->pyr_levels != frames levels");
+  if (cfg->max_tracks > (1 << 24) || cfg->min_tracks > (1 << 24)) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: bad configuration");
+  const int rows = track_rows(*cfg);
+  if (out->cap < rows)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: pairs rows hold %d points, a track list up to %d (max(max_tracks, min_tracks, 1) + 1)",
+                    out->cap, rows);
+  // Slots per lock step: the reset's corner work area holds W*H candidates per slot (~265 MB at 4K); 16 GiB bound it as
+  // they bound the pair calls' chunks.  Chunks are balanced; the last one's spare slots repeat its last segment (unread).
+  int S = 0;
+  if (nseg > 0) {
+    const int md = cfg->min_distance < 0 ? -cfg->min_distance : cfg->min_distance;
+    const size_t per = sfm_corner_work_bytes_md(f->w, f->h, 1, f->w * f->h, md);
+    long long most = (long long)(((size_t)16 << 30) / (per ? per : 1));
+    if (most > 512) most = 512;  // sfmgpu_multitracker_create's limit
+    if (most < 1) most = 1;
+    const int nchunk = (int)((nseg + most - 1) / most);
+    S = (nseg + nchunk - 1) / nchunk;
+  }
+  sfmgpu_multitracker* mt = out->seg;
+  if (mt && S > 0 && (mt->S != S || mt->w != f->w || mt->h != f->h || !same_lkcfg(mt->cfg, *cfg))) {
+    sfmgpu_multitracker_destroy(ctx, mt);
+    out->seg = mt = nullptr;
+  }
+  if (!mt && S > 0) {
+    SFM_TRY(sfmgpu_multitracker_create(ctx, cfg, S, f->w, f->h, &out->seg));
+    mt = out->seg;
+  }
+  if (!out->ids) SFM_CUDA(ctx, cudaMalloc((void**)&out->ids, (size_t)out->max_pairs * out->cap * 4 + 256));
+  const int npairs = nseg * steps;
+  out->last_npairs = npairs;
+  out->ids_valid = true;
+  SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
+  std::vector<int32_t> idx(S);
+  for (int j0 = 0; j0 < nseg; j0 += S) {
+    const int cnt = nseg - j0 < S ? nseg - j0 : S;
+    SFM_TRY(sfmgpu_multitracker_reset(ctx, mt));
+    for (int k = 0; k <= steps; k++) {  // k = 0: reset on the segment's first frame, no result (:341-344)
+      for (int s = 0; s < S; s++) idx[s] = seg_first[j0 + (s < cnt ? s : cnt - 1)] + k;
+      SFM_TRY(sfmgpu_multitracker_step_frames(ctx, mt, f, idx.data(), nullptr, nullptr, nullptr, nullptr));
+      if (k == 0) continue;
+      SFM_LAUNCH(ctx, segment_rows_kernel, dim3(sfm_cdiv(rows, 256), cnt), 256, 0, (const double2*)mt->oa, (const double2*)mt->ob,
+                 (const int*)mt->oid, (const int*)mt->dn, (const int*)mt->dnk, mt->cap, out->li, out->lj, out->ids, out->ncorn, out->nkept,
+                 out->cap, (long long)j0 * steps + (k - 1), steps);
+      SFM_LAUNCH(ctx, totals_kernel, 64, 256, 0, (const int*)mt->dn, (const int*)mt->dnk, (const int*)mt->nit, cnt, mt->cap, out->totals);
+    }
+  }
+  if (sfm_two_view_enabled(out->tv) && npairs > 0) {  // find_E_ransac(K, prev_pts, cur_pts, ...) on every step's survivors (:1739)
+    StageTimer rt(ctx, 4);
+    SFM_TRY(sfm_two_view_stage(ctx, out->tv, out->li, out->lj, out->nkept, out->cap, 0, npairs, nullptr));
+    // a step that reset its segment (no tracks entering it) returns no step: SKIPPED whatever min_points says
+    SFM_TRY(sfm_two_view_skip(ctx, out->tv, out->ncorn, npairs));
+  }
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}

@@ -10,6 +10,7 @@
 // NCCL is bound at run time (dlopen of libnccl.so.2, or SFMGPU_NCCL_LIB): libsfmgpu.so itself has no NCCL dependency, a
 // single-GPU drop-in never loads it, and inside a PyTorch process the already-loaded library is found by its soname.
 #include <dlfcn.h>
+#include <stddef.h>
 #include <nccl.h>
 #include <stdlib.h>
 #include <string.h>
@@ -87,6 +88,8 @@ struct sfmgpu_sched {
   bool own_comm = false;
   DevBuf stage;  // root: gathered arrays of the whole sequence
 };
+// The shard functions read world and rank only: a caller without a device may pass these two ints (sfmgpu/sched.py does).
+static_assert(offsetof(sfmgpu_sched, world) == 0 && offsetof(sfmgpu_sched, rank) == sizeof(int), "sfmgpu_sched head");
 
 #define SFM_NCCL(ctx, api, expr)                                                                                  \
   do {                                                                                                            \
@@ -165,6 +168,87 @@ int sfmgpu_sched_pair_shard(const sfmgpu_sched* s, int n_frames, int* pair_begin
   return 0;
 }
 
+// Segment mode (SURVEY.md §8e): G segments of L = ceil((T-1)/G) steps each, spread evenly over the T-1 frame pairs.  Segment j
+// starts on frame floor(j * (T-1-L) / (G-1)) (G = 1: 0), so the first starts on frame 0, the last ends on frame T-1, neighbouring
+// starts are at most L apart (every pair of the sequence is a step of some segment) and G*L - (T-1) < G steps are done twice.
+int sfmgpu_sched_segment_shard(const sfmgpu_sched* s, int n_frames, int n_segments, int* steps, int* seg_begin, int* seg_end,
+                               int32_t* seg_first, int* frame_begin, int* frame_end) {
+  if (!s || s->world < 1 || s->rank < 0 || s->rank >= s->world) return SFMGPU_E_ARG;
+  const long long T = n_frames, G = n_segments;
+  if (T < 2 || G < 1 || G > T - 1) return SFMGPU_E_ARG;
+  const long long L = (T - 1 + G - 1) / G;
+  auto first = [&](long long j) { return G == 1 ? 0 : j * (T - 1 - L) / (G - 1); };
+  int a = 0, b = 0;
+  shard((int)G, s->world, s->rank, &a, &b);
+  if (steps) *steps = (int)L;
+  if (seg_begin) *seg_begin = a;
+  if (seg_end) *seg_end = b;
+  if (seg_first)
+    for (long long j = 0; j < G; j++) seg_first[j] = (int32_t)first(j);
+  if (frame_begin) *frame_begin = b > a ? (int)first(a) : 0;
+  if (frame_end) *frame_end = b > a ? (int)(first(b - 1) + L + 1) : 0;
+  return 0;
+}
+
+namespace {
+
+struct GatherArr {
+  size_t per_pair;  // bytes per pair
+  const void* src;  // this rank's device array
+  void* host;       // root: destination of the whole sequence (may be null)
+};
+
+// Collective of the gathers: this rank's block of n_pairs_total (sfmgpu_sched_shard's rule) must be the last batch of p.
+// Non-root ranks send and return after the sends have completed (*base = null).  The root receives every block into its
+// staging area (array k at *base + off[k]), queues the D2H copies of the arrays with a host pointer, and returns with them in
+// flight: the caller adds its own copies and synchronises.
+int gather_rows(sfmgpu_ctx* ctx, sfmgpu_sched* s, sfmgpu_pairs* p, int n_pairs_total, int root, const GatherArr* arr, int narr,
+                const char* who, char** base, size_t* off) {
+  *base = nullptr;
+  if (root < 0 || root >= s->world || n_pairs_total < 0) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: bad root / size", who);
+  int a = 0, b = 0;
+  shard(n_pairs_total, s->world, s->rank, &a, &b);
+  if (b - a != p->last_npairs)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "%s: rank %d holds %d pairs, its block [%d,%d) has %d", who, s->rank, p->last_npairs, a, b, b - a);
+  NcclApi* api = s->world > 1 ? nccl_api() : nullptr;
+  if (s->world > 1 && (!api->lib || !s->comm)) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: no communicator", who);
+  if (s->rank != root) {
+    SFM_NCCL(ctx, api, api->GroupStart());
+    for (int k = 0; k < narr; k++)
+      if (b > a) SFM_NCCL(ctx, api, api->Send(arr[k].src, arr[k].per_pair * (size_t)(b - a), ncclUint8, root, s->comm, ctx->stream));
+    SFM_NCCL(ctx, api, api->GroupEnd());
+    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+  }
+  // root: staging area for the whole sequence
+  off[0] = 0;
+  for (int k = 0; k < narr; k++) off[k + 1] = off[k] + ((arr[k].per_pair * (size_t)n_pairs_total + 255) & ~(size_t)255);
+  SFM_TRY(sfm_reserve(ctx, s->stage, off[narr] + 256));
+  char* stage = (char*)s->stage.p;
+  if (s->world > 1) SFM_NCCL(ctx, api, api->GroupStart());
+  for (int r = 0; r < s->world; r++) {
+    int ra = 0, rb = 0;
+    shard(n_pairs_total, s->world, r, &ra, &rb);
+    if (rb <= ra) continue;
+    for (int k = 0; k < narr; k++) {
+      void* dst = stage + off[k] + arr[k].per_pair * (size_t)ra;
+      const size_t bytes = arr[k].per_pair * (size_t)(rb - ra);
+      if (r == root)
+        SFM_CUDA(ctx, cudaMemcpyAsync(dst, arr[k].src, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+      else
+        SFM_NCCL(ctx, api, api->Recv(dst, bytes, ncclUint8, r, s->comm, ctx->stream));
+    }
+  }
+  if (s->world > 1) SFM_NCCL(ctx, api, api->GroupEnd());
+  for (int k = 0; k < narr; k++)
+    if (arr[k].host && n_pairs_total > 0)
+      SFM_CUDA(ctx, cudaMemcpyAsync(arr[k].host, stage + off[k], arr[k].per_pair * (size_t)n_pairs_total, cudaMemcpyDeviceToHost, ctx->stream));
+  *base = stage;
+  return 0;
+}
+
+}  // namespace
+
 // Gather.  Every rank calls it with its pairs object (last batch = its block of pairs, in order); on `root` the host
 // arrays receive the whole sequence: li / lj [n_pairs_total][max_corners][2], n_kept / n_corners [n_pairs_total] and -
 // when with_ransac - status / best_n [n_pairs_total], inliers [n_pairs_total][max_corners], R [..][9], t [..][3].
@@ -183,52 +267,32 @@ int sfmgpu_sched_gather_pairs(sfmgpu_ctx* ctx, sfmgpu_sched* s, sfmgpu_pairs* p,
   if (with_ransac && sfmgpu_pairs_ransac_device_ptrs(p, &d_st, &d_best, &d_inl, &d_R, &d_t) != 0)
     return sfm_fail(ctx, SFMGPU_E_STATE, "sched_gather_pairs: the RANSAC stage has not run on this rank");
   const size_t cap = (size_t)p->cap;
-  // arrays: bytes per pair, this rank's device source
-  struct Arr {
-    size_t per_pair;
-    const void* src;
-    void* host;
-  } arr[9] = {{cap * 16, p->li, li_xy},          {cap * 16, p->lj, lj_xy}, {4, p->nkept, n_kept}, {4, p->ncorn, n_corners},
-              {4, d_st, status},                 {8, d_best, nullptr},     {cap * 4, d_inl, inliers}, {72, d_R, R},
-              {24, d_t, t}};
-  const int narr = with_ransac ? 9 : 4;
-  NcclApi* api = s->world > 1 ? nccl_api() : nullptr;
-  if (s->world > 1 && (!api->lib || !s->comm)) return sfm_fail(ctx, SFMGPU_E_STATE, "sched_gather_pairs: no communicator");
-  if (s->rank != root) {
-    SFM_NCCL(ctx, api, api->GroupStart());
-    for (int k = 0; k < narr; k++)
-      if (b > a) SFM_NCCL(ctx, api, api->Send(arr[k].src, arr[k].per_pair * (size_t)(b - a), ncclUint8, root, s->comm, ctx->stream));
-    SFM_NCCL(ctx, api, api->GroupEnd());
-    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return 0;
-  }
-  // root: staging area for the whole sequence
+  const GatherArr arr[9] = {{cap * 16, p->li, li_xy}, {cap * 16, p->lj, lj_xy}, {4, p->nkept, n_kept}, {4, p->ncorn, n_corners},
+                            {4, d_st, status},        {8, d_best, nullptr},     {cap * 4, d_inl, inliers}, {72, d_R, R},
+                            {24, d_t, t}};
+  char* base = nullptr;
   size_t off[10];
-  off[0] = 0;
-  for (int k = 0; k < narr; k++) off[k + 1] = off[k] + ((arr[k].per_pair * (size_t)n_pairs_total + 255) & ~(size_t)255);
-  SFM_TRY(sfm_reserve(ctx, s->stage, off[narr] + 256));
-  char* base = (char*)s->stage.p;
-  if (s->world > 1) SFM_NCCL(ctx, api, api->GroupStart());
-  for (int r = 0; r < s->world; r++) {
-    int ra = 0, rb = 0;
-    shard(n_pairs_total, s->world, r, &ra, &rb);
-    if (rb <= ra) continue;
-    for (int k = 0; k < narr; k++) {
-      void* dst = base + off[k] + arr[k].per_pair * (size_t)ra;
-      const size_t bytes = arr[k].per_pair * (size_t)(rb - ra);
-      if (r == root)
-        SFM_CUDA(ctx, cudaMemcpyAsync(dst, arr[k].src, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
-      else
-        SFM_NCCL(ctx, api, api->Recv(dst, bytes, ncclUint8, r, s->comm, ctx->stream));
-    }
-  }
-  if (s->world > 1) SFM_NCCL(ctx, api, api->GroupEnd());
-  for (int k = 0; k < narr; k++)
-    if (arr[k].host && n_pairs_total > 0)
-      SFM_CUDA(ctx, cudaMemcpyAsync(arr[k].host, base + off[k], arr[k].per_pair * (size_t)n_pairs_total, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_TRY(gather_rows(ctx, s, p, n_pairs_total, root, arr, with_ransac ? 9 : 4, "sched_gather_pairs", &base, off));
+  if (!base) return 0;  // not the root: the sends have completed
   if (with_ransac && best_n && n_pairs_total > 0)  // best is (winner, count) per pair: the count column
     SFM_CUDA(ctx, cudaMemcpy2DAsync(best_n, 4, base + off[5] + 4, 8, 4, (size_t)n_pairs_total, cudaMemcpyDeviceToHost, ctx->stream));
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+// The track ids of a segment call ([n_pairs_total][max_corners] on the root), gathered as sfmgpu_sched_gather_pairs gathers the
+// rows they belong to.
+int sfmgpu_sched_gather_pair_ids(sfmgpu_ctx* ctx, sfmgpu_sched* s, sfmgpu_pairs* p, int n_pairs_total, int root, int32_t* ids) {
+  SFM_ENTER(ctx);
+  if (!ctx || !s || !p) return SFMGPU_E_ARG;
+  void* d_ids = nullptr;
+  if (sfmgpu_pairs_ids_device_ptr(p, &d_ids) != 0)
+    return sfm_fail(ctx, SFMGPU_E_STATE, "sched_gather_pair_ids: the last batch of rank %d carries no track ids (not a segment call)", s->rank);
+  const GatherArr arr[1] = {{(size_t)p->cap * 4, d_ids, ids}};
+  char* base = nullptr;
+  size_t off[2];
+  SFM_TRY(gather_rows(ctx, s, p, n_pairs_total, root, arr, 1, "sched_gather_pair_ids", &base, off));
+  if (base) SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 

@@ -43,6 +43,8 @@ SYMBOLS = [
     "sfmgpu_multitracker_set_ransac", "sfmgpu_multitracker_ransac_download_all", "sfmgpu_multitracker_ransac_early",
     "sfmgpu_pair_frontend_list", "sfmgpu_descs_create", "sfmgpu_descs_destroy", "sfmgpu_descs_compute", "sfmgpu_descs_upload",
     "sfmgpu_descs_download", "sfmgpu_descs_search",
+    "sfmgpu_multitracker_step_frames", "sfmgpu_pair_frontend_segments", "sfmgpu_pairs_ids_download_all", "sfmgpu_pairs_ids_device_ptr",
+    "sfmgpu_sched_segment_shard", "sfmgpu_sched_gather_pair_ids",
 ]
 
 
@@ -175,6 +177,12 @@ def load_library():
         "sfmgpu_sched_destroy": (None, [_vp, _vp]),
         "sfmgpu_sched_pair_shard": (_i, [_vp, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
         "sfmgpu_sched_gather_pairs": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+        "sfmgpu_multitracker_step_frames": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+        "sfmgpu_pair_frontend_segments": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(LKCfg), _vp]),
+        "sfmgpu_pairs_ids_download_all": (_i, [_vp, _vp, _vp]),
+        "sfmgpu_pairs_ids_device_ptr": (_i, [_vp, C.POINTER(_vp)]),
+        "sfmgpu_sched_segment_shard": (_i, [_vp, _i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), _vp, C.POINTER(_i), C.POINTER(_i)]),
+        "sfmgpu_sched_gather_pair_ids": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
     }
     for name, (res, args) in S.items():
         fn = getattr(lib, name)
@@ -522,6 +530,20 @@ class Pairs:
         self.ctx._ck(self.ctx.lib.sfmgpu_pair_frontend_host(self.ctx.h, frames.h_, host.ctypes.data_as(_vp), host.shape[0], C.byref(cfg),
                                                             self.h_, chunk, _ptr(li), _ptr(lj), _ptr(nkept), _ptr(ncorn)))
 
+    def run_segments(self, frames, seg_first, steps, cfg):
+        """Segment mode: segment j = a fresh KLTTracker reset on frame seg_first[j] and stepped through the next `steps`
+        frames; step k of segment j goes to row j * steps + (k - 1).  The pairs object needs max_corners >=
+        max(max_tracks, min_tracks, 1) + 1."""
+        sf = np.ascontiguousarray(seg_first, np.int32).reshape(-1)
+        self.ctx._ck(self.ctx.lib.sfmgpu_pair_frontend_segments(self.ctx.h, frames.h_, _ptr(sf) if len(sf) else None, len(sf), steps,
+                                                                C.byref(cfg), self.h_))
+
+    def ids_download_all(self, npairs, ids=None):
+        """Track ids [npairs, cap] int32 of the segment call's rows (the first n_kept of each row valid)."""
+        ids = np.zeros((max(npairs, 1), self.cap), np.int32) if ids is None else ids
+        self.ctx._ck(self.ctx.lib.sfmgpu_pairs_ids_download_all(self.ctx.h, self.h_, _ptr(ids)))
+        return ids[:npairs]
+
     def totals(self):
         a, b, c = _ll(0), _ll(0), _ll(0)
         self.ctx._ck(self.ctx.lib.sfmgpu_pairs_totals(self.ctx.h, self.h_, C.byref(a), C.byref(b), C.byref(c)))
@@ -735,6 +757,17 @@ class MultiTracker:
                                                                      self.n.ctypes.data_as(_vp)))
         if not fetch:
             return self.n
+        return [(self.prev[s, :self.n[s]].copy(), self.cur[s, :self.n[s]].copy(), self.ids[s, :self.n[s]].copy()) for s in range(self.S)]
+
+    def step_frames(self, frames, frame_idx, fetch=True):
+        """step() with the next frame of sequence s = frame frame_idx[s] of the resident batch `frames` (pyramids built)."""
+        idx = np.ascontiguousarray(frame_idx, np.int32).reshape(-1)
+        assert len(idx) == self.S, (len(idx), self.S)
+        a = (self.prev, self.cur, self.ids) if fetch else (None, None, None)
+        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_step_frames(self.ctx.h, self.h_, frames.h_, _ptr(idx), _ptr(a[0]), _ptr(a[1]),
+                                                                  _ptr(a[2]), self.n.ctypes.data_as(_vp)))
+        if not fetch:
+            return self.n.copy()
         return [(self.prev[s, :self.n[s]].copy(), self.cur[s, :self.n[s]].copy(), self.ids[s, :self.n[s]].copy()) for s in range(self.S)]
 
     def reset(self):

@@ -7,8 +7,9 @@ The front end shards with NO data-path collective:
                     rank g owns a contiguous block of pairs plus one halo frame (`pair_shard`);
   * sequence mode - whole sequences per rank (a KLTTracker chain cannot be split across frames, :370-371): `shard_range`
                     over the sequences; several sequences per GPU advance in lock step (run_sequences -> sfmgpu_multitracker);
-  * segment mode  - contiguous frame segments of one sequence per rank, each restarting the tracker: `shard_range` over
-                    the frames.  That equals the reference run on each segment separately (track ids restart per
+  * segment mode  - contiguous frame segments of one sequence, each restarting the tracker: `segment_shard` spreads G
+                    segments of equal length over the sequence and gives each rank a block of them (Pairs.run_segments
+                    runs them).  That equals the reference run on each segment separately (track ids restart per
                     segment), NOT the unsegmented run.
 The only communication is the gather of results (tracks, survivor counts, inlier sets) to rank 0: an all_gather of
 per-rank sizes followed by one padded gather (NCCL has no gatherv).  Works on NCCL (GPU tensors) and gloo (CPU tests).
@@ -35,6 +36,25 @@ def pair_shard(n_frames, world, rank):
     """Pairs [p0, p1) of a sequence of n_frames and the frames [p0, p1] (inclusive halo) the rank must hold."""
     p0, p1 = shard_range(max(n_frames - 1, 0), world, rank)
     return p0, p1, (p0, p1 + 1 if p1 > p0 else p0)
+
+
+class _RankOf(C.Structure):
+    """The head of sfmgpu_sched that the shard functions read (csrc/sched.cu asserts the layout)."""
+    _fields_ = [("world", C.c_int), ("rank", C.c_int)]
+
+
+def segment_shard(n_frames, n_segments, world=1, rank=0):
+    """Segment mode: sfmgpu_sched_segment_shard (no GPU needed).  Returns (steps, seg_begin, seg_end, seg_first [n_segments]
+    int32, frame_begin, frame_end): this rank runs segments [seg_begin, seg_end) of `steps` steps each, segment j starting on
+    frame seg_first[j], and must hold frames [frame_begin, frame_end)."""
+    import sfmgpu
+    lib = sfmgpu.load_library()
+    L, a, b, f0, f1 = (C.c_int(0) for _ in range(5))
+    first = np.zeros(max(int(n_segments), 1), np.int32)
+    if lib.sfmgpu_sched_segment_shard(C.byref(_RankOf(int(world), int(rank))), int(n_frames), int(n_segments), C.byref(L), C.byref(a),
+                                      C.byref(b), first.ctypes.data_as(C.c_void_p), C.byref(f0), C.byref(f1)) != 0:
+        raise ValueError(f"segment_shard({n_frames}, {n_segments}, {world}, {rank})")
+    return L.value, a.value, b.value, first[:n_segments], f0.value, f1.value
 
 
 def _dev(t):
