@@ -78,7 +78,8 @@ int sfmgpu_flush_l2(sfmgpu_ctx* ctx, size_t bytes);
 int sfmgpu_profile(sfmgpu_ctx* ctx, int enable);
 int sfmgpu_stage_times(sfmgpu_ctx* ctx, float* ms4);
 /* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac),
- * ms[5] = the frame gather of sfmgpu_pair_frontend_list and sfmgpu_multitracker_step_frames. */
+ * ms[5] = the frame gather of sfmgpu_pair_frontend_list and sfmgpu_multitracker_step_frames, ms[6] = the tile decode of the
+ * packed-input calls (sfmgpu_frames_upload_packed, sfmgpu_pair_frontend_host_packed). */
 int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n);
 /* Measured non-tensor FP64 throughput of this GPU (DFMA micro-benchmark, ~10 ms): the KLT / RANSAC roofline. */
 int sfmgpu_fp64_peak(sfmgpu_ctx* ctx, double* tflops);
@@ -107,6 +108,35 @@ int sfmgpu_frames_download(sfmgpu_ctx* ctx, sfmgpu_frames* f, int frame, int lev
 /* Device address of a level (frame k starts at ptr + k * frame_stride, rows are pitch bytes apart): interop with the
  * caller's own kernels, NCCL, or as an image source for the entry points that accept device pointers. */
 int sfmgpu_frames_device_ptr(const sfmgpu_frames* f, int level, void** ptr, size_t* pitch, size_t* frame_stride);
+
+/* ---- packed frames: a lossless tile codec, encoded and decoded on the device (DESIGN.md §2) -----------------------------
+ * Uploads of raw u8 frames are bound by PCIe; a packed blob moves fewer bytes and decodes on the device to exactly the raw
+ * frame, so every result computed from it is byte-identical.  Blob layout (integers little-endian):
+ *   header     8 x uint32: magic 0x504B4653, version 1, w, h, nframes, tile size 64, 0, 0
+ *   uint64     frame_off[nframes + 1]: frame k is the byte range [frame_off[k], frame_off[k+1]) of the blob, so any frame range
+ *              is one contiguous byte range
+ *   per frame  uint32 tile_off[ntiles + 1] (bytes from the frame's start, 4-byte aligned; tile_off[ntiles] = frame size), then
+ *              the tile records, tiles of 64 x 64 pixels in raster order (edge tiles partial: n = tw * th pixels)
+ * A tile's values are its planar residuals p - left - up + upleft mod 256 (pixels outside the tile = 0), zig-zag mapped to
+ * u in [0, 255], in raster order, in runs of 32 (the last one zero padded), each run with its own Rice parameter k in 0..8
+ * (the fewest bits, the smallest k on a tie).  Coded record, uint32 words: U << 1 (U = unary bits), the k of every run as
+ * nibbles (8 per word), the remainders (u & (2^k - 1), k bits each, LSB first: k words per run), the unary stream (u >> k
+ * one-bits and a zero bit per value, LSB first, zero padded).  Raw record: the word 1, then the n pixels, zero padded - used
+ * when the coded record would not be shorter.  tests/frame_codec.py is the reference encoder and decoder. */
+/* Largest blob nframes frames of w x h can give (every tile raw: the raw size plus about 0.1 %). */
+int sfmgpu_pack_bound(int w, int h, int nframes, size_t* bytes);
+/* Encode level 0 of frames [first, first+count) into out (host memory, cap bytes); *bytes = the blob size.  A cap below it is
+ * SFMGPU_E_CAPACITY with *bytes set (out == NULL asks for the size).  The bytes equal the reference encoder's. */
+int sfmgpu_frames_pack(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count, uint8_t* out, size_t cap, size_t* bytes);
+/* Decode frames [blob_first, blob_first+count) of the blob (host memory, pinned for full speed) into level 0 of frames
+ * [first, first+count) of f: the same bytes sfmgpu_frames_upload writes (w bytes per row, row padding untouched).  Build
+ * the pyramids afterwards, as after an upload.  The header (magic, version, w, h, tile size against f), the frame range and
+ * the frame offsets (monotonic, inside blob_bytes) are checked before any work is queued: SFMGPU_E_ARG.  A tile record that
+ * does not decode (k above 8, a unary stream without one terminator per value, sizes that do not add up, a value above 255,
+ * tile offsets out of order or outside the frame) is not written and makes the call return SFMGPU_E_ARG.  Returns when the
+ * frames are decoded. */
+int sfmgpu_frames_upload_packed(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, const uint8_t* blob, size_t blob_bytes, int blob_first,
+                                int count);
 
 /* ---- corners: shi_tomasi (:237-302) ---------------------------------------------------------------- */
 /* Raster-ordered candidate list {s >= max*quality} of one frame (:274-285): pixel (x,y) and exact score.
@@ -176,6 +206,14 @@ int sfmgpu_pipeline_set(sfmgpu_ctx* ctx, int pairs_per_chunk);
 int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* host_pix, int nframes,
                               const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out, int chunk_frames, double* li_xy, double* lj_xy,
                               int32_t* n_kept, int32_t* n_corners);
+/* Same call on a packed blob (sfmgpu_frames_upload_packed): frames [blob_first, blob_first+nframes) of the blob become frames
+ * [0, nframes) of f.  Same chunks, streams, overlap and outputs: each chunk's blob bytes go up in one copy into one of two
+ * device staging buffers, and are decoded and their pyramids built on the score stream; a staging buffer is refilled only
+ * after the decode that read it.  Results are byte-identical to sfmgpu_pair_frontend_host on the decoded frames.  Blob checks
+ * and refusals as for sfmgpu_frames_upload_packed. */
+int sfmgpu_pair_frontend_host_packed(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* blob, size_t blob_bytes, int blob_first,
+                                     int nframes, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out, int chunk_frames, double* li_xy,
+                                     double* lj_xy, int32_t* n_kept, int32_t* n_corners);
 /* Totals over the last batch: corners detected (= tracks attempted), survivors, LK iterations. */
 int sfmgpu_pairs_totals(sfmgpu_ctx* ctx, sfmgpu_pairs* p, long long* n_corners, long long* n_kept,
                         long long* n_lk_iters);

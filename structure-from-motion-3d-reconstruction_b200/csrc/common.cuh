@@ -67,6 +67,9 @@ struct sfmgpu_ctx {
   DevBuf rs_raw;     // std::mt19937(12345) outputs for single-call sampling (two_view.cu: raw_stream)
   int rs_raw_n = 0;
   DevBuf sv_list;    // screening solver: [0] count, [64...] hypotheses left to the Jacobi emulation (repeated index)
+  DevBuf pk_stage[2];  // packed input (codec.cu): staged blob bytes (two: the streaming call uploads one while it decodes the other)
+  DevBuf pk_fo, pk_flag;  // packed input: frame offsets of the staged range, "a tile record did not decode" flag
+  DevBuf pk_tmp, pk_enc;  // encoder: record sizes / tile tables / frame offsets, and the records of one batch of frames
   int rs_n = 0, rs_H = 0;
   bool rs_screened = false;  // rs_E holds screening hypotheses of the octets in rs_idx8: the winner is re-solved when scored
   int solver_mode = 1;       // device 8-point solver: 1 screening solver for the counts of launches beyond one wave + Jacobi emulation for the winner, 0 Jacobi emulation for every hypothesis, 2 the same by the warp kernel, 3 screening always (2, 3: tests)
@@ -74,7 +77,7 @@ struct sfmgpu_ctx {
   bool profile = false;
   struct StageEv { int stage; cudaEvent_t a, b; };
   std::vector<StageEv> stage_evs;
-  float stage_ms[6] = {0, 0, 0, 0, 0, 0};  // corner score, corner select, KLT, compaction, RANSAC stage, list-call gather
+  float stage_ms[7] = {0, 0, 0, 0, 0, 0, 0};  // corner score, corner select, KLT, compaction, RANSAC stage, list-call gather, packed decode
   void* pinned = nullptr;  // staging for small D2H results
   size_t pinned_cap = 0;
   // kernels whose >48 KB dynamic shared memory opt-in has been set ON THIS CONTEXT'S DEVICE (the attribute is per device)
@@ -123,6 +126,15 @@ int sfm_two_view_download(sfmgpu_ctx* ctx, TwoViewState* tv, int cap, int set_of
 int sfm_two_view_download_all(sfmgpu_ctx* ctx, TwoViewState* tv, int cap, int nsets, int32_t* status, int32_t* best_n, int32_t* inliers,
                               double* R, double* t, const char* who);
 int sfm_two_view_early(sfmgpu_ctx* ctx, TwoViewState* tv, long long* stopped);
+
+// codec.cu: packed frame input
+int sfm_pk_check(sfmgpu_ctx* ctx, const sfmgpu_frames* f, const uint8_t* blob, size_t blob_bytes, int blob_first, int count,
+                 std::vector<uint64_t>& fo, const char* who);
+int sfm_pk_decode(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count, const uint8_t* stage, const unsigned long long* d_fo,
+                  unsigned long long base, int* d_bad);
+int sfm_pk_prepare(sfmgpu_ctx* ctx, const uint8_t* blob, int blob_first, const std::vector<uint64_t>& fo, size_t stage_bytes, int nstage);
+size_t sfm_pk_max_chunk_bytes(const std::vector<uint64_t>& fo, int chunk);
+int sfm_pk_read_flag(sfmgpu_ctx* ctx, const char* who);
 
 int sfm_fail(sfmgpu_ctx* ctx, int code, const char* fmt, ...);
 int sfm_reserve(sfmgpu_ctx* ctx, DevBuf& b, size_t bytes);

@@ -95,7 +95,8 @@ void sfmgpu_destroy(sfmgpu_ctx* ctx) {
   cudaStreamSynchronize(ctx->stream);
   DevBuf* bufs[] = {&ctx->flush,  &ctx->klt_in, &ctx->klt_p1, &ctx->klt_pb,    &ctx->klt_nit, &ctx->klt_keep, &ctx->klt_defer, &ctx->cs_work,
                     &ctx->sel_work, &ctx->misc,   &ctx->rs_xi,  &ctx->rs_xj,     &ctx->rs_E,    &ctx->rs_counts, &ctx->rs_inl,
-                    &ctx->rs_best, &ctx->rs_idx8, &ctx->sv_list, &ctx->rs_raw};
+                    &ctx->rs_best, &ctx->rs_idx8, &ctx->sv_list, &ctx->rs_raw, &ctx->pk_stage[0], &ctx->pk_stage[1],
+                    &ctx->pk_fo,   &ctx->pk_flag, &ctx->pk_tmp, &ctx->pk_enc};
   for (DevBuf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
@@ -299,13 +300,13 @@ extern "C" int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n) {
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   for (auto& e : ctx->stage_evs) {
     float t = 0;
-    if (cudaEventElapsedTime(&t, e.a, e.b) == cudaSuccess && e.stage >= 0 && e.stage < 6) ctx->stage_ms[e.stage] += t;
+    if (cudaEventElapsedTime(&t, e.a, e.b) == cudaSuccess && e.stage >= 0 && e.stage < 7) ctx->stage_ms[e.stage] += t;
     cudaEventDestroy(e.a);
     cudaEventDestroy(e.b);
   }
   ctx->stage_evs.clear();
-  for (int i = 0; i < n; i++) ms[i] = i < 6 ? ctx->stage_ms[i] : 0.f;
-  for (int i = 0; i < 6; i++) ctx->stage_ms[i] = 0;
+  for (int i = 0; i < n; i++) ms[i] = i < 7 ? ctx->stage_ms[i] : 0.f;
+  for (int i = 0; i < 7; i++) ctx->stage_ms[i] = 0;
   return 0;
 }
 

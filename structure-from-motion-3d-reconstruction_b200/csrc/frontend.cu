@@ -619,22 +619,8 @@ int sfmgpu_pair_frontend_list(sfmgpu_ctx* ctx, sfmgpu_frames* f, const int32_t* 
   return pair_fix_overflow(ctx, f, 0, npairs, cfg, out, nullptr, frame_a, frame_b);
 }
 
-// Streaming variant for frames that live in HOST memory: frames [0, nframes) of `f` are filled from host_pix in
-// chunks on a copy stream (which also builds their pyramids); every chunk then flows through the stage pipeline and
-// its results go back on a fifth stream.
-int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* host_pix, int nframes, const sfmgpu_lkcfg* cfg,
-                              sfmgpu_pairs* out, int chunk_frames, double* li_xy, double* lj_xy, int32_t* n_kept,
-                              int32_t* n_corners) {
-  SFM_ENTER(ctx);
-  if (!ctx || !f || !cfg || !out || !host_pix) return SFMGPU_E_ARG;
-  if (nframes < 0 || nframes > f->n) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_host: %d frames do not fit (%d)", nframes, f->n);
-  const int npairs = nframes > 0 ? nframes - 1 : 0;
-  SFM_TRY(pair_args_ok(ctx, f, 0, npairs, cfg, out));
-  out->last_npairs = npairs;
-  out->ids_valid = false;
-  SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
-  if (nframes == 0) return 0;
-  SFM_TRY(pipe_streams(ctx));
+// Frames per upload chunk of the streaming calls (chunk_frames <= 0: the default rule).
+static int host_chunk(const sfmgpu_frames* f, int nframes, int chunk_frames) {
   // default: about 100 frames (50 for large frames), at least 8 chunks for short sequences, at most 20 (40) for long ones.  Smaller chunks shorten the
   // pipeline fill (the first upload and the last chunk's compute are not overlapped), too small ones under-fill the
   // one-block-per-frame kernels.  Measured end to end: C2 (1000 x 1080p) chunks of 84-125 frames 43.0 ms, 167: 44.1, 250: 46.3,
@@ -655,6 +641,26 @@ int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* 
   }
   if (chunk < 2) chunk = 2;
   if (chunk > 1024) chunk = 1024;
+  return chunk;
+}
+
+// Queues level 0 of frames [a, b) (upload chunk c) on the copy stream and makes ctx->stream wait for it; whatever else the
+// frames need before their pyramids (a decode) goes on ctx->stream behind that wait.
+struct ChunkFill {
+  virtual int fill(Pipe& p, sfmgpu_frames* f, int c, int a, int b) = 0;
+};
+
+// The streaming front end: frames [0, nframes) of `f` are filled chunk by chunk by `src` on a copy stream; every chunk's
+// pyramids are built on the score stream, the chunk flows through the stage pipeline and its results go back on a fifth
+// stream.  Argument checks are the caller's.
+static int host_stream(sfmgpu_ctx* ctx, sfmgpu_frames* f, int nframes, int chunk, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out,
+                       ChunkFill& src, double* li_xy, double* lj_xy, int32_t* n_kept, int32_t* n_corners) {
+  const int npairs = nframes > 0 ? nframes - 1 : 0;
+  out->last_npairs = npairs;
+  out->ids_valid = false;
+  SFM_CUDA(ctx, cudaMemsetAsync(out->totals, 0, 64, ctx->stream));
+  if (nframes == 0) return 0;
+  SFM_TRY(pipe_streams(ctx));
   const int nchunks = (nframes + chunk - 1) / chunk;
   SFM_TRY(pipe_reserve(ctx, f, cfg, out, chunk));
   Pipe p;
@@ -670,15 +676,7 @@ int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* 
   const size_t cap = (size_t)out->cap;
   for (int c = 0; c < nchunks; c++) {
     const int a = c * chunk, b = a + chunk < nframes ? a + chunk : nframes;
-    SFM_CUDA(ctx, cudaMemcpy2DAsync(f->lvl[0] + (size_t)a * f->fstride[0], f->pitch[0], host_pix + (size_t)a * f->w * f->h, f->w,
-                                    f->w, (size_t)f->h * (b - a), cudaMemcpyDefault, ctx->copy_stream));
-    cudaEvent_t up = p.next();
-    if (!up) return sfm_fail(ctx, SFMGPU_E_CUDA, "pair_frontend_host: cudaEventCreate failed");
-    // The copy stream carries NOTHING but the uploads, back to back: the call is bound by them.  The chunk's pyramid is built
-    // on the score stream behind the upload's event (on the copy stream it sat between two uploads and, waiting for SMs
-    // behind the running KLT / RANSAC kernels, kept the copy engine idle ~0.35 ms per chunk).
-    SFM_CUDA(ctx, cudaEventRecord(up, ctx->copy_stream));
-    SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, up, 0));
+    SFM_TRY(src.fill(p, f, c, a, b));
     SFM_TRY(sfmgpu_pyramid_build(ctx, f, a, b - a));
     // pairs whose second frame arrived with this chunk
     const int P0 = a > 0 ? a - 1 : 0, P1 = b - 1;
@@ -712,6 +710,82 @@ int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* 
   }
   if (!redone.empty()) SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
+}
+
+struct RawFill : ChunkFill {
+  const uint8_t* pix;
+  int fill(Pipe& p, sfmgpu_frames* f, int, int a, int b) override {
+    sfmgpu_ctx* ctx = p.ctx;
+    SFM_CUDA(ctx, cudaMemcpy2DAsync(f->lvl[0] + (size_t)a * f->fstride[0], f->pitch[0], pix + (size_t)a * f->w * f->h, f->w, f->w,
+                                    (size_t)f->h * (b - a), cudaMemcpyDefault, ctx->copy_stream));
+    cudaEvent_t up = p.next();
+    if (!up) return sfm_fail(ctx, SFMGPU_E_CUDA, "pair_frontend_host: cudaEventCreate failed");
+    // The copy stream carries NOTHING but the uploads, back to back: the call is bound by them.  The chunk's pyramid is built
+    // on the score stream behind the upload's event (on the copy stream it sat between two uploads and, waiting for SMs
+    // behind the running KLT / RANSAC kernels, kept the copy engine idle ~0.35 ms per chunk).
+    SFM_CUDA(ctx, cudaEventRecord(up, ctx->copy_stream));
+    SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, up, 0));
+    return 0;
+  }
+};
+
+// Packed chunks: one cudaMemcpyAsync of the chunk's blob bytes into staging buffer c % 2 on the copy stream, then the decode on
+// the score stream behind the upload's event.  A staging buffer is overwritten only after the decode that read it (chunk c - 2).
+struct PackedFill : ChunkFill {
+  const uint8_t* blob;
+  const std::vector<uint64_t>* fo;  // absolute offsets of the call's frames in the blob
+  const unsigned long long* d_fo;   // the same on the device
+  cudaEvent_t decoded[2] = {nullptr, nullptr};
+  int fill(Pipe& p, sfmgpu_frames* f, int c, int a, int b) override {
+    sfmgpu_ctx* ctx = p.ctx;
+    const int s = c & 1;
+    cudaEvent_t up = p.next(), dec = p.next();
+    if (!up || !dec) return sfm_fail(ctx, SFMGPU_E_CUDA, "pair_frontend_host_packed: cudaEventCreate failed");
+    if (decoded[s]) SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, decoded[s], 0));
+    const uint64_t o0 = (*fo)[a], o1 = (*fo)[b];
+    SFM_CUDA(ctx, cudaMemcpyAsync(ctx->pk_stage[s].p, blob + o0, o1 - o0, cudaMemcpyHostToDevice, ctx->copy_stream));
+    SFM_CUDA(ctx, cudaEventRecord(up, ctx->copy_stream));
+    SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, up, 0));
+    SFM_TRY(sfm_pk_decode(ctx, f, a, b - a, (const uint8_t*)ctx->pk_stage[s].p, d_fo + a, o0, (int*)ctx->pk_flag.p));
+    SFM_CUDA(ctx, cudaEventRecord(dec, ctx->stream));
+    decoded[s] = dec;
+    return 0;
+  }
+};
+
+static int host_args_ok(sfmgpu_ctx* ctx, sfmgpu_frames* f, int nframes, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out, const char* who) {
+  if (nframes < 0 || nframes > f->n) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: %d frames do not fit (%d)", who, nframes, f->n);
+  return pair_args_ok(ctx, f, 0, nframes > 0 ? nframes - 1 : 0, cfg, out);
+}
+
+int sfmgpu_pair_frontend_host(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* host_pix, int nframes, const sfmgpu_lkcfg* cfg,
+                              sfmgpu_pairs* out, int chunk_frames, double* li_xy, double* lj_xy, int32_t* n_kept,
+                              int32_t* n_corners) {
+  SFM_ENTER(ctx);
+  if (!ctx || !f || !cfg || !out || !host_pix) return SFMGPU_E_ARG;
+  SFM_TRY(host_args_ok(ctx, f, nframes, cfg, out, "pair_frontend_host"));
+  RawFill src;
+  src.pix = host_pix;
+  return host_stream(ctx, f, nframes, host_chunk(f, nframes, chunk_frames), cfg, out, src, li_xy, lj_xy, n_kept, n_corners);
+}
+
+int sfmgpu_pair_frontend_host_packed(sfmgpu_ctx* ctx, sfmgpu_frames* f, const uint8_t* blob, size_t blob_bytes, int blob_first,
+                                     int nframes, const sfmgpu_lkcfg* cfg, sfmgpu_pairs* out, int chunk_frames, double* li_xy,
+                                     double* lj_xy, int32_t* n_kept, int32_t* n_corners) {
+  SFM_ENTER(ctx);
+  if (!ctx || !f || !cfg || !out) return SFMGPU_E_ARG;
+  const char* who = "pair_frontend_host_packed";
+  SFM_TRY(host_args_ok(ctx, f, nframes, cfg, out, who));
+  std::vector<uint64_t> fo;
+  SFM_TRY(sfm_pk_check(ctx, f, blob, blob_bytes, blob_first, nframes, fo, who));
+  const int chunk = host_chunk(f, nframes, chunk_frames);
+  if (nframes > 0) SFM_TRY(sfm_pk_prepare(ctx, blob, blob_first, fo, sfm_pk_max_chunk_bytes(fo, chunk), 2));
+  PackedFill src;
+  src.blob = blob;
+  src.fo = &fo;
+  src.d_fo = (const unsigned long long*)ctx->pk_fo.p;
+  SFM_TRY(host_stream(ctx, f, nframes, chunk, cfg, out, src, li_xy, lj_xy, n_kept, n_corners));
+  return nframes > 0 ? sfm_pk_read_flag(ctx, who) : 0;
 }
 
 int sfmgpu_pairs_totals(sfmgpu_ctx* ctx, sfmgpu_pairs* p, long long* n_corners, long long* n_kept, long long* n_lk_iters) {

@@ -45,6 +45,7 @@ SYMBOLS = [
     "sfmgpu_descs_download", "sfmgpu_descs_search",
     "sfmgpu_multitracker_step_frames", "sfmgpu_pair_frontend_segments", "sfmgpu_pairs_ids_download_all", "sfmgpu_pairs_ids_device_ptr",
     "sfmgpu_sched_segment_shard", "sfmgpu_sched_gather_pair_ids",
+    "sfmgpu_pack_bound", "sfmgpu_frames_pack", "sfmgpu_frames_upload_packed", "sfmgpu_pair_frontend_host_packed",
 ]
 
 
@@ -183,6 +184,10 @@ def load_library():
         "sfmgpu_pairs_ids_device_ptr": (_i, [_vp, C.POINTER(_vp)]),
         "sfmgpu_sched_segment_shard": (_i, [_vp, _i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), _vp, C.POINTER(_i), C.POINTER(_i)]),
         "sfmgpu_sched_gather_pair_ids": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
+        "sfmgpu_pack_bound": (_i, [_i, _i, _i, C.POINTER(C.c_size_t)]),
+        "sfmgpu_frames_pack": (_i, [_vp, _vp, _i, _i, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
+        "sfmgpu_frames_upload_packed": (_i, [_vp, _vp, _i, _vp, C.c_size_t, _i, _i]),
+        "sfmgpu_pair_frontend_host_packed": (_i, [_vp, _vp, _vp, C.c_size_t, _i, _i, C.POINTER(LKCfg), _vp, _i, _vp, _vp, _vp, _vp]),
     }
     for name, (res, args) in S.items():
         fn = getattr(lib, name)
@@ -193,6 +198,21 @@ def load_library():
 
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(_vp)
+
+
+def pack_bound(w, h, nframes):
+    """The largest packed blob (bytes) nframes frames of w x h can give."""
+    b = C.c_size_t(0)
+    rc = load_library().sfmgpu_pack_bound(w, h, nframes, C.byref(b))
+    if rc != 0:
+        raise SfmGpuError(rc, f"pack_bound: bad arguments ({w}, {h}, {nframes})")
+    return b.value
+
+
+def _blob(blob):
+    if not (isinstance(blob, np.ndarray) and blob.dtype == np.uint8 and blob.ndim == 1 and blob.flags["C_CONTIGUOUS"]):
+        raise TypeError("a packed blob is a contiguous 1-D np.uint8 array")
+    return blob.ctypes.data_as(_vp), blob.nbytes
 
 
 class Context:
@@ -436,6 +456,24 @@ class Frames:
     def upload_ptr(self, first, count, host_ptr):
         self.ctx._ck(self.ctx.lib.sfmgpu_frames_upload(self.ctx.h, self.h_, first, count, host_ptr))
 
+    def pack(self, first=0, count=None, out=None):
+        """Encode level 0 of frames [first, first+count) on the device -> packed blob (np.uint8).  out: a caller buffer (e.g.
+        Context.pinned_empty(pack_bound(...))); the result is then a view of its first bytes."""
+        count = self.n - first if count is None else count
+        if out is None:
+            out = np.empty(pack_bound(self.w, self.h, count), np.uint8)
+        ptr, cap = _blob(out)
+        nb = C.c_size_t(0)
+        self.ctx._ck(self.ctx.lib.sfmgpu_frames_pack(self.ctx.h, self.h_, first, count, ptr, cap, C.byref(nb)))
+        return out[:nb.value]
+
+    def upload_packed(self, first, blob, blob_first=0, count=None):
+        """Decode frames [blob_first, blob_first+count) of a packed blob into frames [first, first+count) (level 0)."""
+        ptr, nb = _blob(blob)
+        if count is None:
+            count = int(np.frombuffer(blob[16:20].tobytes(), "<u4")[0]) - blob_first if nb >= 20 else 0
+        self.ctx._ck(self.ctx.lib.sfmgpu_frames_upload_packed(self.ctx.h, self.h_, first, ptr, nb, blob_first, count))
+
     def synth(self, first, count, seed, t0):
         self.ctx._ck(self.ctx.lib.sfmgpu_frames_synth(self.ctx.h, self.h_, first, count, seed & 0xFFFFFFFF, t0))
 
@@ -529,6 +567,13 @@ class Pairs:
         assert host.dtype == np.uint8 and host.flags["C_CONTIGUOUS"] and host.shape[1:] == (frames.h, frames.w)
         self.ctx._ck(self.ctx.lib.sfmgpu_pair_frontend_host(self.ctx.h, frames.h_, host.ctypes.data_as(_vp), host.shape[0], C.byref(cfg),
                                                             self.h_, chunk, _ptr(li), _ptr(lj), _ptr(nkept), _ptr(ncorn)))
+
+    def run_host_packed(self, frames, blob, nframes, cfg, li=None, lj=None, nkept=None, ncorn=None, chunk=0, blob_first=0):
+        """run_host on a packed blob (Frames.pack): frames [blob_first, blob_first+nframes) of the blob are streamed and
+        decoded on the device; the outputs are those run_host gives on the decoded frames."""
+        ptr, nb = _blob(blob)
+        self.ctx._ck(self.ctx.lib.sfmgpu_pair_frontend_host_packed(self.ctx.h, frames.h_, ptr, nb, blob_first, nframes, C.byref(cfg),
+                                                                   self.h_, chunk, _ptr(li), _ptr(lj), _ptr(nkept), _ptr(ncorn)))
 
     def run_segments(self, frames, seg_first, steps, cfg):
         """Segment mode: segment j = a fresh KLTTracker reset on frame seg_first[j] and stepped through the next `steps`
