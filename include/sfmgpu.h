@@ -79,7 +79,7 @@ int sfmgpu_profile(sfmgpu_ctx* ctx, int enable);
 int sfmgpu_stage_times(sfmgpu_ctx* ctx, float* ms4);
 /* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac),
  * ms[5] = the frame gather of sfmgpu_pair_frontend_list and sfmgpu_multitracker_step_frames, ms[6] = the tile decode of the
- * packed-input calls (sfmgpu_frames_upload_packed, sfmgpu_pair_frontend_host_packed). */
+ * packed-input calls (sfmgpu_frames_upload_packed, sfmgpu_pair_frontend_host_packed, sfmgpu_multitracker_step_packed). */
 int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n);
 /* Measured non-tensor FP64 throughput of this GPU (DFMA micro-benchmark, ~10 ms): the KLT / RANSAC roofline. */
 int sfmgpu_fp64_peak(sfmgpu_ctx* ctx, double* tflops);
@@ -380,6 +380,26 @@ int sfmgpu_multitracker_step(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint
 int sfmgpu_multitracker_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* host_pix);
 int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* host_pix, const uint8_t* next_host_pix,
                                        double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
+/* Packed frames (the blob format of sfmgpu_frames_upload_packed) as the lock-step tracker's input.  blobs[s] / blob_bytes[s]:
+ * the blob that sequence s reads from (host memory; pinned for overlap).  The same blob may serve several sequences: a
+ * step-major blob holds frame t of sequence s as blob frame t*S + s.  Sequence s's next frame is blob frame blob_frame[s].
+ * The S frame records are copied into the tracker's own staging (one cudaMemcpyAsync per run of records adjacent in host
+ * memory: one copy per step for a step-major blob), decoded in one launch (sfmgpu_stage_times_n ms[6]) and their pyramids
+ * built; results are identical to sfmgpu_multitracker_step with the raw frames.  NULL blobs, blob_bytes or blob_frame, a NULL
+ * entry, a blob that sfmgpu_frames_upload_packed would refuse for the tracker's w x h, a frame index outside its blob or a
+ * frame record larger than sfmgpu_pack_bound allows: SFMGPU_E_ARG, before any work is queued.  Frames already prefetched:
+ * SFMGPU_E_STATE.  The caller keeps the blobs valid and unmodified until the step that consumes the prefetch returns. */
+int sfmgpu_multitracker_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* const* blobs,
+                                        const size_t* blob_bytes, const int32_t* blob_frame);
+/* blob_frame == NULL: step the prefetched frames (raw or packed).  next_blob_frame != NULL: frames of the FOLLOWING step, from
+ * the same blobs, are copied, decoded and their pyramids built on the copy stream while this step computes.  Refusals as
+ * above for both index arrays; blob_frame == NULL with nothing prefetched, or frames given while others are prefetched:
+ * SFMGPU_E_STATE.  Records of the stepped frames that do not decode: SFMGPU_E_ARG with the tracker exactly as before the call
+ * (tracks, ids, totals, RANSAC stage results) and no prefetch pending.  sfmgpu_multitracker_step_pipelined with
+ * host_pix == NULL consumes a packed prefetch the same way. */
+int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* const* blobs,
+                                    const size_t* blob_bytes, const int32_t* blob_frame, const int32_t* next_blob_frame,
+                                    double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 /* Resident frames: the next frame of sequence s is frame frame_idx[s] of f (pyramids built; same w, h and level count as the
  * tracker), any indices, repeats allowed - no host-to-device copy of images.  The S pyramids are copied into the tracker's own
  * slots (about 1.33 * w * h bytes read and written per sequence with 3 levels; sfmgpu_stage_times_n ms[5]).  Results identical to

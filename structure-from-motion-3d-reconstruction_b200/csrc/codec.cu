@@ -479,6 +479,9 @@ int sfm_pk_decode(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count, const
   return 0;
 }
 
+// The largest frame record a blob of w x h frames can hold (every tile raw).
+size_t sfm_pk_frame_bound(int w, int h) { return frame_bound(w, h); }
+
 // Largest staged byte range of frames [a, b) chunks: frames of fo (relative indices) split at `chunk` frames.
 size_t sfm_pk_max_chunk_bytes(const std::vector<uint64_t>& fo, int chunk) {
   size_t m = 0;

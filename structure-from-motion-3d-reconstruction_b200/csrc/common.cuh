@@ -133,6 +133,7 @@ int sfm_pk_check(sfmgpu_ctx* ctx, const sfmgpu_frames* f, const uint8_t* blob, s
 int sfm_pk_decode(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count, const uint8_t* stage, const unsigned long long* d_fo,
                   unsigned long long base, int* d_bad);
 int sfm_pk_prepare(sfmgpu_ctx* ctx, const uint8_t* blob, int blob_first, const std::vector<uint64_t>& fo, size_t stage_bytes, int nstage);
+size_t sfm_pk_frame_bound(int w, int h);
 size_t sfm_pk_max_chunk_bytes(const std::vector<uint64_t>& fo, int chunk);
 int sfm_pk_read_flag(sfmgpu_ctx* ctx, const char* who);
 

@@ -1152,6 +1152,14 @@ struct sfmgpu_multitracker {
   unsigned long long* tot = nullptr;
   TwoViewState* tv = nullptr;       // find_E_ransac on every sequence's survivors inside the step (sfmgpu_multitracker_set_ransac)
   bool tv_fresh = false;            // the last step ran the stage: its results can be downloaded
+  // packed input (sfmgpu_multitracker_step_packed): the tracker's own device buffer [decode flag | staged frame offsets [S+1] |
+  // S frame records back to back], allocated by the first packed call, so that no other call on the context can overwrite a
+  // pending prefetch.  pk_done follows the last decode that read the staging; pk_bad receives the flag.
+  uint8_t* pk = nullptr;
+  int* pk_bad = nullptr;            // page-locked host copy of the decode flag
+  cudaEvent_t pk_done = nullptr;
+  bool pk_used = false;             // pk_done has been recorded
+  bool pf_packed = false;           // the prefetched frames were decoded: their flag is checked before they are stepped
 };
 
 namespace {
@@ -1243,12 +1251,16 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   SFM_ENTER_VOID(ctx);
   if (!t) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
+  if (t->pf_done) cudaEventSynchronize(t->pf_done);  // a prefetch still running on the copy stream
   sfm_two_view_free(ctx, &t->tv);
   void* ptrs[] = {t->trk, t->p1, t->pb, t->oa, t->ob, t->ids, t->oid, t->nit, t->keep, t->fresh, t->ok, t->dn, t->dnk, t->didx, t->scal, t->tot};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   if (t->frames) sfmgpu_frames_destroy(ctx, t->frames);
+  if (t->pk) cudaFree(t->pk);
+  if (t->pk_bad) cudaFreeHost(t->pk_bad);
   if (t->pf_done) cudaEventDestroy(t->pf_done);
+  if (t->pk_done) cudaEventDestroy(t->pk_done);
   delete t;
 }
 
@@ -1271,6 +1283,96 @@ static int multi_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int after_gro
     SFM_CUDA(ctx, cudaEventRecord(t->pf_done, ctx->stream));
   }
   t->prefetched = true;
+  t->pf_packed = false;
+  return 0;
+}
+
+// Packed input: blob frame blob_frame[s] of blobs[s] for every sequence s, checked against the tracker's frames.  The records
+// are staged back to back in sequence order (fo: their offsets in the staging), with one copy per run of records that are
+// adjacent in host memory (a step-major blob: one copy per step).
+struct PkPlan {
+  struct Copy {
+    const uint8_t* src;
+    size_t dst, bytes;
+  };
+  std::vector<unsigned long long> fo;
+  std::vector<Copy> copies;
+};
+
+static int multi_pk_plan(sfmgpu_ctx* ctx, const sfmgpu_multitracker* t, const uint8_t* const* blobs, const size_t* blob_bytes,
+                         const int32_t* blob_frame, PkPlan& p, const char* who) {
+  if (!blobs || !blob_bytes) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null blob array", who);
+  const size_t bound = sfm_pk_frame_bound(t->w, t->h);
+  std::vector<uint64_t> fo;
+  p.fo.assign(1, 0);
+  p.copies.clear();
+  for (int s = 0; s < t->S; s++) {
+    SFM_TRY(sfm_pk_check(ctx, t->frames, blobs[s], blob_bytes[s], blob_frame[s], 1, fo, who));
+    const size_t bytes = fo[1] - fo[0];
+    if (bytes > bound)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequence %d: frame record of %zu bytes, a %dx%d frame holds at most %zu", who, s, bytes,
+                      t->w, t->h, bound);
+    const uint8_t* src = blobs[s] + fo[0];
+    if (!p.copies.empty() && p.copies.back().src + p.copies.back().bytes == src)
+      p.copies.back().bytes += bytes;
+    else
+      p.copies.push_back({src, (size_t)p.fo.back(), bytes});
+    p.fo.push_back(p.fo.back() + bytes);
+  }
+  return 0;
+}
+
+// Copy and decode planned records into slot group g on ctx->stream (the caller may scope it to the copy stream); the flag is
+// copied to t->pk_bad behind the decode.  The staging is refilled only after the decode that last read it, on any stream.
+static int multi_pk_decode(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g, const PkPlan& p) {
+  const int S = t->S;
+  const size_t o_fo = 16, o_stage = (o_fo + 8 * ((size_t)S + 1) + 15) & ~(size_t)15;
+  // each piece on its own: a call after a failed allocation completes what is missing
+  if (!t->pk) SFM_CUDA(ctx, cudaMalloc(&t->pk, o_stage + (size_t)S * sfm_pk_frame_bound(t->w, t->h)));
+  if (!t->pk_bad) SFM_CUDA(ctx, cudaMallocHost(&t->pk_bad, sizeof(int)));
+  if (!t->pk_done) SFM_CUDA(ctx, cudaEventCreateWithFlags(&t->pk_done, cudaEventDisableTiming));
+  int* d_bad = (int*)t->pk;
+  unsigned long long* d_fo = (unsigned long long*)(t->pk + o_fo);
+  uint8_t* stage = t->pk + o_stage;
+  if (t->pk_used) SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, t->pk_done, 0));
+  SFM_CUDA(ctx, cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream));
+  SFM_CUDA(ctx, cudaMemcpyAsync(d_fo, p.fo.data(), 8 * p.fo.size(), cudaMemcpyHostToDevice, ctx->stream));
+  for (const PkPlan::Copy& c : p.copies)
+    SFM_CUDA(ctx, cudaMemcpyAsync(stage + c.dst, c.src, c.bytes, cudaMemcpyHostToDevice, ctx->stream));
+  SFM_TRY(sfm_pk_decode(ctx, t->frames, g * S, S, stage, d_fo, 0, d_bad));
+  SFM_CUDA(ctx, cudaEventRecord(t->pk_done, ctx->stream));
+  t->pk_used = true;
+  SFM_CUDA(ctx, cudaMemcpyAsync(t->pk_bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  return 0;
+}
+
+// multi_prefetch for packed frames: copy, decode and pyramids on the copy stream.
+static int multi_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int after_group, const PkPlan& p) {
+  SFM_TRY(pipe_streams(ctx));
+  if (!t->pf_done && cudaEventCreateWithFlags(&t->pf_done, cudaEventDisableTiming) != cudaSuccess)
+    return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker: cudaEventCreate failed");
+  const int S = t->S, g = (after_group + 1) % 3;
+  {
+    StageScope sc(ctx, ctx->copy_stream);
+    SFM_TRY(multi_pk_decode(ctx, t, g, p));
+    SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, g * S, S));
+    SFM_CUDA(ctx, cudaEventRecord(t->pf_done, ctx->stream));
+  }
+  t->prefetched = true;
+  t->pf_packed = true;
+  return 0;
+}
+
+// Hand the prefetched frames to the step on ctx->stream.  Decoded frames are waited for on the host first: records that do not
+// decode fail the call before the step queues anything, and drop the prefetch.
+static int multi_take_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const char* who) {
+  t->prefetched = false;
+  if (t->pf_packed) {
+    t->pf_packed = false;
+    SFM_CUDA(ctx, cudaEventSynchronize(t->pf_done));
+    if (*t->pk_bad) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: a tile record of the prefetched frames does not decode", who);
+  }
+  SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, t->pf_done, 0));
   return 0;
 }
 
@@ -1282,6 +1384,7 @@ int sfmgpu_multitracker_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   if (ctx->copy_stream) SFM_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
   t->parity = -1;
   t->prefetched = false;
+  t->pf_packed = false;
   t->tv_fresh = false;
   t->n.assign(t->S, 0);
   t->next_id.assign(t->S, 0);
@@ -1311,16 +1414,52 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   if (host_pix && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: frames given but others are prefetched");
   const int S = t->S;
   const int par = multi_next_group(t);
+  if (!host_pix) SFM_TRY(multi_take_prefetch(ctx, t, "multitracker_step"));
   t->tv_fresh = false;
   if (host_pix) {
     SFM_TRY(sfmgpu_frames_upload(ctx, t->frames, par * S, S, host_pix));
     SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, par * S, S));
-  } else {
-    SFM_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, t->pf_done, 0));
-    t->prefetched = false;
   }
   // the frames of the NEXT step travel while this one computes (their slot group is neither previous nor current)
   if (next_host_pix) SFM_TRY(multi_prefetch(ctx, t, par, next_host_pix));
+  return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
+}
+
+int sfmgpu_multitracker_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* const* blobs, const size_t* blob_bytes,
+                                        const int32_t* blob_frame) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  const char* who = "multitracker_prefetch_packed";
+  if (!blob_frame) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null frame index array", who);
+  if (t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: the prefetched frames have not been stepped yet", who);
+  PkPlan p;
+  SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, blob_frame, p, who));
+  return multi_prefetch_packed(ctx, t, t->parity < 0 ? 2 : t->parity, p);
+}
+
+int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* const* blobs, const size_t* blob_bytes,
+                                    const int32_t* blob_frame, const int32_t* next_blob_frame, double* prev_xy, double* cur_xy,
+                                    int32_t* ids, int32_t* n_out) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  const char* who = "multitracker_step_packed";
+  if (!blob_frame && !t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: no frames given and none prefetched", who);
+  if (blob_frame && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: frames given but others are prefetched", who);
+  PkPlan cur, next;
+  if (blob_frame) SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, blob_frame, cur, who));
+  if (next_blob_frame) SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, next_blob_frame, next, who));
+  const int S = t->S;
+  const int par = multi_next_group(t);
+  if (blob_frame) {  // decoded and checked before the step queues anything; the pyramids only for frames that decoded
+    SFM_TRY(multi_pk_decode(ctx, t, par, cur));
+    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (*t->pk_bad) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: a tile record of the frames does not decode", who);
+    SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, par * S, S));
+  } else {
+    SFM_TRY(multi_take_prefetch(ctx, t, who));
+  }
+  t->tv_fresh = false;
+  if (next_blob_frame) SFM_TRY(multi_prefetch_packed(ctx, t, par, next));
   return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
 }
 

@@ -46,6 +46,7 @@ SYMBOLS = [
     "sfmgpu_multitracker_step_frames", "sfmgpu_pair_frontend_segments", "sfmgpu_pairs_ids_download_all", "sfmgpu_pairs_ids_device_ptr",
     "sfmgpu_sched_segment_shard", "sfmgpu_sched_gather_pair_ids",
     "sfmgpu_pack_bound", "sfmgpu_frames_pack", "sfmgpu_frames_upload_packed", "sfmgpu_pair_frontend_host_packed",
+    "sfmgpu_multitracker_prefetch_packed", "sfmgpu_multitracker_step_packed",
 ]
 
 
@@ -188,6 +189,8 @@ def load_library():
         "sfmgpu_frames_pack": (_i, [_vp, _vp, _i, _i, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
         "sfmgpu_frames_upload_packed": (_i, [_vp, _vp, _i, _vp, C.c_size_t, _i, _i]),
         "sfmgpu_pair_frontend_host_packed": (_i, [_vp, _vp, _vp, C.c_size_t, _i, _i, C.POINTER(LKCfg), _vp, _i, _vp, _vp, _vp, _vp]),
+        "sfmgpu_multitracker_prefetch_packed": (_i, [_vp, _vp, _vp, _vp, _vp]),
+        "sfmgpu_multitracker_step_packed": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     }
     for name, (res, args) in S.items():
         fn = getattr(lib, name)
@@ -811,6 +814,45 @@ class MultiTracker:
         a = (self.prev, self.cur, self.ids) if fetch else (None, None, None)
         self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_step_frames(self.ctx.h, self.h_, frames.h_, _ptr(idx), _ptr(a[0]), _ptr(a[1]),
                                                                   _ptr(a[2]), self.n.ctypes.data_as(_vp)))
+        if not fetch:
+            return self.n.copy()
+        return [(self.prev[s, :self.n[s]].copy(), self.cur[s, :self.n[s]].copy(), self.ids[s, :self.n[s]].copy()) for s in range(self.S)]
+
+    def _packed(self, blobs, blob_frames):
+        """(arrays to keep alive, blob pointer array, byte counts, frame indices) of a packed call; blobs: one blob shared by
+        every sequence, a list of S, or None (no frames)."""
+        if blobs is None:
+            return None, None, None, (None if blob_frames is None else np.ascontiguousarray(blob_frames, np.int32).reshape(-1))
+        bl = [blobs] * self.S if isinstance(blobs, np.ndarray) else list(blobs)
+        assert len(bl) == self.S, (len(bl), self.S)
+        ptrs, sizes = zip(*(_blob(b) for b in bl))
+        idx = None
+        if blob_frames is not None:
+            idx = np.ascontiguousarray(blob_frames, np.int32).reshape(-1)
+            assert len(idx) == self.S, (len(idx), self.S)
+        return bl, (_vp * self.S)(*ptrs), (C.c_size_t * self.S)(*sizes), idx
+
+    def prefetch_packed(self, blobs, blob_frames):
+        """prefetch() from packed blobs (Frames.pack): the next frame of sequence s is blob frame blob_frames[s] of its blob;
+        copied, decoded and its pyramids built on the copy stream.  step(None) or step_packed(blobs, None) consumes them."""
+        bl, p, n, idx = self._packed(blobs, blob_frames)
+        # keep the blobs alive while the prefetch is pending; until the call returns, also those of an earlier prefetch that a
+        # refused call leaves pending
+        self._pf = (getattr(self, "_pf", None), bl)
+        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_prefetch_packed(self.ctx.h, self.h_, p, n, _ptr(idx)))
+        self._pf = bl
+
+    def step_packed(self, blobs, blob_frames, next_frames=None, fetch=True):
+        """step() from packed blobs: blob_frames[s] = the blob frame of sequence s (None: the prefetched frames, raw or
+        packed); next_frames: the blob frames of the following step, decoded while this one computes.  Returns as step()."""
+        bl, p, n, idx = self._packed(blobs, blob_frames)
+        nxt = None if next_frames is None else self._packed(bl, next_frames)[3]
+        a = (self.prev, self.cur, self.ids) if fetch else (None, None, None)
+        if next_frames is not None:  # held before the call: a call that fails after queuing the prefetch leaves it pending
+            self._pf = (getattr(self, "_pf", None), bl)
+        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_step_packed(self.ctx.h, self.h_, p, n, _ptr(idx), _ptr(nxt), _ptr(a[0]), _ptr(a[1]),
+                                                                  _ptr(a[2]), self.n.ctypes.data_as(_vp)))
+        self._pf = bl if next_frames is not None else None
         if not fetch:
             return self.n.copy()
         return [(self.prev[s, :self.n[s]].copy(), self.cur[s, :self.n[s]].copy(), self.ids[s, :self.n[s]].copy()) for s in range(self.S)]
