@@ -12,6 +12,31 @@
 // ---- small kernels -----------------------------------------------------------------------------------------------
 namespace {
 
+// Rank of this thread's element among the kept elements of its 1024-element tile, in block order; *total receives the tile's
+// count.  Called by every thread of a 1024-thread block, once per tile: the next call's shared writes come after a barrier
+// that every thread reaches only once it has read this call's results.
+__device__ __forceinline__ int tile_rank(bool k, int* total) {
+  __shared__ int wcnt[32], wpre[32], tile_total;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned m = __ballot_sync(0xffffffffu, k);
+  if (lane == 0) wcnt[warp] = __popc(m);
+  __syncthreads();
+  if (warp == 0) {
+    const int a = wcnt[lane];
+    int ia = a;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, ia, o);
+      if (lane >= o) ia += u;
+    }
+    wpre[lane] = ia - a;
+    if (lane == 31) tile_total = ia;
+  }
+  __syncthreads();
+  *total = tile_total;
+  return wpre[warp] + __popc(m & ((1u << lane) - 1u));
+}
+
 // Ordered compaction of the survivors of one pair / one tracker step: block = one pair.
 // keep == nullptr keeps everything.  Outputs (any may be null): a/b = p0/p1 of survivors, ids_out, n_out.
 __global__ void __launch_bounds__(1024) compact_kernel(const double2* __restrict__ p0, const double2* __restrict__ p1,
@@ -19,46 +44,28 @@ __global__ void __launch_bounds__(1024) compact_kernel(const double2* __restrict
                                                       const int* __restrict__ counts, int cap, double2* __restrict__ oa,
                                                       double2* __restrict__ ob, int* __restrict__ oid,
                                                       int* __restrict__ n_out) {
-  __shared__ int wcnt[32], wpre[32];
-  __shared__ int base, total;
-  const int pair = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int pair = blockIdx.x;
   int n = counts ? counts[pair] : cap;
   n = n < 0 ? 0 : (n > cap ? cap : n);
   const size_t off = (size_t)pair * cap;
-  if (tid == 0) base = 0;
-  __syncthreads();
+  int base = 0;
   for (int s = 0; s < n; s += 1024) {
-    const int i = s + tid;
+    const int i = s + threadIdx.x;
     const bool k = i < n && (keep ? keep[off + i] != 0 : true);
-    const unsigned m = __ballot_sync(0xffffffffu, k);
-    if (lane == 0) wcnt[warp] = __popc(m);
-    __syncthreads();
-    if (warp == 0) {
-      const int a = wcnt[lane];
-      int ia = a;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int u = __shfl_up_sync(0xffffffffu, ia, o);
-        if (lane >= o) ia += u;
-      }
-      wpre[lane] = ia - a;
-      if (lane == 31) total = ia;
-    }
-    __syncthreads();
+    int total;
+    const int r = base + tile_rank(k, &total);
     if (k) {
-      const int r = base + wpre[warp] + __popc(m & ((1u << lane) - 1u));
       if (oa) oa[off + r] = p0[off + i];
       if (ob) ob[off + r] = p1[off + i];
       if (oid) oid[off + r] = ids[off + i];
     }
-    __syncthreads();
-    if (tid == 0) base += total;
-    __syncthreads();
+    base += total;
   }
-  if (tid == 0 && n_out) n_out[pair] = base;
+  if (threadIdx.x == 0 && n_out) n_out[pair] = base;
 }
 
 // totals[0] += sum max(ncorn,0); totals[1] += sum nkept; totals[2] += sum nit; totals[3] += #frames with ncorn < 0
+// (ncorn == nullptr: cap for every pair)
 __global__ void __launch_bounds__(256) totals_kernel(const int* __restrict__ ncorn, const int* __restrict__ nkept,
                                                     const int* __restrict__ nit, int npairs, int cap,
                                                     unsigned long long* __restrict__ totals) {
@@ -66,7 +73,7 @@ __global__ void __launch_bounds__(256) totals_kernel(const int* __restrict__ nco
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)npairs * cap;
        i += (long long)gridDim.x * blockDim.x) {
     const int pair = (int)(i / cap), slot = (int)(i - (long long)pair * cap);
-    const int n = ncorn[pair];
+    const int n = ncorn ? ncorn[pair] : cap;
     if (slot == 0) {
       if (n < 0) bad++;
       c += n > 0 ? n : 0;
@@ -80,11 +87,11 @@ __global__ void __launch_bounds__(256) totals_kernel(const int* __restrict__ nco
   // nit can exceed 32 bits per warp only for absurd sizes; reduce in two halves to be safe
   unsigned lo = __reduce_add_sync(0xffffffffu, (unsigned)(it & 0xFFFFu));
   unsigned hi = __reduce_add_sync(0xffffffffu, (unsigned)(it >> 16));
-  if ((threadIdx.x & 31) == 0) {
-    atomicAdd(&totals[0], c);
-    atomicAdd(&totals[1], k);
-    atomicAdd(&totals[2], (unsigned long long)lo + ((unsigned long long)hi << 16));
-    atomicAdd(&totals[3], bad);
+  if ((threadIdx.x & 31) == 0) {  // zero partials are skipped: only the warps holding slot 0 of a pair count corners
+    if (c) atomicAdd(&totals[0], c);
+    if (k) atomicAdd(&totals[1], k);
+    if (lo | hi) atomicAdd(&totals[2], (unsigned long long)lo + ((unsigned long long)hi << 16));
+    if (bad) atomicAdd(&totals[3], bad);
   }
 }
 
@@ -115,56 +122,30 @@ __global__ void __launch_bounds__(1024) replenish_append_kernel(const double2* _
                                                                const uint8_t* __restrict__ ok, double2* __restrict__ tracks,
                                                                int* __restrict__ ids, int n_tracks, int room, int next_id,
                                                                int* __restrict__ n_added) {
-  __shared__ int wcnt[32], wpre[32];
-  __shared__ int base, total;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nf = *n_fresh;
-  if (tid == 0) base = 0;
-  __syncthreads();
-  for (int s = 0; s < nf; s += 1024) {
-    const int i = s + tid;
+  int base = 0;
+  for (int s = 0; s < nf && base < room; s += 1024) {
+    const int i = s + threadIdx.x;
     const bool k = i < nf && ok[i];
-    const unsigned m = __ballot_sync(0xffffffffu, k);
-    if (lane == 0) wcnt[warp] = __popc(m);
-    __syncthreads();
-    if (warp == 0) {
-      const int a = wcnt[lane];
-      int ia = a;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int u = __shfl_up_sync(0xffffffffu, ia, o);
-        if (lane >= o) ia += u;
-      }
-      wpre[lane] = ia - a;
-      if (lane == 31) total = ia;
+    int total;
+    const int r = base + tile_rank(k, &total);
+    if (k && r < room) {
+      tracks[n_tracks + r] = fresh[i];
+      ids[n_tracks + r] = next_id + r;
     }
-    __syncthreads();
-    if (k) {
-      const int r = base + wpre[warp] + __popc(m & ((1u << lane) - 1u));
-      if (r < room) {
-        tracks[n_tracks + r] = fresh[i];
-        ids[n_tracks + r] = next_id + r;
-      }
-    }
-    __syncthreads();
-    if (tid == 0) base += total;
-    __syncthreads();
-    if (base >= room) break;
+    base += total;
   }
-  if (tid == 0) *n_added = base < room ? base : room;
+  if (threadIdx.x == 0) *n_added = base < room ? base : room;
 }
 
-// out[0] += sum v[0..n)
-__global__ void __launch_bounds__(256) sum_int_kernel(const int* __restrict__ v, int n, unsigned long long* __restrict__ out) {
-  unsigned s = 0;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) s += (unsigned)v[i];
-  s = __reduce_add_sync(0xffffffffu, s);
-  if ((threadIdx.x & 31) == 0 && s) atomicAdd(out, (unsigned long long)s);
-}
-
-__global__ void iota_ids_kernel(int* ids, const int* n, int next_id) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < *n) ids[i] = next_id + i;
+// After a detection into `fresh` (row stride fresh_stride): row s of the track lists = the first n[s] corners with ids
+// first_id[s]...
+__global__ void take_corners_kernel(const double2* __restrict__ fresh, int fresh_stride, const int* __restrict__ n,
+                                    const int* __restrict__ first_id, double2* __restrict__ trk, int* __restrict__ ids, int rows) {
+  const int s = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n[s] || i >= rows) return;
+  trk[(size_t)s * rows + i] = fresh[(size_t)s * fresh_stride + i];
+  ids[(size_t)s * rows + i] = first_id[s] + i;
 }
 
 // Rows of a track list: after reset at most max(max_tracks, 1) entries; replenish appends first and tests the cap afterwards
@@ -193,6 +174,18 @@ int default_cand_cap(int w, int h) {
   if (cap < 65536) cap = 65536;
   if (cap > px) cap = px;
   return (int)cap;
+}
+
+int abs_min_distance(const sfmgpu_lkcfg& c) { return c.min_distance < 0 ? -c.min_distance : c.min_distance; }
+
+// Corners of frames [first, first + count) with the work area sized for the worst case, W*H candidates per frame (a flat image
+// makes every pixel one), so that no frame overflows: out [count][max(max_corners, 1)], counts d_n[count].
+int detect_full(sfmgpu_ctx* ctx, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int first, int count, int max_corners, double2* out,
+                int* d_n) {
+  const int cand_cap = f->w * f->h;
+  SFM_TRY(sfm_reserve(ctx, ctx->cs_work, sfm_corner_work_bytes_md(f->w, f->h, count, cand_cap, abs_min_distance(cfg))));
+  return sfm_corners_batch(ctx, f, first, count, max_corners, cfg.quality, cfg.min_distance, cand_cap, ctx->cs_work.p,
+                           ctx->cs_work.cap, out, d_n);
 }
 
 }  // namespace
@@ -318,7 +311,7 @@ static ChunkArgs chunk_args(sfmgpu_frames* f, int first_frame, int pair_off, int
   c.out = out;
   c.work = work;
   c.cand_cap = default_cand_cap(f->w, f->h);
-  c.md = cfg->min_distance < 0 ? -cfg->min_distance : cfg->min_distance;
+  c.md = abs_min_distance(*cfg);
   c.cf = f;
   c.cfirst = first_frame;
   c.b_off = 1;
@@ -499,11 +492,8 @@ static int pair_fix_overflow(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first_frame,
   for (int p = 0; p < npairs; p++)
     if (hn[p] < 0) bad.push_back(p);
   if (bad.empty()) return 0;
-  const int full_cap = f->w * f->h, md = cfg->min_distance < 0 ? -cfg->min_distance : cfg->min_distance;
-  SFM_TRY(sfm_reserve(ctx, ctx->cs_work, sfm_corner_work_bytes_md(f->w, f->h, 1, full_cap, md)));
   for (int p : bad) {
-    SFM_TRY(sfm_corners_batch(ctx, f, h_fa ? h_fa[p] : first_frame + p, 1, cfg->max_tracks, cfg->quality, cfg->min_distance, full_cap,
-                              ctx->cs_work.p, ctx->cs_work.cap, out->xy0 + (size_t)p * out->cap, out->ncorn + p));
+    SFM_TRY(detect_full(ctx, *cfg, f, h_fa ? h_fa[p] : first_frame + p, 1, cfg->max_tracks, out->xy0 + (size_t)p * out->cap, out->ncorn + p));
     ChunkArgs c = chunk_args(f, first_frame + p, p, 1, cfg, out, nullptr);
     if (h_fa) {
       c.cfirst = h_fa[p];
@@ -886,78 +876,223 @@ int sfmgpu_pairs_download(sfmgpu_ctx* ctx, sfmgpu_pairs* p, int pair, double* li
 
 }  // extern "C"
 
-// ---- stateful tracker -------------------------------------------------------------------------------------------------
+// ---- track lists: the state and the operations of KLTTracker (:323-391) ------------------------------------------------------
+// Both tracker objects run on this one core: sfmgpu_tracker holds one track list, sfmgpu_multitracker S lists that are stepped
+// together.  What differs between them is where the frames come from, how the KLT launch is sized, and what is downloaded.
+namespace {
+
+// S track lists of `rows` entries, list s at entry s * rows, with the device scratch of their steps.
+struct TrackLists {
+  int S = 0, rows = 0, fresh_cap = 0;
+  double2 *trk = nullptr, *p1 = nullptr, *pb = nullptr, *oa = nullptr, *ob = nullptr, *fresh = nullptr;
+  int *ids = nullptr, *oid = nullptr, *nit = nullptr;
+  int *dn = nullptr, *dnk = nullptr;  // per list: tracks entering the last step (KLT_BY_ROWS), its survivors
+  int* rst = nullptr;                 // a reset's per-list corner counts [S] and first ids [S]
+  int* scal = nullptr;                // a replenishment's [1] n_fresh, [2] n_added
+  uint8_t *keep = nullptr, *ok = nullptr;
+  unsigned long long* tot = nullptr;  // totals_kernel's sums over all steps ([2]: LK iterations)
+  std::vector<int> n, next_id;        // host: live tracks and the next id of every list
+  long long track_steps = 0;
+};
+
+int lkcfg_ok(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, const char* who) {
+  if (cfg->pyr_levels < 1 || cfg->pyr_levels > SFM_MAXL || cfg->max_tracks > (1 << 24) || cfg->min_tracks > (1 << 24))
+    return sfm_fail(ctx, SFMGPU_E_ARG, "%s: bad configuration", who);
+  return 0;
+}
+
+cudaError_t lists_alloc(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, int S) {
+  L.S = S;
+  L.rows = track_rows(cfg);
+  L.fresh_cap = 3 * (cfg.max_tracks < 1 ? 1 : cfg.max_tracks);
+  L.n.assign(S, 0);
+  L.next_id.assign(S, 0);
+  cudaError_t e = cudaSuccess;
+  auto al = [&](void** q, size_t bytes) {
+    if (e == cudaSuccess) e = cudaMalloc(q, bytes + 256);
+  };
+  const size_t n = (size_t)L.rows * S;
+  al((void**)&L.trk, n * 16);
+  al((void**)&L.p1, n * 16);
+  al((void**)&L.pb, n * 16);
+  al((void**)&L.oa, n * 16);
+  al((void**)&L.ob, n * 16);
+  al((void**)&L.ids, n * 4);
+  al((void**)&L.oid, n * 4);
+  al((void**)&L.nit, n * 4);
+  al((void**)&L.keep, n);
+  al((void**)&L.fresh, (size_t)L.fresh_cap * 16 * S);
+  al((void**)&L.ok, (size_t)L.fresh_cap);
+  al((void**)&L.dn, (size_t)S * 4);
+  al((void**)&L.dnk, (size_t)S * 4);
+  al((void**)&L.rst, (size_t)S * 8);
+  al((void**)&L.scal, 64);
+  al((void**)&L.tot, 64);
+  if (e == cudaSuccess) e = cudaMemsetAsync(L.tot, 0, 64, ctx->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(L.scal, 0, 64, ctx->stream);
+  return e;
+}
+
+void lists_free(TrackLists& L) {
+  void* ptrs[] = {L.trk, L.p1, L.pb, L.oa, L.ob, L.fresh, L.ids, L.oid, L.nit, L.dn, L.dnk, L.rst, L.scal, L.keep, L.ok, L.tot};
+  for (void* q : ptrs)
+    if (q) cudaFree(q);
+}
+
+// reset(gray) (:327-332) of lists [s0, s0 + count) on frames first + s0, ...: list s = the first corners of its frame
+// (shi_tomasi(gray, max_tracks, ...)) with ids next_id[s]++.  Synchronises the context stream.
+int lists_reset(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int first, int s0, int count,
+                const char* who) {
+  const int stride = cfg.max_tracks < 1 ? 1 : cfg.max_tracks;
+  int *d_n = L.rst + s0, *d_id = L.rst + L.S + s0;
+  SFM_TRY(detect_full(ctx, cfg, f, first + s0, count, cfg.max_tracks, L.fresh, d_n));
+  std::vector<int> n(count);
+  SFM_CUDA(ctx, cudaMemcpyAsync(n.data(), d_n, (size_t)count * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaMemcpyAsync(d_id, L.next_id.data() + s0, (size_t)count * 4, cudaMemcpyHostToDevice, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  for (int j = 0; j < count; j++)
+    if (n[j] < 0) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "%s: candidate capacity exceeded (sequence %d)", who, s0 + j);
+  SFM_LAUNCH(ctx, take_corners_kernel, dim3(sfm_cdiv(stride, 256), count), 256, 0, (const double2*)L.fresh, stride, (const int*)d_n,
+             (const int*)d_id, L.trk + (size_t)s0 * L.rows, L.ids + (size_t)s0 * L.rows, L.rows);
+  for (int j = 0; j < count; j++) {
+    L.n[s0 + j] = n[j];
+    L.next_id[s0 + j] += n[j];
+  }
+  return 0;
+}
+
+// How a step's launches are sized.  sfm_klt_launch picks the kernel family from npairs * cap, and the two families agree to
+// within 1e-6 px, not bit for bit, so each tracker keeps its own rule: the single tracker by its live tracks, the lock-step
+// tracker by all S x rows entries with the live counts uploaded to dn.
+enum KltSizing { KLT_BY_LIVE, KLT_BY_ROWS };
+
+// One step of every list from frame fa0 + s to frame fb0 + s (:346-371): the survivors of list s in track order, (p0, p1, id),
+// go to row s of oa / ob / oid and their count to dnk[s]; the step's sums are added to tot.
+int lists_track(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int fa0, int fb0, KltSizing sizing) {
+  KltLaunch k;
+  k.pv = f->view();
+  k.p0 = L.trk;
+  if (sizing == KLT_BY_LIVE) {  // one list
+    k.counts = nullptr;
+    k.npairs = 1;
+    k.cap = L.n[0];
+  } else {
+    SFM_CUDA(ctx, cudaMemcpyAsync(L.dn, L.n.data(), (size_t)L.S * 4, cudaMemcpyHostToDevice, ctx->stream));
+    k.counts = L.dn;
+    k.npairs = L.S;
+    k.cap = L.rows;
+  }
+  k.fa0 = fa0;
+  k.fa_step = 1;
+  k.fb0 = fb0;
+  k.fb_step = 1;
+  k.radius = cfg.win_radius;
+  k.iters = cfg.iters;
+  k.fb_thresh = cfg.fb_thresh;
+  k.p1 = L.p1;
+  k.pb = L.pb;
+  k.nit = L.nit;
+  k.keep = L.keep;
+  SFM_TRY(sfm_klt_launch(ctx, k));
+  for (int s = 0; s < L.S; s++) L.track_steps += L.n[s];
+  SFM_LAUNCH(ctx, compact_kernel, L.S, 1024, 0, L.trk, L.p1, L.keep, (const int*)L.ids, k.counts, k.cap, L.oa, L.ob, L.oid, L.dnk);
+  const unsigned tb = sfm_cdiv((long long)k.npairs * k.cap, 256);  // no more blocks (and atomics) than entries
+  SFM_LAUNCH(ctx, totals_kernel, tb < 64 ? tb : 64, 256, 0, k.counts, (const int*)L.dnk, (const int*)L.nit, L.S, k.cap, L.tot);
+  return 0;
+}
+
+// tracks_ = kept (:371): the first `entries` entries of the survivor rows become the track lists (the caller sets n).
+// Synchronises the context stream, so downloads queued before it have landed when it returns.
+int lists_commit(sfmgpu_ctx* ctx, TrackLists& L, size_t entries) {
+  if (entries == 0) return 0;
+  SFM_CUDA(ctx, cudaMemcpyAsync(L.trk, L.ob, entries * 16, cudaMemcpyDeviceToDevice, ctx->stream));
+  SFM_CUDA(ctx, cudaMemcpyAsync(L.ids, L.oid, entries * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+// Replenish list s (:374-389): detect need*3 corners on its current frame, drop those within min_distance of a live track,
+// append survivors with consecutive ids until max_tracks (tested after the append: at least one is added).
+int replenish_row(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int frame, int s) {
+  int &n = L.n[s], &next_id = L.next_id[s];
+  double2* trk = L.trk + (size_t)s * L.rows;
+  const int need = cfg.max_tracks - n;
+  long long want = (long long)need * 3;
+  if (want > L.fresh_cap) want = L.fresh_cap;  // fresh_cap = 3*max_tracks >= need*3
+  SFM_TRY(detect_full(ctx, cfg, f, frame, 1, (int)want, L.fresh, L.scal + 1));
+  int nf = 0;
+  SFM_CUDA(ctx, cudaMemcpyAsync(&nf, L.scal + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (nf < 0) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker: candidate capacity exceeded");
+  if (nf > 0) {
+    const double d2 = (double)cfg.min_distance * cfg.min_distance;
+    SFM_LAUNCH(ctx, replenish_filter_kernel, sfm_cdiv(nf, 256), 256, 0, L.fresh, (const int*)(L.scal + 1), trk, n, d2, L.ok);
+    // the reference appends first and tests the cap afterwards (:386-387): at least one corner is added
+    int room = cfg.max_tracks - n;
+    if (room < 1) room = 1;
+    if (n + room > L.rows)  // cannot happen with rows sized by track_rows(); never write past the row
+      return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker: track list of %d + %d exceeds its %d rows", n, room, L.rows);
+    SFM_LAUNCH(ctx, replenish_append_kernel, 1, 1024, 0, L.fresh, (const int*)(L.scal + 1), L.ok, trk, L.ids + (size_t)s * L.rows, n,
+               room, next_id, L.scal + 2);
+    int na = 0;
+    SFM_CUDA(ctx, cudaMemcpyAsync(&na, L.scal + 2, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    n += na;
+    next_id += na;
+  }
+  return 0;
+}
+
+// After a commit, list by list on frames first + s: a list that entered the step without tracks (empty[s]; empty == nullptr:
+// none did) is reset on its frame instead of stepped (:341-344), one frame at a time; a list below min_tracks is replenished.
+int lists_refill(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int first, const std::vector<char>* empty,
+                 const char* who) {
+  for (int s = 0; s < L.S; s++) {
+    if (empty && (*empty)[s])
+      SFM_TRY(lists_reset(ctx, L, cfg, f, first, s, 1, who));
+    else if (L.n[s] < cfg.min_tracks)
+      SFM_TRY(replenish_row(ctx, L, cfg, f, first + s, s));
+  }
+  return 0;
+}
+
+// tracks() of list s: its first n entries into the caller's cap.
+int lists_tracks(sfmgpu_ctx* ctx, const TrackLists& L, int s, double* xy, int32_t* ids, int cap, int* n_out, const char* who) {
+  const int n = L.n[s];
+  if (n_out) *n_out = n;
+  if (n > cap) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "%s: %d tracks, room for %d", who, n, cap);
+  if (n > 0) {
+    if (xy) SFM_CUDA(ctx, cudaMemcpyAsync(xy, L.trk + (size_t)s * L.rows, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, L.ids + (size_t)s * L.rows, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  }
+  return 0;
+}
+
+int lists_totals(sfmgpu_ctx* ctx, const TrackLists& L, long long* n_track_steps, long long* n_lk_iters) {
+  unsigned long long tt[4];
+  SFM_CUDA(ctx, cudaMemcpyAsync(tt, L.tot, sizeof tt, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (n_track_steps) *n_track_steps = L.track_steps;
+  if (n_lk_iters) *n_lk_iters = (long long)tt[2];
+  return 0;
+}
+
+}  // namespace
+
+// ---- stateful tracker: one track list; its frames are read in place from the caller's batch ---------------------------------
 struct sfmgpu_tracker {
   sfmgpu_lkcfg cfg;
   sfmgpu_frames* own = nullptr;     // 2-slot ping-pong used by the host-image entry points
   sfmgpu_frames* prev_frames = nullptr;
   int prev_index = -1;
-  int n = 0;                        // live tracks (host copy)
-  int next_id = 0;
-  int cap = 0;
-  double2 *trk = nullptr, *p1 = nullptr, *pb = nullptr, *oa = nullptr, *ob = nullptr, *fresh = nullptr;
-  int *ids = nullptr, *oid = nullptr, *nit = nullptr, *scal = nullptr;  // scal: [0] n_out, [1] n_fresh, [2] n_added
-  uint8_t *keep = nullptr, *ok = nullptr;
-  int fresh_cap = 0;
-  long long track_steps = 0;
-  unsigned long long* tot = nullptr;
+  TrackLists L;                     // S = 1
 };
 
 namespace {
 
-int tracker_detect(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int frame, int max_corners, double2* out, int* d_n) {
-  const int cand_cap = f->w * f->h;  // single frame: always room for the worst case
-  const int md = t->cfg.min_distance < 0 ? -t->cfg.min_distance : t->cfg.min_distance;
-  const size_t wb = sfm_corner_work_bytes_md(f->w, f->h, 1, cand_cap, md);
-  SFM_TRY(sfm_reserve(ctx, ctx->cs_work, wb));
-  return sfm_corners_batch(ctx, f, frame, 1, max_corners, t->cfg.quality, t->cfg.min_distance, cand_cap, ctx->cs_work.p,
-                           ctx->cs_work.cap, out, d_n);
-}
-
-// Replenish one track list (:374-389): detect need*3 corners on the current frame, drop those within min_distance of a live
-// track, append survivors with consecutive ids until max_tracks (tested after the append: at least one is added).
-int replenish_row(sfmgpu_ctx* ctx, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int frame, double2* trk, int* ids, int* n_io, int* next_id_io,
-                  double2* fresh, int fresh_cap, uint8_t* ok, int* scal, int row_cap) {
-  const int need = cfg.max_tracks - *n_io;
-  long long want = (long long)need * 3;
-  if (want > fresh_cap) want = fresh_cap;  // fresh_cap = 3*max_tracks >= need*3
-  const int cand_cap = f->w * f->h;        // single frame: always room for the worst case
-  const int md = cfg.min_distance < 0 ? -cfg.min_distance : cfg.min_distance;
-  SFM_TRY(sfm_reserve(ctx, ctx->cs_work, sfm_corner_work_bytes_md(f->w, f->h, 1, cand_cap, md)));
-  SFM_TRY(sfm_corners_batch(ctx, f, frame, 1, (int)want, cfg.quality, cfg.min_distance, cand_cap, ctx->cs_work.p, ctx->cs_work.cap, fresh,
-                            scal + 1));
-  int nf = 0;
-  SFM_CUDA(ctx, cudaMemcpyAsync(&nf, scal + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (nf < 0) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker: candidate capacity exceeded");
-  if (nf > 0) {
-    const double d2 = (double)cfg.min_distance * cfg.min_distance;
-    SFM_LAUNCH(ctx, replenish_filter_kernel, sfm_cdiv(nf, 256), 256, 0, fresh, (const int*)(scal + 1), trk, *n_io, d2, ok);
-    // the reference appends first and tests the cap afterwards (:386-387): at least one corner is added
-    int room = cfg.max_tracks - *n_io;
-    if (room < 1) room = 1;
-    if (*n_io + room > row_cap)  // cannot happen with rows sized by track_rows(); never write past the row
-      return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker: track list of %d + %d exceeds its %d rows", *n_io, room, row_cap);
-    SFM_LAUNCH(ctx, replenish_append_kernel, 1, 1024, 0, fresh, (const int*)(scal + 1), ok, trk, ids, *n_io, room, *next_id_io, scal + 2);
-    int na = 0;
-    SFM_CUDA(ctx, cudaMemcpyAsync(&na, scal + 2, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    *n_io += na;
-    *next_id_io += na;
-  }
-  return 0;
-}
-
 int tracker_reset_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int frame) {
-  // reset(gray) :327-332: prev_ = gray; tracks_ = shi_tomasi(...) with ids next_id_++
-  SFM_TRY(tracker_detect(ctx, t, f, frame, t->cfg.max_tracks, t->trk, t->scal + 1));
-  int n = 0;
-  SFM_CUDA(ctx, cudaMemcpyAsync(&n, t->scal + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (n < 0) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker: candidate capacity exceeded");
-  if (n > 0) SFM_LAUNCH(ctx, iota_ids_kernel, sfm_cdiv(n, 256), 256, 0, t->ids, (const int*)(t->scal + 1), t->next_id);
-  t->n = n;
-  t->next_id += n;
+  SFM_TRY(lists_reset(ctx, t->L, t->cfg, f, frame, 0, 1, "tracker"));
   t->prev_frames = f;
   t->prev_index = frame;
   return 0;
@@ -965,54 +1100,28 @@ int tracker_reset_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int f
 
 int tracker_step_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int frame, double* prev_xy, double* cur_xy,
                     int32_t* ids, int cap, int* n_out) {
+  TrackLists& L = t->L;
   if (n_out) *n_out = 0;
-  if (t->prev_index < 0 || t->n == 0) return tracker_reset_on(ctx, t, f, frame);  // :341-344
+  if (t->prev_index < 0 || L.n[0] == 0) return tracker_reset_on(ctx, t, f, frame);  // :341-344
   if (t->prev_frames != f) return sfm_fail(ctx, SFMGPU_E_STATE, "tracker: previous frame lives in another frame batch");
-  KltLaunch k;
-  k.pv = f->view();
-  k.p0 = t->trk;
-  k.counts = nullptr;
-  k.npairs = 1;
-  k.cap = t->n;
-  k.fa0 = t->prev_index;
-  k.fa_step = 0;
-  k.fb0 = frame;
-  k.fb_step = 0;
-  k.radius = t->cfg.win_radius;
-  k.iters = t->cfg.iters;
-  k.fb_thresh = t->cfg.fb_thresh;
-  k.p1 = t->p1;
-  k.pb = t->pb;
-  k.nit = t->nit;
-  k.keep = t->keep;
-  SFM_TRY(sfm_klt_launch(ctx, k));
-  t->track_steps += t->n;
-  SFM_LAUNCH(ctx, sum_int_kernel, 8, 256, 0, (const int*)t->nit, t->n, t->tot + 2);
-  // survivors in track order: (p0, p1, id); tracks_ = kept (:364-371)
-  SFM_LAUNCH(ctx, compact_kernel, 1, 1024, 0, t->trk, t->p1, t->keep, t->ids, (const int*)nullptr, t->n, t->oa, t->ob, t->oid,
-             t->scal);
+  SFM_TRY(lists_track(ctx, L, t->cfg, f, t->prev_index, frame, KLT_BY_LIVE));
   int nk = 0;
-  SFM_CUDA(ctx, cudaMemcpyAsync(&nk, t->scal, 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_CUDA(ctx, cudaMemcpyAsync(&nk, L.dnk, 4, cudaMemcpyDeviceToHost, ctx->stream));
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   if (nk > cap && (prev_xy || cur_xy || ids))
     return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker_step: %d survivors, room for %d", nk, cap);
   if (nk > 0) {
-    if (prev_xy) SFM_CUDA(ctx, cudaMemcpyAsync(prev_xy, t->oa, (size_t)nk * 16, cudaMemcpyDeviceToHost, ctx->stream));
-    if (cur_xy) SFM_CUDA(ctx, cudaMemcpyAsync(cur_xy, t->ob, (size_t)nk * 16, cudaMemcpyDeviceToHost, ctx->stream));
-    if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, t->oid, (size_t)nk * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    SFM_CUDA(ctx, cudaMemcpyAsync(t->trk, t->ob, (size_t)nk * 16, cudaMemcpyDeviceToDevice, ctx->stream));
-    SFM_CUDA(ctx, cudaMemcpyAsync(t->ids, t->oid, (size_t)nk * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-    // the header's promise: results are in the caller's (possibly pinned) buffers when the call returns
-    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (prev_xy) SFM_CUDA(ctx, cudaMemcpyAsync(prev_xy, L.oa, (size_t)nk * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    if (cur_xy) SFM_CUDA(ctx, cudaMemcpyAsync(cur_xy, L.ob, (size_t)nk * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, L.oid, (size_t)nk * 4, cudaMemcpyDeviceToHost, ctx->stream));
   }
-  t->n = nk;
+  // the header's promise: results are in the caller's (possibly pinned) buffers when the call returns
+  SFM_TRY(lists_commit(ctx, L, (size_t)nk));
+  L.n[0] = nk;
   t->prev_frames = f;
   t->prev_index = frame;
   if (n_out) *n_out = nk;
-  // replenish (:374-389)
-  if (t->n < t->cfg.min_tracks)
-    SFM_TRY(replenish_row(ctx, t->cfg, f, frame, t->trk, t->ids, &t->n, &t->next_id, t->fresh, t->fresh_cap, t->ok, t->scal, t->cap));
-  return 0;
+  return lists_refill(ctx, L, t->cfg, f, frame, nullptr, "tracker");
 }
 
 int tracker_own_frames(sfmgpu_ctx* ctx, sfmgpu_tracker* t, int w, int h) {
@@ -1030,32 +1139,10 @@ extern "C" {
 int sfmgpu_tracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, sfmgpu_tracker** out) {
   SFM_ENTER(ctx);
   if (!ctx || !cfg || !out) return SFMGPU_E_ARG;
-  if (cfg->pyr_levels < 1 || cfg->pyr_levels > SFM_MAXL || cfg->max_tracks > (1 << 24) || cfg->min_tracks > (1 << 24))
-    return sfm_fail(ctx, SFMGPU_E_ARG, "tracker_create: bad configuration");
+  SFM_TRY(lkcfg_ok(ctx, cfg, "tracker_create"));
   sfmgpu_tracker* t = new sfmgpu_tracker();
   t->cfg = *cfg;
-  t->cap = track_rows(*cfg);
-  t->fresh_cap = 3 * (cfg->max_tracks < 1 ? 1 : cfg->max_tracks);
-  cudaError_t e = cudaSuccess;
-  auto al = [&](void** q, size_t bytes) {
-    if (e == cudaSuccess) e = cudaMalloc(q, bytes + 256);
-  };
-  const size_t n = (size_t)t->cap;
-  al((void**)&t->trk, n * 16);
-  al((void**)&t->p1, n * 16);
-  al((void**)&t->pb, n * 16);
-  al((void**)&t->oa, n * 16);
-  al((void**)&t->ob, n * 16);
-  al((void**)&t->ids, n * 4);
-  al((void**)&t->oid, n * 4);
-  al((void**)&t->nit, n * 4);
-  al((void**)&t->keep, n);
-  al((void**)&t->fresh, (size_t)t->fresh_cap * 16);
-  al((void**)&t->ok, (size_t)t->fresh_cap);
-  al((void**)&t->scal, 64);
-  al((void**)&t->tot, 64);
-  if (e == cudaSuccess) e = cudaMemsetAsync(t->tot, 0, 64, ctx->stream);
-  if (e == cudaSuccess) e = cudaMemsetAsync(t->scal, 0, 64, ctx->stream);
+  const cudaError_t e = lists_alloc(ctx, t->L, *cfg, 1);
   if (e != cudaSuccess) {
     sfmgpu_tracker_destroy(ctx, t);
     return sfm_fail(ctx, SFMGPU_E_CUDA, "tracker_create: CUDA allocation failed: %s", cudaGetErrorString(e));
@@ -1068,9 +1155,7 @@ void sfmgpu_tracker_destroy(sfmgpu_ctx* ctx, sfmgpu_tracker* t) {
   SFM_ENTER_VOID(ctx);
   if (!t) return;
   if (ctx) cudaStreamSynchronize(ctx->stream);
-  void* ptrs[] = {t->trk, t->p1, t->pb, t->oa, t->ob, t->ids, t->oid, t->nit, t->keep, t->fresh, t->ok, t->scal, t->tot};
-  for (void* q : ptrs)
-    if (q) cudaFree(q);
+  lists_free(t->L);
   if (t->own) sfmgpu_frames_destroy(ctx, t->own);
   delete t;
 }
@@ -1108,48 +1193,31 @@ int sfmgpu_tracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames
 int sfmgpu_tracker_tracks(sfmgpu_ctx* ctx, sfmgpu_tracker* t, double* xy, int32_t* ids, int cap, int* n_out) {
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
-  if (n_out) *n_out = t->n;
-  if (t->n > cap) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "tracker_tracks: %d tracks, room for %d", t->n, cap);
-  if (t->n > 0) {
-    if (xy) SFM_CUDA(ctx, cudaMemcpyAsync(xy, t->trk, (size_t)t->n * 16, cudaMemcpyDeviceToHost, ctx->stream));
-    if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, t->ids, (size_t)t->n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  }
-  return 0;
+  return lists_tracks(ctx, t->L, 0, xy, ids, cap, n_out, "tracker_tracks");
 }
 
 int sfmgpu_tracker_totals(sfmgpu_ctx* ctx, sfmgpu_tracker* t, long long* n_track_steps, long long* n_lk_iters) {
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
-  unsigned long long tt[4];
-  SFM_CUDA(ctx, cudaMemcpyAsync(tt, t->tot, sizeof tt, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (n_track_steps) *n_track_steps = t->track_steps;
-  if (n_lk_iters) *n_lk_iters = (long long)tt[2];
-  return 0;
+  return lists_totals(ctx, t->L, n_track_steps, n_lk_iters);
 }
 
 }  // extern "C"
 
 // ---- lock-step tracker over S independent sequences (BASELINE.json C5: several sequences per GPU) -------------------------------
-// The same KLTTracker semantics per sequence (:323-391), but ONE batched launch per stage and step for all of them: frame t of
-// every sequence arrives together, the S x max_tracks feature-tracks share a KLT launch (large enough for the lane-per-feature
-// kernels), survivors are compacted per sequence.  Results are identical to S separate sfmgpu_tracker objects.  Replenishment
-// (rare: a track list below min_tracks) is done sequence by sequence with the single-tracker code.
+// The same KLTTracker semantics per sequence (:323-391) on the same track-list core, but ONE batched launch per stage and step for
+// all of them: frame t of every sequence arrives together, the S x max_tracks feature-tracks share a KLT launch (large enough
+// for the lane-per-feature kernels), survivors are compacted per sequence.  Results are identical to S separate sfmgpu_tracker
+// objects.  Resets after a total track loss and replenishment (rare) run list by list.
 struct sfmgpu_multitracker {
   sfmgpu_lkcfg cfg;
-  int S = 0, w = 0, h = 0, cap = 0, fresh_cap = 0;
+  int w = 0, h = 0;
   sfmgpu_frames* frames = nullptr;  // 3*S slots: group g of sequence s lives in slot g*S + s (previous / current / prefetched)
   int parity = -1;                  // slot group of the previous frames, -1: nothing tracked yet
   bool prefetched = false;          // group (parity+1)%3 holds the next frames (uploaded + pyramids), ready at pf_done
   cudaEvent_t pf_done = nullptr;
-  std::vector<int> n, next_id;      // host copies
-  double2 *trk = nullptr, *p1 = nullptr, *pb = nullptr, *oa = nullptr, *ob = nullptr, *fresh = nullptr;
-  int *ids = nullptr, *oid = nullptr, *nit = nullptr, *dn = nullptr, *dnk = nullptr, *scal = nullptr;
+  TrackLists L;                     // list s: sequence s
   int* didx = nullptr;              // step_frames: the frame index of every sequence (device copy for the gather)
-  uint8_t *keep = nullptr, *ok = nullptr;
-  long long track_steps = 0;
-  unsigned long long* tot = nullptr;
   TwoViewState* tv = nullptr;       // find_E_ransac on every sequence's survivors inside the step (sfmgpu_multitracker_set_ransac)
   bool tv_fresh = false;            // the last step ran the stage: its results can be downloaded
   // packed input (sfmgpu_multitracker_step_packed): the tracker's own device buffer [decode flag | staged frame offsets [S+1] |
@@ -1162,83 +1230,24 @@ struct sfmgpu_multitracker {
   bool pf_packed = false;           // the prefetched frames were decoded: their flag is checked before they are stepped
 };
 
-namespace {
-
-// after a batched detection: row s of the track list = the first n[s] corners with ids next_id[s]..
-__global__ void multi_take_corners_kernel(const double2* __restrict__ fresh, int fresh_stride, const int* __restrict__ n,
-                                          const int* __restrict__ next_id, double2* __restrict__ trk, int* __restrict__ ids, int cap) {
-  const int s = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n[s] || i >= cap) return;
-  trk[(size_t)s * cap + i] = fresh[(size_t)s * fresh_stride + i];
-  ids[(size_t)s * cap + i] = next_id[s] + i;
-}
-
-int multi_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par) {
-  const int S = t->S, mc = t->cfg.max_tracks, cap_out = mc < 1 ? 1 : mc;
-  const int cand_cap = t->w * t->h;
-  const int md = t->cfg.min_distance < 0 ? -t->cfg.min_distance : t->cfg.min_distance;
-  SFM_TRY(sfm_reserve(ctx, ctx->cs_work, sfm_corner_work_bytes_md(t->w, t->h, S, cand_cap, md)));
-  SFM_TRY(sfm_corners_batch(ctx, t->frames, par * S, S, mc, t->cfg.quality, t->cfg.min_distance, cand_cap, ctx->cs_work.p,
-                            ctx->cs_work.cap, t->fresh, t->dn));
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->n.data(), t->dn, (size_t)S * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->dnk, t->next_id.data(), (size_t)S * 4, cudaMemcpyHostToDevice, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  for (int s = 0; s < S; s++)
-    if (t->n[s] < 0) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "multitracker: candidate capacity exceeded (sequence %d)", s);
-  SFM_LAUNCH(ctx, multi_take_corners_kernel, dim3(sfm_cdiv(cap_out, 256), S), 256, 0, t->fresh, cap_out, (const int*)t->dn,
-             (const int*)t->dnk, t->trk, t->ids, t->cap);
-  for (int s = 0; s < S; s++) t->next_id[s] += t->n[s];
-  t->parity = par;
-  return 0;
-}
-
-}  // namespace
-
 extern "C" {
 
 int sfmgpu_multitracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_sequences, int w, int h, sfmgpu_multitracker** out) {
   SFM_ENTER(ctx);
   if (!ctx || !cfg || !out) return SFMGPU_E_ARG;
-  if (n_sequences < 1 || n_sequences > 512 || w < 1 || h < 1 || cfg->pyr_levels < 1 || cfg->pyr_levels > SFM_MAXL ||
-      cfg->max_tracks > (1 << 24) || cfg->min_tracks > (1 << 24))
-    return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_create: bad configuration");
+  if (n_sequences < 1 || n_sequences > 512 || w < 1 || h < 1) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_create: bad configuration");
+  SFM_TRY(lkcfg_ok(ctx, cfg, "multitracker_create"));
   sfmgpu_multitracker* t = new sfmgpu_multitracker();
   t->cfg = *cfg;
-  t->S = n_sequences;
   t->w = w;
   t->h = h;
-  t->cap = track_rows(*cfg);  // as in sfmgpu_tracker
-  t->fresh_cap = 3 * (cfg->max_tracks < 1 ? 1 : cfg->max_tracks);
-  t->n.assign(n_sequences, 0);
-  t->next_id.assign(n_sequences, 0);
   int rc = sfmgpu_frames_create(ctx, w, h, 3 * n_sequences, cfg->pyr_levels, &t->frames);
   if (rc != 0) {
     delete t;
     return rc;
   }
-  cudaError_t e = cudaSuccess;
-  auto al = [&](void** q, size_t bytes) {
-    if (e == cudaSuccess) e = cudaMalloc(q, bytes + 256);
-  };
-  const size_t n = (size_t)t->cap * n_sequences;
-  al((void**)&t->trk, n * 16);
-  al((void**)&t->p1, n * 16);
-  al((void**)&t->pb, n * 16);
-  al((void**)&t->oa, n * 16);
-  al((void**)&t->ob, n * 16);
-  al((void**)&t->ids, n * 4);
-  al((void**)&t->oid, n * 4);
-  al((void**)&t->nit, n * 4);
-  al((void**)&t->keep, n);
-  al((void**)&t->fresh, (size_t)t->fresh_cap * 16 * n_sequences);
-  al((void**)&t->ok, (size_t)t->fresh_cap);
-  al((void**)&t->dn, (size_t)n_sequences * 4);
-  al((void**)&t->dnk, (size_t)n_sequences * 4);
-  al((void**)&t->didx, (size_t)n_sequences * 4);
-  al((void**)&t->scal, 64);
-  al((void**)&t->tot, 64);
-  if (e == cudaSuccess) e = cudaMemsetAsync(t->tot, 0, 64, ctx->stream);
-  if (e == cudaSuccess) e = cudaMemsetAsync(t->scal, 0, 64, ctx->stream);
+  cudaError_t e = lists_alloc(ctx, t->L, *cfg, n_sequences);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&t->didx, (size_t)n_sequences * 4 + 256);
   if (e != cudaSuccess) {
     sfmgpu_multitracker_destroy(ctx, t);
     return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker_create: CUDA allocation failed: %s", cudaGetErrorString(e));
@@ -1253,9 +1262,8 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   if (ctx) cudaStreamSynchronize(ctx->stream);
   if (t->pf_done) cudaEventSynchronize(t->pf_done);  // a prefetch still running on the copy stream
   sfm_two_view_free(ctx, &t->tv);
-  void* ptrs[] = {t->trk, t->p1, t->pb, t->oa, t->ob, t->ids, t->oid, t->nit, t->keep, t->fresh, t->ok, t->dn, t->dnk, t->didx, t->scal, t->tot};
-  for (void* q : ptrs)
-    if (q) cudaFree(q);
+  lists_free(t->L);
+  if (t->didx) cudaFree(t->didx);
   if (t->frames) sfmgpu_frames_destroy(ctx, t->frames);
   if (t->pk) cudaFree(t->pk);
   if (t->pk_bad) cudaFreeHost(t->pk_bad);
@@ -1273,7 +1281,7 @@ static int multi_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int after_gro
   SFM_TRY(pipe_streams(ctx));
   if (!t->pf_done && cudaEventCreateWithFlags(&t->pf_done, cudaEventDisableTiming) != cudaSuccess)
     return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker: cudaEventCreate failed");
-  const int S = t->S, g = (after_group + 1) % 3;
+  const int S = t->L.S, g = (after_group + 1) % 3;
   sfmgpu_frames* f = t->frames;
   SFM_CUDA(ctx, cudaMemcpy2DAsync(f->lvl[0] + (size_t)g * S * f->fstride[0], f->pitch[0], host_pix, f->w, f->w, (size_t)f->h * S,
                                   cudaMemcpyDefault, ctx->copy_stream));
@@ -1306,7 +1314,7 @@ static int multi_pk_plan(sfmgpu_ctx* ctx, const sfmgpu_multitracker* t, const ui
   std::vector<uint64_t> fo;
   p.fo.assign(1, 0);
   p.copies.clear();
-  for (int s = 0; s < t->S; s++) {
+  for (int s = 0; s < t->L.S; s++) {
     SFM_TRY(sfm_pk_check(ctx, t->frames, blobs[s], blob_bytes[s], blob_frame[s], 1, fo, who));
     const size_t bytes = fo[1] - fo[0];
     if (bytes > bound)
@@ -1325,7 +1333,7 @@ static int multi_pk_plan(sfmgpu_ctx* ctx, const sfmgpu_multitracker* t, const ui
 // Copy and decode planned records into slot group g on ctx->stream (the caller may scope it to the copy stream); the flag is
 // copied to t->pk_bad behind the decode.  The staging is refilled only after the decode that last read it, on any stream.
 static int multi_pk_decode(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g, const PkPlan& p) {
-  const int S = t->S;
+  const int S = t->L.S;
   const size_t o_fo = 16, o_stage = (o_fo + 8 * ((size_t)S + 1) + 15) & ~(size_t)15;
   // each piece on its own: a call after a failed allocation completes what is missing
   if (!t->pk) SFM_CUDA(ctx, cudaMalloc(&t->pk, o_stage + (size_t)S * sfm_pk_frame_bound(t->w, t->h)));
@@ -1351,7 +1359,7 @@ static int multi_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int af
   SFM_TRY(pipe_streams(ctx));
   if (!t->pf_done && cudaEventCreateWithFlags(&t->pf_done, cudaEventDisableTiming) != cudaSuccess)
     return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker: cudaEventCreate failed");
-  const int S = t->S, g = (after_group + 1) % 3;
+  const int S = t->L.S, g = (after_group + 1) % 3;
   {
     StageScope sc(ctx, ctx->copy_stream);
     SFM_TRY(multi_pk_decode(ctx, t, g, p));
@@ -1386,10 +1394,10 @@ int sfmgpu_multitracker_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   t->prefetched = false;
   t->pf_packed = false;
   t->tv_fresh = false;
-  t->n.assign(t->S, 0);
-  t->next_id.assign(t->S, 0);
-  t->track_steps = 0;
-  SFM_CUDA(ctx, cudaMemsetAsync(t->tot, 0, 64, ctx->stream));
+  t->L.n.assign(t->L.S, 0);
+  t->L.next_id.assign(t->L.S, 0);
+  t->L.track_steps = 0;
+  SFM_CUDA(ctx, cudaMemsetAsync(t->L.tot, 0, 64, ctx->stream));
   return 0;
 }
 
@@ -1412,7 +1420,7 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   if (!ctx || !t) return SFMGPU_E_ARG;
   if (!host_pix && !t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: no frames given and none prefetched");
   if (host_pix && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: frames given but others are prefetched");
-  const int S = t->S;
+  const int S = t->L.S;
   const int par = multi_next_group(t);
   if (!host_pix) SFM_TRY(multi_take_prefetch(ctx, t, "multitracker_step"));
   t->tv_fresh = false;
@@ -1448,7 +1456,7 @@ int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, con
   PkPlan cur, next;
   if (blob_frame) SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, blob_frame, cur, who));
   if (next_blob_frame) SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, next_blob_frame, next, who));
-  const int S = t->S;
+  const int S = t->L.S;
   const int par = multi_next_group(t);
   if (blob_frame) {  // decoded and checked before the step queues anything; the pyramids only for frames that decoded
     SFM_TRY(multi_pk_decode(ctx, t, par, cur));
@@ -1475,7 +1483,7 @@ int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfm
   if (f->w != g->w || f->h != g->h || f->levels != g->levels)
     return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: frames are %dx%d with %d levels, the tracker %dx%d with %d", f->w, f->h,
                     f->levels, g->w, g->h, g->levels);
-  const int S = t->S;
+  const int S = t->L.S;
   for (int s = 0; s < S; s++)
     if (frame_idx[s] < 0 || frame_idx[s] >= f->n)
       return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: sequence %d: frame %d outside [0,%d)", s, frame_idx[s], f->n);
@@ -1498,85 +1506,42 @@ int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfm
 
 // One step of every sequence on the frames in slot group `par` (uploaded, prefetched or gathered there).
 static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out) {
-  const int S = t->S, cap = t->cap;
+  TrackLists& L = t->L;
+  const int S = L.S;
   const bool stage = sfm_two_view_enabled(t->tv);
   if (n_out)
     for (int s = 0; s < S; s++) n_out[s] = 0;
   if (t->parity < 0) {  // first frames: reset every sequence (:341-344); find_E_ransac is not called (:1715)
-    SFM_TRY(multi_reset(ctx, t, par));
+    SFM_TRY(lists_reset(ctx, L, t->cfg, t->frames, par * S, 0, S, "multitracker"));
+    t->parity = par;
     if (stage) SFM_TRY(sfm_two_view_skip(ctx, t->tv, nullptr, S));
     t->tv_fresh = stage;
     return 0;
   }
-  std::vector<int> empties;  // sequences without tracks are reset on this frame instead of stepped (:341-344)
-  for (int s = 0; s < S; s++)
-    if (t->n[s] == 0) empties.push_back(s);
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->dn, t->n.data(), (size_t)S * 4, cudaMemcpyHostToDevice, ctx->stream));
-  KltLaunch k;
-  k.pv = t->frames->view();
-  k.p0 = t->trk;
-  k.counts = t->dn;
-  k.npairs = S;
-  k.cap = cap;
-  k.fa0 = t->parity * S;
-  k.fa_step = 1;
-  k.fb0 = par * S;
-  k.fb_step = 1;
-  k.radius = t->cfg.win_radius;
-  k.iters = t->cfg.iters;
-  k.fb_thresh = t->cfg.fb_thresh;
-  k.p1 = t->p1;
-  k.pb = t->pb;
-  k.nit = t->nit;
-  k.keep = t->keep;
-  SFM_TRY(sfm_klt_launch(ctx, k));
-  for (int s = 0; s < S; s++) t->track_steps += t->n[s];
-  // survivors per sequence in track order: (p0, p1, id) (:364-371); LK iterations into the totals
-  SFM_LAUNCH(ctx, compact_kernel, S, 1024, 0, t->trk, t->p1, t->keep, (const int*)t->ids, (const int*)t->dn, cap, t->oa, t->ob, t->oid,
-             t->dnk);
-  SFM_LAUNCH(ctx, totals_kernel, 64, 256, 0, (const int*)t->dn, (const int*)t->dnk, (const int*)t->nit, S, cap, t->tot);
+  std::vector<char> empty(S);  // sequences without tracks are reset on this frame instead of stepped (:341-344)
+  bool any_empty = false;
+  for (int s = 0; s < S; s++) {
+    empty[s] = L.n[s] == 0;
+    any_empty = any_empty || empty[s];
+  }
+  SFM_TRY(lists_track(ctx, L, t->cfg, t->frames, t->parity * S, par * S, KLT_BY_ROWS));
   if (stage) {  // find_E_ransac(K, prev_pts, cur_pts, ...) on every sequence's survivors (:1739), inside the step's one synchronisation
     StageTimer rt(ctx, 4);
-    SFM_TRY(sfm_two_view_stage(ctx, t->tv, t->oa, t->ob, t->dnk, cap, 0, S, nullptr));
+    SFM_TRY(sfm_two_view_stage(ctx, t->tv, L.oa, L.ob, L.dnk, L.rows, 0, S, nullptr));
     // sequences reset on this frame instead of stepped (dn == 0) return no step: SKIPPED whatever min_points says
-    if (!empties.empty()) SFM_TRY(sfm_two_view_skip(ctx, t->tv, t->dn, S));
+    if (any_empty) SFM_TRY(sfm_two_view_skip(ctx, t->tv, L.dn, S));
   }
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->n.data(), t->dnk, (size_t)S * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  const size_t rows = (size_t)S * cap;
-  if (prev_xy) SFM_CUDA(ctx, cudaMemcpyAsync(prev_xy, t->oa, rows * 16, cudaMemcpyDeviceToHost, ctx->stream));
-  if (cur_xy) SFM_CUDA(ctx, cudaMemcpyAsync(cur_xy, t->ob, rows * 16, cudaMemcpyDeviceToHost, ctx->stream));
-  if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, t->oid, rows * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->trk, t->ob, rows * 16, cudaMemcpyDeviceToDevice, ctx->stream));
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->ids, t->oid, rows * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  SFM_CUDA(ctx, cudaMemcpyAsync(L.n.data(), L.dnk, (size_t)S * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  const size_t rows = (size_t)S * L.rows;
+  if (prev_xy) SFM_CUDA(ctx, cudaMemcpyAsync(prev_xy, L.oa, rows * 16, cudaMemcpyDeviceToHost, ctx->stream));
+  if (cur_xy) SFM_CUDA(ctx, cudaMemcpyAsync(cur_xy, L.ob, rows * 16, cudaMemcpyDeviceToHost, ctx->stream));
+  if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, L.oid, rows * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  SFM_TRY(lists_commit(ctx, L, rows));
   t->parity = par;
   t->tv_fresh = stage;
   if (n_out)
-    for (int s = 0; s < S; s++) n_out[s] = t->n[s];
-  for (int s : empties) {
-    // reset(gray): tracks_ = shi_tomasi(gray, max_tracks, ...) with ids next_id_++; the step returns nothing for it
-    const int cand_cap = t->w * t->h;
-    const int md = t->cfg.min_distance < 0 ? -t->cfg.min_distance : t->cfg.min_distance;
-    SFM_TRY(sfm_reserve(ctx, ctx->cs_work, sfm_corner_work_bytes_md(t->w, t->h, 1, cand_cap, md)));
-    SFM_TRY(sfm_corners_batch(ctx, t->frames, par * S + s, 1, t->cfg.max_tracks, t->cfg.quality, t->cfg.min_distance, cand_cap,
-                              ctx->cs_work.p, ctx->cs_work.cap, t->trk + (size_t)s * cap, t->scal + 1));
-    int n = 0;
-    SFM_CUDA(ctx, cudaMemcpyAsync(&n, t->scal + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (n < 0) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "multitracker: candidate capacity exceeded (sequence %d)", s);
-    if (n > 0) SFM_LAUNCH(ctx, iota_ids_kernel, sfm_cdiv(n, 256), 256, 0, t->ids + (size_t)s * cap, (const int*)(t->scal + 1), t->next_id[s]);
-    t->n[s] = n;
-    t->next_id[s] += n;
-    if (n_out) n_out[s] = 0;
-  }
-  for (int s = 0; s < S; s++) {
-    bool was_empty = false;
-    for (int e : empties) was_empty = was_empty || e == s;
-    if (!was_empty && t->n[s] < t->cfg.min_tracks)
-      SFM_TRY(replenish_row(ctx, t->cfg, t->frames, par * S + s, t->trk + (size_t)s * cap, t->ids + (size_t)s * cap, &t->n[s],
-                            &t->next_id[s], t->fresh, t->fresh_cap, t->ok, t->scal, cap));
-  }
-  return 0;
+    for (int s = 0; s < S; s++) n_out[s] = L.n[s];
+  return lists_refill(ctx, L, t->cfg, t->frames, par * S, &empty, "multitracker");
 }
 
 extern "C" {
@@ -1585,7 +1550,7 @@ int sfmgpu_multitracker_set_ransac(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, cons
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
   t->tv_fresh = false;  // results of earlier steps are not those of this configuration
-  return sfm_two_view_configure(ctx, &t->tv, t->S, t->cap, K, rc, "multitracker_set_ransac");
+  return sfm_two_view_configure(ctx, &t->tv, t->L.S, t->L.rows, K, rc, "multitracker_set_ransac");
 }
 
 int sfmgpu_multitracker_ransac_download_all(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int32_t* status, int32_t* best_n, int32_t* inliers,
@@ -1594,7 +1559,7 @@ int sfmgpu_multitracker_ransac_download_all(sfmgpu_ctx* ctx, sfmgpu_multitracker
   if (!ctx || !t) return SFMGPU_E_ARG;
   if (!t->tv || !t->tv_fresh)
     return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_ransac_download_all: the last step ran without the RANSAC stage");
-  return sfm_two_view_download_all(ctx, t->tv, t->cap, t->S, status, best_n, inliers, R, tr, "multitracker_ransac");
+  return sfm_two_view_download_all(ctx, t->tv, t->L.rows, t->L.S, status, best_n, inliers, R, tr, "multitracker_ransac");
 }
 
 int sfmgpu_multitracker_ransac_early(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long long* sets_stopped) {
@@ -1606,27 +1571,14 @@ int sfmgpu_multitracker_ransac_early(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, lo
 int sfmgpu_multitracker_tracks(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int sequence, double* xy, int32_t* ids, int cap, int* n_out) {
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
-  if (sequence < 0 || sequence >= t->S) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_tracks: bad sequence index");
-  const int n = t->n[sequence];
-  if (n_out) *n_out = n;
-  if (n > cap) return sfm_fail(ctx, SFMGPU_E_CAPACITY, "multitracker_tracks: %d tracks, room for %d", n, cap);
-  if (n > 0) {
-    if (xy) SFM_CUDA(ctx, cudaMemcpyAsync(xy, t->trk + (size_t)sequence * t->cap, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
-    if (ids) SFM_CUDA(ctx, cudaMemcpyAsync(ids, t->ids + (size_t)sequence * t->cap, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  }
-  return 0;
+  if (sequence < 0 || sequence >= t->L.S) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_tracks: bad sequence index");
+  return lists_tracks(ctx, t->L, sequence, xy, ids, cap, n_out, "multitracker_tracks");
 }
 
 int sfmgpu_multitracker_totals(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long long* n_track_steps, long long* n_lk_iters) {
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
-  unsigned long long tt[4];
-  SFM_CUDA(ctx, cudaMemcpyAsync(tt, t->tot, sizeof tt, cudaMemcpyDeviceToHost, ctx->stream));
-  SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (n_track_steps) *n_track_steps = t->track_steps;
-  if (n_lk_iters) *n_lk_iters = (long long)tt[2];
-  return 0;
+  return lists_totals(ctx, t->L, n_track_steps, n_lk_iters);
 }
 
 }  // extern "C"
@@ -1678,7 +1630,7 @@ extern "C" int sfmgpu_pair_frontend_segments(sfmgpu_ctx* ctx, sfmgpu_frames* f, 
       return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: segment %d = frames [%d, %lld] outside [0,%d)", j, seg_first[j],
                       (long long)seg_first[j] + steps, f->n);
   if (cfg->pyr_levels != f->levels) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: cfg->pyr_levels != frames levels");
-  if (cfg->max_tracks > (1 << 24) || cfg->min_tracks > (1 << 24)) return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: bad configuration");
+  SFM_TRY(lkcfg_ok(ctx, cfg, "pair_frontend_segments"));
   const int rows = track_rows(*cfg);
   if (out->cap < rows)
     return sfm_fail(ctx, SFMGPU_E_ARG, "pair_frontend_segments: pairs rows hold %d points, a track list up to %d (max(max_tracks, min_tracks, 1) + 1)",
@@ -1687,8 +1639,7 @@ extern "C" int sfmgpu_pair_frontend_segments(sfmgpu_ctx* ctx, sfmgpu_frames* f, 
   // they bound the pair calls' chunks.  Chunks are balanced; the last one's spare slots repeat its last segment (unread).
   int S = 0;
   if (nseg > 0) {
-    const int md = cfg->min_distance < 0 ? -cfg->min_distance : cfg->min_distance;
-    const size_t per = sfm_corner_work_bytes_md(f->w, f->h, 1, f->w * f->h, md);
+    const size_t per = sfm_corner_work_bytes_md(f->w, f->h, 1, f->w * f->h, abs_min_distance(*cfg));
     long long most = (long long)(((size_t)16 << 30) / (per ? per : 1));
     if (most > 512) most = 512;  // sfmgpu_multitracker_create's limit
     if (most < 1) most = 1;
@@ -1696,7 +1647,7 @@ extern "C" int sfmgpu_pair_frontend_segments(sfmgpu_ctx* ctx, sfmgpu_frames* f, 
     S = (nseg + nchunk - 1) / nchunk;
   }
   sfmgpu_multitracker* mt = out->seg;
-  if (mt && S > 0 && (mt->S != S || mt->w != f->w || mt->h != f->h || !same_lkcfg(mt->cfg, *cfg))) {
+  if (mt && S > 0 && (mt->L.S != S || mt->w != f->w || mt->h != f->h || !same_lkcfg(mt->cfg, *cfg))) {
     sfmgpu_multitracker_destroy(ctx, mt);
     out->seg = mt = nullptr;
   }
@@ -1717,10 +1668,11 @@ extern "C" int sfmgpu_pair_frontend_segments(sfmgpu_ctx* ctx, sfmgpu_frames* f, 
       for (int s = 0; s < S; s++) idx[s] = seg_first[j0 + (s < cnt ? s : cnt - 1)] + k;
       SFM_TRY(sfmgpu_multitracker_step_frames(ctx, mt, f, idx.data(), nullptr, nullptr, nullptr, nullptr));
       if (k == 0) continue;
-      SFM_LAUNCH(ctx, segment_rows_kernel, dim3(sfm_cdiv(rows, 256), cnt), 256, 0, (const double2*)mt->oa, (const double2*)mt->ob,
-                 (const int*)mt->oid, (const int*)mt->dn, (const int*)mt->dnk, mt->cap, out->li, out->lj, out->ids, out->ncorn, out->nkept,
+      const TrackLists& L = mt->L;
+      SFM_LAUNCH(ctx, segment_rows_kernel, dim3(sfm_cdiv(rows, 256), cnt), 256, 0, (const double2*)L.oa, (const double2*)L.ob,
+                 (const int*)L.oid, (const int*)L.dn, (const int*)L.dnk, L.rows, out->li, out->lj, out->ids, out->ncorn, out->nkept,
                  out->cap, (long long)j0 * steps + (k - 1), steps);
-      SFM_LAUNCH(ctx, totals_kernel, 64, 256, 0, (const int*)mt->dn, (const int*)mt->dnk, (const int*)mt->nit, cnt, mt->cap, out->totals);
+      SFM_LAUNCH(ctx, totals_kernel, 64, 256, 0, (const int*)L.dn, (const int*)L.dnk, (const int*)L.nit, cnt, L.rows, out->totals);
     }
   }
   if (sfm_two_view_enabled(out->tv) && npairs > 0) {  // find_E_ransac(K, prev_pts, cur_pts, ...) on every step's survivors (:1739)
