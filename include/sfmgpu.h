@@ -164,9 +164,18 @@ int sfmgpu_select_set_mode(sfmgpu_ctx* ctx, int mode);
  * per point); n_iters (optional) = LK iterations executed. */
 int sfmgpu_klt_track(sfmgpu_ctx* ctx, sfmgpu_frames* f, int frame_a, int frame_b, const double* p0_xy, int n,
                      int win_radius, int iters, double* p1_xy, double* p0_back_xy, int32_t* n_iters);
+/* The same with image A = frame_a of fa and image B = frame_b of fb: two batches of any sizes, as the reference's
+ * track_one accepts any two pyramids with the same level count.  Each image is sampled against its own level sizes (a tap
+ * outside that image zeroes the sample, :183-198).  fa == fb is sfmgpu_klt_track.  Otherwise the warp-per-feature kernel
+ * runs whatever sfmgpu_klt_set_mode says.  Level counts that differ, a bad index or count, or a NULL pointer: SFMGPU_E_ARG. */
+int sfmgpu_klt_track_between(sfmgpu_ctx* ctx, sfmgpu_frames* fa, int frame_a, sfmgpu_frames* fb, int frame_b,
+                             const double* p0_xy, int n, int win_radius, int iters, double* p1_xy, double* p0_back_xy,
+                             int32_t* n_iters);
 /* Kernel selection for every KLT launch of this context (tests and profiling; results agree within the parity
  * budget either way): 0 = automatic (lane-per-feature kernel for batches of >= 6000 features with win_radius 5,
- * warp-per-feature otherwise), 1 = warp-per-feature only, 2 = lane-per-feature whenever win_radius is 5. */
+ * warp-per-feature otherwise), 1 = warp-per-feature only, 2 = lane-per-feature whenever win_radius is 5.  A launch
+ * between two frame batches (sfmgpu_klt_track_between, a tracker step across an image-size change) always runs the
+ * warp-per-feature kernel. */
 int sfmgpu_klt_set_mode(sfmgpu_ctx* ctx, int mode);
 
 /* ---- stateless two-view front end over a batch of pairs (:1836-1857) -------------------------------- */
@@ -352,9 +361,15 @@ int sfmgpu_tracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, sfmgpu_track
 void sfmgpu_tracker_destroy(sfmgpu_ctx* ctx, sfmgpu_tracker* t);
 /* reset(gray) :327-332 */
 int sfmgpu_tracker_reset(sfmgpu_ctx* ctx, sfmgpu_tracker* t, const uint8_t* host_pix, int w, int h);
-/* step(gray) :340-391.  Survivors (prev, cur, id) in track order; *n_out = 0 on the first frame. */
+/* step(gray) :340-391.  Survivors (prev, cur, id) in track order; *n_out = 0 on the first frame.  An image of another size
+ * than the previous one: SFMGPU_E_ARG for reset and step, unless sfmgpu_tracker_set_size_change is on. */
 int sfmgpu_tracker_step(sfmgpu_ctx* ctx, sfmgpu_tracker* t, const uint8_t* host_pix, int w, int h,
                         double* prev_xy, double* cur_xy, int32_t* ids, int cap, int* n_out);
+/* follow = 1: reset and step take any w x h, as the reference's KLTTracker does: a step at a new size tracks from the previous
+ * image at its own size to the new one (:345-346, the warp-per-feature KLT kernel between the two frame batches, see
+ * sfmgpu_klt_set_mode) and replenishes on the new image.  follow = 0 (default): a new size is SFMGPU_E_ARG.  Other values:
+ * SFMGPU_E_ARG.  The C++ drop-in's KLTTracker turns it on. */
+int sfmgpu_tracker_set_size_change(sfmgpu_ctx* ctx, sfmgpu_tracker* t, int follow);
 /* Same with the frame already resident (frame index into `f`, pyramid built): no H2D in the step. */
 int sfmgpu_tracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int frame, double* prev_xy,
                                double* cur_xy, int32_t* ids, int cap, int* n_out);

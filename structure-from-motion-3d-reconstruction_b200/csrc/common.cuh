@@ -214,7 +214,7 @@ static inline unsigned sfm_cdiv(long long a, long long b) { return (unsigned)((a
 // ---- internal cross-file entry points (device-pointer level) --------------------------------------------
 // klt.cu
 struct KltLaunch {
-  PyrView pv;
+  PyrView pv;            // image A: frame fa0 + k*fa_step of this batch
   const double2* p0;     // [npairs*cap] (or [n] when npairs == 1)
   const int* counts;     // per-pair valid count, or nullptr (all cap valid)
   int npairs, cap;
@@ -225,6 +225,10 @@ struct KltLaunch {
   double2* pb;           // backward result
   int* nit;              // optional
   uint8_t* keep;         // optional: !(fb >= fb_thresh)
+  // Image B: frame fb0 + k*fb_step of this batch.  Callers that track within one batch set it equal to pv.  A launch whose
+  // two views differ (two batches, of any sizes, with equal level counts) always runs the two-geometry warp-per-feature
+  // kernel; the lane kernels and the context's KLT mode only apply to one-batch launches.
+  PyrView pvb;
 };
 int sfm_klt_launch(sfmgpu_ctx* ctx, const KltLaunch& k);
 

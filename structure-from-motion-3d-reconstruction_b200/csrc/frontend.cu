@@ -267,6 +267,7 @@ static int stage_klt(sfmgpu_ctx* ctx, const ChunkArgs& c) {
   const size_t so = (size_t)c.pair_off * out->cap;
   KltLaunch k;
   k.pv = c.cf->view();
+  k.pvb = k.pv;
   k.p0 = out->xy0 + so;
   k.counts = out->ncorn + c.pair_off;
   k.npairs = c.npairs;
@@ -966,11 +967,14 @@ int lists_reset(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_
 // tracker by all S x rows entries with the live counts uploaded to dn.
 enum KltSizing { KLT_BY_LIVE, KLT_BY_ROWS };
 
-// One step of every list from frame fa0 + s to frame fb0 + s (:346-371): the survivors of list s in track order, (p0, p1, id),
-// go to row s of oa / ob / oid and their count to dnk[s]; the step's sums are added to tot.
-int lists_track(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int fa0, int fb0, KltSizing sizing) {
+// One step of every list from frame fa0 + s of fa to frame fb0 + s of fb (:346-371): the survivors of list s in track order,
+// (p0, p1, id), go to row s of oa / ob / oid and their count to dnk[s]; the step's sums are added to tot.  fa != fb (the single
+// tracker across an image-size change) runs the two-geometry KLT kernel.
+int lists_track(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* fa, sfmgpu_frames* fb, int fa0, int fb0,
+                KltSizing sizing) {
   KltLaunch k;
-  k.pv = f->view();
+  k.pv = fa->view();
+  k.pvb = fb->view();
   k.p0 = L.trk;
   if (sizing == KLT_BY_LIVE) {  // one list
     k.counts = nullptr;
@@ -1086,6 +1090,7 @@ struct sfmgpu_tracker {
   sfmgpu_frames* own = nullptr;     // 2-slot ping-pong used by the host-image entry points
   sfmgpu_frames* prev_frames = nullptr;
   int prev_index = -1;
+  bool size_change = false;         // host images of a new size: followed (sfmgpu_tracker_set_size_change) or refused
   TrackLists L;                     // S = 1
 };
 
@@ -1098,13 +1103,15 @@ int tracker_reset_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int f
   return 0;
 }
 
-int tracker_step_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int frame, double* prev_xy, double* cur_xy,
-                    int32_t* ids, int cap, int* n_out) {
+// Steps from the previous frame, which must live in fprev, to frame `frame` of f: fprev == f except across an image-size change
+// of the host-image entry points, where fprev is the tracker's old batch and f its new one.
+int tracker_step_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* fprev, sfmgpu_frames* f, int frame, double* prev_xy,
+                    double* cur_xy, int32_t* ids, int cap, int* n_out) {
   TrackLists& L = t->L;
   if (n_out) *n_out = 0;
   if (t->prev_index < 0 || L.n[0] == 0) return tracker_reset_on(ctx, t, f, frame);  // :341-344
-  if (t->prev_frames != f) return sfm_fail(ctx, SFMGPU_E_STATE, "tracker: previous frame lives in another frame batch");
-  SFM_TRY(lists_track(ctx, L, t->cfg, f, t->prev_index, frame, KLT_BY_LIVE));
+  if (t->prev_frames != fprev) return sfm_fail(ctx, SFMGPU_E_STATE, "tracker: previous frame lives in another frame batch");
+  SFM_TRY(lists_track(ctx, L, t->cfg, fprev, f, t->prev_index, frame, KLT_BY_LIVE));
   int nk = 0;
   SFM_CUDA(ctx, cudaMemcpyAsync(&nk, L.dnk, 4, cudaMemcpyDeviceToHost, ctx->stream));
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1124,12 +1131,32 @@ int tracker_step_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int fr
   return lists_refill(ctx, L, t->cfg, f, frame, nullptr, "tracker");
 }
 
-int tracker_own_frames(sfmgpu_ctx* ctx, sfmgpu_tracker* t, int w, int h) {
-  if (t->own && (t->own->w != w || t->own->h != h))
-    return sfm_fail(ctx, SFMGPU_E_ARG, "tracker: image size changed from %dx%d to %dx%d (not supported)", t->own->w, t->own->h, w,
-                    h);
+// A host image of the tracker's size goes to the slot of its 2-slot batch that does not hold the previous frame.
+int tracker_own_slot(sfmgpu_ctx* ctx, sfmgpu_tracker* t, const uint8_t* host_pix, int w, int h, int* slot) {
   if (!t->own) SFM_TRY(sfmgpu_frames_create(ctx, w, h, 2, t->cfg.pyr_levels, &t->own));
-  return 0;
+  *slot = (t->prev_frames == t->own && t->prev_index == 0) ? 1 : 0;
+  SFM_TRY(sfmgpu_frames_upload(ctx, t->own, *slot, 1, host_pix));
+  return sfmgpu_pyramid_build(ctx, t->own, *slot, 1);
+}
+
+// A host image of another size (:345-346 build the two pyramids at their own sizes): it goes to slot 0 of a new 2-slot batch,
+// the tracker resets or steps onto it (the step tracks from the old batch), and the new batch replaces the old one once it
+// holds the previous frame.  So no more than two batches are alive, and a call that fails before the step commits keeps the
+// tracker on its old batch.
+int tracker_resized(sfmgpu_ctx* ctx, sfmgpu_tracker* t, const uint8_t* host_pix, int w, int h, bool reset, double* prev_xy,
+                    double* cur_xy, int32_t* ids, int cap, int* n_out) {
+  if (!t->size_change)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "tracker: image size changed from %dx%d to %dx%d (sfmgpu_tracker_set_size_change not set)",
+                    t->own->w, t->own->h, w, h);
+  sfmgpu_frames* nb = nullptr;
+  SFM_TRY(sfmgpu_frames_create(ctx, w, h, 2, t->cfg.pyr_levels, &nb));
+  int r = sfmgpu_frames_upload(ctx, nb, 0, 1, host_pix);
+  if (r == 0) r = sfmgpu_pyramid_build(ctx, nb, 0, 1);
+  if (r == 0)
+    r = reset ? tracker_reset_on(ctx, t, nb, 0) : tracker_step_on(ctx, t, t->own, nb, 0, prev_xy, cur_xy, ids, cap, n_out);
+  if (t->prev_frames == nb) std::swap(t->own, nb);
+  sfmgpu_frames_destroy(ctx, nb);  // synchronises the context stream first
+  return r;
 }
 
 }  // namespace
@@ -1160,13 +1187,21 @@ void sfmgpu_tracker_destroy(sfmgpu_ctx* ctx, sfmgpu_tracker* t) {
   delete t;
 }
 
+int sfmgpu_tracker_set_size_change(sfmgpu_ctx* ctx, sfmgpu_tracker* t, int follow) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  if (follow != 0 && follow != 1) return sfm_fail(ctx, SFMGPU_E_ARG, "tracker_set_size_change: %d not in {0,1}", follow);
+  t->size_change = follow == 1;
+  return 0;
+}
+
 int sfmgpu_tracker_reset(sfmgpu_ctx* ctx, sfmgpu_tracker* t, const uint8_t* host_pix, int w, int h) {
   SFM_ENTER(ctx);
   if (!ctx || !t || !host_pix) return SFMGPU_E_ARG;
-  SFM_TRY(tracker_own_frames(ctx, t, w, h));
-  const int slot = (t->prev_frames == t->own && t->prev_index == 0) ? 1 : 0;
-  SFM_TRY(sfmgpu_frames_upload(ctx, t->own, slot, 1, host_pix));
-  SFM_TRY(sfmgpu_pyramid_build(ctx, t->own, slot, 1));
+  if (t->own && (t->own->w != w || t->own->h != h))
+    return tracker_resized(ctx, t, host_pix, w, h, true, nullptr, nullptr, nullptr, 0, nullptr);
+  int slot = 0;
+  SFM_TRY(tracker_own_slot(ctx, t, host_pix, w, h, &slot));
   return tracker_reset_on(ctx, t, t->own, slot);
 }
 
@@ -1174,11 +1209,11 @@ int sfmgpu_tracker_step(sfmgpu_ctx* ctx, sfmgpu_tracker* t, const uint8_t* host_
                         double* cur_xy, int32_t* ids, int cap, int* n_out) {
   SFM_ENTER(ctx);
   if (!ctx || !t || !host_pix) return SFMGPU_E_ARG;
-  SFM_TRY(tracker_own_frames(ctx, t, w, h));
-  const int slot = (t->prev_frames == t->own && t->prev_index == 0) ? 1 : 0;
-  SFM_TRY(sfmgpu_frames_upload(ctx, t->own, slot, 1, host_pix));
-  SFM_TRY(sfmgpu_pyramid_build(ctx, t->own, slot, 1));
-  return tracker_step_on(ctx, t, t->own, slot, prev_xy, cur_xy, ids, cap, n_out);
+  if (t->own && (t->own->w != w || t->own->h != h))
+    return tracker_resized(ctx, t, host_pix, w, h, false, prev_xy, cur_xy, ids, cap, n_out);
+  int slot = 0;
+  SFM_TRY(tracker_own_slot(ctx, t, host_pix, w, h, &slot));
+  return tracker_step_on(ctx, t, t->own, t->own, slot, prev_xy, cur_xy, ids, cap, n_out);
 }
 
 int sfmgpu_tracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* f, int frame, double* prev_xy,
@@ -1187,7 +1222,7 @@ int sfmgpu_tracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames
   if (!ctx || !t || !f) return SFMGPU_E_ARG;
   if (frame < 0 || frame >= f->n) return sfm_fail(ctx, SFMGPU_E_ARG, "tracker_step_frames: bad frame index");
   if (f->levels != t->cfg.pyr_levels) return sfm_fail(ctx, SFMGPU_E_ARG, "tracker_step_frames: pyramid levels differ from cfg");
-  return tracker_step_on(ctx, t, f, frame, prev_xy, cur_xy, ids, cap, n_out);
+  return tracker_step_on(ctx, t, f, f, frame, prev_xy, cur_xy, ids, cap, n_out);
 }
 
 int sfmgpu_tracker_tracks(sfmgpu_ctx* ctx, sfmgpu_tracker* t, double* xy, int32_t* ids, int cap, int* n_out) {
@@ -1524,7 +1559,7 @@ static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, doubl
     empty[s] = L.n[s] == 0;
     any_empty = any_empty || empty[s];
   }
-  SFM_TRY(lists_track(ctx, L, t->cfg, t->frames, t->parity * S, par * S, KLT_BY_ROWS));
+  SFM_TRY(lists_track(ctx, L, t->cfg, t->frames, t->frames, t->parity * S, par * S, KLT_BY_ROWS));
   if (stage) {  // find_E_ransac(K, prev_pts, cur_pts, ...) on every sequence's survivors (:1739), inside the step's one synchronisation
     StageTimer rt(ctx, 4);
     SFM_TRY(sfm_two_view_stage(ctx, t->tv, L.oa, L.ob, L.dnk, L.rows, 0, S, nullptr));

@@ -37,7 +37,7 @@ struct KltSmem {
   static constexpr int TW = ((2 * R + 17 + 3) / 4) * 4;        // cached tile row bytes, origin 4-aligned (28 for R = 5)
   static constexpr int WPR = TW / 4;
   double cfy[NC + 3];      // per grid row: fractional weight of the lower tap row
-  int cvy[NC + 3];         // per grid row: both tap rows inside the image
+  int cvy[NC + 3];         // per grid row: both tap rows inside the image (two geometries: bit 0 image A, bit 1 image B)
   uint32_t t0[TH * WPR];   // cached u8 tile of image A around the window (rows of TW bytes)
   uint32_t t1[TH * WPR];   // same for image B
 };
@@ -85,10 +85,12 @@ __device__ __forceinline__ void stage_tile(uint32_t* tile, const uint8_t* __rest
 }
 
 // The window walk of one LK iteration for this lane (see track_one).  INTERIOR: every tap is inside the image, so
-// the per-sample bounds logic (:188) is compiled out.
-template <int R, bool FIXED, bool INTERIOR>
+// the per-sample bounds logic (:188) is compiled out.  TWO: images A and B have their own bounds; vx / bit 1 of cvy test
+// B's, vx0 / bit 0 of cvy test A's.
+template <int R, bool FIXED, bool INTERIOR, bool TWO = false>
 __device__ __forceinline__ void walk_rows(const KltSmem<R>& sm, int NK, int nc, int rowbase, int col, int p0, int p1, bool pix_col,
-                                          bool vx, double fx, double& a00, double& a01, double& a11, double& b0, double& b1) {
+                                          bool vx, double fx, double& a00, double& a01, double& a11, double& b0, double& b1,
+                                          bool vx0 = false) {
   constexpr int TW = KltSmem<R>::TW;
   const uint8_t* q1 = reinterpret_cast<const uint8_t*>(sm.t1) + rowbase * TW + col;
   const uint8_t* q0 = reinterpret_cast<const uint8_t*>(sm.t0) + rowbase * TW + col;
@@ -105,7 +107,11 @@ __device__ __forceinline__ void walk_rows(const KltSmem<R>& sm, int NK, int nc, 
       const double fy = sm.cfy[j];
       double s1c = __fma_rn(fy, h1 - h1p, h1p);
       double s0c = __fma_rn(fy, h0 - h0p, h0p);
-      if (!INTERIOR) {
+      if (!INTERIOR && TWO) {
+        const int cy = sm.cvy[j];
+        s1c = (vx && (cy & 2)) ? s1c : 0.0;  // a sample of B is zeroed by B's bounds, a sample of A by A's
+        s0c = (vx0 && (cy & 1)) ? s0c : 0.0;
+      } else if (!INTERIOR) {
         const bool ok = vx && sm.cvy[j];
         s1c = ok ? s1c : 0.0;  // any out-of-range tap zeroes the whole sample (:188)
         s0c = ok ? s0c : 0.0;
@@ -147,9 +153,14 @@ __device__ __forceinline__ void walk_rows(const KltSmem<R>& sm, int NK, int nc, 
 // case where fl(x+i') rounds up to the next integer the reference's own floor moves by one and its fraction is
 // 0; f == 1 on the regular pair selects exactly the same tap (weights 0 and 1), so no special case is needed
 // for the value, only for the bounds test, which uses the reference's floor.
-template <int R, bool FIXED>
+//
+// TWO: image A (frame fa of pva) and image B (frame fb of pv) have their own level sizes, as the reference's
+// track(Pyr A, Pyr B) allows: each tile is staged from its own image and each sample is zeroed by its own image's
+// bounds (:188).  The step is zero whenever B has fewer than 2 columns or rows (no gradient); an A that small only
+// zeroes its own samples.  Without TWO, pva is pv.
+template <int R, bool FIXED, bool TWO = false>
 __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int radius_rt, int iters, double& px, double& py,
-                          int& n_it, int lane) {
+                          int& n_it, int lane, const PyrView& pva) {
   constexpr int TH = KltSmem<R>::TH, TW = KltSmem<R>::TW;
   const int radius = FIXED ? R : radius_rt;  // compile-time window for the default radius
   const int nc = 2 * radius + 3;
@@ -166,8 +177,11 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
 
   for (int l = pv.levels - 1; l >= 0; --l) {
     const int w = pv.w[l], h = pv.h[l], pitch = pv.pitch[l];
-    const uint8_t* I0 = pv.base[l] + (size_t)fa * pv.fstride[l];
+    const PyrView& va = TWO ? pva : pv;
+    const uint8_t* I0 = va.base[l] + (size_t)fa * va.fstride[l];
     const uint8_t* I1 = pv.base[l] + (size_t)fb * pv.fstride[l];
+    const int w0 = TWO ? pva.w[l] : w, h0 = TWO ? pva.h[l] : h;
+    const bool a_ok = !TWO || (w0 >= 2 && h0 >= 2);  // otherwise no sample of A is inside A: its tile is not staged
     const double scale = 1.0 / (double)(1 << l);
     const double plx = px * scale, ply = py * scale;
     double dlx = 0.0, dly = 0.0;
@@ -188,11 +202,12 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
           tx0 = (FX - radius - 1 - KLT_MARGIN) & ~3;
           ty0 = FY - radius - 1 - KLT_MARGIN;
           __syncwarp();
-          stage_tile<R>(sm.t0, I0, h, pitch, tx0, ty0, lane);
+          if (a_ok) stage_tile<R>(sm.t0, I0, h0, TWO ? pva.pitch[l] : pitch, tx0, ty0, lane);
           stage_tile<R>(sm.t1, I1, h, pitch, tx0, ty0, lane);
           have_tile = true;
         }
-        const bool interior = FX - radius - 1 >= 0 && FX + radius + 3 <= w - 1 && FY - radius - 1 >= 0 && FY + radius + 3 <= h - 1;
+        bool interior = FX - radius - 1 >= 0 && FX + radius + 3 <= w - 1 && FY - radius - 1 >= 0 && FY + radius + 3 <= h - 1;
+        if (TWO) interior = interior && FX + radius + 3 <= w0 - 1 && FY + radius + 3 <= h0 - 1;
         // per-row weight table (lanes 0..nc-1), per-column weights in registers
         if (lane < nc) {
           const double reg = fyy + off_i;            // off_i == lane - r - 1 here
@@ -200,7 +215,10 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
           sm.cfy[lane] = f;
           if (!interior) {
             const double tf = f == 1.0 ? reg + 1.0 : reg;
-            sm.cvy[lane] = (tf >= 0.0 && tf <= (double)(h - 2)) ? 1 : 0;
+            if (TWO)
+              sm.cvy[lane] = ((tf >= 0.0 && tf <= (double)(h0 - 2)) ? 1 : 0) | ((tf >= 0.0 && tf <= (double)(h - 2)) ? 2 : 0);
+            else
+              sm.cvy[lane] = (tf >= 0.0 && tf <= (double)(h - 2)) ? 1 : 0;
           }
         }
         const double regx = fxx + off_i;
@@ -215,7 +233,12 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
         } else {
           const double tfx = fx == 1.0 ? regx + 1.0 : regx;
           const bool vx = col_active && tfx >= 0.0 && tfx <= (double)(w - 2);
-          walk_rows<R, FIXED, false>(sm, NK, nc, rowbase, col, p0, p1, pix_col, vx, fx, a00, a01, a11, b0, b1);
+          if (TWO) {
+            const bool vx0 = col_active && tfx >= 0.0 && tfx <= (double)(w0 - 2);
+            walk_rows<R, FIXED, false, true>(sm, NK, nc, rowbase, col, p0, p1, pix_col, vx, fx, a00, a01, a11, b0, b1, vx0);
+          } else {
+            walk_rows<R, FIXED, false>(sm, NK, nc, rowbase, col, p0, p1, pix_col, vx, fx, a00, a01, a11, b0, b1);
+          }
         }
         reduce5(a00, a01, a11, b0, b1, lane);
         // a** = 4*A, b* = 2*b of :444-448 (exact power-of-two scalings): det' = 16 det, step = 2 * A'^-1 b'
@@ -239,7 +262,8 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
 
 // list == nullptr: one warp per slot of the launch (grid covers them all).  list != nullptr: the warps of a
 // fixed-size grid walk the deferred-feature list written by klt_lane_kernel (count read from device memory).
-template <int R, bool FIXED>
+// TWO: image A from k.pv, image B from k.pvb (two batches, any sizes); the backward track swaps the two views.
+template <int R, bool FIXED, bool TWO>
 __global__ void __launch_bounds__(128, (R <= 5 ? 6 : 3)) klt_kernel(KltLaunch k, const int* __restrict__ list,
                                                                     const int* __restrict__ list_count) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -255,10 +279,11 @@ __global__ void __launch_bounds__(128, (R <= 5 ? 6 : 3)) klt_kernel(KltLaunch k,
     int n_it = 0;
     double x = p0.x, y = p0.y;
     __syncwarp();
-    track_one<R, FIXED>(sm, k.pv, fa, fb, k.radius, k.iters, x, y, n_it, lane);
+    track_one<R, FIXED, TWO>(sm, TWO ? k.pvb : k.pv, fa, fb, k.radius, k.iters, x, y, n_it, lane, k.pv);
     const double x1 = x, y1 = y;
     __syncwarp();
-    if (k.pb) track_one<R, FIXED>(sm, k.pv, fb, fa, k.radius, k.iters, x, y, n_it, lane);  // pb == null: forward only
+    if (k.pb)  // pb == null: forward only
+      track_one<R, FIXED, TWO>(sm, k.pv, fb, fa, k.radius, k.iters, x, y, n_it, lane, TWO ? k.pvb : k.pv);
     if (lane == 0) {
       k.p1[g] = make_double2(x1, y1);
       if (k.pb) k.pb[g] = make_double2(x, y);
@@ -271,12 +296,15 @@ __global__ void __launch_bounds__(128, (R <= 5 ? 6 : 3)) klt_kernel(KltLaunch k,
   }
 }
 
-template <int R, bool FIXED>
+template <int R, bool FIXED, bool TWO = false>
 int launch_r(sfmgpu_ctx* ctx, const KltLaunch& k, const int* list, const int* list_count) {
   const int warps_per_block = 4;
-  const size_t smem = sizeof(KltSmem<R>) * warps_per_block;
+  // Without FIXED, the last row group of a window of radius 1..3 walks up to two tap rows past the rows its pixels need
+  // (G * chunk exceeds 2r + 2), which can lie past the tile; those samples are never accumulated, and the pad keeps the
+  // last warp's reads inside the block's shared memory.
+  const size_t smem = sizeof(KltSmem<R>) * warps_per_block + (FIXED ? 0 : 2 * KltSmem<R>::TW);
   static const int cfg_id = sfm_next_cfg_id();  // one per template instantiation
-  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_kernel<R, FIXED>), smem);
+  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_kernel<R, FIXED, TWO>), smem);
   const long long total = (long long)k.npairs * k.cap;
   if (total == 0) return 0;
   unsigned grid = sfm_cdiv(total, warps_per_block);
@@ -284,7 +312,7 @@ int launch_r(sfmgpu_ctx* ctx, const KltLaunch& k, const int* list, const int* li
     const unsigned cap = (unsigned)ctx->n_sm * 24;  // deferred features are a few % of the batch: a resident grid walks the list
     grid = grid < cap ? grid : cap;
   }
-  SFM_LAUNCH(ctx, (klt_kernel<R, FIXED>), grid, warps_per_block * 32, smem, k, list, list_count);
+  SFM_LAUNCH(ctx, (klt_kernel<R, FIXED, TWO>), grid, warps_per_block * 32, smem, k, list, list_count);
   return 0;
 }
 
@@ -299,10 +327,25 @@ int sfm_klt_lane_masked_launch(sfmgpu_ctx* ctx, const KltLaunch& k, const int* i
 // features to fill 148 SMs); smaller ones (a single tracker step) keep one warp per feature.
 static const long long KLT_LANE_MIN = 6000;
 
+static bool same_view(const PyrView& a, const PyrView& b) {
+  if (a.levels != b.levels) return false;
+  for (int l = 0; l < a.levels; l++)
+    if (a.base[l] != b.base[l] || a.w[l] != b.w[l] || a.h[l] != b.h[l] || a.pitch[l] != b.pitch[l] || a.fstride[l] != b.fstride[l])
+      return false;
+  return true;
+}
+
 int sfm_klt_launch(sfmgpu_ctx* ctx, const KltLaunch& k) {
   if (k.radius < 1 || k.radius > 10)
     return sfm_fail(ctx, SFMGPU_E_ARG, "klt: win_radius %d outside the supported range [1,10]", k.radius);
   if (k.iters < 0) return sfm_fail(ctx, SFMGPU_E_ARG, "klt: negative iteration count");
+  if (!same_view(k.pv, k.pvb)) {  // two batches: the lane kernels assume one geometry, so the mode does not apply
+    if (k.pv.levels != k.pvb.levels) return sfm_fail(ctx, SFMGPU_E_ARG, "klt: pyramid level counts differ (%d, %d)", k.pv.levels, k.pvb.levels);
+    if (k.radius == 5) return launch_r<5, true, true>(ctx, k, nullptr, nullptr);
+    if (k.radius < 5) return launch_r<5, false, true>(ctx, k, nullptr, nullptr);
+    if (k.radius == 10) return launch_r<10, true, true>(ctx, k, nullptr, nullptr);
+    return launch_r<10, false, true>(ctx, k, nullptr, nullptr);
+  }
   const long long total = (long long)k.npairs * k.cap;
   const int* list = nullptr;
   const int* list_count = nullptr;
@@ -339,14 +382,9 @@ extern "C" int sfmgpu_klt_set_mode(sfmgpu_ctx* ctx, int mode) {
   return 0;
 }
 
-extern "C" int sfmgpu_klt_track(sfmgpu_ctx* ctx, sfmgpu_frames* f, int frame_a, int frame_b, const double* p0_xy, int n,
-                                int win_radius, int iters, double* p1_xy, double* p0_back_xy, int32_t* n_iters) {
-  SFM_ENTER(ctx);
-  if (!ctx || !f) return SFMGPU_E_ARG;
-  if (frame_a < 0 || frame_a >= f->n || frame_b < 0 || frame_b >= f->n || n < 0)
-    return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track: bad frame index or count");
-  if (n == 0) return 0;
-  if (!p0_xy || !p1_xy) return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track: null pointer");
+// Host points in, host results out: frame_a of view a -> frame_b of view b and back.
+static int klt_track_host(sfmgpu_ctx* ctx, const PyrView& va, int frame_a, const PyrView& vb, int frame_b, const double* p0_xy, int n,
+                          int win_radius, int iters, double* p1_xy, double* p0_back_xy, int32_t* n_iters) {
   const size_t pb = (size_t)n * sizeof(double2);
   SFM_TRY(sfm_reserve(ctx, ctx->klt_in, pb));
   SFM_TRY(sfm_reserve(ctx, ctx->klt_p1, pb));
@@ -354,7 +392,8 @@ extern "C" int sfmgpu_klt_track(sfmgpu_ctx* ctx, sfmgpu_frames* f, int frame_a, 
   SFM_TRY(sfm_reserve(ctx, ctx->klt_nit, (size_t)n * sizeof(int)));
   SFM_CUDA(ctx, cudaMemcpyAsync(ctx->klt_in.p, p0_xy, pb, cudaMemcpyHostToDevice, ctx->stream));
   KltLaunch k;
-  k.pv = f->view();
+  k.pv = va;
+  k.pvb = vb;
   k.p0 = (const double2*)ctx->klt_in.p;
   k.counts = nullptr;
   k.npairs = 1;
@@ -377,4 +416,31 @@ extern "C" int sfmgpu_klt_track(sfmgpu_ctx* ctx, sfmgpu_frames* f, int frame_a, 
     SFM_CUDA(ctx, cudaMemcpyAsync(n_iters, ctx->klt_nit.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
+}
+
+extern "C" int sfmgpu_klt_track(sfmgpu_ctx* ctx, sfmgpu_frames* f, int frame_a, int frame_b, const double* p0_xy, int n,
+                                int win_radius, int iters, double* p1_xy, double* p0_back_xy, int32_t* n_iters) {
+  SFM_ENTER(ctx);
+  if (!ctx || !f) return SFMGPU_E_ARG;
+  if (frame_a < 0 || frame_a >= f->n || frame_b < 0 || frame_b >= f->n || n < 0)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track: bad frame index or count");
+  if (n == 0) return 0;
+  if (!p0_xy || !p1_xy) return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track: null pointer");
+  const PyrView v = f->view();
+  return klt_track_host(ctx, v, frame_a, v, frame_b, p0_xy, n, win_radius, iters, p1_xy, p0_back_xy, n_iters);
+}
+
+extern "C" int sfmgpu_klt_track_between(sfmgpu_ctx* ctx, sfmgpu_frames* fa, int frame_a, sfmgpu_frames* fb, int frame_b,
+                                        const double* p0_xy, int n, int win_radius, int iters, double* p1_xy, double* p0_back_xy,
+                                        int32_t* n_iters) {
+  SFM_ENTER(ctx);
+  if (!ctx || !fa || !fb) return SFMGPU_E_ARG;
+  if (fa == fb) return sfmgpu_klt_track(ctx, fa, frame_a, frame_b, p0_xy, n, win_radius, iters, p1_xy, p0_back_xy, n_iters);
+  if (frame_a < 0 || frame_a >= fa->n || frame_b < 0 || frame_b >= fb->n || n < 0)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track_between: bad frame index or count");
+  if (fa->levels != fb->levels)
+    return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track_between: pyramid level counts differ (%d, %d)", fa->levels, fb->levels);
+  if (n == 0) return 0;
+  if (!p0_xy || !p1_xy) return sfm_fail(ctx, SFMGPU_E_ARG, "klt_track_between: null pointer");
+  return klt_track_host(ctx, fa->view(), frame_a, fb->view(), frame_b, p0_xy, n, win_radius, iters, p1_xy, p0_back_xy, n_iters);
 }

@@ -114,7 +114,7 @@ inline sfmgpu_ctx* context() {
 }
 
 // Device twin of one Pyramid: a slot in a small pool of equally sized frames, so that two pyramids of the same
-// size (the only case the reference ever tracks between) live in one batch.
+// size usually live in one batch (the one-batch KLT kernels apply); pyramids of two pools are tracked between the batches.
 struct Pool {
   sfmgpu_frames* frames = nullptr;
   int w = 0, h = 0, levels = 0;
@@ -295,12 +295,13 @@ struct Track {
   Vec2 p;
 };
 
-// Batched form of the loop at :1845-1849: forward a->b and backward b->a for all points in one launch.
+// Batched form of the loop at :1845-1849: forward a->b and backward b->a for all points in one launch.  Pyramids of
+// different pools (different sizes, or more live pyramids of one size than a pool holds) are tracked between their two batches,
+// as the reference tracks between any two pyramids with the same level count.
 static void track_pairs(const Pyramid& a, const Pyramid& b, const std::vector<Vec2>& p0, int win_radius, int iters,
                         std::vector<Vec2>& p1, std::vector<Vec2>* p0_back) {
   using namespace sfmgpu_shim;
-  if (!a.dev || !b.dev || a.dev->pool != b.dev->pool)
-    throw std::runtime_error("sfmgpu: track: pyramids must come from build_pyr and have the same size / levels");
+  if (!a.dev || !b.dev) throw std::runtime_error("sfmgpu: track: pyramids must come from build_pyr");
   sfmgpu_ctx* ctx = context();
   const int n = (int)p0.size();
   p1.resize(p0.size());
@@ -308,9 +309,9 @@ static void track_pairs(const Pyramid& a, const Pyramid& b, const std::vector<Ve
   if (n == 0) return;
   static_assert(sizeof(Vec2) == 2 * sizeof(double), "Vec2 must be two packed doubles");
   check(ctx,
-        sfmgpu_klt_track(ctx, a.dev->pool->frames, a.dev->slot, b.dev->slot, reinterpret_cast<const double*>(p0.data()), n,
-                         win_radius, iters, reinterpret_cast<double*>(p1.data()),
-                         p0_back ? reinterpret_cast<double*>(p0_back->data()) : nullptr, nullptr),
+        sfmgpu_klt_track_between(ctx, a.dev->pool->frames, a.dev->slot, b.dev->pool->frames, b.dev->slot,
+                                 reinterpret_cast<const double*>(p0.data()), n, win_radius, iters, reinterpret_cast<double*>(p1.data()),
+                                 p0_back ? reinterpret_cast<double*>(p0_back->data()) : nullptr, nullptr),
         "klt_track");
 }
 
@@ -329,6 +330,8 @@ class KLTTracker {
     sfmgpu_tracker* t = nullptr;
     sfmgpu_shim::check(sfmgpu_shim::context(), sfmgpu_tracker_create(sfmgpu_shim::context(), &c, &t), "tracker_create");
     trk_ = std::shared_ptr<sfmgpu_tracker>(t, [](sfmgpu_tracker* p) { sfmgpu_tracker_destroy(sfmgpu_shim::context(), p); });
+    // the reference's step() takes an image of any size and tracks from the previous one at its own size (:345-346)
+    sfmgpu_shim::check(sfmgpu_shim::context(), sfmgpu_tracker_set_size_change(sfmgpu_shim::context(), t, 1), "tracker_set_size_change");
     cap_ = sfmgpu_shim::track_rows(cfg.max_tracks, cfg.min_tracks);
   }
   // The device state is owned, not shared: a copy would alias one tracker (stepping the copy would advance the

@@ -27,9 +27,9 @@ SYMBOLS = [
     "sfmgpu_host_free", "sfmgpu_frames_create", "sfmgpu_frames_destroy", "sfmgpu_frames_upload",
     "sfmgpu_frames_upload_device", "sfmgpu_frames_synth", "sfmgpu_pyramid_build", "sfmgpu_frames_level_size",
     "sfmgpu_frames_download", "sfmgpu_corner_candidates", "sfmgpu_corners", "sfmgpu_sort_perm_desc",
-    "sfmgpu_klt_track", "sfmgpu_klt_set_mode", "sfmgpu_select_set_mode", "sfmgpu_pairs_create", "sfmgpu_pairs_destroy", "sfmgpu_pair_frontend", "sfmgpu_pipeline_set", "sfmgpu_pair_frontend_host", "sfmgpu_pairs_totals",
+    "sfmgpu_klt_track", "sfmgpu_klt_track_between", "sfmgpu_klt_set_mode", "sfmgpu_select_set_mode", "sfmgpu_pairs_create", "sfmgpu_pairs_destroy", "sfmgpu_pair_frontend", "sfmgpu_pipeline_set", "sfmgpu_pair_frontend_host", "sfmgpu_pairs_totals",
     "sfmgpu_pairs_download", "sfmgpu_pairs_download_all", "sfmgpu_pairs_device_ptrs", "sfmgpu_tracker_create", "sfmgpu_tracker_destroy", "sfmgpu_tracker_reset",
-    "sfmgpu_tracker_step", "sfmgpu_tracker_step_frames", "sfmgpu_tracker_tracks", "sfmgpu_tracker_totals",
+    "sfmgpu_tracker_step", "sfmgpu_tracker_set_size_change", "sfmgpu_tracker_step_frames", "sfmgpu_tracker_tracks", "sfmgpu_tracker_totals",
     "sfmgpu_multitracker_create", "sfmgpu_multitracker_destroy", "sfmgpu_multitracker_step", "sfmgpu_multitracker_tracks",
     "sfmgpu_multitracker_prefetch", "sfmgpu_multitracker_step_pipelined",
     "sfmgpu_multitracker_totals",
@@ -115,6 +115,7 @@ def load_library():
         "sfmgpu_corners": (_i, [_vp, _vp, _i, _i, _d, _i, _f64p, C.POINTER(_i)]),
         "sfmgpu_sort_perm_desc": (_i, [_vp, _f64p, _i, _i32p]),
         "sfmgpu_klt_track": (_i, [_vp, _vp, _i, _i, _f64p, _i, _i, _i, _f64p, _f64p, _vp]),
+        "sfmgpu_klt_track_between": (_i, [_vp, _vp, _i, _vp, _i, _f64p, _i, _i, _i, _f64p, _f64p, _vp]),
         "sfmgpu_klt_set_mode": (_i, [_vp, _i]),
         "sfmgpu_select_set_mode": (_i, [_vp, _i]),
         "sfmgpu_pairs_create": (_i, [_vp, _i, _i, C.POINTER(_vp)]),
@@ -130,6 +131,7 @@ def load_library():
         "sfmgpu_tracker_destroy": (None, [_vp, _vp]),
         "sfmgpu_tracker_reset": (_i, [_vp, _vp, _u8p, _i, _i]),
         "sfmgpu_tracker_step": (_i, [_vp, _vp, _u8p, _i, _i, _vp, _vp, _vp, _i, C.POINTER(_i)]),
+        "sfmgpu_tracker_set_size_change": (_i, [_vp, _vp, _i]),
         "sfmgpu_tracker_step_frames": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _i, C.POINTER(_i)]),
         "sfmgpu_tracker_tracks": (_i, [_vp, _vp, _f64p, _i32p, _i, C.POINTER(_i)]),
         "sfmgpu_tracker_totals": (_i, [_vp, _vp, C.POINTER(_ll), C.POINTER(_ll)]),
@@ -531,6 +533,16 @@ class Frames:
                                                    radius, iters, p1, pb, _ptr(nit)))
         return (p1[:n], pb[:n], nit[:n]) if count else (p1[:n], pb[:n])
 
+    def klt_track_between(self, frame_a, other, frame_b, p0, radius=5, iters=10, count=False):
+        """klt_track from frame_a of this batch to frame_b of `other`, a batch of any size with the same level count."""
+        p0 = np.ascontiguousarray(p0, np.float64).reshape(-1, 2)
+        n = len(p0)
+        p1, pb = np.zeros((max(n, 1), 2)), np.zeros((max(n, 1), 2))
+        nit = np.zeros(max(n, 1), np.int32)
+        self.ctx._ck(self.ctx.lib.sfmgpu_klt_track_between(self.ctx.h, self.h_, frame_a, other.h_, frame_b,
+                                                           p0 if n else np.zeros((1, 2)), n, radius, iters, p1, pb, _ptr(nit)))
+        return (p1[:n], pb[:n], nit[:n]) if count else (p1[:n], pb[:n])
+
 
 class Pairs:
     """sfmgpu_pairs: device-resident results of a batch of frame pairs."""
@@ -920,6 +932,10 @@ class Tracker:
             self.close()
         except Exception:
             pass
+
+    def set_size_change(self, follow=True):
+        """follow=True: reset / step take images of any size, as the reference's KLTTracker does (default: refused)."""
+        self.ctx._ck(self.ctx.lib.sfmgpu_tracker_set_size_change(self.ctx.h, self.h_, 1 if follow else 0))
 
     def reset(self, img):
         img = np.ascontiguousarray(img, np.uint8)
