@@ -382,8 +382,19 @@ int sfmgpu_tracker_totals(sfmgpu_ctx* ctx, sfmgpu_tracker* t, long long* n_track
 /* Per sequence exactly KLTTracker::step (:340-391); one batched launch per stage for all sequences.  All images are
  * w x h.  The first step resets every sequence (n_out = 0 everywhere). */
 int sfmgpu_multitracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_sequences, int w, int h, sfmgpu_multitracker** out);
+/* Sequences of different image sizes (several cameras) in one lock step: sequence s has images of w[s] x h[s].  n_sequences in
+ * [1, 512] and every size in [1, 32767], else SFMGPU_E_ARG (also for NULL w or h).  With all sizes equal this is
+ * sfmgpu_multitracker_create and every entry point behaves exactly as on such a tracker.  Otherwise the tracker is "mixed": the
+ * sequences of one size share a frame batch, uploads and pyramids run per size, and the KLT stage is still one chain of launches
+ * for all S sequences (per-sequence geometry), so sequence s gives, byte for byte, what a one-sequence tracker of its size gives
+ * under the same kernel family (sfmgpu_klt_set_mode).  Every output keeps its [S][ROWS] layout in sequence order.  Not built yet
+ * for mixed trackers: packed and resident input - sfmgpu_multitracker_step_frames, _prefetch_packed and _step_packed return
+ * SFMGPU_E_ARG before any work is queued. */
+int sfmgpu_multitracker_create_sized(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_sequences, const int32_t* w, const int32_t* h,
+                                     sfmgpu_multitracker** out);
 void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t);
-/* host_pix: [n_sequences][h][w], the next frame of every sequence.  With ROWS = max(max_tracks, min_tracks, 1) + 1 (the
+/* host_pix: the next frame of every sequence, back to back in sequence order, frame s w[s] * h[s] bytes with row stride w[s]
+ * ([n_sequences][h][w] when all sizes are equal).  With ROWS = max(max_tracks, min_tracks, 1) + 1 (the
  * longest a track list can get: replenish appends before it tests the cap, :386-387): prev_xy / cur_xy are
  * [n_sequences][ROWS][2], ids [n_sequences][ROWS], n_out [n_sequences] survivors per sequence (any output may be NULL). */
 int sfmgpu_multitracker_step(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* host_pix, double* prev_xy, double* cur_xy,
@@ -432,6 +443,11 @@ int sfmgpu_multitracker_totals(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, long lon
  * the context) and runs before the step's one synchronisation.  A sequence that the step resets instead of tracking (the
  * first step, the first after sfmgpu_multitracker_reset, a sequence without tracks) is SFMGPU_TV_SKIPPED. */
 int sfmgpu_multitracker_set_ransac(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const double* K, const sfmgpu_ransac_cfg* rc);
+/* Same with one camera per sequence: find_E_ransac(K_s, prev_pts, cur_pts, ...) for sequence s, K [n_sequences][9] row-major
+ * (any tracker, mixed or not).  Same stage, results and layout; with S copies of one K the results equal set_ransac(K) byte for
+ * byte.  A singular K_s is SFMGPU_E_ARG naming s, NULL K SFMGPU_E_ARG; a refused call leaves the previous configuration and the
+ * last step's results in force.  rc == NULL: off. */
+int sfmgpu_multitracker_set_ransac_cameras(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const double* K, const sfmgpu_ransac_cfg* rc);
 /* Results of the last step: status / best_n [S], inliers [S][ROWS] (indices into that step's survivor list, ascending),
  * R [S][9], t [S][3] (valid for SFMGPU_TV_OK); any may be NULL.  SFMGPU_E_STATE when the last step ran without the stage
  * (never enabled, switched off, or no step since set_ransac / reset). */

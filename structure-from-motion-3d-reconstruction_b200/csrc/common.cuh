@@ -119,6 +119,9 @@ void sfm_two_view_free(sfmgpu_ctx* ctx, TwoViewState** tv);
 bool sfm_two_view_enabled(const TwoViewState* tv);
 int sfm_two_view_configure(sfmgpu_ctx* ctx, TwoViewState** tv, int max_sets, int cap, const double* K, const sfmgpu_ransac_cfg* rc,
                            const char* who);
+// Same with one camera per set: K [max_sets][9], set s normalised with the inverse of K + 9 s.
+int sfm_two_view_configure_sets(sfmgpu_ctx* ctx, TwoViewState** tv, int max_sets, int cap, const double* K, const sfmgpu_ransac_cfg* rc,
+                                const char* who);
 int sfm_two_view_stage(sfmgpu_ctx* ctx, TwoViewState* tv, const double2* li, const double2* lj, const int* nkept, int cap, int set_off,
                        int nsets, const double* E_host);
 int sfm_two_view_skip(sfmgpu_ctx* ctx, TwoViewState* tv, const int* n_in, int nsets);
@@ -213,6 +216,16 @@ static inline unsigned sfm_cdiv(long long a, long long b) { return (unsigned)((a
 
 // ---- internal cross-file entry points (device-pointer level) --------------------------------------------
 // klt.cu
+// Geometry of one list (pair) of a KLT launch whose lists have their own image sizes (the lock-step tracker over sequences of
+// different sizes): level l of image A starts at lv[l].a, of image B at lv[l].b; both are w x h with row pitch `pitch`.
+struct KltGeoLevel {
+  const uint8_t* a;
+  const uint8_t* b;
+  int w, h, pitch, pad;
+};
+struct KltGeo {
+  KltGeoLevel lv[SFM_MAXL];
+};
 struct KltLaunch {
   PyrView pv;            // image A: frame fa0 + k*fa_step of this batch
   const double2* p0;     // [npairs*cap] (or [n] when npairs == 1)
@@ -229,6 +242,10 @@ struct KltLaunch {
   // two views differ (two batches, of any sizes, with equal level counts) always runs the two-geometry warp-per-feature
   // kernel; the lane kernels and the context's KLT mode only apply to one-batch launches.
   PyrView pvb;
+  // Optional device table [npairs]: list k reads its images from geo[k] instead of pv / pvb and the frame indices (pv gives
+  // the level count; pvb must equal pv).  Such launches take the same kernel family as one-batch launches, through
+  // instantiations of their own.
+  const KltGeo* geo = nullptr;
 };
 int sfm_klt_launch(sfmgpu_ctx* ctx, const KltLaunch& k);
 

@@ -969,12 +969,14 @@ enum KltSizing { KLT_BY_LIVE, KLT_BY_ROWS };
 
 // One step of every list from frame fa0 + s of fa to frame fb0 + s of fb (:346-371): the survivors of list s in track order,
 // (p0, p1, id), go to row s of oa / ob / oid and their count to dnk[s]; the step's sums are added to tot.  fa != fb (the single
-// tracker across an image-size change) runs the two-geometry KLT kernel.
+// tracker across an image-size change) runs the two-geometry KLT kernel.  geo != nullptr (the lock-step tracker over sequences of
+// different sizes): list s reads its two images from geo[s], fa only gives the level count.
 int lists_track(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* fa, sfmgpu_frames* fb, int fa0, int fb0,
-                KltSizing sizing) {
+                KltSizing sizing, const KltGeo* geo = nullptr) {
   KltLaunch k;
   k.pv = fa->view();
   k.pvb = fb->view();
+  k.geo = geo;
   k.p0 = L.trk;
   if (sizing == KLT_BY_LIVE) {  // one list
     k.counts = nullptr;
@@ -997,7 +999,10 @@ int lists_track(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_
   k.pb = L.pb;
   k.nit = L.nit;
   k.keep = L.keep;
-  SFM_TRY(sfm_klt_launch(ctx, k));
+  {
+    StageTimer st(ctx, 2);
+    SFM_TRY(sfm_klt_launch(ctx, k));
+  }
   for (int s = 0; s < L.S; s++) L.track_steps += L.n[s];
   SFM_LAUNCH(ctx, compact_kernel, L.S, 1024, 0, L.trk, L.p1, L.keep, (const int*)L.ids, k.counts, k.cap, L.oa, L.ob, L.oid, L.dnk);
   const unsigned tb = sfm_cdiv((long long)k.npairs * k.cap, 256);  // no more blocks (and atomics) than entries
@@ -1047,15 +1052,19 @@ int replenish_row(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgp
   return 0;
 }
 
-// After a commit, list by list on frames first + s: a list that entered the step without tracks (empty[s]; empty == nullptr:
-// none did) is reset on its frame instead of stepped (:341-344), one frame at a time; a list below min_tracks is replenished.
-int lists_refill(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, sfmgpu_frames* f, int first, const std::vector<char>* empty,
-                 const char* who) {
+// After a commit, list by list on its current frame (where(s, &batch, &index)): a list that entered the step without tracks
+// (empty[s]; empty == nullptr: none did) is reset on its frame instead of stepped (:341-344), one frame at a time; a list below
+// min_tracks is replenished.
+template <class Where>
+int lists_refill(sfmgpu_ctx* ctx, TrackLists& L, const sfmgpu_lkcfg& cfg, Where where, const std::vector<char>* empty, const char* who) {
   for (int s = 0; s < L.S; s++) {
+    sfmgpu_frames* f = nullptr;
+    int frame = 0;
+    where(s, &f, &frame);
     if (empty && (*empty)[s])
-      SFM_TRY(lists_reset(ctx, L, cfg, f, first, s, 1, who));
+      SFM_TRY(lists_reset(ctx, L, cfg, f, frame - s, s, 1, who));
     else if (L.n[s] < cfg.min_tracks)
-      SFM_TRY(replenish_row(ctx, L, cfg, f, first + s, s));
+      SFM_TRY(replenish_row(ctx, L, cfg, f, frame, s));
   }
   return 0;
 }
@@ -1128,7 +1137,11 @@ int tracker_step_on(sfmgpu_ctx* ctx, sfmgpu_tracker* t, sfmgpu_frames* fprev, sf
   t->prev_frames = f;
   t->prev_index = frame;
   if (n_out) *n_out = nk;
-  return lists_refill(ctx, L, t->cfg, f, frame, nullptr, "tracker");
+  auto where = [&](int, sfmgpu_frames** wf, int* wi) {
+    *wf = f;
+    *wi = frame;
+  };
+  return lists_refill(ctx, L, t->cfg, where, nullptr, "tracker");
 }
 
 // A host image of the tracker's size goes to the slot of its 2-slot batch that does not hold the previous frame.
@@ -1244,10 +1257,30 @@ int sfmgpu_tracker_totals(sfmgpu_ctx* ctx, sfmgpu_tracker* t, long long* n_track
 // all of them: frame t of every sequence arrives together, the S x max_tracks feature-tracks share a KLT launch (large enough
 // for the lane-per-feature kernels), survivors are compacted per sequence.  Results are identical to S separate sfmgpu_tracker
 // objects.  Resets after a total track loss and replenishment (rare) run list by list.
+//
+// Sequences may have different image sizes (sfmgpu_multitracker_create_sized).  The sequences of one size form a size class with
+// its own frame batch; the KLT chain still runs once over all S lists, reading every list's images through a per-list geometry
+// table, and everything after it (compaction, totals, commit, the RANSAC stage) works on the [S][ROWS] lists as before.
 struct sfmgpu_multitracker {
   sfmgpu_lkcfg cfg;
-  int w = 0, h = 0;
-  sfmgpu_frames* frames = nullptr;  // 3*S slots: group g of sequence s lives in slot g*S + s (previous / current / prefetched)
+  int w = 0, h = 0;                 // class 0's size (every sequence's, unless the tracker is mixed)
+  sfmgpu_frames* frames = nullptr;  // class 0's batch
+  // Size class: 3*n slots, group g of its i-th sequence in slot g*n + i (previous / current / prefetched).  With one class,
+  // sequence s is its s-th: group g of sequence s lives in slot g*S + s.
+  struct SizeClass {
+    int w, h, n;
+    sfmgpu_frames* frames;
+  };
+  // Adjacent sequences of one class: one upload.  host_off: where sequence s0's frame starts in the caller's S frames.
+  struct Run {
+    int s0, count, cls, i0;
+    size_t host_off;
+  };
+  std::vector<SizeClass> cls;
+  std::vector<Run> runs;
+  std::vector<int> cls_of, idx_in;  // per sequence: its class and its index in that class
+  KltGeo* geo = nullptr;            // mixed: [3][S] geometry tables, steps from group g to group (g+1)%3 read entries g*S ...
+  bool mixed() const { return cls.size() > 1; }
   int parity = -1;                  // slot group of the previous frames, -1: nothing tracked yet
   bool prefetched = false;          // group (parity+1)%3 holds the next frames (uploaded + pyramids), ready at pf_done
   cudaEvent_t pf_done = nullptr;
@@ -1267,28 +1300,98 @@ struct sfmgpu_multitracker {
 
 extern "C" {
 
+}  // extern "C"
+
+// Per-list geometry of the KLT launches of a mixed tracker: table g, entry s = sequence s from group g to group (g+1)%3.
+static std::vector<KltGeo> multi_geo_tables(const sfmgpu_multitracker* t) {
+  const int S = t->L.S;
+  std::vector<KltGeo> geo((size_t)3 * S);
+  for (int g = 0; g < 3; g++)
+    for (int s = 0; s < S; s++) {
+      const sfmgpu_multitracker::SizeClass& c = t->cls[t->cls_of[s]];
+      const sfmgpu_frames* f = c.frames;
+      const size_t sa = (size_t)g * c.n + t->idx_in[s], sb = (size_t)((g + 1) % 3) * c.n + t->idx_in[s];
+      KltGeo& e = geo[(size_t)g * S + s];
+      for (int l = 0; l < SFM_MAXL; l++) {
+        const bool in = l < f->levels;
+        e.lv[l].a = in ? f->lvl[l] + sa * f->fstride[l] : nullptr;
+        e.lv[l].b = in ? f->lvl[l] + sb * f->fstride[l] : nullptr;
+        e.lv[l].w = in ? f->lw[l] : 0;
+        e.lv[l].h = in ? f->lh[l] : 0;
+        e.lv[l].pitch = in ? f->pitch[l] : 0;
+        e.lv[l].pad = 0;
+      }
+    }
+  return geo;
+}
+
+// Sequence s has images of w[s] x h[s] (checked by the caller).
+static int multi_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int S, const int32_t* w, const int32_t* h, sfmgpu_multitracker** out,
+                        const char* who) {
+  SFM_TRY(lkcfg_ok(ctx, cfg, who));
+  sfmgpu_multitracker* t = new sfmgpu_multitracker();
+  t->cfg = *cfg;
+  t->cls_of.resize(S);
+  t->idx_in.resize(S);
+  size_t off = 0;
+  for (int s = 0; s < S; s++) {
+    int c = 0;
+    while (c < (int)t->cls.size() && (t->cls[c].w != w[s] || t->cls[c].h != h[s])) c++;
+    if (c == (int)t->cls.size()) t->cls.push_back({w[s], h[s], 0, nullptr});
+    t->cls_of[s] = c;
+    t->idx_in[s] = t->cls[c].n++;
+    if (s > 0 && t->cls_of[s - 1] == c)
+      t->runs.back().count++;
+    else
+      t->runs.push_back({s, 1, c, t->idx_in[s], off});
+    off += (size_t)w[s] * h[s];
+  }
+  for (sfmgpu_multitracker::SizeClass& c : t->cls) {
+    const int rc = sfmgpu_frames_create(ctx, c.w, c.h, 3 * c.n, cfg->pyr_levels, &c.frames);
+    if (rc != 0) {
+      sfmgpu_multitracker_destroy(ctx, t);
+      return rc;
+    }
+  }
+  t->frames = t->cls[0].frames;
+  t->w = t->cls[0].w;
+  t->h = t->cls[0].h;
+  cudaError_t e = lists_alloc(ctx, t->L, *cfg, S);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&t->didx, (size_t)S * 4 + 256);
+  if (e == cudaSuccess && t->mixed()) {
+    const std::vector<KltGeo> geo = multi_geo_tables(t);
+    e = cudaMalloc((void**)&t->geo, geo.size() * sizeof(KltGeo));
+    if (e == cudaSuccess) e = cudaMemcpy(t->geo, geo.data(), geo.size() * sizeof(KltGeo), cudaMemcpyHostToDevice);
+  }
+  if (e != cudaSuccess) {
+    sfmgpu_multitracker_destroy(ctx, t);
+    return sfm_fail(ctx, SFMGPU_E_CUDA, "%s: CUDA allocation failed: %s", who, cudaGetErrorString(e));
+  }
+  *out = t;
+  return 0;
+}
+
+extern "C" {
+
 int sfmgpu_multitracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_sequences, int w, int h, sfmgpu_multitracker** out) {
   SFM_ENTER(ctx);
   if (!ctx || !cfg || !out) return SFMGPU_E_ARG;
   if (n_sequences < 1 || n_sequences > 512 || w < 1 || h < 1) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_create: bad configuration");
-  SFM_TRY(lkcfg_ok(ctx, cfg, "multitracker_create"));
-  sfmgpu_multitracker* t = new sfmgpu_multitracker();
-  t->cfg = *cfg;
-  t->w = w;
-  t->h = h;
-  int rc = sfmgpu_frames_create(ctx, w, h, 3 * n_sequences, cfg->pyr_levels, &t->frames);
-  if (rc != 0) {
-    delete t;
-    return rc;
-  }
-  cudaError_t e = lists_alloc(ctx, t->L, *cfg, n_sequences);
-  if (e == cudaSuccess) e = cudaMalloc((void**)&t->didx, (size_t)n_sequences * 4 + 256);
-  if (e != cudaSuccess) {
-    sfmgpu_multitracker_destroy(ctx, t);
-    return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker_create: CUDA allocation failed: %s", cudaGetErrorString(e));
-  }
-  *out = t;
-  return 0;
+  const std::vector<int32_t> ws(n_sequences, w), hs(n_sequences, h);
+  return multi_create(ctx, cfg, n_sequences, ws.data(), hs.data(), out, "multitracker_create");
+}
+
+int sfmgpu_multitracker_create_sized(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_sequences, const int32_t* w, const int32_t* h,
+                                     sfmgpu_multitracker** out) {
+  SFM_ENTER(ctx);
+  const char* who = "multitracker_create_sized";
+  if (!ctx || !cfg || !out) return SFMGPU_E_ARG;
+  if (!w || !h) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null size array", who);
+  if (n_sequences < 1 || n_sequences > 512) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: %d sequences, not in [1, 512]", who, n_sequences);
+  for (int s = 0; s < n_sequences; s++)
+    if (w[s] < 1 || w[s] > 32767 || h[s] < 1 || h[s] > 32767)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequence %d is %d x %d, sizes must lie in [1, 32767]", who, s, w[s], h[s]);
+  return multi_create(ctx, cfg, n_sequences, w, h, out, who);
 }
 
 void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
@@ -1299,7 +1402,9 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   sfm_two_view_free(ctx, &t->tv);
   lists_free(t->L);
   if (t->didx) cudaFree(t->didx);
-  if (t->frames) sfmgpu_frames_destroy(ctx, t->frames);
+  if (t->geo) cudaFree(t->geo);
+  for (sfmgpu_multitracker::SizeClass& c : t->cls)
+    if (c.frames) sfmgpu_frames_destroy(ctx, c.frames);
   if (t->pk) cudaFree(t->pk);
   if (t->pk_bad) cudaFreeHost(t->pk_bad);
   if (t->pf_done) cudaEventDestroy(t->pf_done);
@@ -1311,18 +1416,26 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
 static int multi_next_group(const sfmgpu_multitracker* t) { return t->parity < 0 ? 0 : (t->parity + 1) % 3; }
 static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 
+// The S frames of one step (back to back in sequence order, frame s of w[s] x h[s] bytes) into slot group g, one copy per run of
+// adjacent sequences of one size, then the pyramids of every class, on ctx->stream.
+static int multi_upload(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g, const uint8_t* host_pix) {
+  for (const sfmgpu_multitracker::Run& r : t->runs) {
+    const sfmgpu_multitracker::SizeClass& c = t->cls[r.cls];
+    SFM_TRY(sfmgpu_frames_upload(ctx, c.frames, g * c.n + r.i0, r.count, host_pix + r.host_off));
+  }
+  for (const sfmgpu_multitracker::SizeClass& c : t->cls) SFM_TRY(sfmgpu_pyramid_build(ctx, c.frames, g * c.n, c.n));
+  return 0;
+}
+
 // Upload + pyramids of the frames of a LATER step on the copy stream, into the slot group after `after_group`.
 static int multi_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int after_group, const uint8_t* host_pix) {
   SFM_TRY(pipe_streams(ctx));
   if (!t->pf_done && cudaEventCreateWithFlags(&t->pf_done, cudaEventDisableTiming) != cudaSuccess)
     return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker: cudaEventCreate failed");
-  const int S = t->L.S, g = (after_group + 1) % 3;
-  sfmgpu_frames* f = t->frames;
-  SFM_CUDA(ctx, cudaMemcpy2DAsync(f->lvl[0] + (size_t)g * S * f->fstride[0], f->pitch[0], host_pix, f->w, f->w, (size_t)f->h * S,
-                                  cudaMemcpyDefault, ctx->copy_stream));
+  const int g = (after_group + 1) % 3;
   {
     StageScope sc(ctx, ctx->copy_stream);
-    SFM_TRY(sfmgpu_pyramid_build(ctx, f, g * S, S));
+    SFM_TRY(multi_upload(ctx, t, g, host_pix));
     SFM_CUDA(ctx, cudaEventRecord(t->pf_done, ctx->stream));
   }
   t->prefetched = true;
@@ -1455,14 +1568,10 @@ int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, 
   if (!ctx || !t) return SFMGPU_E_ARG;
   if (!host_pix && !t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: no frames given and none prefetched");
   if (host_pix && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step: frames given but others are prefetched");
-  const int S = t->L.S;
   const int par = multi_next_group(t);
   if (!host_pix) SFM_TRY(multi_take_prefetch(ctx, t, "multitracker_step"));
   t->tv_fresh = false;
-  if (host_pix) {
-    SFM_TRY(sfmgpu_frames_upload(ctx, t->frames, par * S, S, host_pix));
-    SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, par * S, S));
-  }
+  if (host_pix) SFM_TRY(multi_upload(ctx, t, par, host_pix));
   // the frames of the NEXT step travel while this one computes (their slot group is neither previous nor current)
   if (next_host_pix) SFM_TRY(multi_prefetch(ctx, t, par, next_host_pix));
   return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
@@ -1473,6 +1582,8 @@ int sfmgpu_multitracker_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t,
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
   const char* who = "multitracker_prefetch_packed";
+  if (t->mixed())
+    return sfm_fail(ctx, SFMGPU_E_ARG, "%s: the sequences have different image sizes; packed and resident input take one size", who);
   if (!blob_frame) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null frame index array", who);
   if (t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: the prefetched frames have not been stepped yet", who);
   PkPlan p;
@@ -1486,6 +1597,8 @@ int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, con
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
   const char* who = "multitracker_step_packed";
+  if (t->mixed())
+    return sfm_fail(ctx, SFMGPU_E_ARG, "%s: the sequences have different image sizes; packed and resident input take one size", who);
   if (!blob_frame && !t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: no frames given and none prefetched", who);
   if (blob_frame && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: frames given but others are prefetched", who);
   PkPlan cur, next;
@@ -1512,6 +1625,9 @@ int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfm
                                     double* cur_xy, int32_t* ids, int32_t* n_out) {
   SFM_ENTER(ctx);
   if (!ctx || !t || !f) return SFMGPU_E_ARG;
+  if (t->mixed())
+    return sfm_fail(ctx, SFMGPU_E_ARG,
+                    "multitracker_step_frames: the sequences have different image sizes; packed and resident input take one size");
   if (!frame_idx) return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: null frame index array");
   if (t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "multitracker_step_frames: frames are prefetched; step them first");
   const sfmgpu_frames* g = t->frames;
@@ -1547,7 +1663,10 @@ static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, doubl
   if (n_out)
     for (int s = 0; s < S; s++) n_out[s] = 0;
   if (t->parity < 0) {  // first frames: reset every sequence (:341-344); find_E_ransac is not called (:1715)
-    SFM_TRY(lists_reset(ctx, L, t->cfg, t->frames, par * S, 0, S, "multitracker"));
+    for (const sfmgpu_multitracker::Run& r : t->runs) {
+      const sfmgpu_multitracker::SizeClass& c = t->cls[r.cls];
+      SFM_TRY(lists_reset(ctx, L, t->cfg, c.frames, par * c.n + r.i0 - r.s0, r.s0, r.count, "multitracker"));
+    }
     t->parity = par;
     if (stage) SFM_TRY(sfm_two_view_skip(ctx, t->tv, nullptr, S));
     t->tv_fresh = stage;
@@ -1559,7 +1678,8 @@ static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, doubl
     empty[s] = L.n[s] == 0;
     any_empty = any_empty || empty[s];
   }
-  SFM_TRY(lists_track(ctx, L, t->cfg, t->frames, t->frames, t->parity * S, par * S, KLT_BY_ROWS));
+  SFM_TRY(lists_track(ctx, L, t->cfg, t->frames, t->frames, t->parity * S, par * S, KLT_BY_ROWS,
+                      t->mixed() ? t->geo + (size_t)t->parity * S : nullptr));
   if (stage) {  // find_E_ransac(K, prev_pts, cur_pts, ...) on every sequence's survivors (:1739), inside the step's one synchronisation
     StageTimer rt(ctx, 4);
     SFM_TRY(sfm_two_view_stage(ctx, t->tv, L.oa, L.ob, L.dnk, L.rows, 0, S, nullptr));
@@ -1576,7 +1696,12 @@ static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, doubl
   t->tv_fresh = stage;
   if (n_out)
     for (int s = 0; s < S; s++) n_out[s] = L.n[s];
-  return lists_refill(ctx, L, t->cfg, t->frames, par * S, &empty, "multitracker");
+  auto where = [&](int s, sfmgpu_frames** f, int* frame) {
+    const sfmgpu_multitracker::SizeClass& c = t->cls[t->cls_of[s]];
+    *f = c.frames;
+    *frame = par * c.n + t->idx_in[s];
+  };
+  return lists_refill(ctx, L, t->cfg, where, &empty, "multitracker");
 }
 
 extern "C" {
@@ -1586,6 +1711,14 @@ int sfmgpu_multitracker_set_ransac(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, cons
   if (!ctx || !t) return SFMGPU_E_ARG;
   t->tv_fresh = false;  // results of earlier steps are not those of this configuration
   return sfm_two_view_configure(ctx, &t->tv, t->L.S, t->L.rows, K, rc, "multitracker_set_ransac");
+}
+
+int sfmgpu_multitracker_set_ransac_cameras(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const double* K, const sfmgpu_ransac_cfg* rc) {
+  SFM_ENTER(ctx);
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  SFM_TRY(sfm_two_view_configure_sets(ctx, &t->tv, t->L.S, t->L.rows, K, rc, "multitracker_set_ransac_cameras"));
+  t->tv_fresh = false;  // results of earlier steps are not those of this configuration (a refused call keeps them)
+  return 0;
 }
 
 int sfmgpu_multitracker_ransac_download_all(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int32_t* status, int32_t* best_n, int32_t* inliers,

@@ -158,9 +158,12 @@ __device__ __forceinline__ void walk_rows(const KltSmem<R>& sm, int NK, int nc, 
 // track(Pyr A, Pyr B) allows: each tile is staged from its own image and each sample is zeroed by its own image's
 // bounds (:188).  The step is zero whenever B has fewer than 2 columns or rows (no gradient); an A that small only
 // zeroes its own samples.  Without TWO, pva is pv.
-template <int R, bool FIXED, bool TWO = false>
+//
+// GEO: the list's own geometry table `geo` (one size for both images) replaces pv's sizes and the frame indices; back = true
+// tracks from its image B to its image A.
+template <int R, bool FIXED, bool TWO = false, bool GEO = false>
 __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int radius_rt, int iters, double& px, double& py,
-                          int& n_it, int lane, const PyrView& pva) {
+                          int& n_it, int lane, const PyrView& pva, const KltGeoLevel* geo = nullptr, bool back = false) {
   constexpr int TH = KltSmem<R>::TH, TW = KltSmem<R>::TW;
   const int radius = FIXED ? R : radius_rt;  // compile-time window for the default radius
   const int nc = 2 * radius + 3;
@@ -176,10 +179,23 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
   const double off_i = (double)(i - radius - 1);
 
   for (int l = pv.levels - 1; l >= 0; --l) {
-    const int w = pv.w[l], h = pv.h[l], pitch = pv.pitch[l];
-    const PyrView& va = TWO ? pva : pv;
-    const uint8_t* I0 = va.base[l] + (size_t)fa * va.fstride[l];
-    const uint8_t* I1 = pv.base[l] + (size_t)fb * pv.fstride[l];
+    int w, h, pitch;
+    const uint8_t *I0, *I1;
+    if constexpr (GEO) {
+      const KltGeoLevel g = geo[l];
+      w = g.w;
+      h = g.h;
+      pitch = g.pitch;
+      I0 = back ? g.b : g.a;
+      I1 = back ? g.a : g.b;
+    } else {
+      w = pv.w[l];
+      h = pv.h[l];
+      pitch = pv.pitch[l];
+      const PyrView& va = TWO ? pva : pv;
+      I0 = va.base[l] + (size_t)fa * va.fstride[l];
+      I1 = pv.base[l] + (size_t)fb * pv.fstride[l];
+    }
     const int w0 = TWO ? pva.w[l] : w, h0 = TWO ? pva.h[l] : h;
     const bool a_ok = !TWO || (w0 >= 2 && h0 >= 2);  // otherwise no sample of A is inside A: its tile is not staged
     const double scale = 1.0 / (double)(1 << l);
@@ -263,7 +279,8 @@ __device__ void track_one(KltSmem<R>& sm, const PyrView& pv, int fa, int fb, int
 // list == nullptr: one warp per slot of the launch (grid covers them all).  list != nullptr: the warps of a
 // fixed-size grid walk the deferred-feature list written by klt_lane_kernel (count read from device memory).
 // TWO: image A from k.pv, image B from k.pvb (two batches, any sizes); the backward track swaps the two views.
-template <int R, bool FIXED, bool TWO>
+// GEO: both images of pair k from k.geo[k].
+template <int R, bool FIXED, bool TWO, bool GEO = false>
 __global__ void __launch_bounds__(128, (R <= 5 ? 6 : 3)) klt_kernel(KltLaunch k, const int* __restrict__ list,
                                                                     const int* __restrict__ list_count) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -279,11 +296,20 @@ __global__ void __launch_bounds__(128, (R <= 5 ? 6 : 3)) klt_kernel(KltLaunch k,
     int n_it = 0;
     double x = p0.x, y = p0.y;
     __syncwarp();
-    track_one<R, FIXED, TWO>(sm, TWO ? k.pvb : k.pv, fa, fb, k.radius, k.iters, x, y, n_it, lane, k.pv);
+    if constexpr (GEO) {
+      const KltGeoLevel* geo = k.geo[pair].lv;
+      track_one<R, FIXED, false, true>(sm, k.pv, 0, 0, k.radius, k.iters, x, y, n_it, lane, k.pv, geo, false);
+    } else {
+      track_one<R, FIXED, TWO>(sm, TWO ? k.pvb : k.pv, fa, fb, k.radius, k.iters, x, y, n_it, lane, k.pv);
+    }
     const double x1 = x, y1 = y;
     __syncwarp();
-    if (k.pb)  // pb == null: forward only
-      track_one<R, FIXED, TWO>(sm, k.pv, fb, fa, k.radius, k.iters, x, y, n_it, lane, TWO ? k.pvb : k.pv);
+    if (k.pb) {  // pb == null: forward only
+      if constexpr (GEO)
+        track_one<R, FIXED, false, true>(sm, k.pv, 0, 0, k.radius, k.iters, x, y, n_it, lane, k.pv, k.geo[pair].lv, true);
+      else
+        track_one<R, FIXED, TWO>(sm, k.pv, fb, fa, k.radius, k.iters, x, y, n_it, lane, TWO ? k.pvb : k.pv);
+    }
     if (lane == 0) {
       k.p1[g] = make_double2(x1, y1);
       if (k.pb) k.pb[g] = make_double2(x, y);
@@ -296,7 +322,7 @@ __global__ void __launch_bounds__(128, (R <= 5 ? 6 : 3)) klt_kernel(KltLaunch k,
   }
 }
 
-template <int R, bool FIXED, bool TWO = false>
+template <int R, bool FIXED, bool TWO = false, bool GEO = false>
 int launch_r(sfmgpu_ctx* ctx, const KltLaunch& k, const int* list, const int* list_count) {
   const int warps_per_block = 4;
   // Without FIXED, the last row group of a window of radius 1..3 walks up to two tap rows past the rows its pixels need
@@ -304,7 +330,7 @@ int launch_r(sfmgpu_ctx* ctx, const KltLaunch& k, const int* list, const int* li
   // last warp's reads inside the block's shared memory.
   const size_t smem = sizeof(KltSmem<R>) * warps_per_block + (FIXED ? 0 : 2 * KltSmem<R>::TW);
   static const int cfg_id = sfm_next_cfg_id();  // one per template instantiation
-  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_kernel<R, FIXED, TWO>), smem);
+  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_kernel<R, FIXED, TWO, GEO>), smem);
   const long long total = (long long)k.npairs * k.cap;
   if (total == 0) return 0;
   unsigned grid = sfm_cdiv(total, warps_per_block);
@@ -312,7 +338,7 @@ int launch_r(sfmgpu_ctx* ctx, const KltLaunch& k, const int* list, const int* li
     const unsigned cap = (unsigned)ctx->n_sm * 24;  // deferred features are a few % of the batch: a resident grid walks the list
     grid = grid < cap ? grid : cap;
   }
-  SFM_LAUNCH(ctx, (klt_kernel<R, FIXED, TWO>), grid, warps_per_block * 32, smem, k, list, list_count);
+  SFM_LAUNCH(ctx, (klt_kernel<R, FIXED, TWO, GEO>), grid, warps_per_block * 32, smem, k, list, list_count);
   return 0;
 }
 
@@ -339,7 +365,7 @@ int sfm_klt_launch(sfmgpu_ctx* ctx, const KltLaunch& k) {
   if (k.radius < 1 || k.radius > 10)
     return sfm_fail(ctx, SFMGPU_E_ARG, "klt: win_radius %d outside the supported range [1,10]", k.radius);
   if (k.iters < 0) return sfm_fail(ctx, SFMGPU_E_ARG, "klt: negative iteration count");
-  if (!same_view(k.pv, k.pvb)) {  // two batches: the lane kernels assume one geometry, so the mode does not apply
+  if (!k.geo && !same_view(k.pv, k.pvb)) {  // two batches: the lane kernels assume one geometry, so the mode does not apply
     if (k.pv.levels != k.pvb.levels) return sfm_fail(ctx, SFMGPU_E_ARG, "klt: pyramid level counts differ (%d, %d)", k.pv.levels, k.pvb.levels);
     if (k.radius == 5) return launch_r<5, true, true>(ctx, k, nullptr, nullptr);
     if (k.radius < 5) return launch_r<5, false, true>(ctx, k, nullptr, nullptr);
@@ -366,6 +392,12 @@ int sfm_klt_launch(sfmgpu_ctx* ctx, const KltLaunch& k) {
       list = dlist2;
       list_count = dcount + 1;
     }
+  }
+  if (k.geo) {  // per-list geometry: the same chain through the table instantiations
+    if (k.radius == 5) return launch_r<5, true, false, true>(ctx, k, list, list_count);
+    if (k.radius < 5) return launch_r<5, false, false, true>(ctx, k, list, list_count);
+    if (k.radius == 10) return launch_r<10, true, false, true>(ctx, k, list, list_count);
+    return launch_r<10, false, false, true>(ctx, k, list, list_count);
   }
   if (k.radius == 5) return launch_r<5, true>(ctx, k, list, list_count);
   if (k.radius < 5) return launch_r<5, false>(ctx, k, list, list_count);

@@ -197,7 +197,8 @@ __device__ __forceinline__ void stage_store(const StageRegs& r, unsigned char* t
 //                 masks; what it still cannot do exactly (non-finite positions, a fractional part so close to 1 that
 //                 the reference's own floor(fl(x + dx)) may land on the next integer, degenerate level sizes) is
 //                 deferred once more, to the warp-per-feature kernel of klt.cu.
-template <int ACC, int MINB, int LSTAGE, bool MASKED>
+// GEO: every lane reads its pair's images and level sizes from k.geo (lanes of a warp may belong to pairs of different sizes).
+template <int ACC, int MINB, int LSTAGE, bool MASKED, bool GEO = false>
 __global__ void __launch_bounds__(32 * LWARPS, MINB) klt_lane_kernel(KltLaunch k, const int* __restrict__ in_list,
                                                                      const int* __restrict__ in_count, int* __restrict__ defer_count,
                                                                      int* __restrict__ defer_list) {
@@ -225,7 +226,7 @@ __global__ void __launch_bounds__(32 * LWARPS, MINB) klt_lane_kernel(KltLaunch k
 
   for (int dir = 0; dir < ndir; dir++) {
     for (int l = k.pv.levels - 1; l >= 0; --l) {
-      const int w = k.pv.w[l], h = k.pv.h[l], pitch = k.pv.pitch[l];
+      const int w = GEO ? k.geo[pair].lv[l].w : k.pv.w[l], h = GEO ? k.geo[pair].lv[l].h : k.pv.h[l], pitch = k.pv.pitch[l];
       const uint8_t* lbase = k.pv.base[l];
       const size_t fstride = k.pv.fstride[l];
       const double scale = 1.0 / (double)(1 << l);
@@ -281,9 +282,15 @@ __global__ void __launch_bounds__(32 * LWARPS, MINB) klt_lane_kernel(KltLaunch k
               const int sFX = __shfl_sync(FULL, FX, src), sFY = __shfl_sync(FULL, FY, src), spair = __shfl_sync(FULL, pair, src);
               const int sA = k.fa0 + spair * k.fa_step, sB = k.fb0 + spair * k.fb_step;
               sx0[j] = sFX - LR - 1;
+              if constexpr (GEO) {
+                const KltGeoLevel& q = k.geo[spair].lv[l];
+                if (ss[j] >= 0 && lane < 2 * LN)
+                  stage_load<MASKED>(sr[j], dir ? q.b : q.a, dir ? q.a : q.b, q.pitch, q.h, sx0[j], sFY - LR - 1, lane);
+              } else {
               if (ss[j] >= 0 && lane < 2 * LN)
                 stage_load<MASKED>(sr[j], lbase + (size_t)(dir ? sB : sA) * fstride, lbase + (size_t)(dir ? sA : sB) * fstride, pitch, h,
                                    sx0[j], sFY - LR - 1, lane);
+              }
             }
 #pragma unroll
             for (int j = 0; j < LSTAGE; j++)
@@ -728,7 +735,8 @@ __device__ __forceinline__ void quad_eval(const double* m, double fx, double fy,
 __device__ unsigned long long klt_round_hist[2][33];  // [0]: build rounds by lanes building, [1]: iteration rounds by lanes iterating
 #endif
 
-template <int MINB, int LSTAGE, typename T>
+// GEO: every lane reads its pair's images and level sizes from k.geo, as klt_lane_kernel does.
+template <int MINB, int LSTAGE, typename T, bool GEO = false>
 __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __restrict__ defer_count, int* __restrict__ defer_list) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const unsigned FULL = 0xffffffffu;
@@ -792,7 +800,7 @@ __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __
       int FX = 0, FY = 0;
       bool act = canwork;
       if (act) {
-        const int w = k.pv.w[l], h = k.pv.h[l];
+        const int w = GEO ? k.geo[pair].lv[l].w : k.pv.w[l], h = GEO ? k.geo[pair].lv[l].h : k.pv.h[l];
         const bool finite_ok = (fabs(fxx) < 1.0e9) && (fabs(fyy) < 1.0e9);
         FX = finite_ok ? (int)fxx : 0;
         FY = finite_ok ? (int)fyy : 0;
@@ -852,9 +860,14 @@ __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __
           const uint8_t* lbase = k.pv.base[sl];
           const size_t fstride = k.pv.fstride[sl];
           sx0[j] = sFX - LR - 1;
+          if constexpr (GEO) {
+            const KltGeoLevel& q = k.geo[spair].lv[sl];
+            if (ss[j] >= 0 && lane < 2 * LN) stage_load<false>(sr[j], sdir ? q.b : q.a, sdir ? q.a : q.b, q.pitch, q.h, sx0[j], sFY - LR - 1, lane);
+          } else {
           if (ss[j] >= 0 && lane < 2 * LN)
             stage_load<false>(sr[j], lbase + (size_t)(sdir ? sB : sA) * fstride, lbase + (size_t)(sdir ? sA : sB) * fstride,
                               k.pv.pitch[sl], k.pv.h[sl], sx0[j], sFY - LR - 1, lane);
+          }
         }
 #pragma unroll
         for (int j = 0; j < LSTAGE; j++)
@@ -895,11 +908,11 @@ __global__ void __launch_bounds__(32, MINB) klt_quad_kernel(KltLaunch k, int* __
 
 }  // namespace
 
-template <int ACC, int MINB, int LSTAGE, bool MASKED>
+template <int ACC, int MINB, int LSTAGE, bool MASKED, bool GEO = false>
 static int lane_launch(sfmgpu_ctx* ctx, const KltLaunch& k, const int* in_list, const int* in_count, int* defer_count, int* defer_list) {
   const size_t smem = (size_t)LWARPS * 32 * LSTRIDE;
   static const int cfg_id = sfm_next_cfg_id();  // one per template instantiation
-  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_lane_kernel<ACC, MINB, LSTAGE, MASKED>), smem);
+  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_lane_kernel<ACC, MINB, LSTAGE, MASKED, GEO>), smem);
   const long long total = (long long)k.npairs * k.cap;
   if (total == 0) return 0;
   unsigned grid = sfm_cdiv(total, 32 * LWARPS);
@@ -907,24 +920,25 @@ static int lane_launch(sfmgpu_ctx* ctx, const KltLaunch& k, const int* in_list, 
     const unsigned cap = (unsigned)ctx->n_sm * 8;
     grid = grid < cap ? grid : cap;
   }
-  SFM_LAUNCH(ctx, (klt_lane_kernel<ACC, MINB, LSTAGE, MASKED>), grid, 32 * LWARPS, smem, k, in_list, in_count, defer_count, defer_list);
+  SFM_LAUNCH(ctx, (klt_lane_kernel<ACC, MINB, LSTAGE, MASKED, GEO>), grid, 32 * LWARPS, smem, k, in_list, in_count, defer_count, defer_list);
   return 0;
 }
 
 // Interior windows of every slot; features it cannot handle are appended to defer_list (device), count in
 // *defer_count (device, zeroed by the caller on the same stream).  variant: tuning builds (A/B runs).
-template <int MINB, int LSTAGE, typename T>
+template <int MINB, int LSTAGE, typename T, bool GEO = false>
 static int quad_launch(sfmgpu_ctx* ctx, const KltLaunch& k, int* defer_count, int* defer_list) {
   const size_t smem = (size_t)32 * LSTRIDE + (std::is_same<T, GramBuild>::value ? GRAM_SCRATCH : 0);
   static const int cfg_id = sfm_next_cfg_id();  // one per template instantiation
-  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_quad_kernel<MINB, LSTAGE, T>), smem);
+  SFM_SMEM_OPTIN(ctx, cfg_id, (klt_quad_kernel<MINB, LSTAGE, T, GEO>), smem);
   const long long total = (long long)k.npairs * k.cap;
   if (total == 0) return 0;
-  SFM_LAUNCH(ctx, (klt_quad_kernel<MINB, LSTAGE, T>), sfm_cdiv(total, 32), 32, smem, k, defer_count, defer_list);
+  SFM_LAUNCH(ctx, (klt_quad_kernel<MINB, LSTAGE, T, GEO>), sfm_cdiv(total, 32), 32, smem, k, defer_count, defer_list);
   return 0;
 }
 
 int sfm_klt_lane_launch(sfmgpu_ctx* ctx, const KltLaunch& k, int* defer_count, int* defer_list, int variant) {
+  if (k.geo) return quad_launch<14, 2, GramBuild, true>(ctx, k, defer_count, defer_list);  // per-list geometry: the default only
   // Measured on B200, C2 shape (scripts/klt_ab.py, KLT stage incl. the deferred pass, 238k tracks): <1,12,4> 4.43 ms
   // (168 registers, spills), <1,8,4> 3.57 ms, <2,8,4> 3.66 ms, <2,8,8> 3.97 ms: the schedule wants registers, not warps.
   switch (variant) {
@@ -949,6 +963,7 @@ int sfm_klt_lane_launch(sfmgpu_ctx* ctx, const KltLaunch& k, int* defer_count, i
 // Border windows: the features of in_list with the out-of-bounds rule as masks; the rest goes to defer_list.
 int sfm_klt_lane_masked_launch(sfmgpu_ctx* ctx, const KltLaunch& k, const int* in_list, const int* in_count, int* defer_count,
                                int* defer_list) {
+  if (k.geo) return lane_launch<1, 8, 4, true, true>(ctx, k, in_list, in_count, defer_count, defer_list);
   return lane_launch<1, 8, 4, true>(ctx, k, in_list, in_count, defer_count, defer_list);
 }
 

@@ -25,6 +25,9 @@ struct TwoViewState {
   bool enabled = false;  // run the stage inside sfmgpu_pair_frontend(_host)
   sfmgpu_ransac_cfg rc{};
   double Kinv[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  bool per_set = false;                  // set s is normalised with kinv_sets + 9 s instead of Kinv (one camera per set)
+  double* kinv_sets = nullptr;           // [max_sets][9], allocated by the first per-set configuration
+  std::vector<double> kinv_host;         // its host copy (the source of the upload)
   double2 *xi = nullptr, *xj = nullptr;  // [max_pairs][cap] normalised survivors
   int *neff = nullptr;                   // [max_pairs] points entering RANSAC (0: skipped by min_points)
   int *status = nullptr, *best = nullptr, *inl = nullptr;  // [max_pairs], [max_pairs][2], [max_pairs][cap]
@@ -45,10 +48,13 @@ constexpr int TV_CHUNK = 1024;  // pairs per launch set: bounds the scratch (102
                                 // The small kernels of a set (sampler, repeated-index and winner solves, argmax, mask, pose) are
                                 // latency-bound, ~0.6 ms per set: 256 pairs per set cost C3 (1999 pairs) 8 x that, C2 4 x
 
+// PER_SET: set `pair` reads its K^-1 from kset + 9 * pair (k0..k8 unused); the same operations in the same order.
+template <bool PER_SET>
 __global__ void __launch_bounds__(256) tv_normalize_kernel(const double2* __restrict__ li, const double2* __restrict__ lj,
                                                           const int* __restrict__ nkept, int cap, int min_points, double k0, double k1,
                                                           double k2, double k3, double k4, double k5, double k6, double k7, double k8,
-                                                          double2* __restrict__ xi, double2* __restrict__ xj, int* __restrict__ neff) {
+                                                          double2* __restrict__ xi, double2* __restrict__ xj, int* __restrict__ neff,
+                                                          const double* __restrict__ kset) {
   const int pair = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
   int n = nkept[pair];
   n = n < 0 ? 0 : (n > cap ? cap : n);
@@ -56,6 +62,10 @@ __global__ void __launch_bounds__(256) tv_normalize_kernel(const double2* __rest
   if (i == 0) neff[pair] = n;
   if (i >= n) return;
   const size_t o = (size_t)pair * cap + i;
+  if (PER_SET) {
+    const double* q = kset + 9 * (size_t)pair;
+    k0 = q[0], k1 = q[1], k2 = q[2], k3 = q[3], k4 = q[4], k5 = q[5], k6 = q[6], k7 = q[7], k8 = q[8];
+  }
   // Kinv * (u, v, 1) then divide by z (:498-501; Mat33 * Vec3 of linalg.hpp:70-76: left-to-right sums, no contraction)
   const double2 p = li[o], q = lj[o];
   const double pa = k0 * p.x + k1 * p.y + k2 * 1.0, pb = k3 * p.x + k4 * p.y + k5 * 1.0, pc = k6 * p.x + k7 * p.y + k8 * 1.0;
@@ -226,7 +236,8 @@ void sfm_two_view_free(sfmgpu_ctx* ctx, TwoViewState** tvp) {
   (void)ctx;
   TwoViewState* tv = *tvp;
   if (!tv) return;
-  void* ptrs[] = {tv->xi, tv->xj, tv->inl, tv->neff, tv->status, tv->best, tv->bestE, tv->R, tv->t, tv->flags, tv->idx8.p, tv->E.p, tv->counts.p, tv->neff2.p, tv->raw.p};
+  void* ptrs[] = {tv->xi, tv->xj, tv->inl, tv->neff, tv->status, tv->best, tv->bestE, tv->R, tv->t, tv->flags, tv->idx8.p, tv->E.p, tv->counts.p, tv->neff2.p, tv->raw.p,
+                  tv->kinv_sets};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   delete tv;
@@ -259,8 +270,12 @@ int sfm_two_view_stage(sfmgpu_ctx* ctx, TwoViewState* tv, const double2* li, con
   for (int c0 = 0; c0 < npairs; c0 += chunk) {
     const int pc = npairs - c0 < chunk ? npairs - c0 : chunk, po = pair_off + c0;
     const size_t so = (size_t)po * cap;
-    SFM_LAUNCH(ctx, tv_normalize_kernel, dim3(sfm_cdiv(cap, 256), pc), 256, 0, li + so, lj + so, nkept + po, cap, mp, k[0], k[1], k[2],
-               k[3], k[4], k[5], k[6], k[7], k[8], tv->xi + so, tv->xj + so, tv->neff + po);
+    if (tv->per_set)
+      SFM_LAUNCH(ctx, tv_normalize_kernel<true>, dim3(sfm_cdiv(cap, 256), pc), 256, 0, li + so, lj + so, nkept + po, cap, mp, 0.0, 0.0, 0.0,
+                 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, tv->xi + so, tv->xj + so, tv->neff + po, (const double*)(tv->kinv_sets + 9 * (size_t)po));
+    else
+      SFM_LAUNCH(ctx, tv_normalize_kernel<false>, dim3(sfm_cdiv(cap, 256), pc), 256, 0, li + so, lj + so, nkept + po, cap, mp, k[0], k[1],
+                 k[2], k[3], k[4], k[5], k[6], k[7], k[8], tv->xi + so, tv->xj + so, tv->neff + po, (const double*)nullptr);
     if (H > 0) {
       if (E_host) {
         SFM_CUDA(ctx, cudaMemcpyAsync(tv->E.p, E_host + (size_t)c0 * H * 9, (size_t)pc * H * 72, cudaMemcpyHostToDevice, ctx->stream));
@@ -349,6 +364,31 @@ int sfm_two_view_configure(sfmgpu_ctx* ctx, TwoViewState** tvp, int max_sets, in
   TwoViewState* tv = *tvp;
   tv->rc = *rc;
   for (int i = 0; i < 9; i++) tv->Kinv[i] = Ki[i];
+  tv->per_set = false;
+  tv->enabled = true;
+  return 0;
+}
+
+// Every K is checked before anything changes, so a refused call leaves the previous configuration (and its results) in force.
+int sfm_two_view_configure_sets(sfmgpu_ctx* ctx, TwoViewState** tvp, int max_sets, int cap, const double* K, const sfmgpu_ransac_cfg* rc,
+                                const char* who) {
+  if (!rc) {
+    if (*tvp) (*tvp)->enabled = false;
+    return 0;
+  }
+  if (!K) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null K", who);
+  if (rc->iters < 0 || rc->iters > (1 << 24)) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: bad iteration count", who);
+  std::vector<double> ki((size_t)max_sets * 9);
+  for (int s = 0; s < max_sets; s++)
+    if (!invert_K_host(K + 9 * (size_t)s, ki.data() + 9 * (size_t)s))
+      return sfm_fail(ctx, SFMGPU_E_ARG, "%s: Singular K of sequence %d", who, s);  // the reference throws "Singular K" (:474)
+  SFM_TRY(tv_alloc(ctx, tvp, max_sets, cap));
+  TwoViewState* tv = *tvp;
+  if (!tv->kinv_sets) SFM_CUDA(ctx, cudaMalloc((void**)&tv->kinv_sets, (size_t)max_sets * 72));
+  tv->kinv_host.swap(ki);  // kept until the next configuration: the copy below reads it asynchronously
+  SFM_CUDA(ctx, cudaMemcpyAsync(tv->kinv_sets, tv->kinv_host.data(), (size_t)max_sets * 72, cudaMemcpyHostToDevice, ctx->stream));
+  tv->rc = *rc;
+  tv->per_set = true;
   tv->enabled = true;
   return 0;
 }

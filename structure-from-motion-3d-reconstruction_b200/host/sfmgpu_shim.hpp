@@ -32,6 +32,7 @@
 #include <random>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <thread>
 #include <unordered_map>
 #include <vector>
@@ -445,39 +446,30 @@ class KLTTracker {
 
 // S KLTTrackers advanced in lock step (no counterpart in the reference, which tracks one sequence: this is the C++ face of
 // sfmgpu_multitracker for callers with several independent sequences per GPU).  Per sequence the results equal a
-// KLTTracker's; all images must be w x h.
+// KLTTracker's.  The (cfg, n, w, h) form takes w x h images for every sequence; the (cfg, sizes) form gives sequence s images of
+// sizes[s] = {w, h} (cameras of different resolutions in one lock step).  Packed and resident input are not offered for the
+// latter (the C ABI refuses them for sequences of different sizes).
 class MultiKLTTracker {
  public:
   MultiKLTTracker(const MultiKLTTracker&) = delete;
   MultiKLTTracker& operator=(const MultiKLTTracker&) = delete;
-  MultiKLTTracker(LKConfig cfg, int n_sequences, int w, int h) : S_(n_sequences), w_(w), h_(h) {
-    sfmgpu_lkcfg c;
-    c.max_tracks = cfg.max_tracks;
-    c.min_tracks = cfg.min_tracks;
-    c.quality = cfg.quality;
-    c.min_distance = cfg.min_distance;
-    c.pyr_levels = cfg.pyr_levels;
-    c.win_radius = cfg.win_radius;
-    c.iters = cfg.iters;
-    c.fb_thresh = cfg.fb_thresh;
-    sfmgpu_multitracker* t = nullptr;
-    auto* ctx = sfmgpu_shim::context();
-    sfmgpu_shim::check(ctx, sfmgpu_multitracker_create(ctx, &c, n_sequences, w, h, &t), "multitracker_create");
-    trk_ = std::shared_ptr<sfmgpu_multitracker>(t, [](sfmgpu_multitracker* p) { sfmgpu_multitracker_destroy(sfmgpu_shim::context(), p); });
-    cap_ = sfmgpu_shim::track_rows(cfg.max_tracks, cfg.min_tracks);
-    void* pin = nullptr;  // page-locked staging for the S frames of a step
-    sfmgpu_shim::check(ctx, sfmgpu_host_alloc(ctx, (size_t)S_ * w * h, &pin), "host_alloc");
-    stage_ = std::shared_ptr<uint8_t>((uint8_t*)pin, [](uint8_t* p) { sfmgpu_host_free(sfmgpu_shim::context(), p); });
-  }
+  MultiKLTTracker(LKConfig cfg, int n_sequences, int w, int h)
+      : MultiKLTTracker(cfg, std::vector<std::pair<int, int>>((size_t)(n_sequences > 0 ? n_sequences : 0), {w, h}), false) {}
+  MultiKLTTracker(LKConfig cfg, std::vector<std::pair<int, int>> sizes) : MultiKLTTracker(cfg, std::move(sizes), true) {}
 
   // frames[s] = the next frame of sequence s; returns one StepOut per sequence (empty on the first call)
   std::vector<KLTTracker::StepOut> step(const std::vector<const GrayImage*>& frames) {
     auto* ctx = sfmgpu_shim::context();
     if ((int)frames.size() != S_) throw std::runtime_error("sfmgpu: MultiKLTTracker::step: one frame per sequence expected");
-    const size_t px = (size_t)w_ * h_;
+    size_t off = 0;
     for (int s = 0; s < S_; s++) {
-      if (!frames[s] || frames[s]->w != w_ || frames[s]->h != h_) throw std::runtime_error("sfmgpu: MultiKLTTracker::step: frame size differs");
-      std::copy(frames[s]->pix.begin(), frames[s]->pix.begin() + px, stage_.get() + (size_t)s * px);
+      const int w = sizes_[s].first, h = sizes_[s].second;
+      if (!frames[s] || frames[s]->w != w || frames[s]->h != h)
+        throw std::runtime_error("sfmgpu: MultiKLTTracker::step: frame " + std::to_string(s) + " is not " + std::to_string(w) + "x" +
+                                 std::to_string(h));
+      const size_t px = (size_t)w * h;
+      std::copy(frames[s]->pix.begin(), frames[s]->pix.begin() + px, stage_.get() + off);
+      off += px;
     }
     std::vector<double> prev(2 * (size_t)S_ * cap_), cur(2 * (size_t)S_ * cap_);
     std::vector<std::int32_t> ids((size_t)S_ * cap_), n((size_t)S_);
@@ -515,13 +507,53 @@ class MultiKLTTracker {
     const sfmgpu_ransac_cfg rc{iters, thr, min_inliers, 1};
     sfmgpu_shim::check(ctx, sfmgpu_multitracker_set_ransac(ctx, trk_.get(), K.a.data(), &rc), "multitracker_set_ransac");
   }
+  // Same with one camera per sequence: find_E_ransac(K[s], ...) for sequence s
+  void set_two_view(const std::vector<Mat33>& K, int iters, double thr, int min_inliers) {
+    auto* ctx = sfmgpu_shim::context();
+    if ((int)K.size() != S_) throw std::runtime_error("sfmgpu: MultiKLTTracker::set_two_view: one K per sequence expected");
+    std::vector<double> k9(9 * (size_t)S_);
+    for (int s = 0; s < S_; s++) std::copy(K[s].a.begin(), K[s].a.end(), k9.begin() + 9 * (size_t)s);
+    const sfmgpu_ransac_cfg rc{iters, thr, min_inliers, 1};
+    sfmgpu_shim::check(ctx, sfmgpu_multitracker_set_ransac_cameras(ctx, trk_.get(), k9.data(), &rc), "multitracker_set_ransac_cameras");
+  }
 
   sfmgpu_multitracker* handle() const { return trk_.get(); }
   int n_sequences() const { return S_; }
   int rows() const { return cap_; }
 
  private:
-  int S_, w_, h_, cap_ = 0;
+  MultiKLTTracker(LKConfig cfg, std::vector<std::pair<int, int>> sizes, bool sized) : S_((int)sizes.size()), sizes_(std::move(sizes)) {
+    sfmgpu_lkcfg c;
+    c.max_tracks = cfg.max_tracks;
+    c.min_tracks = cfg.min_tracks;
+    c.quality = cfg.quality;
+    c.min_distance = cfg.min_distance;
+    c.pyr_levels = cfg.pyr_levels;
+    c.win_radius = cfg.win_radius;
+    c.iters = cfg.iters;
+    c.fb_thresh = cfg.fb_thresh;
+    sfmgpu_multitracker* t = nullptr;
+    auto* ctx = sfmgpu_shim::context();
+    size_t px = 0;
+    std::vector<std::int32_t> ws((size_t)S_), hs((size_t)S_);
+    for (int s = 0; s < S_; s++) {
+      ws[s] = sizes_[s].first;
+      hs[s] = sizes_[s].second;
+      px += (size_t)(ws[s] > 0 ? ws[s] : 0) * (size_t)(hs[s] > 0 ? hs[s] : 0);
+    }
+    if (sized)
+      sfmgpu_shim::check(ctx, sfmgpu_multitracker_create_sized(ctx, &c, S_, ws.data(), hs.data(), &t), "multitracker_create_sized");
+    else
+      sfmgpu_shim::check(ctx, sfmgpu_multitracker_create(ctx, &c, S_, S_ > 0 ? ws[0] : 0, S_ > 0 ? hs[0] : 0, &t), "multitracker_create");
+    trk_ = std::shared_ptr<sfmgpu_multitracker>(t, [](sfmgpu_multitracker* p) { sfmgpu_multitracker_destroy(sfmgpu_shim::context(), p); });
+    cap_ = sfmgpu_shim::track_rows(cfg.max_tracks, cfg.min_tracks);
+    void* pin = nullptr;  // page-locked staging for the S frames of a step, back to back
+    sfmgpu_shim::check(ctx, sfmgpu_host_alloc(ctx, px, &pin), "host_alloc");
+    stage_ = std::shared_ptr<uint8_t>((uint8_t*)pin, [](uint8_t* p) { sfmgpu_host_free(sfmgpu_shim::context(), p); });
+  }
+
+  int S_, cap_ = 0;
+  std::vector<std::pair<int, int>> sizes_;
   std::shared_ptr<sfmgpu_multitracker> trk_;
   std::shared_ptr<uint8_t> stage_;
 };

@@ -47,6 +47,7 @@ SYMBOLS = [
     "sfmgpu_sched_segment_shard", "sfmgpu_sched_gather_pair_ids",
     "sfmgpu_pack_bound", "sfmgpu_frames_pack", "sfmgpu_frames_upload_packed", "sfmgpu_pair_frontend_host_packed",
     "sfmgpu_multitracker_prefetch_packed", "sfmgpu_multitracker_step_packed",
+    "sfmgpu_multitracker_create_sized", "sfmgpu_multitracker_set_ransac_cameras",
 ]
 
 
@@ -192,6 +193,8 @@ def load_library():
         "sfmgpu_frames_upload_packed": (_i, [_vp, _vp, _i, _vp, C.c_size_t, _i, _i]),
         "sfmgpu_pair_frontend_host_packed": (_i, [_vp, _vp, _vp, C.c_size_t, _i, _i, C.POINTER(LKCfg), _vp, _i, _vp, _vp, _vp, _vp]),
         "sfmgpu_multitracker_prefetch_packed": (_i, [_vp, _vp, _vp, _vp, _vp]),
+        "sfmgpu_multitracker_create_sized": (_i, [_vp, C.POINTER(LKCfg), _i, _vp, _vp, C.POINTER(_vp)]),
+        "sfmgpu_multitracker_set_ransac_cameras": (_i, [_vp, _vp, _vp, C.POINTER(RansacCfg)]),
         "sfmgpu_multitracker_step_packed": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     }
     for name, (res, args) in S.items():
@@ -427,6 +430,7 @@ class Context:
         return Tracker(self, cfg if cfg is not None else lkcfg(**kw))
 
     def multitracker(self, n_sequences, w, h, cfg=None, **kw):
+        """w, h: one size for all sequences, or length-S sequences (sequence s has w[s] x h[s] images)."""
         return MultiTracker(self, n_sequences, w, h, cfg if cfg is not None else lkcfg(**kw))
 
 
@@ -766,8 +770,18 @@ class MultiTracker:
     def __init__(self, ctx, n_sequences, w, h, cfg):
         self.ctx, self.cfg, self.S, self.w, self.h = ctx, cfg, n_sequences, w, h
         p = _vp()
-        ctx._ck(ctx.lib.sfmgpu_multitracker_create(ctx.h, C.byref(cfg), n_sequences, w, h, C.byref(p)))
+        if np.ndim(w) or np.ndim(h):  # per-sequence sizes: sfmgpu_multitracker_create_sized
+            ws = np.ascontiguousarray(np.broadcast_to(np.asarray(w), (n_sequences,)), np.int32)
+            hs = np.ascontiguousarray(np.broadcast_to(np.asarray(h), (n_sequences,)), np.int32)
+            ctx._ck(ctx.lib.sfmgpu_multitracker_create_sized(ctx.h, C.byref(cfg), n_sequences, _ptr(ws), _ptr(hs), C.byref(p)))
+            self.sizes = [(int(a), int(b)) for a, b in zip(ws, hs)]
+            if len(set(self.sizes)) == 1:  # one size: [S, h, w] arrays are accepted as by create
+                self.w, self.h = self.sizes[0]
+        else:
+            ctx._ck(ctx.lib.sfmgpu_multitracker_create(ctx.h, C.byref(cfg), n_sequences, w, h, C.byref(p)))
+            self.sizes = [(w, h)] * n_sequences
         self.h_ = p
+        self._stage, self._si = None, 0  # page-locked staging for frames given as a list (three: current, prefetch, previous prefetch)
         self.cap = max(1, cfg.max_tracks, cfg.min_tracks) + 1
         self.prev = ctx.pinned_empty((n_sequences, self.cap, 2), np.float64)
         self.cur = ctx.pinned_empty((n_sequences, self.cap, 2), np.float64)
@@ -788,17 +802,32 @@ class MultiTracker:
     def _frames(self, imgs):
         if imgs is None:
             return None
+        if isinstance(imgs, (list, tuple)):  # per-sequence 2-D arrays: packed back to back into page-locked staging
+            assert len(imgs) == self.S, (len(imgs), self.S)
+            if self._stage is None:
+                total = sum(w * h for w, h in self.sizes)
+                self._stage = [self.ctx.pinned_empty((total,), np.uint8) for _ in range(3)]
+            buf = self._stage[self._si]
+            self._si = (self._si + 1) % 3
+            o = 0
+            for (w, h), im in zip(self.sizes, imgs):
+                assert im.shape == (h, w), (im.shape, (h, w))
+                buf[o:o + w * h].reshape(h, w)[...] = im
+                o += w * h
+            return buf
         imgs = np.ascontiguousarray(imgs, np.uint8)
         assert imgs.shape == (self.S, self.h, self.w)
         return imgs
 
     def prefetch(self, imgs):
-        """Start uploading the frames of the next step (page-locked memory for the overlap); step(None, ...) consumes them."""
+        """Start uploading the frames of the next step (page-locked memory for the overlap); step(None, ...) consumes them.
+        imgs: [S, h, w] uint8, or a list of S per-sequence 2-D arrays (any tracker; the only form for mixed sizes)."""
         self._pf = self._frames(imgs)  # keep the buffer alive while the copy runs
         self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_prefetch(self.ctx.h, self.h_, _ptr(self._pf)))
 
     def step(self, imgs, fetch=True, next_imgs=None):
-        """imgs: [S, h, w] uint8, the next frame of every sequence (None: the prefetched ones); next_imgs: the frames of
+        """imgs: [S, h, w] uint8 or a list of S 2-D arrays of the sequences' own sizes, the next frame of every sequence (None:
+        the prefetched ones); next_imgs: the frames of
         the following step, uploaded while this one computes.  Returns per sequence (prev_xy, cur_xy, ids) of the
         survivors (copies), or the survivor counts when fetch is False."""
         imgs, self._pf = self._frames(imgs), self._frames(next_imgs)
@@ -875,12 +904,18 @@ class MultiTracker:
     # ---- RANSAC stage: find_E_ransac(K, prev_pts, cur_pts, ...) on every sequence's survivors inside the step -------------
     def set_ransac(self, K, iters=2500, thr=1e-3, min_inliers=60, min_points=1):
         """Make find_E_ransac(K, prev_pts, cur_pts, iters, thr, min_inliers) part of every later step (K None: off again);
-        min_points=1 skips sequences without survivors, as the reference's `prev_pts.empty()` guard does."""
+        min_points=1 skips sequences without survivors, as the reference's `prev_pts.empty()` guard does.  K: one (3, 3)
+        camera, or (S, 3, 3): camera K[s] for sequence s (sfmgpu_multitracker_set_ransac_cameras)."""
         if K is None:
             self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_set_ransac(self.ctx.h, self.h_, None, None))
             return
-        K = np.ascontiguousarray(K, np.float64).reshape(9)
+        K = np.ascontiguousarray(K, np.float64)
         rc = RansacCfg(iters, thr, min_inliers, min_points)
+        if K.ndim == 3:
+            assert K.shape == (self.S, 3, 3), K.shape
+            self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_set_ransac_cameras(self.ctx.h, self.h_, K.ctypes.data_as(_vp), C.byref(rc)))
+            return
+        K = K.reshape(9)
         self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_set_ransac(self.ctx.h, self.h_, K.ctypes.data_as(_vp), C.byref(rc)))
 
     def ransac_results(self):
