@@ -78,7 +78,7 @@ int sfmgpu_flush_l2(sfmgpu_ctx* ctx, size_t bytes);
 int sfmgpu_profile(sfmgpu_ctx* ctx, int enable);
 int sfmgpu_stage_times(sfmgpu_ctx* ctx, float* ms4);
 /* Same with n values: ms[4] = the RANSAC stage of the two-view unit (sfmgpu_pairs_set_ransac, sfmgpu_multitracker_set_ransac),
- * ms[5] = the frame gather of sfmgpu_pair_frontend_list and sfmgpu_multitracker_step_frames, ms[6] = the tile decode of the
+ * ms[5] = the frame gather of sfmgpu_pair_frontend_list and sfmgpu_multitracker_step_frames(_sized), ms[6] = the tile decode of the
  * packed-input calls (sfmgpu_frames_upload_packed, sfmgpu_pair_frontend_host_packed, sfmgpu_multitracker_step_packed). */
 int sfmgpu_stage_times_n(sfmgpu_ctx* ctx, float* ms, int n);
 /* Measured non-tensor FP64 throughput of this GPU (DFMA micro-benchmark, ~10 ms): the KLT / RANSAC roofline. */
@@ -387,9 +387,10 @@ int sfmgpu_multitracker_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_s
  * sfmgpu_multitracker_create and every entry point behaves exactly as on such a tracker.  Otherwise the tracker is "mixed": the
  * sequences of one size share a frame batch, uploads and pyramids run per size, and the KLT stage is still one chain of launches
  * for all S sequences (per-sequence geometry), so sequence s gives, byte for byte, what a one-sequence tracker of its size gives
- * under the same kernel family (sfmgpu_klt_set_mode).  Every output keeps its [S][ROWS] layout in sequence order.  Not built yet
- * for mixed trackers: packed and resident input - sfmgpu_multitracker_step_frames, _prefetch_packed and _step_packed return
- * SFMGPU_E_ARG before any work is queued. */
+ * under the same kernel family (sfmgpu_klt_set_mode).  Every output keeps its [S][ROWS] layout in sequence order.  Packed input
+ * (_step_packed, _prefetch_packed) reads sequence s's frames at its own size; resident input takes one frame batch per sequence
+ * (sfmgpu_multitracker_step_frames_sized), since sfmgpu_multitracker_step_frames' single batch holds one size (it refuses a
+ * mixed tracker with SFMGPU_E_ARG). */
 int sfmgpu_multitracker_create_sized(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int n_sequences, const int32_t* w, const int32_t* h,
                                      sfmgpu_multitracker** out);
 void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t);
@@ -407,13 +408,15 @@ int sfmgpu_multitracker_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const 
 int sfmgpu_multitracker_step_pipelined(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* host_pix, const uint8_t* next_host_pix,
                                        double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 /* Packed frames (the blob format of sfmgpu_frames_upload_packed) as the lock-step tracker's input.  blobs[s] / blob_bytes[s]:
- * the blob that sequence s reads from (host memory; pinned for overlap).  The same blob may serve several sequences: a
- * step-major blob holds frame t of sequence s as blob frame t*S + s.  Sequence s's next frame is blob frame blob_frame[s].
+ * the blob that sequence s reads from (host memory; pinned for overlap), holding frames of sequence s's size.  The same blob
+ * may serve several sequences of one size: a step-major blob holds frame t of sequence s as blob frame t*S + s (with sizes that
+ * differ, one step-major blob per size).  Sequence s's next frame is blob frame blob_frame[s].
  * The S frame records are copied into the tracker's own staging (one cudaMemcpyAsync per run of records adjacent in host
  * memory: one copy per step for a step-major blob), decoded in one launch (sfmgpu_stage_times_n ms[6]) and their pyramids
  * built; results are identical to sfmgpu_multitracker_step with the raw frames.  NULL blobs, blob_bytes or blob_frame, a NULL
- * entry, a blob that sfmgpu_frames_upload_packed would refuse for the tracker's w x h, a frame index outside its blob or a
- * frame record larger than sfmgpu_pack_bound allows: SFMGPU_E_ARG, before any work is queued.  Frames already prefetched:
+ * entry, one blob given to sequences of different sizes, a blob that sfmgpu_frames_upload_packed would refuse for sequence s's
+ * size, a frame index outside its blob or a frame record larger than sfmgpu_pack_bound allows for sequence s's size:
+ * SFMGPU_E_ARG (the message names s), before any work is queued.  Frames already prefetched:
  * SFMGPU_E_STATE.  The caller keeps the blobs valid and unmodified until the step that consumes the prefetch returns. */
 int sfmgpu_multitracker_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, const uint8_t* const* blobs,
                                         const size_t* blob_bytes, const int32_t* blob_frame);
@@ -428,11 +431,20 @@ int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, con
                                     double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 /* Resident frames: the next frame of sequence s is frame frame_idx[s] of f (pyramids built; same w, h and level count as the
  * tracker), any indices, repeats allowed - no host-to-device copy of images.  The S pyramids are copied into the tracker's own
- * slots (about 1.33 * w * h bytes read and written per sequence with 3 levels; sfmgpu_stage_times_n ms[5]).  Results identical to
+ * slots by one launch (about 1.33 * w * h bytes read and written per sequence with 3 levels; sfmgpu_stage_times_n ms[5]).
+ * The tracker's sequences must have one size (SFMGPU_E_ARG otherwise: see _step_frames_sized).  Results identical to
  * sfmgpu_multitracker_step with those images.  Prefetched frames pending: SFMGPU_E_STATE; a NULL frame_idx, an index outside
  * [0, f->n) or a size / level mismatch: SFMGPU_E_ARG; both before any work is queued. */
 int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* f, const int32_t* frame_idx,
                                     double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
+/* Resident frames for any tracker, mixed or not: sequence s's next frame is frame frame_idx[s] of batch f[s] (pyramids built).
+ * f[s] is w[s] x h[s] with the tracker's level count; one batch may serve several sequences, indices may repeat.  The S
+ * pyramids are copied into the tracker's slots by one launch (sfmgpu_stage_times_n ms[5]).  Results equal
+ * sfmgpu_multitracker_step with those images.  A NULL f, frame_idx or entry of f, a size or level mismatch of f[s] or an index
+ * outside [0, f[s]->n): SFMGPU_E_ARG (the message names s); prefetched frames pending: SFMGPU_E_STATE; all before any work is
+ * queued. */
+int sfmgpu_multitracker_step_frames_sized(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* const* f, const int32_t* frame_idx,
+                                          double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 /* Back to the state after create (the next step resets every sequence, ids restart at 0). */
 int sfmgpu_multitracker_reset(sfmgpu_ctx* ctx, sfmgpu_multitracker* t);
 int sfmgpu_multitracker_tracks(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int sequence, double* xy, int32_t* ids, int cap, int* n_out);

@@ -246,10 +246,24 @@ __global__ void __launch_bounds__(NT) pk_write_kernel(const uint8_t* __restrict_
 // ---- decoder: one block per tile --------------------------------------------------------------------------------------
 // stage holds blob bytes from absolute offset `base` on; fo[k] = absolute offset of frame k of the launch (the host has checked
 // fo against the blob, and that every frame holds its tile table).  A tile whose record does not decode sets *bad and writes
-// nothing.
+// nothing.  TABLE = false: frames [first, first + gridDim.y) of one batch, grid (ntiles, frames).  TABLE = true: frames of any
+// sizes, frame k of the launch into frames[k] (lvl0 ... ntiles are taken from there, fstride and first are 0); grid (the largest
+// tile count, frames), and blocks past their frame's tile count return at once.
+template <bool TABLE>
 __global__ void __launch_bounds__(NT) pk_decode_kernel(const uint8_t* __restrict__ stage, const unsigned long long* __restrict__ fo,
                                                        unsigned long long base, uint8_t* __restrict__ lvl0, int pitch, size_t fstride,
-                                                       int first, int w, int h, int tiles_x, int ntiles, int* __restrict__ bad) {
+                                                       int first, int w, int h, int tiles_x, int ntiles, int* __restrict__ bad,
+                                                       const PkDst* __restrict__ frames) {
+  if constexpr (TABLE) {
+    const PkDst d = frames[blockIdx.y];
+    if ((int)blockIdx.x >= d.ntiles) return;
+    lvl0 = d.lvl0;
+    pitch = d.pitch;
+    w = d.w;
+    h = d.h;
+    tiles_x = d.tiles_x;
+    ntiles = d.ntiles;
+  }
   __shared__ uint32_t rec[RAW_MAX_WORDS + 1];
   __shared__ uint32_t tile[TILE][TILE + 1];
   __shared__ uint16_t zpos[MAXV];
@@ -473,10 +487,25 @@ int sfm_pk_decode(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count, const
   const int nt = ntiles_of(f->w, f->h);
   for (int k = 0; k < count; k += 65535) {
     const int c = count - k < 65535 ? count - k : 65535;
-    SFM_LAUNCH(ctx, pk_decode_kernel, dim3(nt, c), NT, 0, stage, d_fo + k, base, f->lvl[0], f->pitch[0], f->fstride[0], first + k,
-               f->w, f->h, tiles_x_of(f->w), nt, d_bad);
+    SFM_LAUNCH(ctx, pk_decode_kernel<false>, dim3(nt, c), NT, 0, stage, d_fo + k, base, f->lvl[0], f->pitch[0], f->fstride[0], first + k,
+               f->w, f->h, tiles_x_of(f->w), nt, d_bad, (const PkDst*)nullptr);
   }
   return 0;
+}
+
+// Decode of `count` frames of any sizes on ctx->stream: frame k (records staged from offset 0 on, d_fo its count + 1 offsets)
+// into d_dst[k]; max_tiles = the largest tile count of the entries.
+int sfm_pk_decode_table(sfmgpu_ctx* ctx, const PkDst* d_dst, int count, int max_tiles, const uint8_t* stage,
+                        const unsigned long long* d_fo, int* d_bad) {
+  StageTimer st(ctx, 6);
+  if (count > 0)
+    SFM_LAUNCH(ctx, pk_decode_kernel<true>, dim3(max_tiles, count), NT, 0, stage, d_fo, 0ull, (uint8_t*)nullptr, 0, (size_t)0, 0, 0, 0, 0,
+               0, d_bad, d_dst);
+  return 0;
+}
+
+PkDst sfm_pk_dst(const sfmgpu_frames* f, int frame) {
+  return {f->lvl[0] + (size_t)frame * f->fstride[0], f->pitch[0], f->w, f->h, tiles_x_of(f->w), ntiles_of(f->w, f->h)};
 }
 
 // The largest frame record a blob of w x h frames can hold (every tile raw).

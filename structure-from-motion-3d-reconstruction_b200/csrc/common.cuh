@@ -136,6 +136,14 @@ int sfm_pk_check(sfmgpu_ctx* ctx, const sfmgpu_frames* f, const uint8_t* blob, s
 int sfm_pk_decode(sfmgpu_ctx* ctx, sfmgpu_frames* f, int first, int count, const uint8_t* stage, const unsigned long long* d_fo,
                   unsigned long long base, int* d_bad);
 int sfm_pk_prepare(sfmgpu_ctx* ctx, const uint8_t* blob, int blob_first, const std::vector<uint64_t>& fo, size_t stage_bytes, int nstage);
+// Level-0 destination of one frame of a decode over frames of different sizes (sfm_pk_decode_table).
+struct PkDst {
+  uint8_t* lvl0;  // the frame's level-0 base
+  int pitch, w, h, tiles_x, ntiles;
+};
+PkDst sfm_pk_dst(const sfmgpu_frames* f, int frame);
+int sfm_pk_decode_table(sfmgpu_ctx* ctx, const PkDst* d_dst, int count, int max_tiles, const uint8_t* stage,
+                        const unsigned long long* d_fo, int* d_bad);
 size_t sfm_pk_frame_bound(int w, int h);
 size_t sfm_pk_max_chunk_bytes(const std::vector<uint64_t>& fo, int chunk);
 int sfm_pk_read_flag(sfmgpu_ctx* ctx, const char* who);

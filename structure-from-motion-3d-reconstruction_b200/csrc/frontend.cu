@@ -4,6 +4,8 @@
 // Everything stays on the device between stages; only survivors / counts are copied back when the caller asks.
 #include <stdlib.h>
 
+#include <string>
+#include <unordered_map>
 #include <utility>
 #include <vector>
 
@@ -166,6 +168,21 @@ __global__ void __launch_bounds__(256) gather_frames_kernel(const uint8_t* __res
   const uint4* s = reinterpret_cast<const uint4*>(src + (size_t)sf * fstride);
   uint4* d = reinterpret_cast<uint4*>(dst + (size_t)df * fstride);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (size_t)gridDim.x * blockDim.x) d[i] = s[i];
+}
+
+// One whole-frame copy of a pyramid level: n16 16-byte words from src to dst.
+struct FrameCopy {
+  const uint4* src;
+  uint4* dst;
+  unsigned long long n16;
+};
+
+// Lock-step tracker, resident input: copy tab[blockIdx.y] for every (sequence, level) entry of the table in one launch, 16 B per
+// thread and step.
+__global__ void __launch_bounds__(256) copy_frames_kernel(const FrameCopy* __restrict__ tab) {
+  const FrameCopy c = tab[blockIdx.y];
+#pragma unroll 4
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < c.n16; i += (size_t)gridDim.x * blockDim.x) c.dst[i] = c.src[i];
 }
 
 int default_cand_cap(int w, int h) {
@@ -1270,6 +1287,7 @@ struct sfmgpu_multitracker {
   struct SizeClass {
     int w, h, n;
     sfmgpu_frames* frames;
+    size_t pk_bound;  // the largest packed record of a w x h frame (sfm_pk_frame_bound)
   };
   // Adjacent sequences of one class: one upload.  host_off: where sequence s0's frame starts in the caller's S frames.
   struct Run {
@@ -1280,17 +1298,20 @@ struct sfmgpu_multitracker {
   std::vector<Run> runs;
   std::vector<int> cls_of, idx_in;  // per sequence: its class and its index in that class
   KltGeo* geo = nullptr;            // mixed: [3][S] geometry tables, steps from group g to group (g+1)%3 read entries g*S ...
+  PkDst* pkdst = nullptr;           // mixed: [3][S] packed-decode destinations, group g of sequence s at g*S + s
+  int pk_tiles = 0;                 // mixed: the largest tile count of a sequence's frame
   bool mixed() const { return cls.size() > 1; }
   int parity = -1;                  // slot group of the previous frames, -1: nothing tracked yet
   bool prefetched = false;          // group (parity+1)%3 holds the next frames (uploaded + pyramids), ready at pf_done
   cudaEvent_t pf_done = nullptr;
   TrackLists L;                     // list s: sequence s
-  int* didx = nullptr;              // step_frames: the frame index of every sequence (device copy for the gather)
+  FrameCopy* gtab = nullptr;        // resident input: the gather's (sequence, level) table, [S][levels] entries at most
   TwoViewState* tv = nullptr;       // find_E_ransac on every sequence's survivors inside the step (sfmgpu_multitracker_set_ransac)
   bool tv_fresh = false;            // the last step ran the stage: its results can be downloaded
   // packed input (sfmgpu_multitracker_step_packed): the tracker's own device buffer [decode flag | staged frame offsets [S+1] |
-  // S frame records back to back], allocated by the first packed call, so that no other call on the context can overwrite a
-  // pending prefetch.  pk_done follows the last decode that read the staging; pk_bad receives the flag.
+  // S frame records back to back, sum over s of the bound of a w[s] x h[s] record], allocated by the first packed call, so that
+  // no other call on the context can overwrite a pending prefetch.  pk_done follows the last decode that read the staging;
+  // pk_bad receives the flag.
   uint8_t* pk = nullptr;
   int* pk_bad = nullptr;            // page-locked host copy of the decode flag
   cudaEvent_t pk_done = nullptr;
@@ -1337,7 +1358,7 @@ static int multi_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int S, const i
   for (int s = 0; s < S; s++) {
     int c = 0;
     while (c < (int)t->cls.size() && (t->cls[c].w != w[s] || t->cls[c].h != h[s])) c++;
-    if (c == (int)t->cls.size()) t->cls.push_back({w[s], h[s], 0, nullptr});
+    if (c == (int)t->cls.size()) t->cls.push_back({w[s], h[s], 0, nullptr, sfm_pk_frame_bound(w[s], h[s])});
     t->cls_of[s] = c;
     t->idx_in[s] = t->cls[c].n++;
     if (s > 0 && t->cls_of[s - 1] == c)
@@ -1357,11 +1378,21 @@ static int multi_create(sfmgpu_ctx* ctx, const sfmgpu_lkcfg* cfg, int S, const i
   t->w = t->cls[0].w;
   t->h = t->cls[0].h;
   cudaError_t e = lists_alloc(ctx, t->L, *cfg, S);
-  if (e == cudaSuccess) e = cudaMalloc((void**)&t->didx, (size_t)S * 4 + 256);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&t->gtab, (size_t)S * SFM_MAXL * sizeof(FrameCopy));
   if (e == cudaSuccess && t->mixed()) {
     const std::vector<KltGeo> geo = multi_geo_tables(t);
     e = cudaMalloc((void**)&t->geo, geo.size() * sizeof(KltGeo));
     if (e == cudaSuccess) e = cudaMemcpy(t->geo, geo.data(), geo.size() * sizeof(KltGeo), cudaMemcpyHostToDevice);
+    // packed input: level 0 of group g of sequence s, decoded by one launch over all S frames of a step
+    std::vector<PkDst> dst((size_t)3 * S);
+    for (int g = 0; g < 3; g++)
+      for (int s = 0; s < S; s++) {
+        const sfmgpu_multitracker::SizeClass& c = t->cls[t->cls_of[s]];
+        dst[(size_t)g * S + s] = sfm_pk_dst(c.frames, g * c.n + t->idx_in[s]);
+        if (dst[(size_t)g * S + s].ntiles > t->pk_tiles) t->pk_tiles = dst[(size_t)g * S + s].ntiles;
+      }
+    if (e == cudaSuccess) e = cudaMalloc((void**)&t->pkdst, dst.size() * sizeof(PkDst));
+    if (e == cudaSuccess) e = cudaMemcpy(t->pkdst, dst.data(), dst.size() * sizeof(PkDst), cudaMemcpyHostToDevice);
   }
   if (e != cudaSuccess) {
     sfmgpu_multitracker_destroy(ctx, t);
@@ -1401,8 +1432,9 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
   if (t->pf_done) cudaEventSynchronize(t->pf_done);  // a prefetch still running on the copy stream
   sfm_two_view_free(ctx, &t->tv);
   lists_free(t->L);
-  if (t->didx) cudaFree(t->didx);
+  if (t->gtab) cudaFree(t->gtab);
   if (t->geo) cudaFree(t->geo);
+  if (t->pkdst) cudaFree(t->pkdst);
   for (sfmgpu_multitracker::SizeClass& c : t->cls)
     if (c.frames) sfmgpu_frames_destroy(ctx, c.frames);
   if (t->pk) cudaFree(t->pk);
@@ -1416,15 +1448,20 @@ void sfmgpu_multitracker_destroy(sfmgpu_ctx* ctx, sfmgpu_multitracker* t) {
 static int multi_next_group(const sfmgpu_multitracker* t) { return t->parity < 0 ? 0 : (t->parity + 1) % 3; }
 static int multi_step_on(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int par, double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out);
 
+// The pyramids of slot group g (level 0 written), one build per size class, on ctx->stream.
+static int multi_pyramids(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g) {
+  for (const sfmgpu_multitracker::SizeClass& c : t->cls) SFM_TRY(sfmgpu_pyramid_build(ctx, c.frames, g * c.n, c.n));
+  return 0;
+}
+
 // The S frames of one step (back to back in sequence order, frame s of w[s] x h[s] bytes) into slot group g, one copy per run of
-// adjacent sequences of one size, then the pyramids of every class, on ctx->stream.
+// adjacent sequences of one size, then the pyramids, on ctx->stream.
 static int multi_upload(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g, const uint8_t* host_pix) {
   for (const sfmgpu_multitracker::Run& r : t->runs) {
     const sfmgpu_multitracker::SizeClass& c = t->cls[r.cls];
     SFM_TRY(sfmgpu_frames_upload(ctx, c.frames, g * c.n + r.i0, r.count, host_pix + r.host_off));
   }
-  for (const sfmgpu_multitracker::SizeClass& c : t->cls) SFM_TRY(sfmgpu_pyramid_build(ctx, c.frames, g * c.n, c.n));
-  return 0;
+  return multi_pyramids(ctx, t, g);
 }
 
 // Upload + pyramids of the frames of a LATER step on the copy stream, into the slot group after `after_group`.
@@ -1443,9 +1480,9 @@ static int multi_prefetch(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int after_gro
   return 0;
 }
 
-// Packed input: blob frame blob_frame[s] of blobs[s] for every sequence s, checked against the tracker's frames.  The records
-// are staged back to back in sequence order (fo: their offsets in the staging), with one copy per run of records that are
-// adjacent in host memory (a step-major blob: one copy per step).
+// Packed input: blob frame blob_frame[s] of blobs[s] for every sequence s, checked against the frames of sequence s's size.  The
+// records are staged back to back in sequence order (fo: their offsets in the staging), with one copy per run of records that
+// are adjacent in host memory (a step-major blob: one copy per step).
 struct PkPlan {
   struct Copy {
     const uint8_t* src;
@@ -1458,16 +1495,29 @@ struct PkPlan {
 static int multi_pk_plan(sfmgpu_ctx* ctx, const sfmgpu_multitracker* t, const uint8_t* const* blobs, const size_t* blob_bytes,
                          const int32_t* blob_frame, PkPlan& p, const char* who) {
   if (!blobs || !blob_bytes) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null blob array", who);
-  const size_t bound = sfm_pk_frame_bound(t->w, t->h);
+  if (t->mixed()) {  // a blob's header holds one size: one blob read by sequences of two sizes is never valid
+    std::unordered_map<const uint8_t*, int> first;  // blob -> the first sequence that reads it
+    for (int s = 0; s < t->L.S; s++) {
+      if (!blobs[s]) continue;
+      const int s0 = first.emplace(blobs[s], s).first->second;
+      if (t->cls_of[s0] != t->cls_of[s])
+        return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequences %d and %d have different image sizes (%dx%d, %dx%d) but read one blob", who, s0,
+                        s, t->cls[t->cls_of[s0]].w, t->cls[t->cls_of[s0]].h, t->cls[t->cls_of[s]].w, t->cls[t->cls_of[s]].h);
+    }
+  }
   std::vector<uint64_t> fo;
   p.fo.assign(1, 0);
   p.copies.clear();
   for (int s = 0; s < t->L.S; s++) {
-    SFM_TRY(sfm_pk_check(ctx, t->frames, blobs[s], blob_bytes[s], blob_frame[s], 1, fo, who));
+    const sfmgpu_multitracker::SizeClass& c = t->cls[t->cls_of[s]];
+    if (sfm_pk_check(ctx, c.frames, blobs[s], blob_bytes[s], blob_frame[s], 1, fo, who) != 0) {
+      const std::string m = ctx->err;
+      return sfm_fail(ctx, SFMGPU_E_ARG, "%s (sequence %d, %dx%d)", m.c_str(), s, c.w, c.h);
+    }
     const size_t bytes = fo[1] - fo[0];
-    if (bytes > bound)
+    if (bytes > c.pk_bound)
       return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequence %d: frame record of %zu bytes, a %dx%d frame holds at most %zu", who, s, bytes,
-                      t->w, t->h, bound);
+                      c.w, c.h, c.pk_bound);
     const uint8_t* src = blobs[s] + fo[0];
     if (!p.copies.empty() && p.copies.back().src + p.copies.back().bytes == src)
       p.copies.back().bytes += bytes;
@@ -1484,7 +1534,11 @@ static int multi_pk_decode(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g, const
   const int S = t->L.S;
   const size_t o_fo = 16, o_stage = (o_fo + 8 * ((size_t)S + 1) + 15) & ~(size_t)15;
   // each piece on its own: a call after a failed allocation completes what is missing
-  if (!t->pk) SFM_CUDA(ctx, cudaMalloc(&t->pk, o_stage + (size_t)S * sfm_pk_frame_bound(t->w, t->h)));
+  if (!t->pk) {
+    size_t records = 0;
+    for (const sfmgpu_multitracker::SizeClass& c : t->cls) records += (size_t)c.n * c.pk_bound;
+    SFM_CUDA(ctx, cudaMalloc(&t->pk, o_stage + records));
+  }
   if (!t->pk_bad) SFM_CUDA(ctx, cudaMallocHost(&t->pk_bad, sizeof(int)));
   if (!t->pk_done) SFM_CUDA(ctx, cudaEventCreateWithFlags(&t->pk_done, cudaEventDisableTiming));
   int* d_bad = (int*)t->pk;
@@ -1495,7 +1549,10 @@ static int multi_pk_decode(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int g, const
   SFM_CUDA(ctx, cudaMemcpyAsync(d_fo, p.fo.data(), 8 * p.fo.size(), cudaMemcpyHostToDevice, ctx->stream));
   for (const PkPlan::Copy& c : p.copies)
     SFM_CUDA(ctx, cudaMemcpyAsync(stage + c.dst, c.src, c.bytes, cudaMemcpyHostToDevice, ctx->stream));
-  SFM_TRY(sfm_pk_decode(ctx, t->frames, g * S, S, stage, d_fo, 0, d_bad));
+  if (t->mixed())  // all S frames in one launch, each into its own size class's slot
+    SFM_TRY(sfm_pk_decode_table(ctx, t->pkdst + (size_t)g * S, S, t->pk_tiles, stage, d_fo, d_bad));
+  else
+    SFM_TRY(sfm_pk_decode(ctx, t->frames, g * S, S, stage, d_fo, 0, d_bad));
   SFM_CUDA(ctx, cudaEventRecord(t->pk_done, ctx->stream));
   t->pk_used = true;
   SFM_CUDA(ctx, cudaMemcpyAsync(t->pk_bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1507,11 +1564,11 @@ static int multi_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, int af
   SFM_TRY(pipe_streams(ctx));
   if (!t->pf_done && cudaEventCreateWithFlags(&t->pf_done, cudaEventDisableTiming) != cudaSuccess)
     return sfm_fail(ctx, SFMGPU_E_CUDA, "multitracker: cudaEventCreate failed");
-  const int S = t->L.S, g = (after_group + 1) % 3;
+  const int g = (after_group + 1) % 3;
   {
     StageScope sc(ctx, ctx->copy_stream);
     SFM_TRY(multi_pk_decode(ctx, t, g, p));
-    SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, g * S, S));
+    SFM_TRY(multi_pyramids(ctx, t, g));
     SFM_CUDA(ctx, cudaEventRecord(t->pf_done, ctx->stream));
   }
   t->prefetched = true;
@@ -1582,8 +1639,6 @@ int sfmgpu_multitracker_prefetch_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t,
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
   const char* who = "multitracker_prefetch_packed";
-  if (t->mixed())
-    return sfm_fail(ctx, SFMGPU_E_ARG, "%s: the sequences have different image sizes; packed and resident input take one size", who);
   if (!blob_frame) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null frame index array", who);
   if (t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: the prefetched frames have not been stepped yet", who);
   PkPlan p;
@@ -1597,20 +1652,17 @@ int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, con
   SFM_ENTER(ctx);
   if (!ctx || !t) return SFMGPU_E_ARG;
   const char* who = "multitracker_step_packed";
-  if (t->mixed())
-    return sfm_fail(ctx, SFMGPU_E_ARG, "%s: the sequences have different image sizes; packed and resident input take one size", who);
   if (!blob_frame && !t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: no frames given and none prefetched", who);
   if (blob_frame && t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: frames given but others are prefetched", who);
   PkPlan cur, next;
   if (blob_frame) SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, blob_frame, cur, who));
   if (next_blob_frame) SFM_TRY(multi_pk_plan(ctx, t, blobs, blob_bytes, next_blob_frame, next, who));
-  const int S = t->L.S;
   const int par = multi_next_group(t);
   if (blob_frame) {  // decoded and checked before the step queues anything; the pyramids only for frames that decoded
     SFM_TRY(multi_pk_decode(ctx, t, par, cur));
     SFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     if (*t->pk_bad) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: a tile record of the frames does not decode", who);
-    SFM_TRY(sfmgpu_pyramid_build(ctx, t->frames, par * S, S));
+    SFM_TRY(multi_pyramids(ctx, t, par));
   } else {
     SFM_TRY(multi_take_prefetch(ctx, t, who));
   }
@@ -1619,8 +1671,43 @@ int sfmgpu_multitracker_step_packed(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, con
   return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
 }
 
-// Resident frames: the pyramids of frame frame_idx[s] of f are copied into the current slot group (one gather launch per level),
-// so that every kernel of the step reads its frames exactly as it reads uploaded ones.
+}  // extern "C"
+
+// Resident frames: the pyramid of frame idx[s] of f[s] (checked by the caller: sequence s's size, the tracker's levels, an index
+// inside f[s]) is copied into sequence s's slot of the current group by one launch over a (sequence, level) table, so that every
+// kernel of the step reads its frames exactly as it reads uploaded ones.  Batches of one size and level count have one layout,
+// so every entry is a whole-frame copy.
+static int multi_step_resident(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* const* f, const int32_t* idx, double* prev_xy,
+                               double* cur_xy, int32_t* ids, int32_t* n_out) {
+  const int S = t->L.S, par = multi_next_group(t);
+  std::vector<FrameCopy> tab;
+  tab.reserve((size_t)S * t->cfg.pyr_levels);
+  unsigned long long most = 0;
+  for (int s = 0; s < S; s++) {
+    const sfmgpu_multitracker::SizeClass& c = t->cls[t->cls_of[s]];
+    const sfmgpu_frames* g = c.frames;
+    const size_t slot = (size_t)par * c.n + t->idx_in[s];
+    for (int l = 0; l < g->levels; l++) {
+      if (g->fstride[l] == 0) continue;  // level of zero size
+      const unsigned long long n16 = g->fstride[l] / 16;  // pitch is a multiple of 16
+      tab.push_back({reinterpret_cast<const uint4*>(f[s]->lvl[l] + (size_t)idx[s] * g->fstride[l]),
+                     reinterpret_cast<uint4*>(g->lvl[l] + slot * g->fstride[l]), n16});
+      if (n16 > most) most = n16;
+    }
+  }
+  t->tv_fresh = false;
+  SFM_CUDA(ctx, cudaMemcpyAsync(t->gtab, tab.data(), tab.size() * sizeof(FrameCopy), cudaMemcpyHostToDevice, ctx->stream));
+  {
+    StageTimer st(ctx, 5);
+    if (!tab.empty())
+      SFM_LAUNCH(ctx, copy_frames_kernel, dim3(sfm_cdiv((long long)most, 256 * 8), (unsigned)tab.size(), 1), 256, 0,
+                 (const FrameCopy*)t->gtab);
+  }
+  return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
+}
+
+extern "C" {
+
 int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* f, const int32_t* frame_idx, double* prev_xy,
                                     double* cur_xy, int32_t* ids, int32_t* n_out) {
   SFM_ENTER(ctx);
@@ -1638,19 +1725,29 @@ int sfmgpu_multitracker_step_frames(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfm
   for (int s = 0; s < S; s++)
     if (frame_idx[s] < 0 || frame_idx[s] >= f->n)
       return sfm_fail(ctx, SFMGPU_E_ARG, "multitracker_step_frames: sequence %d: frame %d outside [0,%d)", s, frame_idx[s], f->n);
-  const int par = multi_next_group(t);
-  t->tv_fresh = false;
-  SFM_CUDA(ctx, cudaMemcpyAsync(t->didx, frame_idx, (size_t)S * 4, cudaMemcpyHostToDevice, ctx->stream));
-  {
-    StageTimer st(ctx, 5);
-    for (int l = 0; l < g->levels; l++) {
-      if (g->fstride[l] == 0) continue;  // level of zero size
-      const unsigned gx = sfm_cdiv((long long)(g->fstride[l] / 16), 256 * 8);
-      SFM_LAUNCH(ctx, gather_frames_kernel, dim3(gx, S, 1), 256, 0, f->lvl[l], g->lvl[l] + (size_t)par * S * g->fstride[l], g->fstride[l],
-                 (const int*)t->didx, (const int*)t->didx, 0);
-    }
+  const std::vector<sfmgpu_frames*> fs(S, f);
+  return multi_step_resident(ctx, t, fs.data(), frame_idx, prev_xy, cur_xy, ids, n_out);
+}
+
+int sfmgpu_multitracker_step_frames_sized(sfmgpu_ctx* ctx, sfmgpu_multitracker* t, sfmgpu_frames* const* f, const int32_t* frame_idx,
+                                          double* prev_xy, double* cur_xy, int32_t* ids, int32_t* n_out) {
+  SFM_ENTER(ctx);
+  const char* who = "multitracker_step_frames_sized";
+  if (!ctx || !t) return SFMGPU_E_ARG;
+  if (!f || !frame_idx) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: null frame batch or index array", who);
+  const int S = t->L.S;
+  for (int s = 0; s < S; s++)
+    if (!f[s]) return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequence %d: null frame batch", who, s);
+  if (t->prefetched) return sfm_fail(ctx, SFMGPU_E_STATE, "%s: frames are prefetched; step them first", who);
+  for (int s = 0; s < S; s++) {
+    const sfmgpu_multitracker::SizeClass& c = t->cls[t->cls_of[s]];
+    if (f[s]->w != c.w || f[s]->h != c.h || f[s]->levels != t->cfg.pyr_levels)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequence %d: frames are %dx%d with %d levels, the sequence %dx%d with %d", who, s, f[s]->w,
+                      f[s]->h, f[s]->levels, c.w, c.h, t->cfg.pyr_levels);
+    if (frame_idx[s] < 0 || frame_idx[s] >= f[s]->n)
+      return sfm_fail(ctx, SFMGPU_E_ARG, "%s: sequence %d: frame %d outside [0,%d)", who, s, frame_idx[s], f[s]->n);
   }
-  return multi_step_on(ctx, t, par, prev_xy, cur_xy, ids, n_out);
+  return multi_step_resident(ctx, t, f, frame_idx, prev_xy, cur_xy, ids, n_out);
 }
 
 }  // extern "C"

@@ -447,8 +447,9 @@ class KLTTracker {
 // S KLTTrackers advanced in lock step (no counterpart in the reference, which tracks one sequence: this is the C++ face of
 // sfmgpu_multitracker for callers with several independent sequences per GPU).  Per sequence the results equal a
 // KLTTracker's.  The (cfg, n, w, h) form takes w x h images for every sequence; the (cfg, sizes) form gives sequence s images of
-// sizes[s] = {w, h} (cameras of different resolutions in one lock step).  Packed and resident input are not offered for the
-// latter (the C ABI refuses them for sequences of different sizes).
+// sizes[s] = {w, h} (cameras of different resolutions in one lock step).  Neither form offers packed or resident input; callers
+// who want them use the C ABI (sfmgpu_multitracker_step_packed, sfmgpu_multitracker_step_frames_sized), which takes them for
+// both.
 class MultiKLTTracker {
  public:
   MultiKLTTracker(const MultiKLTTracker&) = delete;

@@ -47,7 +47,7 @@ SYMBOLS = [
     "sfmgpu_sched_segment_shard", "sfmgpu_sched_gather_pair_ids",
     "sfmgpu_pack_bound", "sfmgpu_frames_pack", "sfmgpu_frames_upload_packed", "sfmgpu_pair_frontend_host_packed",
     "sfmgpu_multitracker_prefetch_packed", "sfmgpu_multitracker_step_packed",
-    "sfmgpu_multitracker_create_sized", "sfmgpu_multitracker_set_ransac_cameras",
+    "sfmgpu_multitracker_create_sized", "sfmgpu_multitracker_set_ransac_cameras", "sfmgpu_multitracker_step_frames_sized",
 ]
 
 
@@ -183,6 +183,7 @@ def load_library():
         "sfmgpu_sched_pair_shard": (_i, [_vp, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
         "sfmgpu_sched_gather_pairs": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
         "sfmgpu_multitracker_step_frames": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+        "sfmgpu_multitracker_step_frames_sized": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
         "sfmgpu_pair_frontend_segments": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(LKCfg), _vp]),
         "sfmgpu_pairs_ids_download_all": (_i, [_vp, _vp, _vp]),
         "sfmgpu_pairs_ids_device_ptr": (_i, [_vp, C.POINTER(_vp)]),
@@ -849,12 +850,20 @@ class MultiTracker:
         return [(self.prev[s, :self.n[s]].copy(), self.cur[s, :self.n[s]].copy(), self.ids[s, :self.n[s]].copy()) for s in range(self.S)]
 
     def step_frames(self, frames, frame_idx, fetch=True):
-        """step() with the next frame of sequence s = frame frame_idx[s] of the resident batch `frames` (pyramids built)."""
+        """step() with the next frame of sequence s = frame frame_idx[s] of the resident batch `frames` (pyramids built), or,
+        with a list of S batches, of frames[s] (sfmgpu_multitracker_step_frames_sized: any tracker, one batch per sequence
+        of its size; a batch may serve several sequences)."""
         idx = np.ascontiguousarray(frame_idx, np.int32).reshape(-1)
         assert len(idx) == self.S, (len(idx), self.S)
         a = (self.prev, self.cur, self.ids) if fetch else (None, None, None)
-        self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_step_frames(self.ctx.h, self.h_, frames.h_, _ptr(idx), _ptr(a[0]), _ptr(a[1]),
-                                                                  _ptr(a[2]), self.n.ctypes.data_as(_vp)))
+        if isinstance(frames, (list, tuple)):
+            assert len(frames) == self.S, (len(frames), self.S)
+            fs = (_vp * self.S)(*[None if f is None else f.h_ for f in frames])
+            self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_step_frames_sized(self.ctx.h, self.h_, fs, _ptr(idx), _ptr(a[0]), _ptr(a[1]),
+                                                                            _ptr(a[2]), self.n.ctypes.data_as(_vp)))
+        else:
+            self.ctx._ck(self.ctx.lib.sfmgpu_multitracker_step_frames(self.ctx.h, self.h_, frames.h_, _ptr(idx), _ptr(a[0]), _ptr(a[1]),
+                                                                      _ptr(a[2]), self.n.ctypes.data_as(_vp)))
         if not fetch:
             return self.n.copy()
         return [(self.prev[s, :self.n[s]].copy(), self.cur[s, :self.n[s]].copy(), self.ids[s, :self.n[s]].copy()) for s in range(self.S)]
